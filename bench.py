@@ -7,7 +7,7 @@ shape of BASELINE.json configs[1] (YOOCHOOSE ADER, --batch_size=512): 512 train 
 exemplar rows per step, V = 18 661 items, V_prev = 17 421, table 25 959 rows (period 4 of the
 shipped split, SURVEY A.4), synthetic sessions with the YOOCHOOSE length histogram.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 N > 1 (under torchrun): data parallel, one rank per GPU, per-rank batch fixed (weak scaling); the gradients
 are summed and Adam applied by one kernel over NVLink peer memory (csrc/dp.cu; ADER_B200_DP=nccl selects the
@@ -161,19 +161,11 @@ def reference_arm(args):
     if WL["V"] > 200000:     # [M, V] fp32 logits + the one-hot of the restated graph: ~40 GB of host memory per step at 1M items
         print(json.dumps({"impl": "reference", "unavailable": "CPU restatement not run at the 1M-item shape (materialises [5120, 1M] fp32 twice)"}))
         return
-    # bounded: as many of the K requested steps as fit in ~150 s of CPU time (one step is seconds)
-    step, M, cores = cpu_step_fn()
-    t0 = time.perf_counter(); step(); t1 = time.perf_counter() - t0
-    steps = int(max(1, min(args.steps, 150.0 / max(t1, 1e-3))))
-    t0 = time.perf_counter()
-    for _ in range(steps):
-        step()
-    dt = time.perf_counter() - t0
-    val, ms = M * steps / dt, dt / steps * 1e3
-    sample = ("%d full steps (of %d requested; bounded to ~150 s) of %d rows, dense over 50 slots, [M,V] logits "
-              "materialised, torch-CPU fp32 restatement of the reference graph" % (steps, args.steps, M))
+    val, ms, cores, M = run_cpu(args.steps, args.warmup)
+    sample = ("%d full steps after %d warm-up steps of %d rows, dense over 50 slots, [M,V] logits "
+              "materialised, torch-CPU fp32 restatement of the reference graph" % (args.steps, args.warmup, M))
     line = {"impl": "reference", "metric": "train sessions/sec", "value": val, "unit": "sessions/s", "n_gpus": args.gpus,
-            "steps": steps, "warmup": args.warmup, "ms_per_step": ms, "higher_is_better": True, "scaling": "weak",
+            "steps": args.steps, "warmup": args.warmup, "ms_per_step": ms, "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": workload_config(1),
             "cpu_baseline": {"value": val, "unit": "sessions/s", "cores": cores, "kind": "port", "sample": sample},
@@ -336,6 +328,24 @@ def cpu_components(budget_s=6.0):
 
 
 GROUP = int(os.environ.get("ADER_B200_GRAPH_STEPS", "1"))      # steps per graph replay of the resident region (the product default: 1)
+DUMP_MAX_ELEMS = 1 << 22       # per dumped array (16 MiB in fp32): the 1M-item table is sampled, the YOOCHOOSE one is not
+
+
+def step_outputs(model, loss):
+    """What a train step hands its caller, on the host: the step's loss, the parameters it leaves and the gradient it
+    computed.  Arrays longer than DUMP_MAX_ELEMS keep one element of each of DUMP_MAX_ELEMS equal strata of their index
+    range, at an offset drawn from np.random.default_rng(0): the same sample in every run and every build."""
+    import torch
+    n = model.theta.numel()
+    idx = None
+    if n > DUMP_MAX_ELEMS:
+        edges = np.arange(DUMP_MAX_ELEMS + 1, dtype=np.int64) * n // DUMP_MAX_ELEMS
+        offs = (np.random.default_rng(0).random(DUMP_MAX_ELEMS) * np.diff(edges)).astype(np.int64)
+        idx = torch.from_numpy(edges[:-1] + offs).to(model.device)
+    out = {"loss": loss.detach().reshape(-1).cpu().numpy()}
+    for name, t in (("theta", model.theta), ("grad", model.grad)):
+        out[name] = (t if idx is None else t[idx]).detach().cpu().numpy()
+    return out
 
 
 def workload_config(n):
@@ -463,26 +473,31 @@ def gpu_arm(args):
 
     # ---- value: inputs resident in HBM -----------------------------------------------------------
     def resident_run(lo, hi):
-        """Steps [lo, hi) of the resident region: the queued epoch loop of the product (GROUP steps per graph replay)."""
+        """Steps [lo, hi) of the resident region: the queued epoch loop of the product (GROUP steps per graph replay).
+        Returns the device loss of the last step."""
+        loss = None
         if gs is None:
             for i in range(lo, hi):
-                resident_step(i)
-            return
+                loss = resident_step(i)
+            return loss
         i = lo
         while i < hi:
             n = GROUP if (GROUP > 1 and i + GROUP <= hi) else 1
-            gs.run_queued(max(ntok[i:i + n]), nsteps=n)
+            loss = gs.run_queued(max(ntok[i:i + n]), nsteps=n)
             i += n
+        return loss
 
     resident_run(0, W)
     barrier()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     w0 = time.time()
     e0.record()
-    resident_run(W, W + K)
+    last_step_loss = resident_run(W, W + K)
     e1.record()
     barrier()
     windows.append((w0, time.time()))
+    # the later regions keep training the same model: take the outputs of the timed region's last step now
+    outputs = step_outputs(model, last_step_loss) if args.dump_outputs and rank == 0 else None
     ms_total = e0.elapsed_time(e1)
     if world > 1:
         t = torch.tensor([ms_total], device=dev)
@@ -735,6 +750,10 @@ def gpu_arm(args):
                 "cpu_baseline": None if big else
                                 {"value": cpu_val, "unit": "sessions/s", "cores": cores, "kind": "port",
                                  "sample": "2 full steps of %d rows after 1 warm-up, torch-CPU fp32 restatement" % M}}
+        if outputs is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in outputs.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
         print(json.dumps(line))
         sys.stdout.flush()
     if world > 1:
@@ -750,7 +769,7 @@ def gpu_arm(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=200, help="timed steps, after --warmup untimed ones (with --impl reference too)")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="ader_b200")
     ap.add_argument("--no-graph", dest="no_graph", action="store_true", help="issue the step's launches eagerly")
@@ -759,7 +778,15 @@ def main():
     ap.add_argument("--config", default="yoochoose_p4", choices=["yoochoose_p4", "synthetic1m", "synthetic1m_full"],
                     help="workload: BASELINE configs[1] shape (default, the headline) or configs[4] (1M-item vocabulary; session "
                          "lengths from the YOOCHOOSE histogram, or _full: all 50 slots of every row filled)")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default=None,
+                    help="write the loss, parameters and gradient of the last timed step as DIR/<name>.npy (float32; at most "
+                         "%d elements per array, a fixed seeded sample beyond that) to compare two builds output for output"
+                    % DUMP_MAX_ELEMS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU step's outputs: it does not apply to --impl reference")
     if args.config.startswith("synthetic1m"):
         WL.update(WL_SYNTH1M)
         if args.config.endswith("_full"):
