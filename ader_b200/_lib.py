@@ -11,7 +11,7 @@ import os
 
 from . import build as _build
 
-ABI_VERSION = 1
+ABI_VERSION = 2
 
 
 class AderError(RuntimeError):
@@ -28,7 +28,8 @@ class AderLossArgs(C.Structure):
                 ("V_prev", C.c_int32), ("mode", C.c_int32), ("lambda_", C.c_float),
                 ("pos", C.c_void_p), ("ex_pos", C.c_void_p), ("teacher", C.c_void_p),
                 ("teacher_row", C.c_void_p), ("teacher_ld", C.c_int64),
-                ("n_train_global", C.c_int32), ("n_ex_global", C.c_int32)]
+                ("n_train_global", C.c_int32), ("n_ex_global", C.c_int32),
+                ("teacher_rep", C.c_void_p), ("teacher_table", C.c_void_p), ("teacher_table16", C.c_void_p)]
 
 
 class AderAdamArgs(C.Structure):
@@ -79,6 +80,8 @@ SIGNATURES = {
                                           _P, C.c_float, C.c_uint64, _P, C.c_int32, _P]),
     "ader_train_step_tc": (C.c_int32, [_MP, _P, _P, C.c_int32, C.c_int32, C.POINTER(AderLossArgs), _P, _P, _P, _P, _P, _P, _P,
                                        _P, C.c_float, C.c_uint64, _P, _P, _P, _P, C.POINTER(AderAdamArgs), C.c_int32, _P]),
+    "ader_table16_ws_bytes": (C.c_size_t, [_MP, C.c_int32]),
+    "ader_pack_table16": (C.c_int32, [_MP, _P, C.c_int32, _P, _P]),
     "ader_logits": (C.c_int32, [_MP, _P, _P, C.c_int32, C.c_int32, _P, C.c_int64, _P]),
     "ader_adam_step": (C.c_int32, [_MP, _P, _P, _P, _P, _P, C.POINTER(AderAdamArgs), _P]),
     "ader_eval_ws_bytes": (C.c_size_t, [_MP, C.c_int32, C.c_int32]),

@@ -58,6 +58,19 @@ static inline int check_model(const AderModel* m) {
   return 0;
 }
 
+// Teacher of a distillation (mode 1) call: stored logits (`teacher`) or a frozen snapshot (`teacher_rep` + the table the
+// entry reads: fp32 rows for the exact entry, the bf16 shadow for the tcgen05 ones) -- exactly one of the two.
+static inline int check_teacher(const AderLossArgs* a, const char* who, bool tc) {
+  const bool stored = a->teacher != nullptr, frozen = a->teacher_rep != nullptr;
+  if (stored == frozen)
+    return fail(-1, "%s: mode 1 takes exactly one teacher source: teacher (stored logits) or teacher_rep (frozen snapshot)", who);
+  if (a->V_prev < 1 || a->V_prev > a->V) return fail(-1, "%s: bad teacher (V_prev=%d, V=%d)", who, a->V_prev, a->V);
+  if (stored && a->teacher_ld < a->V_prev) return fail(-1, "%s: bad teacher (teacher_ld %lld < V_prev %d)", who, (long long)a->teacher_ld, a->V_prev);
+  if (frozen && !tc && !a->teacher_table) return fail(-1, "%s: frozen teacher without teacher_table", who);
+  if (frozen && tc && !a->teacher_table16) return fail(-1, "%s: frozen teacher without teacher_table16 (see ader_pack_table16)", who);
+  return 0;
+}
+
 // ---- programmatic dependent launch (PDL) -----------------------------------------------------------------
 // Chain kernels call pdl_wait() before their first access to data of the preceding kernel (a no-op for a normal
 // launch) and pdl_go() right behind it; launch_chain() sets the programmatic-stream-serialization attribute when

@@ -28,6 +28,10 @@
 //              bulk-copied instead of computed)   -> loss dot = rep.uc / coef,  d_rep -= uc
 //   MODE_DE  : after its row-tile loop the CTA of a vocabulary tile < V_prev runs one more second-MMA per exemplar
 //              row tile with the A operand NEGATED in the instruction descriptor: dE[v] -= Pc^T . rep
+// A frozen teacher (AderLossArgs.teacher_rep) builds Pc from a snapshot of the previous model instead of stored logits:
+// T = trep . E_prev^T tiles go through MODE_FWD on the snapshot's operands (label-free rows of width V_prev: the teacher's
+// online (max, sumexp) per chunk, merged into lse_t), then
+//   MODE_TP  : recomputes the T tiles and writes Pc = coef * exp(T - lse_t) as bf16 straight into the matrix MODE_TU / MODE_DE read
 #include "tc_common.cuh"
 #include <stdlib.h>
 
@@ -42,8 +46,9 @@ constexpr int KSTEPS1 = KP / 16;              // 10 MMAs per S tile
 constexpr int KSTEPS2 = TILE / 16;            // 8 MMAs per gradient tile
 constexpr float LOG2E = 1.4426950408889634f;
 
-enum { MODE_FWD = 0, MODE_DREP = 1, MODE_DE = 2, MODE_TU = 3 };
-__host__ __device__ constexpr bool is_teach(int mode) { return mode >= MODE_TU; }
+enum { MODE_FWD = 0, MODE_DREP = 1, MODE_DE = 2, MODE_TU = 3, MODE_TP = 4 };
+__host__ __device__ constexpr bool is_teach(int mode) { return mode == MODE_TU; }
+__host__ __device__ constexpr bool fwd_like(int mode) { return mode == MODE_FWD || mode == MODE_TP; }   // S tiles only, no second product
 
 struct TcArgs {
   const uint8_t* rep_tiles;     // [n_mtiles][TILE_BYTES]
@@ -68,6 +73,9 @@ struct TcArgs {
   int x0_t, n_et, n_vtp, n_chunks_t;   // first row tile holding exemplar rows, their count, teacher vocab tiles, TU chunks
   float* u_part;                // TU: [n_chunks_t][n_et*128][160]
   int n2;                       // tc2: N of the gradient products (160, or 192 = three whole swizzle atoms; ADER_B200_TC2_N2)
+  // MODE_TP (frozen teacher): output Pc matrix [n_mtiles*128][n_vtiles*128] bf16; rows [t_row_lo, t_row_hi) are exemplars
+  __nv_bfloat16* pt_out;
+  int t_row_lo, t_row_hi;
 };
 
 // one T128 tile as LOAD_SPLIT independent bulk copies (a single 40 KB bulk copy keeps only a few
@@ -489,7 +497,7 @@ constexpr int TILE2_BYTES = 3 * REG2;        // 49152
 constexpr int DS2_BYTES = 2 * REG2;          // 32768
 constexpr int ROW16 = KP;                    // bf16 row pitch (elements) of the HBM operand matrices
 __host__ __device__ constexpr int n_stages2(int mode) { return 3; }
-__host__ __device__ constexpr int n_ds2(int mode) { return mode == MODE_FWD ? 0 : 1; }
+__host__ __device__ constexpr int n_ds2(int mode) { return fwd_like(mode) ? 0 : 1; }
 constexpr int smem_tc2(int mode) { return 1024 + (1 + n_stages2(mode)) * TILE2_BYTES + n_ds2(mode) * DS2_BYTES + 256; }
 
 // 128 rows x 160 (192) k starting at matrix row `row0`
@@ -567,7 +575,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_tc2(TcArgs a, const __grid_cons
     asm volatile("prefetch.tensormap [%0];" ::"l"(tmY) : "memory");
     if (is_teach(MODE) || MODE == MODE_DE) asm volatile("prefetch.tensormap [%0];" ::"l"(&tm_pt) : "memory");
   }
-  constexpr uint32_t TMEM_COLS = (MODE == MODE_FWD) ? 256u : 512u;
+  constexpr uint32_t TMEM_COLS = fwd_like(MODE) ? 256u : 512u;
   if (warp == 1) {
     asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(TMEM_COLS) : "memory");
     asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
@@ -633,13 +641,13 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_tc2(TcArgs a, const __grid_cons
 #pragma unroll
         for (int k = 0; k < KSTEPS1; ++k)
           umma_bf16(tmem + s * 128, desc_kmajor(A, k), desc_kmajor(B, k), IDESC1, k > 0);
-        if (MODE == MODE_FWD) umma_commit(BAR(B_YEMPTY + ys));
+        if (fwd_like(MODE)) umma_commit(BAR(B_YEMPTY + ys));
         umma_commit(BAR(B_TFULL + s));
       };
       if (!is_teach(MODE)) { mbar_wait(BAR(B_XFULL), 0, a.err); issue_s(0); }
       for (int it = 0; it < n_it; ++it) {
         if (!is_teach(MODE) && it + 1 < n_it) issue_s(it + 1);
-        if (MODE != MODE_FWD) {
+        if (!fwd_like(MODE)) {
           const int s = it % NDS; const uint32_t ph = (it / NDS) & 1;
           const int ys = it % NST;
           if (is_teach(MODE)) mbar_wait(BAR(B_YFULL + ys), (it / NST) & 1, a.err);
@@ -677,7 +685,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_tc2(TcArgs a, const __grid_cons
           umma_commit(BAR(B_DSEMPTY + s));
         }
       }
-      if (MODE != MODE_FWD) umma_commit(BAR(B_ACC));
+      if (!fwd_like(MODE)) umma_commit(BAR(B_ACC));
     }
     __syncwarp();
   } else {
@@ -691,6 +699,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_tc2(TcArgs a, const __grid_cons
     if (is_teach(MODE)) { ri = RowInfo(); ri_next = RowInfo(); }
     else if (MODE != MODE_DE) ri = row_info(a, x_tile * TILE + row, MODE != MODE_FWD);
     else ri_next = row_info(a, y_lo * TILE + row, true);
+    if (MODE == MODE_TP && (x_tile * TILE + row < a.t_row_lo || x_tile * TILE + row >= a.t_row_hi)) ri.kind = 0;   // zero row
     for (int it = 0; it < (is_teach(MODE) ? 0 : n_it); ++it) {
       const int s = it & 1; const uint32_t ph = (it >> 1) & 1;
       int v0;
@@ -787,7 +796,11 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_tc2(TcArgs a, const __grid_cons
         }
       }
       if (threadIdx.x == 64 && it == 2) TL2(5);
-      if (MODE != MODE_FWD) {
+      if (MODE == MODE_TP) {                   // Pc row segment: 64 bf16 = 128 contiguous bytes of this thread's row
+        uint4* o = reinterpret_cast<uint4*>(a.pt_out + (size_t)(x_tile * TILE + row) * ((size_t)a.n_vtiles * TILE) + vb0);
+#pragma unroll
+        for (int j = 0; j < 8; ++j) o[j] = make_uint4(pk[4 * j], pk[4 * j + 1], pk[4 * j + 2], pk[4 * j + 3]);
+      } else if (MODE != MODE_FWD) {
         const int sd = it % NDS; const uint32_t dph = (it / NDS) & 1;
         // the exponentials above overlap the second product of the previous tile; only the stores wait for its dS buffer
         mbar_wait(BAR(B_DSEMPTY + sd), dph ^ 1, a.err);
@@ -808,7 +821,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_tc2(TcArgs a, const __grid_cons
         float4 o = make_float4(mx, sum, lab, dot);
         *reinterpret_cast<float4*>(a.stats + ((size_t)(chunk * 2 + half) * a.M + gm) * 4) = o;
       }
-    } else if (n_it > 0) {
+    } else if (MODE != MODE_TP && n_it > 0) {
       mbar_wait(BAR(B_ACC), 0, a.err);
       tc_fence_after();
       // accumulator [128 rows, 160] -> the (now idle) Y stages, row pitch DE_LD floats (conflict-free 16-byte row writes) ...
@@ -880,6 +893,27 @@ __global__ void k_pack_rows16(const float* __restrict__ src, long long ld, int n
     pk[i] = *reinterpret_cast<uint32_t*>(&h);
   }
   *reinterpret_cast<uint4*>(out + row * ROW16 + kc * 8) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
+}
+
+// frozen teacher: the exemplar rows' snapshot reps as the row-major bf16 [n_et*128][160] operand of the teacher passes, in
+// the row convention of Pc (row = step row - x0*128; rows that are not exemplar rows and columns >= d are zero)
+__global__ void k_pack_trep16(const float* __restrict__ trep, const int* __restrict__ teacher_row, int n_train, int M, int x0,
+                              int d, int rows_pad, __nv_bfloat16* __restrict__ out) {
+  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= (long long)rows_pad * (ROW16 / 8)) return;
+  const int kc = (int)(idx % (ROW16 / 8));
+  const int row = (int)(idx / (ROW16 / 8));
+  const int e = x0 * TILE + row - n_train;
+  const float* src = (e >= 0 && e + n_train < M) ? trep + (long long)(teacher_row ? teacher_row[e] : e) * d : nullptr;
+  uint32_t pk[4];
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const int k = kc * 8 + i * 2;
+    const float v0 = (src && k < d) ? src[k] : 0.f, v1 = (src && k + 1 < d) ? src[k + 1] : 0.f;
+    __nv_bfloat162 h = __floats2bfloat162_rn(v0, v1);
+    pk[i] = *reinterpret_cast<uint32_t*>(&h);
+  }
+  *reinterpret_cast<uint4*>(out + (long long)row * ROW16 + kc * 8) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
 }
 
 // Pc = coef * softmax(teacher) as ONE row-major bf16 matrix [n_et*128][n_vtp*128] (row = step row - x0*128, column = local
@@ -1077,6 +1111,25 @@ __global__ void __launch_bounds__(256) k_merge_stats(const float* __restrict__ s
   row_loss[i] = kd ? l - dot : l - lab;
 }
 
+// frozen teacher: lse_t[r] of every packed exemplar row from the per-chunk (max, sumexp) partials of the MODE_FWD pass over
+// the snapshot (k_merge_stats without label, distillation and row-loss terms).  Warp per row, fixed butterfly order.
+__global__ void __launch_bounds__(256) k_merge_lse(const float* __restrict__ stats, int rows, int n_chunks, float* __restrict__ lse) {
+  const int i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+  if (i >= rows) return;
+  float mx = -INFINITY;
+  for (int c = lane; c < n_chunks; c += 32) mx = fmaxf(mx, stats[((size_t)c * rows + i) * 4]);
+#pragma unroll
+  for (int o = 16; o; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+  float sum = 0.f;
+  for (int c = lane; c < n_chunks; c += 32) {
+    const float2 s = *reinterpret_cast<const float2*>(stats + ((size_t)c * rows + i) * 4);
+    if (s.x > -INFINITY) sum += s.y * expf(s.x - mx);
+  }
+#pragma unroll
+  for (int o = 16; o; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
+  if (lane == 0) lse[i] = mx + logf(sum);
+}
+
 // d_rep[M, d] = sum over chunks of the padded partials  (- uc = coef_ex * P.E for distillation rows)
 __global__ void k_reduce_drep(const float* __restrict__ part, int n_chunks, int rows_pad, int M, int d,
                               float* __restrict__ d_rep, const float* __restrict__ u, int x0, int n_train) {
@@ -1115,6 +1168,8 @@ namespace ader { int launch_loss_reduce(const float* row_loss, int n_train, int 
 struct TcWs {
   uint8_t *rep_tiles, *e_tiles, *pt_tiles;
   float *stats, *lse, *lse_t, *drep_part, *u_part, *u, *udot;
+  uint8_t* trep16;                         // frozen teacher: packed exemplar reps [n_et*128][160] bf16
+  float *tstats, *lse_tt;                  // ... its per-chunk statistics and log-sum-exp per packed row
   int* err;
   int x0_t, n_et, n_vtp, n_chunks_t;       // teacher products (0 tiles when the step has no distillation rows)
   size_t bytes;
@@ -1132,7 +1187,7 @@ static int tc_chunks(int n_mtiles, int n_vtiles) {
   return best;
 }
 // V = columns of this shard (local), Vp_local = how many of them are teacher columns (0 = no distillation)
-static TcWs carve_tc(const AderModel* m, int M, int V, int n_ex, int Vp_local, char* base) {
+static TcWs carve_tc(const AderModel* m, int M, int V, int n_ex, int Vp_local, char* base, bool frozen = false) {
   TcWs w; size_t o = 0;
   auto take = [&](size_t n) { char* p = base ? base + o : nullptr; o += align_up(n); return p; };
   const int nm = cdiv(M, TILE), nv = cdiv(V, TILE), nc = tc_chunks(nm, nv);
@@ -1152,13 +1207,22 @@ static TcWs carve_tc(const AderModel* m, int M, int V, int n_ex, int Vp_local, c
   w.u = (float*)take(sizeof(float) * ((size_t)w.n_et * TILE * KP + 4));
   w.udot = (float*)take(sizeof(float) * ((size_t)w.n_et * TILE + 4));
   w.err = (int*)take(sizeof(int) * 4);
+  const bool fz = frozen && kd;
+  w.trep16 = fz ? (uint8_t*)take((size_t)w.n_et * TILE * ROW16 * 2) : nullptr;
+  w.tstats = fz ? (float*)take(sizeof(float) * 4 * (size_t)w.n_chunks_t * 2 * w.n_et * TILE) : nullptr;
+  w.lse_tt = fz ? (float*)take(sizeof(float) * (size_t)w.n_et * TILE) : nullptr;
   w.bytes = o;
   return w;
 }
 
 extern "C" size_t ader_loss_tc_ws_bytes(const AderModel* m, const AderLossArgs* a) {
   if (check_model(m) || !a || a->M <= 0 || a->V <= 0) return 0;
-  return carve_tc(m, a->M, a->V, a->n_ex, a->mode == 1 ? a->V_prev : 0, nullptr).bytes;
+  return carve_tc(m, a->M, a->V, a->n_ex, a->mode == 1 ? a->V_prev : 0, nullptr, a->teacher_rep != nullptr).bytes;
+}
+
+extern "C" size_t ader_table16_ws_bytes(const AderModel* m, int32_t V) {
+  if (check_model(m) || V <= 0 || m->d > KP) return 0;
+  return (size_t)cdiv(V, TILE) * TILE * ROW16 * 2;
 }
 
 // ---- tc2: TMA tensor maps over the row-major bf16 operand matrices ---------------------------------------------------
@@ -1173,7 +1237,7 @@ static int tc2_n2() {
   if (!n) { const char* e = getenv("ADER_B200_TC2_N2"); n = (e && atoi(e) == 192) ? 192 : 160; }
   return n;
 }
-struct TcMaps { CUtensorMap rep, e, pt; };
+struct TcMaps { CUtensorMap rep, e, pt, trep, ttab; };     // trep / ttab: frozen teacher only
 static int make_tc_maps(const TcWs& w, int nm, int nv, TcMaps& mp) {
   if (int e = make_map2d(&mp.rep, w.rep_tiles, ROW16, (uint64_t)nm * TILE, ROW16 * 2)) return e;
   if (int e = make_map2d(&mp.e, w.e_tiles, ROW16, (uint64_t)nv * TILE, ROW16 * 2)) return e;
@@ -1196,12 +1260,33 @@ static void set_tc_attrs() {
   cudaFuncSetAttribute(k_tc2<MODE_DREP>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tc2(MODE_DREP));
   cudaFuncSetAttribute(k_tc2<MODE_DE>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tc2(MODE_DE));
   cudaFuncSetAttribute(k_tc2<MODE_TU>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tc2(MODE_TU));
+  cudaFuncSetAttribute(k_tc2<MODE_TP>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tc2(MODE_TP));
   attr_set = true;
 }
 constexpr int SMEM_FWD = (1 + n_stages(MODE_FWD)) * TILE_BYTES + 256;
 constexpr int SMEM_BWD = (1 + n_stages(MODE_DREP)) * TILE_BYTES + 2 * DS_BYTES + 256;
 // teacher statistics + tiles + uc partials (rep-independent), then u = sum of partials and udot = rep . u
+// frozen teacher: Pc from the snapshot (packed reps -> MODE_FWD statistics of T = trep . E_prev^T -> lse_t -> MODE_TP tiles)
+static void launch_teacher_frozen(const AderLossArgs* a, const TcWs& w, const TcArgs& t, int d, cudaStream_t st, const TcMaps& mp) {
+  const int rows = w.n_et * TILE;
+  k_pack_trep16<<<cdiv((long long)rows * (ROW16 / 8), 256), 256, 0, st>>>(a->teacher_rep, a->teacher_row, a->n_train, a->M, w.x0_t, d,
+                                                                         rows, reinterpret_cast<__nv_bfloat16*>(w.trep16));
+  TcArgs tt = t;                          // every packed row is a label-free softmax row of width V_prev over the snapshot's table
+  tt.M = rows; tt.V = a->V_prev; tt.V_total = a->V_prev; tt.v_off = 0;
+  tt.n_mtiles = w.n_et; tt.n_vtiles = w.n_vtp; tt.n_chunks = w.n_chunks_t;
+  tt.n_train = 0; tt.mode = 1; tt.stats = w.tstats; tt.lse = w.lse_tt; tt.drep_part = nullptr; tt.grad_table = nullptr;
+  tt.pt_out = reinterpret_cast<__nv_bfloat16*>(w.pt_tiles);
+  tt.t_row_lo = a->n_train - w.x0_t * TILE; tt.t_row_hi = a->M - w.x0_t * TILE;
+  k_tc2<MODE_FWD><<<w.n_et * w.n_chunks_t, NTHREADS, smem_tc2(MODE_FWD), st>>>(tt, mp.trep, mp.ttab, mp.pt);
+  k_merge_lse<<<cdiv((long long)rows * 32, 256), 256, 0, st>>>(w.tstats, rows, w.n_chunks_t * 2, w.lse_tt);
+  k_tc2<MODE_TP><<<w.n_et * w.n_chunks_t, NTHREADS, smem_tc2(MODE_TP), st>>>(tt, mp.trep, mp.ttab, mp.pt);
+}
 static void launch_teacher_tu(const AderLossArgs* a, const TcWs& w, const TcArgs& t, int v_off, cudaStream_t st, const TcMaps* mp) {
+  if (a->teacher_rep) {                   // frozen teacher (tc2 only, single GPU: v_off == 0)
+    launch_teacher_frozen(a, w, t, t.d, st, *mp);
+    k_tc2<MODE_TU><<<w.n_et * w.n_chunks_t, NTHREADS, smem_tc2(MODE_TU), st>>>(t, mp->rep, mp->e, mp->pt);
+    return;
+  }
   k_teacher_lse<<<a->n_ex, 256, 0, st>>>(a->teacher, a->teacher_row, a->teacher_ld, a->V_prev, w.lse_t);
   if (mp) {
     k_teacher_rows16<<<dim3(w.n_vtp, w.n_et), 256, 0, st>>>(a->teacher, a->teacher_row, a->teacher_ld, t.teacher_vec4, w.lse_t,
@@ -1261,13 +1346,16 @@ int ader::loss_tc_run(const AderModel* m, const float* theta, const float* rep, 
   ADER_CHECK_ARG(a->n_train == 0 || a->pos, "loss_fwd_bwd_tc: pos is NULL");
   if (a->n_ex > 0) {
     ADER_CHECK_ARG(a->mode != 0, "loss_fwd_bwd_tc: exemplar rows given in vanilla mode");
-    if (a->mode == 1) ADER_CHECK_ARG(a->teacher && a->V_prev >= 1 && a->V_prev <= a->V && a->teacher_ld >= a->V_prev, "loss_fwd_bwd_tc: bad teacher");
+    if (a->mode == 1) {
+      if (int e = check_teacher(a, "loss_fwd_bwd_tc", true)) return e;
+      ADER_CHECK_ARG(!a->teacher_rep || tc_gen() == 2, "loss_fwd_bwd_tc: a frozen teacher needs the second-generation kernels (ADER_B200_TC=1 is set)");
+    }
     if (a->mode == 2) ADER_CHECK_ARG(a->ex_pos, "loss_fwd_bwd_tc: exemplar_pos is NULL");
   }
   cudaStream_t st = f.main, sb = f.b;
   const int d = m->d, M = a->M, V = a->V;
   const bool kd = a->n_ex > 0 && a->mode == 1;
-  TcWs w = carve_tc(m, M, V, a->n_ex, kd ? a->V_prev : 0, (char*)ws);
+  TcWs w = carve_tc(m, M, V, a->n_ex, kd ? a->V_prev : 0, (char*)ws, a->teacher_rep != nullptr);
   const int nm = cdiv(M, TILE), nv = cdiv(V, TILE), nc = tc_chunks(nm, nv);
   const int smem_fwd = SMEM_FWD, smem_bwd = SMEM_BWD;
   set_tc_attrs();
@@ -1282,10 +1370,15 @@ int ader::loss_tc_run(const AderModel* m, const float* theta, const float* rep, 
   t.lse = w.lse; t.lse_t = w.lse_t; t.stats = w.stats; t.drep_part = w.drep_part; t.grad_table = grad ? grad + d : nullptr;
   t.d = d; t.err = w.err;
   t.pt_tiles = w.pt_tiles; t.x0_t = w.x0_t; t.n_et = w.n_et; t.n_vtp = w.n_vtp; t.n_chunks_t = w.n_chunks_t; t.u_part = w.u_part; t.n2 = tc2_n2();
+  t.pt_out = nullptr; t.t_row_lo = t.t_row_hi = 0;
 
   const bool g2 = tc_gen() == 2;
   TcMaps mp;
   if (g2) { if (int e = make_tc_maps(w, nm, nv, mp)) return e; }
+  if (kd && a->teacher_rep) {
+    if (int e = make_map2d(&mp.trep, w.trep16, ROW16, (uint64_t)w.n_et * TILE, ROW16 * 2)) return e;
+    if (int e = make_map2d(&mp.ttab, a->teacher_table16, ROW16, (uint64_t)w.n_vtp * TILE, ROW16 * 2)) return e;
+  }
   if (phase_mask == 4) {      // measurement only: the three tensor-core kernels on an already prepared workspace
     if (g2) {               // launched as in the step: programmatic dependent launches along the chain (ADER_B200_PDL=0: plain)
       const char* pe = getenv("ADER_B200_PDL");
@@ -1383,6 +1476,7 @@ static int vp_setup(const AderModel* m, const float* theta, const float* rep, co
   t.lse = w.lse; t.lse_t = w.lse_t; t.stats = w.stats; t.drep_part = w.drep_part; t.grad_table = nullptr;
   t.d = d; t.err = w.err;
   t.pt_tiles = w.pt_tiles; t.x0_t = w.x0_t; t.n_et = w.n_et; t.n_vtp = w.n_vtp; t.n_chunks_t = w.n_chunks_t; t.u_part = w.u_part; t.n2 = tc2_n2();
+  t.pt_out = nullptr; t.t_row_lo = t.t_row_hi = 0;
   if (pack && w.n_et > 0) launch_teacher_u(a, w, t, v_lo, rep, d, st, tc_gen() == 2 ? &mp : nullptr);
   return 0;
 }
@@ -1393,12 +1487,13 @@ static int vp_check(const AderModel* m, const AderLossArgs* a, int v_lo, int v_h
   ADER_CHECK_ARG(a->V >= 1 && a->V < m->v_tab && a->mode >= 0 && a->mode <= 2, "loss_tc_vp: bad V / mode");
   ADER_CHECK_ARG(v_lo >= 0 && v_lo < v_hi && v_hi <= a->V && v_lo % TILE == 0, "loss_tc_vp: shard [%d,%d) must be 128-aligned inside [0,%d)", v_lo, v_hi, a->V);
   ADER_CHECK_ARG(m->d <= KP, "loss_tc_vp: hidden_units too large");
+  ADER_CHECK_ARG(!a->teacher_rep, "loss_tc_vp: a frozen teacher (teacher_rep) is not supported by the vocab-parallel entries");
   if (a->n_ex > 0 && a->mode == 1) ADER_CHECK_ARG(a->teacher && a->V_prev >= 1 && a->V_prev <= a->V, "loss_tc_vp: bad teacher");
   return 0;
 }
 
 extern "C" size_t ader_loss_tc_vp_ws_bytes(const AderModel* m, const AderLossArgs* a, int32_t v_lo, int32_t v_hi) {
-  if (check_model(m) || !a || a->M <= 0 || v_hi <= v_lo) return 0;
+  if (check_model(m) || !a || a->M <= 0 || v_hi <= v_lo || a->teacher_rep) return 0;
   return carve_tc(m, a->M, v_hi - v_lo, a->n_ex, vp_teacher_cols(a, v_lo, v_hi), nullptr).bytes;
 }
 
@@ -1440,5 +1535,17 @@ extern "C" int32_t ader_loss_tc_vp_bwd(const AderModel* m, const float* theta, c
     else k_tc_logits<MODE_DE><<<t.n_vtiles, NTHREADS, smem_bwd, st>>>(t);
   }
   ADER_CHECK_LAUNCH("loss_tc_vp_bwd");
+  return 0;
+}
+
+extern "C" int32_t ader_pack_table16(const AderModel* m, const float* rows, int32_t V, void* out, void* stream) {
+  if (int e = check_model(m)) return e;
+  ADER_CHECK_ARG(rows && out, "pack_table16: NULL pointer");
+  ADER_CHECK_ARG(V >= 1 && V < m->v_tab, "pack_table16: V=%d outside the table of %d rows", V, m->v_tab);
+  ADER_CHECK_ARG(m->d <= KP, "pack_table16: hidden_units must be <= %d", KP);
+  const long long rows_pad = (long long)cdiv(V, TILE) * TILE;
+  k_pack_rows16<<<cdiv(rows_pad * (ROW16 / 8), 256), 256, 0, (cudaStream_t)stream>>>(rows, m->d, V, m->d, (int)rows_pad,
+                                                                                     reinterpret_cast<__nv_bfloat16*>(out), nullptr);
+  ADER_CHECK_LAUNCH("pack_table16");
   return 0;
 }

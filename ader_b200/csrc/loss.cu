@@ -107,15 +107,28 @@ int launch_loss_reduce(const float* row_loss, int n_train, int n_ex, float lambd
 
 static long long logits_ld(int V) { return ((long long)V + 3) / 4 * 4; }
 
-static int run_logits(const AderModel* m, const float* theta, const float* rep, int M, int V, float* out,
-                      long long ld, cudaStream_t st) {
+// rows = fp32 row of item 1 (theta + d, or a frozen teacher_table), row stride d
+static int run_logits_rows(const AderModel* m, const float* rows, const float* rep, int M, int V, float* out,
+                           long long ld, cudaStream_t st) {
   GemmArgs g; gemm_defaults(g);
   const int d = m->d;
   g.A = rep; g.a_rs = d; g.a_cs = 1;
-  g.B = theta + d; g.b_rs = 1; g.b_cs = d;        // B(k=c, n=v) = E[(v+1)*d + c]  (ADER.py:90-91)
+  g.B = rows; g.b_rs = 1; g.b_cs = d;             // B(k=c, n=v) = E[(v+1)*d + c]  (ADER.py:90-91)
   g.C = out; g.c_rs = ld; g.c_cs = 1;
   g.M = M; g.N = V; g.K = d;
   return launch_gemm(g, st);
+}
+static int run_logits(const AderModel* m, const float* theta, const float* rep, int M, int V, float* out,
+                      long long ld, cudaStream_t st) {
+  return run_logits_rows(m, theta + m->d, rep, M, V, out, ld, st);
+}
+
+// frozen teacher: out[e, :] = src[teacher_row[e], :] (identity when teacher_row is NULL)
+__global__ void k_gather_rep(const float* __restrict__ src, const int* __restrict__ row, int n, int d, float* __restrict__ out) {
+  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= (long long)n * d) return;
+  const int e = (int)(idx / d), c = (int)(idx % d);
+  out[idx] = src[(long long)(row ? row[e] : e) * d + c];
 }
 
 // ---- evaluation rows: rank of the ground truth + top-k (ADER.py:103, util.py:323-339) -------
@@ -176,10 +189,16 @@ __global__ void __launch_bounds__(256) k_rank_topk_rows(const float* __restrict_
 
 using namespace ader;
 
+static bool frozen_kd(const AderLossArgs* a) { return a->mode == 1 && a->n_ex > 0 && a->teacher_rep; }
+
 extern "C" size_t ader_loss_ws_bytes(const AderModel* m, const AderLossArgs* a) {
   if (check_model(m) || !a || a->M <= 0 || a->V <= 0) return 0;
   size_t o = align_up(sizeof(float) * (size_t)a->M * logits_ld(a->V));
   o += align_up(sizeof(float) * (size_t)DR_SPLITS * a->M * m->d);
+  if (frozen_kd(a) && a->V_prev > 0) {      // gathered exemplar reps + their teacher logits [n_ex, V_prev]
+    o += align_up(sizeof(float) * (size_t)a->n_ex * m->d);
+    o += align_up(sizeof(float) * (size_t)a->n_ex * logits_ld(a->V_prev));
+  }
   return o;
 }
 
@@ -194,8 +213,7 @@ extern "C" int32_t ader_loss_fwd_bwd(const AderModel* m, const float* theta, con
   ADER_CHECK_ARG(a->n_train == 0 || a->pos, "loss_fwd_bwd: pos is NULL");
   if (a->n_ex > 0) {
     ADER_CHECK_ARG(a->mode != 0, "loss_fwd_bwd: exemplar rows given in vanilla mode");
-    if (a->mode == 1) ADER_CHECK_ARG(a->teacher && a->V_prev >= 1 && a->V_prev <= a->V && a->teacher_ld >= a->V_prev,
-                                     "loss_fwd_bwd: bad teacher (V_prev=%d, V=%d)", a->V_prev, a->V);
+    if (a->mode == 1) { if (int e = check_teacher(a, "loss_fwd_bwd", false)) return e; }
     if (a->mode == 2) ADER_CHECK_ARG(a->ex_pos, "loss_fwd_bwd: exemplar_pos is NULL");
   }
   cudaStream_t st = (cudaStream_t)stream;
@@ -203,8 +221,21 @@ extern "C" int32_t ader_loss_fwd_bwd(const AderModel* m, const float* theta, con
   const long long ld = logits_ld(V);
   float* S = (float*)ws;
   float* part = (float*)((char*)ws + align_up(sizeof(float) * (size_t)M * ld));
+  AderLossArgs ka = *a;
+  if (frozen_kd(a)) {
+    // teacher logits of the exemplar rows from the snapshot, by the same SGEMM as ader_logits (each element is a
+    // sequential k-sum independent of M and of the row's position), so the rows match stored logits bit for bit
+    char* p = (char*)part + align_up(sizeof(float) * (size_t)DR_SPLITS * M * d);
+    float* trep = (float*)p;
+    float* tl = (float*)(p + align_up(sizeof(float) * (size_t)a->n_ex * d));
+    const long long tld = logits_ld(a->V_prev);
+    k_gather_rep<<<cdiv((long long)a->n_ex * d, 256), 256, 0, st>>>(a->teacher_rep, a->teacher_row, a->n_ex, d, trep);
+    ADER_CHECK_LAUNCH("gather teacher reps");
+    if (int e = run_logits_rows(m, a->teacher_table, trep, a->n_ex, a->V_prev, tl, tld, st)) return e;
+    ka.teacher = tl; ka.teacher_row = nullptr; ka.teacher_ld = tld;
+  }
   if (int e = run_logits(m, theta, rep, M, V, S, ld, st)) return e;
-  k_ce_kd_rows<<<M, 256, 0, st>>>(S, ld, *a, row_loss);
+  k_ce_kd_rows<<<M, 256, 0, st>>>(S, ld, ka, row_loss);
   if (int e = launch_loss_reduce(row_loss, a->n_train, a->n_ex, a->lambda_, loss, st, a->n_train_global, a->n_ex_global)) return e;
   ADER_CHECK_LAUNCH("loss rows");
   if (d_rep) {   // d_rep = dS . E[1..V]   (split-K over the vocabulary, fixed-order reduce)

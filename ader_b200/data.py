@@ -250,11 +250,50 @@ class Sampler:
 
 
 # ---- exemplar store ------------------------------------------------------------------------------
+class FrozenTeacher:
+    """The distillation teacher as a frozen snapshot of the model that selected the exemplars: every stored logit row is
+    rep_prev(session) . E_prev[1..V_prev]^T, so the exemplar reps and a copy of the item table carry the same information
+    as the [E, V_prev] logit matrix in O(E*d + V_prev*d) bytes.  The loss kernels recompute the teacher logits per step.
+
+    rep [E, d] fp32 (exact encoder, at selection time); table [V_prev, d] fp32 = rows 1..V_prev of the table (a copy, never a
+    view of the live parameters); table16 = its bf16 operand shadow for the tcgen05 kernels (ops.pack_table16); width = V_prev."""
+
+    def __init__(self, model, rep: torch.Tensor, width: int):
+        d = model.hp.hidden_units
+        self.ms, self.width = model.ms, int(width)
+        self.rep = rep.detach().to(torch.float32).contiguous()
+        # rows 0..V_prev of the table in one buffer: `table` (rows 1..V_prev) is a view of this copy, and the whole buffer has
+        # the layout of a parameter vector's table, so ops.logits can materialise the teacher rows from it (logits()).
+        self._rows = model.theta[:(self.width + 1) * d].clone()
+        self.table = self._rows[d:].view(self.width, d)
+        self.table16 = None
+        if d <= 160:
+            self.table16 = torch.empty(ops.table16_bytes(model.ms, self.width), dtype=torch.uint8, device=model.device)
+            ops.pack_table16(model.ms, self.table, self.width, self.table16)
+
+    def __len__(self):
+        return self.rep.shape[0]
+
+    def nbytes(self) -> int:
+        return sum(t.numel() * t.element_size() for t in (self.rep, self._rows, self.table16) if t is not None)
+
+    def logits(self, rows: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """The stored-logit matrix this snapshot stands for, [len(rows) or E, V_prev] fp32 (bit-identical to what the
+        previous model's ``logits`` gave at selection time).  O(E * V_prev) memory: small sizes and tests only."""
+        r = self.rep if rows is None else self.rep.index_select(0, rows.to(self.rep.device, torch.int64))
+        ld = (self.width + 3) // 4 * 4
+        out = torch.empty((r.shape[0], ld), dtype=torch.float32, device=self.rep.device)[:, :self.width]
+        if r.shape[0]:
+            ops.logits(self.ms, self._rows, r.contiguous(), self.width, out)
+        return out
+
+
 class ExemplarSet:
     """Flattened exemplars of one period: sessions in the order main.py:54-65 (`load_exemplars`)
-    would yield them, and their stored logits as ONE device matrix [E, V] fp32 (SURVEY S11)."""
+    would yield them, and their teacher: stored logits as ONE device matrix [E, V] fp32 (SURVEY S11), or a
+    ``FrozenTeacher`` snapshot of the selecting model."""
 
-    def __init__(self, sessions: List[List[int]], teacher: Optional[torch.Tensor], by_item: Optional[dict] = None):
+    def __init__(self, sessions: List[List[int]], teacher, by_item: Optional[dict] = None):
         self.sessions = sessions
         self.teacher = teacher
         self.by_item = by_item or {}
@@ -264,7 +303,7 @@ class ExemplarSet:
 
     def as_reference_list(self):
         """[[session, logits_list], ...] exactly like load_exemplars (small sizes only)."""
-        t = self.teacher.cpu().numpy()
+        t = (self.teacher.logits() if isinstance(self.teacher, FrozenTeacher) else self.teacher).cpu().numpy()
         return [[s, t[i].tolist()] for i, s in enumerate(self.sessions)]
 
 
@@ -385,7 +424,11 @@ class Evaluator:
 # ---- util.py:353-522 -----------------------------------------------------------------------------
 class ExemplarGenerator:
     def __init__(self, data: list, exemplar_size: int, disable_m: bool, batch_size: int, maxlen: int,
-                 dropout_rate: float, max_item: int, chunk_rows: int = 16384):
+                 dropout_rate: float, max_item: int, chunk_rows: int = 16384, teacher: str = "logits"):
+        """teacher: "logits" keeps the [E, max_item] teacher logits of the exemplars, "frozen" a FrozenTeacher snapshot."""
+        if teacher not in ("logits", "frozen"):
+            raise ValueError("teacher must be 'logits' or 'frozen', got %r" % (teacher,))
+        self.teacher_form = teacher
         self.m, self.max_item, self.maxlen = exemplar_size, max_item, maxlen
         self.dropout_rate = dropout_rate
         self.chunk_rows = chunk_rows
@@ -432,13 +475,17 @@ class ExemplarGenerator:
         return torch.cat(reps) if reps else torch.zeros((0, model.hp.hidden_units), device=model.device)
 
     def _store(self, model, picked_rows: np.ndarray, reps: Optional[torch.Tensor], by_item=None) -> int:
-        """Keep sessions (non-zero entries of [input, label], util.py:433) and their logits rows."""
+        """Keep sessions (non-zero entries of [input, label], util.py:433) and their logits rows (or, in the frozen form,
+        their reps and a snapshot of the table: no [E, max_item] matrix is built)."""
         sessions = [self.rows[r][-(self.maxlen + 1):] for r in picked_rows.tolist()]
         dev = model.device
         if len(picked_rows):
             idx = torch.from_numpy(picked_rows.astype(np.int64)).to(dev)
             r = reps[idx] if reps is not None else model.rep(self.ids[picked_rows], n_tokens=int(self.n_in[picked_rows].sum()))
-            teacher = model.logits(r.contiguous(), self.max_item)
+            teacher = (FrozenTeacher(model, r, self.max_item) if self.teacher_form == "frozen"
+                       else model.logits(r.contiguous(), self.max_item))
+        elif self.teacher_form == "frozen":
+            teacher = FrozenTeacher(model, torch.zeros((0, model.hp.hidden_units), device=dev), self.max_item)
         else:
             teacher = torch.zeros((0, self.max_item), device=dev)
         self.exemplars = ExemplarSet(sessions, teacher, by_item)

@@ -324,6 +324,9 @@ class VocabParallelLoss:
         ops, m = self.ops, self.model
         M, n_train = rep.shape[0], pos.numel()
         n_ex = M - n_train
+        if teacher is not None and not isinstance(teacher, torch.Tensor):
+            raise ValueError("the vocab-parallel loss takes stored teacher logits only (a frozen teacher would need its "
+                             "statistics all-reduced over the vocabulary shards)")
         v_prev = teacher.shape[1] if teacher is not None else 0
         a = ops.make_loss_args(M, n_train, n_ex, max_item, v_prev, mode if n_ex > 0 else 0, lambda_, pos, ex_pos, teacher, teacher_rows)
         v_lo, v_hi = self.shard(max_item)

@@ -20,7 +20,7 @@ import numpy as np
 import torch
 
 from . import ops
-from .data import DataLoader, Evaluator, ExemplarGenerator, ExemplarSet, Sampler, pack_rows
+from .data import DataLoader, Evaluator, ExemplarGenerator, ExemplarSet, FrozenTeacher, Sampler, pack_rows
 from .model import Ader, Ewc
 
 ITEM_NUM = {"DIGINETICA": 43136, "YOOCHOOSE": 25958}     # main.py:133-138
@@ -65,6 +65,9 @@ def build_parser() -> argparse.ArgumentParser:             # main.py:75-108 (typ
     p.add_argument("--max_periods", default=0, type=int)
     p.add_argument("--item_num", default=0, type=int)
     p.add_argument("--loss_impl", default="tc", choices=["tc", "exact"], type=str)      # logits+CE+KD: tcgen05 bf16 / fp32
+    # distillation teacher: the exemplars' stored [E, V_prev] logits, or a frozen snapshot (exemplar reps + a copy of the item
+    # table) from which the loss recomputes them every step -- O(E*d + V_prev*d) memory instead of O(E*V_prev)
+    p.add_argument("--teacher", default="logits", choices=["logits", "frozen"], type=str)
     p.add_argument("--encoder_impl", default=None, choices=["tc", "exact"], type=str)  # training encoder (default follows loss_impl)
     p.add_argument("--infer_encoder_impl", default="exact", choices=["tc", "exact"], type=str)  # eval / herding encoder
     # SURVEY 8(f)1/3: per-period checkpoint + resume (the reference cannot resume a run), binary cache of the period files
@@ -337,7 +340,8 @@ CKPT_NAME = "checkpoint.pt"
 
 PROTOCOL_KEYS = ("dataset", "exemplar_size", "lambda_", "finetune", "dropout", "ewc", "joint", "ewc_sample_num", "selection",
                  "disable_distillation", "equal_exemplar", "fix_lambda", "batch_size", "lr", "num_blocks", "num_heads",
-                 "random_seed", "hidden_units", "maxlen", "dropout_rate", "item_num")
+                 "random_seed", "hidden_units", "maxlen", "dropout_rate", "item_num", "teacher")
+PROTOCOL_DEFAULTS = {"teacher": "logits"}         # value of a key a checkpoint written before the key existed stands for
 
 
 def protocol_args(args) -> dict:
@@ -354,7 +358,8 @@ def save_period_checkpoint(path: str, period: int, model, dataloader, fast_exemp
                                                       for k, v in model.state_dict().items()},
           "item_set": np.array(sorted(dataloader.item_set), dtype=np.int64),
           "exemplar_sessions": None if fast_exemplar is None else [list(map(int, x)) for x in fast_exemplar.sessions],
-          "teacher_width": None if fast_exemplar is None or fast_exemplar.teacher is None else int(fast_exemplar.teacher.shape[1]),
+          "teacher_width": None if fast_exemplar is None or fast_exemplar.teacher is None else _teacher_cols(fast_exemplar.teacher),
+          "teacher_form": "frozen" if fast_exemplar is not None and isinstance(fast_exemplar.teacher, FrozenTeacher) else "logits",
           "carry": carry, "py_random": random.getstate(), "np_random": np.random.get_state()}
     if isinstance(model, Ewc):
         st["ewc"] = {"fisher": None if model.fisher is None else model.fisher.cpu(),
@@ -364,13 +369,22 @@ def save_period_checkpoint(path: str, period: int, model, dataloader, fast_exemp
     os.replace(tmp, path)
 
 
-def rebuild_exemplars(model, sessions, teacher_width: int, maxlen: int, chunk: int = 4096) -> ExemplarSet:
+def _teacher_cols(teacher) -> int:
+    return teacher.width if isinstance(teacher, FrozenTeacher) else int(teacher.shape[1])
+
+
+def rebuild_exemplars(model, sessions, teacher_width: int, maxlen: int, chunk: int = 4096, form: str = "logits") -> ExemplarSet:
     """Exemplar store of a resumed run: stored logits = logits of the saved sessions under the restored weights
-    (what ExemplarGenerator._store computed with the same weights at the end of the period, util.py:433)."""
+    (what ExemplarGenerator._store computed with the same weights at the end of the period, util.py:433); in the frozen
+    form the snapshot of those weights (the sessions' reps and the table), which is what _store kept."""
     rows = [list(x) for x in sessions]
     if teacher_width is None:
         return ExemplarSet(rows, None)
     ids, _, n_in = pack_rows(rows, maxlen)
+    if form == "frozen":
+        reps = [model.rep(ids[lo:lo + chunk], n_tokens=int(n_in[lo:lo + chunk].sum())).clone() for lo in range(0, len(rows), chunk)]
+        rep = torch.cat(reps) if reps else torch.zeros((0, model.hp.hidden_units), device=model.device)
+        return ExemplarSet(rows, FrozenTeacher(model, rep, teacher_width))
     # one [E, ld] buffer with 16-byte aligned rows (ld % 4 == 0), as ExemplarGenerator._store builds it: the teacher kernels
     # read stored logits with 128-bit loads only then
     ld = (teacher_width + 3) // 4 * 4
@@ -387,7 +401,8 @@ def load_period_checkpoint(path: str, model, dataloader, maxlen: int, args=None)
         raise ValueError("%s: unknown checkpoint format" % path)
     if args is not None and st.get("args") is not None:      # refuse to continue a run under a different protocol
         now = protocol_args(args)
-        diff = {k: (st["args"].get(k), now[k]) for k in now if st["args"].get(k) != now[k]}
+        diff = {k: (st["args"].get(k, PROTOCOL_DEFAULTS.get(k)), now[k]) for k in now
+                if st["args"].get(k, PROTOCOL_DEFAULTS.get(k)) != now[k]}
         if diff:
             raise ValueError("%s was written by a run with different flags (saved, now): %s" % (path, diff))
     model.load_state_dict({k: (v.to(model.device) if isinstance(v, torch.Tensor) else v) for k, v in st["model"].items()})
@@ -398,7 +413,7 @@ def load_period_checkpoint(path: str, model, dataloader, maxlen: int, args=None)
         model.theta_star = None if e["theta_star"] is None else e["theta_star"].to(model.device)
     ex = None
     if st["exemplar_sessions"] is not None:
-        ex = rebuild_exemplars(model, st["exemplar_sessions"], st["teacher_width"], maxlen)
+        ex = rebuild_exemplars(model, st["exemplar_sessions"], st["teacher_width"], maxlen, form=st.get("teacher_form", "logits"))
     random.setstate(st["py_random"])
     np.random.set_state(st["np_random"])
     return st["period"], ex, st["carry"]
@@ -594,8 +609,10 @@ def run(args) -> dict:
             cand = train_subseq
             cand.extend(valid_subseq)
             cand.extend(exemplar_subseq)
+            # the frozen teacher stands in for the distillation logits only: one-hot replay / EWC runs keep the stored form
+            form = "frozen" if getattr(args, "teacher", "logits") == "frozen" and not (args.disable_distillation or args.ewc) else "logits"
             gen = ExemplarGenerator(cand, args.exemplar_size, args.equal_exemplar, args.batch_size, args.maxlen,
-                                    args.dropout_rate, max_item)
+                                    args.dropout_rate, max_item, teacher=form)
             if args.selection == "herding":
                 saved = gen.herding_selection(None, model)
             elif args.selection == "loss":

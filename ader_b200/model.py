@@ -171,7 +171,9 @@ class Ader:
                       global_counts=None, _device_step: bool = False, _opt=None) -> torch.Tensor:
         """Forward + backward of the current loss; fills ``self.grad`` (flat).  Returns the device
         scalar loss.  ``exemplar_logits`` is either a host array / list [M_e, V_prev] (reference feed,
-        ADER.py:20) or a device tensor [E, V_prev] indexed by ``teacher_rows`` [M_e]."""
+        ADER.py:20), a device tensor [E, V_prev] indexed by ``teacher_rows`` [M_e], or a ``data.FrozenTeacher``
+        whose reps ``teacher_rows`` indexes the same way."""
+        from .data import FrozenTeacher
         mode = self.mode if mode is None else mode
         lam = self.lambda_ if lambda_ is None else lambda_
         ids = _to_ids(seq, self.hp.maxlen, self.device)
@@ -179,12 +181,19 @@ class Ader:
         M, n_train = ids.shape[0], pos_t.numel()
         n_ex = M - n_train
         teacher = trow = ex_pos_t = None
+        frozen = None
         v_prev = 0
         if n_ex > 0:
             if mode == self.KD:
                 if exemplar_logits is None:
                     raise ValueError("KD loss needs exemplar_logits")
-                if isinstance(exemplar_logits, torch.Tensor):
+                if isinstance(exemplar_logits, FrozenTeacher):
+                    frozen = exemplar_logits
+                    n_rows = len(frozen)
+                    v_prev = frozen.width
+                    if self.loss_impl == "tc" and frozen.table16 is None:
+                        raise ValueError("the tcgen05 loss needs the snapshot's bf16 table (hidden_units <= 160)")
+                elif isinstance(exemplar_logits, torch.Tensor):
                     teacher = exemplar_logits
                 else:
                     a = np.asarray(exemplar_logits, dtype=np.float32)
@@ -192,15 +201,17 @@ class Ader:
                     buf = np.zeros((a.shape[0], ld), np.float32)
                     buf[:, :a.shape[1]] = a
                     teacher = torch.from_numpy(buf).pin_memory().to(self.device, non_blocking=True)[:, :a.shape[1]]
-                if teacher.dim() != 2 or teacher.stride(1) != 1 or teacher.dtype != torch.float32:
-                    raise ValueError("exemplar_logits must be a 2-D fp32 row-major matrix")
-                v_prev = teacher.shape[1]
+                if teacher is not None:
+                    if teacher.dim() != 2 or teacher.stride(1) != 1 or teacher.dtype != torch.float32:
+                        raise ValueError("exemplar_logits must be a 2-D fp32 row-major matrix")
+                    v_prev = teacher.shape[1]
+                    n_rows = teacher.shape[0]
                 if teacher_rows is not None:
                     trow = _to_i32(teacher_rows, self.device)
                     if trow.numel() != n_ex:
                         raise ValueError("teacher_rows must have one entry per exemplar row")
-                elif teacher.shape[0] != n_ex:
-                    raise ValueError("exemplar_logits rows (%d) != exemplar rows (%d)" % (teacher.shape[0], n_ex))
+                elif n_rows != n_ex:
+                    raise ValueError("exemplar_logits rows (%d) != exemplar rows (%d)" % (n_rows, n_ex))
             elif mode == self.ER:
                 if exemplar_pos is None:
                     raise ValueError("one-hot exemplar loss needs exemplar_pos")
@@ -213,7 +224,8 @@ class Ader:
         seed = (self.seed << 32) + (0 if _device_step else self.global_step)
         gc = global_counts if global_counts is not None else self.global_counts
         a = ops.make_loss_args(M, n_train, n_ex, max_item, v_prev, mode if n_ex > 0 else self.VANILLA, lam,
-                               pos_t, ex_pos_t, teacher, trow, *(gc or (0, 0)))
+                               pos_t, ex_pos_t, teacher, trow, *(gc or (0, 0)),
+                               *((frozen.rep, frozen.table, frozen.table16) if frozen is not None else ()))
         row_loss = torch.empty(M, dtype=torch.float32, device=self.device)
         if self.step_impl != "groups" and self.encoder_impl == "tc" and self.loss_impl == "tc" and not _events:
             # one C call: the three groups as a fork/join DAG over library-owned side streams (same kernels, same bits)
@@ -239,7 +251,7 @@ class Ader:
             if self.grad_sync is not None:
                 self.grad_sync()
             self.last_row_loss = row_loss
-            self._keep = (ids, pos_t, teacher, trow, ex_pos_t, rep, d_rep)
+            self._keep = (ids, pos_t, teacher, trow, ex_pos_t, rep, d_rep, frozen)
             return self._loss
         rep, tcap = self.encode(ids, n_tokens, dropout_rate, seed, impl=self.encoder_impl, d_step=d_step)
         if _events:
@@ -261,7 +273,7 @@ class Ader:
         if self.grad_sync is not None:      # data parallel: NCCL all-reduce of the flat gradient
             self.grad_sync()
         self.last_row_loss = row_loss
-        self._keep = (ids, pos_t, teacher, trow, ex_pos_t, rep, d_rep)   # keep alive until the stream is done
+        self._keep = (ids, pos_t, teacher, trow, ex_pos_t, rep, d_rep, frozen)   # keep alive until the stream is done
         return self._loss
 
     def apply_gradients(self, max_item: int, lr: float, ewc_lambda: float = 0.0, fisher=None, theta_star=None):

@@ -99,7 +99,10 @@ def encoder_bwd(ms: AderModel, theta, ids, Tcap: int, ws, bwd_ws, d_rep, grad, d
 
 
 def make_loss_args(M, n_train, n_ex, V, V_prev=0, mode=0, lambda_=0.0, pos=None, ex_pos=None,
-                   teacher=None, teacher_row=None, n_train_global=0, n_ex_global=0) -> AderLossArgs:
+                   teacher=None, teacher_row=None, n_train_global=0, n_ex_global=0,
+                   teacher_rep=None, teacher_table=None, teacher_table16=None) -> AderLossArgs:
+    """Distillation (mode 1) takes stored logits ``teacher`` [*, V_prev] or a frozen snapshot: ``teacher_rep`` [*, d] fp32,
+    ``teacher_table`` fp32 rows of items 1..V_prev (exact entry) and ``teacher_table16`` (``pack_table16``, tcgen05 entries)."""
     a = AderLossArgs()
     a.M, a.n_train, a.n_ex, a.V, a.V_prev, a.mode, a.lambda_ = M, n_train, n_ex, V, V_prev, mode, lambda_
     a.pos = pos.data_ptr() if pos is not None else None
@@ -108,6 +111,9 @@ def make_loss_args(M, n_train, n_ex, V, V_prev=0, mode=0, lambda_=0.0, pos=None,
     a.teacher_row = teacher_row.data_ptr() if teacher_row is not None else None
     a.teacher_ld = teacher.stride(0) if teacher is not None else 0
     a.n_train_global, a.n_ex_global = n_train_global, n_ex_global
+    a.teacher_rep = teacher_rep.data_ptr() if teacher_rep is not None else None
+    a.teacher_table = teacher_table.data_ptr() if teacher_table is not None else None
+    a.teacher_table16 = teacher_table16.data_ptr() if teacher_table16 is not None else None
     return a
 
 
@@ -187,6 +193,21 @@ def loss_tc_vp_bwd(ms: AderModel, theta, rep, a: AderLossArgs, v_lo: int, v_hi: 
     _require_cuda(theta, rep, ws, lse, d_rep_partial, grad)
     check(_lib.load().ader_loss_tc_vp_bwd(C.byref(ms), _ptr(theta), _ptr(rep), C.byref(a), v_lo, v_hi, _ptr(ws), _ptr(lse),
                                           _ptr(d_rep_partial), _ptr(grad), _stream()), "loss_tc_vp_bwd")
+
+
+def table16_bytes(ms: AderModel, V: int) -> int:
+    n = _lib.load().ader_table16_ws_bytes(C.byref(ms), V)
+    if n == 0:
+        raise _lib.AderError("table16_ws_bytes: bad model / sizes")
+    return n
+
+
+def pack_table16(ms: AderModel, rows, V: int, out):
+    """out (uint8, table16_bytes(ms, V)) = bf16 [ceil(V/128)*128][160] shadow of ``rows`` (fp32 rows of items 1..V, stride d)."""
+    _require_cuda(rows, out)
+    if out.numel() * out.element_size() < table16_bytes(ms, V):
+        raise _lib.AderError("pack_table16: output buffer too small")
+    check(_lib.load().ader_pack_table16(C.byref(ms), _ptr(rows), V, _ptr(out), _stream()), "pack_table16")
 
 
 def logits(ms: AderModel, theta, rep, V: int, out):
@@ -366,7 +387,7 @@ def queue_advance(counter):
 # (CUDA key only: there is no CPU implementation to fall back to).  The POD structs of the C ABI are flattened:
 #   model  = int[5]   (v_tab, d, maxlen, num_blocks, num_heads)
 #   loss   = int[8]   (M, n_train, n_ex, V, V_prev, mode, n_train_global, n_ex_global) + float lambda_ + Tensor? pos, ex_pos,
-#                     teacher, teacher_row
+#                     teacher, teacher_row (+ trailing Tensor? teacher_rep, teacher_table, teacher_table16 = None: frozen teacher)
 #   dp comm = int rank, int world, int[] theta_ptrs, int[] grad_ptrs, int[] flag_ptrs  (peer-mapped device addresses)
 # Workspace-size queries, IPC plumbing and status reads are host-only helpers and stay plain Python functions.
 _registered = False
@@ -376,12 +397,13 @@ _SCHEMAS = {
     "encoder_fwd_tc": "(int[] model, Tensor theta, Tensor ids, int Tcap, Tensor(a!) ws, Tensor(b!) rep, float dropout_rate, int seed, Tensor? d_step) -> ()",
     "encoder_bwd": "(int[] model, Tensor theta, Tensor ids, int Tcap, Tensor ws, Tensor(a!) bwd_ws, Tensor d_rep, Tensor(b!) grad, float dropout_rate, int seed) -> ()",
     "encoder_bwd_tc": "(int[] model, Tensor theta, Tensor ids, int Tcap, Tensor ws, Tensor(a!) bwd_ws, Tensor d_rep, Tensor(b!) grad, float dropout_rate, int seed, Tensor? d_step) -> ()",
-    "loss_fwd_bwd": "(int[] model, Tensor theta, Tensor rep, int[] loss_dims, float lambda_, Tensor? pos, Tensor? ex_pos, Tensor? teacher, Tensor? teacher_row, Tensor(a!) ws, Tensor(b!) loss, Tensor(c!) row_loss, Tensor(d!) d_rep, Tensor(e!) grad) -> ()",
-    "loss_fwd_bwd_tc": "(int[] model, Tensor theta, Tensor rep, int[] loss_dims, float lambda_, Tensor? pos, Tensor? ex_pos, Tensor? teacher, Tensor? teacher_row, Tensor(a!) ws, Tensor(b!) loss, Tensor(c!) row_loss, Tensor(d!) d_rep, Tensor(e!) grad) -> ()",
+    "loss_fwd_bwd": "(int[] model, Tensor theta, Tensor rep, int[] loss_dims, float lambda_, Tensor? pos, Tensor? ex_pos, Tensor? teacher, Tensor? teacher_row, Tensor(a!) ws, Tensor(b!) loss, Tensor(c!) row_loss, Tensor(d!) d_rep, Tensor(e!) grad, Tensor? teacher_rep=None, Tensor? teacher_table=None, Tensor? teacher_table16=None) -> ()",
+    "loss_fwd_bwd_tc": "(int[] model, Tensor theta, Tensor rep, int[] loss_dims, float lambda_, Tensor? pos, Tensor? ex_pos, Tensor? teacher, Tensor? teacher_row, Tensor(a!) ws, Tensor(b!) loss, Tensor(c!) row_loss, Tensor(d!) d_rep, Tensor(e!) grad, Tensor? teacher_rep=None, Tensor? teacher_table=None, Tensor? teacher_table16=None) -> ()",
     "loss_tc_vp_fwd": "(int[] model, Tensor theta, Tensor rep, int[] loss_dims, float lambda_, Tensor? pos, Tensor? ex_pos, Tensor? teacher, Tensor? teacher_row, int v_lo, int v_hi, Tensor(a!) ws, Tensor(b!) stats) -> ()",
     "loss_tc_vp_bwd": "(int[] model, Tensor theta, Tensor rep, int[] loss_dims, float lambda_, Tensor? pos, Tensor? ex_pos, Tensor? teacher, Tensor? teacher_row, int v_lo, int v_hi, Tensor(a!) ws, Tensor lse, Tensor(b!) d_rep_partial, Tensor(c!) grad) -> ()",
-    "train_fwd_bwd_tc": "(int[] model, Tensor theta, Tensor ids, int Tcap, int[] loss_dims, float lambda_, Tensor? pos, Tensor? ex_pos, Tensor? teacher, Tensor? teacher_row, Tensor(a!) enc_ws, Tensor(b!) bwd_ws, Tensor(c!) loss_ws, Tensor(d!) rep, Tensor(e!) loss, Tensor(f!) row_loss, Tensor(g!) d_rep, Tensor(h!) grad, float dropout_rate, int seed, Tensor? d_step, bool serial) -> ()",
-    "train_step_tc": "(int[] model, Tensor(a!) theta, Tensor ids, int Tcap, int[] loss_dims, float lambda_, Tensor? pos, Tensor? ex_pos, Tensor? teacher, Tensor? teacher_row, Tensor(b!) enc_ws, Tensor(c!) bwd_ws, Tensor(d!) loss_ws, Tensor(e!) rep, Tensor(f!) loss, Tensor(g!) row_loss, Tensor(h!) d_rep, Tensor(i!) grad, Tensor(j!) adam_m, Tensor(k!) adam_v, Tensor(l!) state, int V, float lr, float dropout_rate, int seed, Tensor? d_step, float ewc_lambda, Tensor? fisher, Tensor? theta_star, bool serial) -> ()",
+    "train_fwd_bwd_tc": "(int[] model, Tensor theta, Tensor ids, int Tcap, int[] loss_dims, float lambda_, Tensor? pos, Tensor? ex_pos, Tensor? teacher, Tensor? teacher_row, Tensor(a!) enc_ws, Tensor(b!) bwd_ws, Tensor(c!) loss_ws, Tensor(d!) rep, Tensor(e!) loss, Tensor(f!) row_loss, Tensor(g!) d_rep, Tensor(h!) grad, float dropout_rate, int seed, Tensor? d_step, bool serial, Tensor? teacher_rep=None, Tensor? teacher_table=None, Tensor? teacher_table16=None) -> ()",
+    "train_step_tc": "(int[] model, Tensor(a!) theta, Tensor ids, int Tcap, int[] loss_dims, float lambda_, Tensor? pos, Tensor? ex_pos, Tensor? teacher, Tensor? teacher_row, Tensor(b!) enc_ws, Tensor(c!) bwd_ws, Tensor(d!) loss_ws, Tensor(e!) rep, Tensor(f!) loss, Tensor(g!) row_loss, Tensor(h!) d_rep, Tensor(i!) grad, Tensor(j!) adam_m, Tensor(k!) adam_v, Tensor(l!) state, int V, float lr, float dropout_rate, int seed, Tensor? d_step, float ewc_lambda, Tensor? fisher, Tensor? theta_star, bool serial, Tensor? teacher_rep=None, Tensor? teacher_table=None, Tensor? teacher_table16=None) -> ()",
+    "pack_table16": "(int[] model, Tensor rows, int V, Tensor(a!) out) -> ()",
     "logits": "(int[] model, Tensor theta, Tensor rep, int V, Tensor(a!) out) -> ()",
     "adam_step": "(int[] model, Tensor(a!) theta, Tensor(b!) m, Tensor(c!) v, Tensor grad, Tensor(d!) state, int V, float lr, float ewc_lambda, Tensor? fisher, Tensor? theta_star) -> ()",
     "dp_wait": "(int rank, int world, int[] theta_ptrs, int[] grad_ptrs, int[] flag_ptrs, Tensor(a!) flags) -> ()",
@@ -410,9 +432,9 @@ def register_torch_ops() -> None:
     def _ms(model):
         return AderModel(*[int(x) for x in model])
 
-    def _la(dims, lam, pos, ex_pos, teacher, teacher_row):
+    def _la(dims, lam, pos, ex_pos, teacher, teacher_row, fz=(None, None, None)):
         M, n_train, n_ex, V, V_prev, mode, ntg, neg = [int(x) for x in dims]
-        return make_loss_args(M, n_train, n_ex, V, V_prev, mode, lam, pos, ex_pos, teacher, teacher_row, ntg, neg)
+        return make_loss_args(M, n_train, n_ex, V, V_prev, mode, lam, pos, ex_pos, teacher, teacher_row, ntg, neg, *fz)
 
     def _comm(rank, world, tp, gp, fp):
         return dp_comm(int(rank), int(world), list(tp), list(gp), list(fp))
@@ -422,18 +444,19 @@ def register_torch_ops() -> None:
         "encoder_fwd_tc": lambda model, theta, ids, Tcap, ws, rep, p, seed, d_step: encoder_fwd(_ms(model), theta, ids, Tcap, ws, rep, p, seed, impl="tc", d_step=d_step),
         "encoder_bwd": lambda model, theta, ids, Tcap, ws, bws, d_rep, grad, p, seed: encoder_bwd(_ms(model), theta, ids, Tcap, ws, bws, d_rep, grad, p, seed),
         "encoder_bwd_tc": lambda model, theta, ids, Tcap, ws, bws, d_rep, grad, p, seed, d_step: encoder_bwd(_ms(model), theta, ids, Tcap, ws, bws, d_rep, grad, p, seed, impl="tc", d_step=d_step),
-        "loss_fwd_bwd": lambda model, theta, rep, dims, lam, pos, ex_pos, teacher, trow, ws, loss, row_loss, d_rep, grad:
-            loss_fwd_bwd(_ms(model), theta, rep, _la(dims, lam, pos, ex_pos, teacher, trow), ws, loss, row_loss, d_rep, grad),
-        "loss_fwd_bwd_tc": lambda model, theta, rep, dims, lam, pos, ex_pos, teacher, trow, ws, loss, row_loss, d_rep, grad:
-            loss_fwd_bwd_tc(_ms(model), theta, rep, _la(dims, lam, pos, ex_pos, teacher, trow), ws, loss, row_loss, d_rep, grad),
+        "loss_fwd_bwd": lambda model, theta, rep, dims, lam, pos, ex_pos, teacher, trow, ws, loss, row_loss, d_rep, grad, *fz:
+            loss_fwd_bwd(_ms(model), theta, rep, _la(dims, lam, pos, ex_pos, teacher, trow, fz), ws, loss, row_loss, d_rep, grad),
+        "loss_fwd_bwd_tc": lambda model, theta, rep, dims, lam, pos, ex_pos, teacher, trow, ws, loss, row_loss, d_rep, grad, *fz:
+            loss_fwd_bwd_tc(_ms(model), theta, rep, _la(dims, lam, pos, ex_pos, teacher, trow, fz), ws, loss, row_loss, d_rep, grad),
         "loss_tc_vp_fwd": lambda model, theta, rep, dims, lam, pos, ex_pos, teacher, trow, v_lo, v_hi, ws, stats:
             loss_tc_vp_fwd(_ms(model), theta, rep, _la(dims, lam, pos, ex_pos, teacher, trow), v_lo, v_hi, ws, stats),
         "loss_tc_vp_bwd": lambda model, theta, rep, dims, lam, pos, ex_pos, teacher, trow, v_lo, v_hi, ws, lse, d_part, grad:
             loss_tc_vp_bwd(_ms(model), theta, rep, _la(dims, lam, pos, ex_pos, teacher, trow), v_lo, v_hi, ws, lse, d_part, grad),
-        "train_fwd_bwd_tc": lambda model, theta, ids, Tcap, dims, lam, pos, ex_pos, teacher, trow, ews, bws, lws, rep, loss, row_loss, d_rep, grad, p, seed, d_step, serial:
-            train_fwd_bwd_tc(_ms(model), theta, ids, Tcap, _la(dims, lam, pos, ex_pos, teacher, trow), ews, bws, lws, rep, loss, row_loss, d_rep, grad, p, seed, d_step, serial),
-        "train_step_tc": lambda model, theta, ids, Tcap, dims, lam, pos, ex_pos, teacher, trow, ews, bws, lws, rep, loss, row_loss, d_rep, grad, am, av, state, V, lr, p, seed, d_step, ewc_lambda, fisher, theta_star, serial:
-            train_step_tc(_ms(model), theta, ids, Tcap, _la(dims, lam, pos, ex_pos, teacher, trow), ews, bws, lws, rep, loss, row_loss, d_rep, grad, am, av, state, V, lr, p, seed, d_step, ewc_lambda, fisher, theta_star, serial=serial),
+        "train_fwd_bwd_tc": lambda model, theta, ids, Tcap, dims, lam, pos, ex_pos, teacher, trow, ews, bws, lws, rep, loss, row_loss, d_rep, grad, p, seed, d_step, serial, *fz:
+            train_fwd_bwd_tc(_ms(model), theta, ids, Tcap, _la(dims, lam, pos, ex_pos, teacher, trow, fz), ews, bws, lws, rep, loss, row_loss, d_rep, grad, p, seed, d_step, serial),
+        "train_step_tc": lambda model, theta, ids, Tcap, dims, lam, pos, ex_pos, teacher, trow, ews, bws, lws, rep, loss, row_loss, d_rep, grad, am, av, state, V, lr, p, seed, d_step, ewc_lambda, fisher, theta_star, serial, *fz:
+            train_step_tc(_ms(model), theta, ids, Tcap, _la(dims, lam, pos, ex_pos, teacher, trow, fz), ews, bws, lws, rep, loss, row_loss, d_rep, grad, am, av, state, V, lr, p, seed, d_step, ewc_lambda, fisher, theta_star, serial=serial),
+        "pack_table16": lambda model, rows, V, out: pack_table16(_ms(model), rows, V, out),
         "logits": lambda model, theta, rep, V, out: logits(_ms(model), theta, rep, V, out),
         "adam_step": lambda model, theta, m, v, grad, state, V, lr, ewc_lambda, fisher, theta_star: adam_step(_ms(model), theta, m, v, grad, state, V, lr, ewc_lambda, fisher, theta_star),
         "dp_wait": lambda rank, world, tp, gp, fp, flags: dp_wait(_comm(rank, world, tp, gp, fp)),

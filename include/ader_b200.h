@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define ADER_ABI_VERSION 1
+#define ADER_ABI_VERSION 2
 
 typedef struct AderModel {
   int32_t v_tab;       /* rows of the item table = item_num + 1   (ADER.py:29-38)           */
@@ -99,11 +99,18 @@ typedef struct AderLossArgs {
   float   lambda_;         /* main.py:196-200                                                  */
   const int32_t* pos;      /* [n_train] labels 1..V                                            */
   const int32_t* ex_pos;   /* [n_ex] labels (mode 2)                                           */
-  const float*   teacher;  /* [*, V_prev] fp32 stored exemplar logits (mode 1)                 */
-  const int32_t* teacher_row; /* [n_ex] row of `teacher` per exemplar row, or NULL = identity  */
+  const float*   teacher;  /* [*, V_prev] fp32 stored exemplar logits (mode 1), or NULL with teacher_rep */
+  const int32_t* teacher_row; /* [n_ex] row of `teacher` (or `teacher_rep`) per exemplar row, or NULL = identity */
   int64_t teacher_ld;      /* row stride of `teacher` in elements (>= V_prev)                  */
   int32_t n_train_global;  /* data parallel: denominators of the two means over ALL ranks (0 = local   */
   int32_t n_ex_global;     /* counts); gradients and loss are then summed, not averaged, across ranks  */
+  /* Frozen teacher (mode 1, instead of `teacher`): a snapshot of the previous model.  Teacher logits are recomputed per
+   * step as teacher_rep[teacher_row[e]] . table^T over items 1..V_prev, so the library never holds an [E, V_prev] matrix.
+   * Exactly one of `teacher` / `teacher_rep` is set in mode 1. */
+  const float* teacher_rep;      /* [*, d] fp32 exemplar representations (exact encoder, taken at selection time) */
+  const float* teacher_table;    /* fp32 rows of items 1..V_prev of the frozen item table, row stride d (exact entry) */
+  const void*  teacher_table16;  /* bf16 [ceil(V_prev/128)*128][160] shadow of the same rows (ader_pack_table16;
+                                    tcgen05 entries) */
 } AderLossArgs;
 
 size_t  ader_loss_ws_bytes(const AderModel* m, const AderLossArgs* a);
@@ -116,7 +123,9 @@ int32_t ader_loss_fwd_bwd(const AderModel* m, const float* theta, const float* r
  * logits + online-softmax CE + distillation, [M, V] logits never materialised in HBM.  Distillation
  * rows enter by linearity: bf16 tiles of coef * softmax(teacher) are MMA operands (uc = Pc.E for the loss and
  * d_rep, dE -= Pc^T.rep), so the hot kernels never read the fp32 teacher.  Results agree with
- * ader_loss_fwd_bwd to bf16 operand rounding (tests state the tolerance). */
+ * ader_loss_fwd_bwd to bf16 operand rounding (tests state the tolerance).
+ * With a frozen teacher (teacher_rep + teacher_table16) two more tcgen05 passes over the snapshot give the teacher's
+ * log-sum-exp and then the same bf16 Pc tiles, on the side of the step that does not depend on `rep`. */
 size_t  ader_loss_tc_ws_bytes(const AderModel* m, const AderLossArgs* a);
 int32_t ader_loss_fwd_bwd_tc(const AderModel* m, const float* theta, const float* rep,
                              const AderLossArgs* a, void* ws, float* loss, float* row_loss,
@@ -129,7 +138,8 @@ int32_t ader_debug_loss_tc_kernels(const AderModel* m, const float* theta, const
  *   fwd  -> stats [M,4] = this shard's per-row (max, sum exp(s - max), label logit or 0, KD dot);
  *           the caller all-reduces them (max; rescaled sum; sums) into lse [M];
  *   bwd  -> d_rep_partial [M,d] (to be all-reduce-summed) and grad rows v_lo+1 .. v_hi of the item table.
- * `a->V` stays the GLOBAL max_item.  The workspace must persist between the two calls. */
+ * `a->V` stays the GLOBAL max_item.  The workspace must persist between the two calls.  Stored teacher logits only
+ * (a frozen teacher is rejected). */
 size_t  ader_loss_tc_vp_ws_bytes(const AderModel* m, const AderLossArgs* a, int32_t v_lo, int32_t v_hi);
 int32_t ader_loss_tc_vp_fwd(const AderModel* m, const float* theta, const float* rep, const AderLossArgs* a,
                             int32_t v_lo, int32_t v_hi, void* ws, float* stats, void* stream);
@@ -153,6 +163,12 @@ int32_t ader_train_fwd_bwd_tc(const AderModel* m, const float* theta, const int3
                               const AderLossArgs* a, void* enc_ws, void* bwd_ws, void* loss_ws, float* rep,
                               float* loss, float* row_loss, float* d_rep, float* grad, float dropout_rate,
                               uint64_t seed, const int32_t* d_step, int32_t serial, void* stream);
+
+/* bf16 shadow of table rows for the tcgen05 entries: `rows` = fp32 rows of items 1..V, row stride d (theta + d for the
+ * live table, or a frozen AderLossArgs.teacher_table) -> out bf16 [ceil(V/128)*128][160], rows >= V and columns >= d zero
+ * (the operand layout of the tcgen05 loss kernels).  ader_table16_ws_bytes = bytes of `out`.  Needs hidden_units <= 160. */
+size_t  ader_table16_ws_bytes(const AderModel* m, int32_t V);
+int32_t ader_pack_table16(const AderModel* m, const float* rows, int32_t V, void* out, void* stream);
 
 /* logits [M, V] fp32 = rep . E[1..V]^T  (fetch `logits`, util.py:452,482,514). ld = row stride. */
 int32_t ader_logits(const AderModel* m, const float* theta, const float* rep, int32_t M, int32_t V,
