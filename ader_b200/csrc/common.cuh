@@ -115,9 +115,6 @@ struct AdamPlan {
 };
 int adam_prep_early(const AdamPlan& p, cudaStream_t st);                       // state[1] = lr_t(state[0] + 1); no increment
 int adam_table_part(const AderModel* m, const AdamPlan& p, cudaStream_t st);   // item-table rows 1..V
-// item-table rows 1..V that no input token of this step touches (touched[row] == 0): their gradient is final as soon as the
-// dE kernel is done, so this part of the update runs beside the scatter; the touched rows follow it (k_adam_touched)
-int adam_table_untouched(const AderModel* m, const AdamPlan& p, const uint8_t* touched, cudaStream_t st);
 
 // d_rep reduction folded into the final-LayerNorm backward (fused step only): the loss group hands its split partials over
 // instead of launching k_reduce_drep; part is [n_chunks][rows_pad][kp] fp32, u the [.,kp] teacher term of the distillation rows
@@ -135,12 +132,11 @@ struct Fork {
   cudaEvent_t plan_ready;                  // recorded on `c` behind the scatter plan (sorted ids)
   bool plan_done;
   bool pdl;                                // launch the kernel-to-kernel chain links of `main` as programmatic dependent launches
-  bool split_adam;                         // fused step: Adam on the untouched table rows beside the scatter, on the touched rows behind it
   bool fuse_drep, has_drep;                // fused step: the d_rep partials are summed by the final-LayerNorm backward kernel
   DrepFuse drep;
   static Fork serial(cudaStream_t st) {
     Fork f; f.main = f.a = f.b = f.c = st; f.wg[0] = f.wg[1] = f.wg[2] = st; f.ev = nullptr; f.n_ev = f.next_ev = 0; f.pdl = false; f.adam = nullptr;
-    f.split_adam = f.fuse_drep = f.has_drep = false; f.drep = DrepFuse();
+    f.fuse_drep = f.has_drep = false; f.drep = DrepFuse();
     f.table_ready = f.tok_ready = f.plan_ready = nullptr; f.has_table_ready = f.has_tok_ready = f.plan_done = false;
     return f;
   }
@@ -162,7 +158,6 @@ int enc_bwd_tc_run(const AderModel* m, const float* theta, const int32_t* ids, i
                    const float* d_rep, float* grad, float dropout_rate, uint64_t seed, const int32_t* d_step, Fork& f);
 // the scatter's sort of (item id, token) pairs on f.c, as soon as the token ids are packed (parallel plans only)
 int enc_scatter_plan_run(const AderModel* m, int M, int Tcap, const void* ws, void* bwd_ws, Fork& f);
-bool enc_chain_enabled(const AderModel* m);      // ADER_B200_CHAIN=1 and the model fits the chained kernels
 // phase 0: everything that does not need `rep` (table tiles, teacher statistics / tiles, uc partials) on f.b;
 // phase 1: the rest (rep tiles, forward statistics, loss, d_rep on f.main; dE on f.b)
 int loss_tc_run(const AderModel* m, const float* theta, const float* rep, const AderLossArgs* a, void* ws, float* loss,

@@ -8,21 +8,15 @@
 // step is stream-ordered with no host synchronisation; grids are sized for the capacity Tcap and
 // surplus CTAs exit at once.
 #include "common.cuh"
-#include <stdlib.h>
 
 namespace ader {
 
 constexpr int NSLOT = 8;          // per-block [Tcap,d] activation slots
 constexpr int SPLITS = 21;        // split-K partials for weight / LN / bias gradients (21 x 7 problems = 147 CTAs: one wave of 148 SMs)
-constexpr int CHAIN_SPLITS = 14;  // chained encoder path: 14 splits x 10 weight matrices = 140 CTAs in ONE launch
 constexpr int PG_LANES = 6;       // token lanes per column in the LN / position gradient reductions (160 x 6 = 960 threads)
 
-// workspace flag words: [0..3] packing / overflow flags, then the neighbour flags of the chained encoder kernels
-// (encoder_chain.cuh): forward [block][CTA], backward [block][CTA], backward completion counter.  k_row_len (first
-// kernel of every forward) zeroes all of them.
-constexpr int CHF_STRIDE = 160;                    // >= CTAs of a chained kernel (one per SM)
-constexpr int CHF_FWD = 4, CHF_BWD = CHF_FWD + 2 * CHF_STRIDE, CHF_DONE = CHF_BWD + 2 * CHF_STRIDE;
-constexpr int N_WS_FLAGS = CHF_DONE + 4;
+// workspace flag words: packing / overflow flags.  k_row_len (first kernel of every forward) zeroes them.
+constexpr int N_WS_FLAGS = 4;
 
 struct EncWs {
   int *row_len, *row_off, *tok_row, *tok_id, *flags;
@@ -61,7 +55,6 @@ struct BwdWs {
   int *keys[2], *vals[2], *hist;
   float* Dv;             // fused path: per-token softmax-backward row dots
   float* spart; int* scount;   // windowed scatter: partial slots [windows][2][SPAD], arrival counters [windows]
-  uint8_t* touched;            // [v_tab] 1 = an input token of this step carries the item (written by the scatter plan)
   int2* sbounds;               // [windows] segment head of a window's first run / segment end of its last run (scatter plan)
   float* g2[8];          // fused path: second set of gO..gQ1 (blocks alternate sets, so the weight-gradient kernel of
                          // block b may still read its set while block b-1's data-gradient kernels write the other)
@@ -80,7 +73,6 @@ static BwdWs carve_bwd(const AderModel* m, int M, int Tcap, char* base) {
   for (int i = 0; i < 8; ++i) w.g2[i] = (float*)take(sizeof(float) * (size_t)Tcap * m->d);
   w.spart = (float*)take(sizeof(float) * (size_t)cdiv(Tcap, 16) * 2 * 256);
   w.scount = (int*)take(sizeof(int) * (size_t)cdiv(Tcap, 16));
-  w.touched = (uint8_t*)take(align_up((size_t)m->v_tab, 16));
   w.sbounds = (int2*)take(sizeof(int2) * (size_t)cdiv(Tcap, 16));
   w.bytes = o;
   return w;
@@ -133,64 +125,6 @@ __global__ void __launch_bounds__(1024) k_scan_rows(const int* __restrict__ row_
     int T = carry;
     if (T > Tcap) { flags[0] = T; T = Tcap; }   // overflow: host checks flags[0] lazily
     row_off[M] = T;
-  }
-}
-
-// The three packing kernels above as ONE single-CTA kernel for batches of up to 1024 rows: the id matrix is staged in shared
-// memory with one coalesced pass, lengths / offsets / token lists come from there.  Same integers.  Opt-in
-// (ADER_B200_PACK=1), because it is SLOWER in the step: 0.2818 / 0.2820 ms against 0.2765 / 0.2759 for the three launches
-// (same box, alternating runs) -- one SM pulling 130 KB through its own L2 port and walking 650 rows with 32 warps takes
-// longer than three 3 us kernels spread over the chip, launch gaps included.
-constexpr int PACK1_THR = 1024;
-__global__ void __launch_bounds__(PACK1_THR) k_pack_small(const int* __restrict__ ids, int M, int L, int Tcap, int* __restrict__ row_len,
-                                                          int* __restrict__ row_off, int* __restrict__ tok_row, int* __restrict__ tok_id,
-                                                          int* __restrict__ flags) {
-  extern __shared__ int pk_sm[];
-  int* ids_s = pk_sm;                       // [M * L]
-  int* len_s = ids_s + M * L;               // [1024]
-  int* off_s = len_s + PACK1_THR;           // [1024]
-  __shared__ int warp_sum[32];
-  const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-  for (int i = tid; i < N_WS_FLAGS; i += PACK1_THR) flags[i] = 0;
-  for (int i = tid; i < M * L; i += PACK1_THR) ids_s[i] = ids[i];
-  __syncthreads();
-  for (int r = wid; r < M; r += PACK1_THR / 32) {        // row lengths: warp per row
-    int c = 0;
-    for (int j = lane; j < L; j += 32) c += (ids_s[r * L + j] != 0);
-#pragma unroll
-    for (int o = 16; o; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
-    if (lane == 0) { len_s[r] = c; row_len[r] = c; }
-  }
-  __syncthreads();
-  const int v = (tid < M) ? len_s[tid] : 0;              // exclusive scan over the rows (M <= 1024: one element per thread)
-  int x = v;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) { int y = __shfl_up_sync(0xffffffffu, x, o); if (lane >= o) x += y; }
-  if (lane == 31) warp_sum[wid] = x;
-  __syncthreads();
-  if (wid == 0) {
-    int t = warp_sum[lane];
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) { int y = __shfl_up_sync(0xffffffffu, t, o); if (lane >= o) t += y; }
-    warp_sum[lane] = t;
-  }
-  __syncthreads();
-  const int excl = (wid ? warp_sum[wid - 1] : 0) + x - v;
-  if (tid < M) { off_s[tid] = excl; row_off[tid] = excl; }
-  if (tid == 0) {
-    int T = warp_sum[31];
-    if (T > Tcap) { flags[0] = T; T = Tcap; }            // overflow: checked by the host (ader_b200/model.py)
-    row_off[M] = T;
-  }
-  __syncthreads();
-  for (int r = wid; r < M; r += PACK1_THR / 32) {        // token lists: real tokens are the suffix (util.py:161-169)
-    const int n = len_s[r], off = off_s[r];
-    for (int i = lane; i < n; i += 32) {
-      if (off + i < Tcap) {
-        tok_row[off + i] = r;
-        tok_id[off + i] = ids_s[r * L + (L - n + i)];
-      }
-    }
   }
 }
 
@@ -789,15 +723,14 @@ __global__ void k_pos_grad(const float* __restrict__ gx, const int* __restrict__
 // ------------------------------------------------------------------------------------------
 constexpr int SORT_TILE = 2048;
 
-// start of the plan: arrival counters and the touched-row flags back to zero (a memset node costs ~10 us in a graph)
-__global__ void k_plan_zero(uint4* __restrict__ touched16, int n16, int* __restrict__ scount, int n_count) {
+// start of the plan: arrival counters back to zero (a memset node costs ~10 us in a graph)
+__global__ void k_plan_zero(int* __restrict__ scount, int n_count) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n16) touched16[i] = make_uint4(0u, 0u, 0u, 0u);
   if (i < n_count) scount[i] = 0;
 }
 
 __global__ void __launch_bounds__(256) k_sort_hist(const int* __restrict__ keys, const int* __restrict__ dT,
-                                                   int shift, int ntiles, int* __restrict__ hist, uint8_t* __restrict__ touched) {
+                                                   int shift, int ntiles, int* __restrict__ hist) {
   __shared__ int h[256];
   h[threadIdx.x] = 0;
   __syncthreads();
@@ -805,11 +738,7 @@ __global__ void __launch_bounds__(256) k_sort_hist(const int* __restrict__ keys,
   const int base = blockIdx.x * SORT_TILE;
   for (int r = 0; r < SORT_TILE / 256; ++r) {
     int i = base + r * 256 + threadIdx.x;
-    if (i < T) {
-      const int key = keys[i];
-      atomicAdd(&h[(key >> shift) & 255], 1);                  // integer atomics: order-independent result
-      if (touched) touched[key] = 1;                           // first pass: rows the scatter will add into
-    }
+    if (i < T) atomicAdd(&h[(keys[i] >> shift) & 255], 1);    // integer atomics: order-independent result
   }
   __syncthreads();
   hist[threadIdx.x * ntiles + blockIdx.x] = h[threadIdx.x];
@@ -1019,125 +948,17 @@ __global__ void __launch_bounds__(256) k_scatter_apply(const int* __restrict__ k
   }
 }
 
-// Shared-memory form of the windowed reduction (opt-in: ADER_B200_SCATTER=2; measured equal to slightly slower in the step:
-// its 40 KB of shared memory do not fit beside the weight-gradient CTAs the tail runs next to).  k_scatter_apply
-// keeps a window's 16 gradient rows in registers, which forces the 16-step run loop to be unrolled: 49 KB of straight-line
-// code that every warp executes exactly once -- the kernel (30 CTAs, on the tail of the step) was bound by instruction
-// fetch, not by its three dependent memory trips.  Here the rows go to shared memory with cp.async (one batch, no register
-// staging) and the run loop is a real loop over the window: a few hundred instructions.  Same sums in the same order.
-constexpr int SW2_WARPS = 4;
-template <int NEL>
-__global__ void __launch_bounds__(SW2_WARPS * 32) k_scatter_apply2(const int* __restrict__ keys, const int* __restrict__ vals,
-                                                                   const int* __restrict__ dT, const float* __restrict__ gx, int d, float scale,
-                                                                   float* __restrict__ gtable, float* __restrict__ part, int* __restrict__ counter,
-                                                       const int2* __restrict__ bounds) {
-  __shared__ float rows[SW2_WARPS][SW][NEL * 32];
-  const int T = *dT;
-  const int w = (int)((blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
-  const int p0 = w * SW;
-  if (p0 >= T) return;
-  float (*my)[NEL * 32] = rows[threadIdx.x >> 5];
-  const int n = min(SW, T - p0);
-  const int key_l = (lane < n) ? keys[p0 + lane] : -1;
-  const int val_l = (lane < n) ? vals[p0 + lane] : 0;
-  const int key_prev = (p0 > 0) ? keys[p0 - 1] : -1;
-  const int key_next = (p0 + n < T) ? keys[p0 + n] : -1;
-#pragma unroll 1
-  for (int u = 0; u < n; ++u) {
-    const long long o = (long long)__shfl_sync(0xffffffffu, val_l, u) * d;
-#pragma unroll
-    for (int i = 0; i < NEL; ++i) {
-      const int c = lane + 32 * i;
-      const bool ok = c < d;
-      asm volatile("cp.async.ca.shared.global [%0], [%1], 4, %2;" ::"r"((uint32_t)__cvta_generic_to_shared(&my[u][c])),
-                   "l"(ok ? gx + o + c : gx), "r"(ok ? 4 : 0) : "memory");
-    }
-  }
-  asm volatile("cp.async.commit_group;\n cp.async.wait_group 0;" ::: "memory");
-  __syncwarp();
-  float acc[NEL];
-#pragma unroll
-  for (int i = 0; i < NEL; ++i) acc[i] = 0.f;
-  int run_start = 0;
-#pragma unroll 1
-  for (int u = 0; u < n; ++u) {
-    const int ku = __shfl_sync(0xffffffffu, key_l, u);
-    const int kn = __shfl_sync(0xffffffffu, key_l, (u + 1) & 31);
-#pragma unroll
-    for (int i = 0; i < NEL; ++i) acc[i] += my[u][lane + 32 * i];
-    const bool last_in_window = (u + 1 == n);
-    if (last_in_window || kn != ku) {                              // the run [run_start, u] of item ku ends here
-      const bool cont_after = last_in_window && key_next == ku;
-      const bool cont_before = run_start == 0 && key_prev == ku;
-      if (!cont_after && !cont_before) {
-#pragma unroll
-        for (int i = 0; i < NEL; ++i) { const int c = lane + 32 * i; if (c < d) atomicAdd(gtable + (long long)ku * d + c, scale * acc[i]); }
-      } else {
-        scatter_piece<NEL>(p0, w, lane, ku, run_start, u, cont_before, cont_after, acc, gtable, d, scale, part, counter, bounds);
-      }
-#pragma unroll
-      for (int i = 0; i < NEL; ++i) acc[i] = 0.f;
-      run_start = u + 1;
-    }
-  }
-}
-
-// Fused step with the split table update (f.split_adam): TF1 Adam on the table rows the scatter added into, one warp per
-// sorted position that starts a segment (= one warp per distinct item of the batch).  The other rows 1..V were updated by
-// k_adam_untouched beside the scatter; same arithmetic (adam_update_elem), so the step's bits do not depend on the split.
-__global__ void __launch_bounds__(256) k_adam_touched(const int* __restrict__ keys, const int* __restrict__ dT, int d, int V,
-                                                      const float* __restrict__ gtable, float* __restrict__ theta, float* __restrict__ am,
-                                                      float* __restrict__ av, const int* __restrict__ state, float beta1, float beta2,
-                                                      float eps, float ewc_lambda, const float* __restrict__ fisher,
-                                                      const float* __restrict__ theta_star) {
-  const int p = (int)((blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
-  if (p >= *dT) return;
-  const int key = keys[p];
-  if ((p > 0 && keys[p - 1] == key) || key < 1 || key > V) return;
-  const float lr_t = __int_as_float(state[1]);
-  const long long o = (long long)key * d;
-  for (int c0 = 0; c0 < d; c0 += 128) {          // four elements per lane in flight
-    float g[4], th[4], m[4], v[4], fi[4], ts[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int c = c0 + lane + 32 * i; const bool ok = c < d;
-      g[i] = ok ? gtable[o + c] : 0.f; th[i] = ok ? theta[o + c] : 0.f; m[i] = ok ? am[o + c] : 0.f; v[i] = ok ? av[o + c] : 0.f;
-      fi[i] = (ok && ewc_lambda != 0.f) ? fisher[o + c] : 0.f; ts[i] = (ok && ewc_lambda != 0.f) ? theta_star[o + c] : 0.f;
-    }
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int c = c0 + lane + 32 * i;
-      if (c < d) {
-        adam_update_elem(g[i], th[i], m[i], v[i], lr_t, beta1, beta2, eps, ewc_lambda, fi[i], ts[i]);
-        theta[o + c] = th[i]; am[o + c] = m[i]; av[o + c] = v[i];
-      }
-    }
-  }
-}
-
 static int key_bits(int v_tab) { int b = 1; while ((1LL << b) < v_tab) ++b; return b; }
 
 }  // namespace ader
 #include "encoder_fused.cuh"
-#include "encoder_chain.cuh"
 namespace ader {
 
 // ------------------------------------------------------------------------------------------
 // group entry points
 // ------------------------------------------------------------------------------------------
-// packed token lists of a batch (row_len, row_off, tok_row, tok_id): three small launches; ADER_B200_PACK=1 selects the
-// single-CTA kernel for batches of up to 1024 rows (measured slower, see k_pack_small)
+// packed token lists of a batch (row_len, row_off, tok_row, tok_id): three small launches
 static void launch_pack_tokens(const int32_t* ids, int M, int L, int Tcap, const EncWs& w, cudaStream_t st) {
-  static int three = -1;
-  if (three < 0) {
-    const char* e = getenv("ADER_B200_PACK"); three = (e && e[0] == '1') ? 0 : 1;
-    cudaFuncSetAttribute(k_pack_small, cudaFuncAttributeMaxDynamicSharedMemorySize, 216 * 1024);
-  }
-  const size_t smem = sizeof(int) * ((size_t)M * L + 2 * PACK1_THR);
-  if (!three && M <= PACK1_THR && smem <= 216 * 1024) {
-    k_pack_small<<<1, PACK1_THR, smem, st>>>(ids, M, L, Tcap, w.row_len, w.row_off, w.tok_row, w.tok_id, w.flags);
-    return;
-  }
   k_row_len<<<cdiv((long long)M * 32, 256), 256, 0, st>>>(ids, M, L, w.row_len, w.flags);
   k_scan_rows<<<1, 1024, 0, st>>>(w.row_len, M, Tcap, w.row_off, w.flags);
   k_fill_tok<<<cdiv((long long)M * 32, 256), 256, 0, st>>>(ids, w.row_len, w.row_off, M, L, Tcap, w.tok_row, w.tok_id);
@@ -1199,13 +1020,13 @@ static int run_scatter_plan(const AderModel* m, const EncWs& w, const BwdWs& g, 
   const int* dT = w.row_off + M;
   const int ntiles = sort_tiles(Tcap);
   const int bits = key_bits(m->v_tab);
-  const int n16 = cdiv(m->v_tab, 16), n_count = cdiv(Tcap, SW);
-  k_plan_zero<<<cdiv(n16 > n_count ? n16 : n_count, 256), 256, 0, st>>>(reinterpret_cast<uint4*>(g.touched), n16, g.scount, n_count);
+  const int n_count = cdiv(Tcap, SW);
+  k_plan_zero<<<cdiv(n_count, 256), 256, 0, st>>>(g.scount, n_count);
   int cur = 0;
   const int* kin = w.tok_id; const int* vin = nullptr;
   int pass = 0;
   for (int shift = 0; shift < bits; shift += 8, ++pass) {
-    k_sort_hist<<<ntiles, 256, 0, st>>>(kin, dT, shift, ntiles, g.hist, pass == 0 ? g.touched : nullptr);
+    k_sort_hist<<<ntiles, 256, 0, st>>>(kin, dT, shift, ntiles, g.hist);
     k_sort_scan<<<1, 1024, 0, st>>>(g.hist, 256 * ntiles);
     k_sort_scatter<<<ntiles, 256, 0, st>>>(kin, vin, dT, shift, ntiles, g.hist, pass == 0, g.keys[cur], g.vals[cur]);
     kin = g.keys[cur]; vin = g.vals[cur]; cur ^= 1;
@@ -1219,32 +1040,12 @@ static int run_scatter_apply(const AderModel* m, const Layout& l, const EncWs& w
   const int d = m->d;
   const int* dT = w.row_off + M;
   const int fin = (sort_passes(m) - 1) & 1;
-  static int gen = -1;
-  if (gen < 0) { const char* e = getenv("ADER_B200_SCATTER"); gen = (e && e[0] == '2') ? 2 : 1; }
-  if (gen == 2 && d <= 160) {        // rows staged in shared memory, rolled run loop (40 KB static shared memory per CTA): opt-in
-    k_scatter_apply2<5><<<cdiv(cdiv(Tcap, SW), SW2_WARPS), SW2_WARPS * 32, 0, st>>>(g.keys[fin], g.vals[fin], dT, gX, d, sqrtf((float)d),
-                                                                                   grad + l.off_table, g.spart, g.scount, g.sbounds);
-    ADER_CHECK_LAUNCH("scatter apply");
-    return 0;
-  }
   const int grid = cdiv((long long)cdiv(Tcap, SW) * 32, 256);
   if (d <= 160)
     k_scatter_apply<5><<<grid, 256, 0, st>>>(g.keys[fin], g.vals[fin], dT, gX, d, sqrtf((float)d), grad + l.off_table, g.spart, g.scount, g.sbounds);
   else
     k_scatter_apply<LN_MAXE><<<grid, 256, 0, st>>>(g.keys[fin], g.vals[fin], dT, gX, d, sqrtf((float)d), grad + l.off_table, g.spart, g.scount, g.sbounds);
   ADER_CHECK_LAUNCH("scatter apply");
-  return 0;
-}
-// Adam on the touched table rows (behind the scatter, split update)
-static int run_adam_touched(const AderModel* m, const Layout& l, const EncWs& w, const BwdWs& g, int M, int Tcap, const AdamPlan& ap,
-                            cudaStream_t st) {
-  const int fin = (sort_passes(m) - 1) & 1;
-  k_adam_touched<<<cdiv((long long)Tcap * 32, 256), 256, 0, st>>>(g.keys[fin], w.row_off + M, m->d, ap.a.V, ap.grad + l.off_table,
-                                                                 ap.theta + l.off_table, ap.m + l.off_table, ap.v + l.off_table, ap.state,
-                                                                 ap.a.beta1, ap.a.beta2, ap.a.eps, ap.a.ewc_lambda,
-                                                                 ap.a.fisher ? ap.a.fisher + l.off_table : nullptr,
-                                                                 ap.a.theta_star ? ap.a.theta_star + l.off_table : nullptr);
-  ADER_CHECK_LAUNCH("adam table (touched rows)");
   return 0;
 }
 static int run_table_scatter(const AderModel* m, const Layout& l, const EncWs& w, const BwdWs& g, const float* gX,
@@ -1755,33 +1556,11 @@ static void fused_attrs() {
   cudaFuncSetAttribute(fz::k_ffn_fwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fz::FFN_FWD_SMEM);
   cudaFuncSetAttribute(fz::k_ffn_bwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fz::FFN_BWD_SMEM);
   cudaFuncSetAttribute(fz::k_qkv_bwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fz::QKV_BWD_SMEM);
-  cudaFuncSetAttribute(fz::k_wgrad, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fz::WGRAD_SMEM);
   cudaFuncSetAttribute(fz::k_wgrad2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fz::WGRAD2_SMEM);
   cudaFuncSetAttribute(fz::k_attn_ln_fwd, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * fz::att_rows_cap(64) * fz::KP * 4);
   cudaFuncSetAttribute(fz::k_attn_bwd_s1, cudaFuncAttributeMaxDynamicSharedMemorySize, fz::att_bwd_smem(64, fz::KP));
-  cudaFuncSetAttribute(fz::k_attn_ln_fwd_team, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fz::att_tile_smem(64));
-  cudaFuncSetAttribute(fz::k_chain_fwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fz::CHAIN_FWD_SMEM);
-  cudaFuncSetAttribute(fz::k_chain_bwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fz::CHAIN_BWD_SMEM);
   done = true;
 }
-// The chained kernels (encoder_chain.cuh) apply when the attention staging fits beside the weight slots, the model has at
-// most CH_MAXB blocks and one head (the reference's configuration); ADER_B200_CHAIN=0 keeps the per-sub-layer kernels.
-static bool chain_ok(const AderModel* m) {
-  // Opt-in (ADER_B200_CHAIN=1): measured slower than the per-sub-layer kernels at the reference's batch sizes (DESIGN.md
-  // section 3.6).  Read per call: tests compare the two paths in one process.
-  const char* e = getenv("ADER_B200_CHAIN");
-  if (!(e && e[0] == '1') || m->num_blocks > fz::CH_MAXB || m->num_heads != 1 || (m->d & 1)) return false;
-  const size_t stage = sizeof(float) * 2 * (size_t)fz::att_rows_cap(m->maxlen) * m->d;
-  return fz::att_tile_smem(m->maxlen) <= fz::CHAIN_FWD_STAGE && stage <= fz::CHAIN_BWD_STAGE && m->d <= fz::TEAM * fz::TE;
-}
-// attention with a team of 8 lanes per query (encoder_chain.cuh) instead of a warp per query: single head, d <= 152.
-// Opt-in (ADER_B200_TEAM_ATTN=1): as a kernel of its own it has 4x fewer warps in flight than the warp-per-query kernel and
-// measured slower (21 vs 17 us per launch at the bench shape); it is what the chained kernels use.
-static bool team_attention(const AderModel* m) {
-  const char* e = getenv("ADER_B200_TEAM_ATTN");
-  return (e && e[0] == '1') && m->num_heads == 1 && m->d <= fz::TEAM * fz::TE && !(m->d & 1);
-}
-static int chain_grid(int Tcap) { return max(1, min(min(sm_count(), CHF_STRIDE), cdiv(Tcap, 16))); }
 static const fz::op_t* shadow_of(const EncWs& w, int b, int which, int orient) {
   return (const fz::op_t*)w.wshadow + (size_t)((b * 5 + which) * 2 + orient) * (fz::KP * fz::LDS);
 }
@@ -1826,8 +1605,6 @@ int ader::enc_fwd_tc_run(const AderModel* m, const float* theta, const int32_t* 
   const int tile_grid = min(cdiv(Tcap, fz::TM), sm_count());
   const int warp_grid = cdiv(Tcap, fz::ATT_TOK);
   const size_t att_smem = sizeof(float) * 2 * (size_t)fz::att_rows_cap(L) * d;
-  const bool chain = chain_ok(m);
-  fz::ChainFwdArgs ca;
   for (int b = 0; b < m->num_blocks; ++b) {
     const float* P = theta + l.block(b);
     float* X = w.slot[b][0]; float* Q1 = w.slot[b][1]; float* Qp = w.slot[b][2]; float* Kp = w.slot[b][3];
@@ -1853,20 +1630,10 @@ int ader::enc_fwd_tc_run(const AderModel* m, const float* theta, const int32_t* 
     fa.Z = Z; fa.H = H; fa.Xn = Xn; fa.W1 = shadow_of(w, b, 3, 0); fa.W2 = shadow_of(w, b, 4, 0);
     fa.b1 = P + l.b1; fa.b2 = P + l.b2; fa.dT = dT; fa.d = d;
     fa.drop_p = dropout_rate; fa.seed = seed; fa.d_step = d_step; fa.site1 = 2u + 3u * b; fa.site2 = 3u + 3u * b;
-    if (chain) { ca.q[b] = qa; ca.at[b] = aa; ca.f[b] = fa; continue; }
     launch_chain(fz::k_qkv_fwd, dim3(tile_grid), dim3(fz::NTHR), fz::QKV_FWD_SMEM, st, f.pdl && b > 0, qa);
-    if (team_attention(m)) launch_chain(fz::k_attn_ln_fwd_team, dim3(cdiv(Tcap, fz::TM)), dim3(fz::NTHR), fz::att_tile_smem(L), st, f.pdl, aa);
-    else launch_chain(fz::k_attn_ln_fwd, dim3(warp_grid), dim3(256), att_smem, st, f.pdl, aa);
+    launch_chain(fz::k_attn_ln_fwd, dim3(warp_grid), dim3(256), att_smem, st, f.pdl, aa);
     launch_chain(fz::k_ffn_fwd, dim3(tile_grid), dim3(fz::NTHR), fz::FFN_FWD_SMEM, st, f.pdl, fa);
     ADER_CHECK_LAUNCH("encoder_fwd_tc/block");
-  }
-  if (chain) {       // all blocks + the final LayerNorm in one persistent kernel: a CTA owns whole sessions
-    ca.nb = m->num_blocks; ca.M = M; ca.xfinal = w.xfinal; ca.rep = rep; ca.meanf = w.meanf; ca.rstdf = w.rstdf;
-    ca.lnf_b = theta + l.off_lnf; ca.lnf_g = theta + l.off_lnf + d;
-    ca.flags = w.flags + CHF_FWD; ca.flag_stride = CHF_STRIDE;
-    launch_chain(fz::k_chain_fwd, dim3(chain_grid(Tcap)), dim3(fz::NTHR), fz::CHAIN_FWD_SMEM, st, false, ca);
-    ADER_CHECK_LAUNCH("encoder_fwd_tc/chain");
-    return 0;
   }
   launch_chain(k_ln_last_fwd, dim3(cdiv((long long)M * 32, 256)), dim3(256), 0, st, f.pdl, (const float*)w.xfinal, (const int*)w.row_len,
                (const int*)w.row_off, M, rep, w.meanf, w.rstdf, theta + l.off_lnf, theta + l.off_lnf + d, d);
@@ -1874,13 +1641,9 @@ int ader::enc_fwd_tc_run(const AderModel* m, const float* theta, const int32_t* 
   return 0;
 }
 
-// weight / LayerNorm-parameter gradient launch: second generation (two 4-warp CTAs per GEMM problem and split, bulk-copied
-// tiles) unless ADER_B200_WGRAD=1
-static void launch_wgrad(const fz::WgradArgs& wa, int splits, cudaStream_t st) {
-  static int gen = -1;
-  if (gen < 0) { const char* e = getenv("ADER_B200_WGRAD"); gen = (e && e[0] == '1') ? 1 : 2; }
-  if (gen == 1) fz::k_wgrad<<<dim3(splits, wa.n_gemm + wa.n_ln), fz::NTHR, fz::WGRAD_SMEM, st>>>(wa);
-  else fz::k_wgrad2<<<dim3(splits, 2 * wa.n_gemm + wa.n_ln), fz::WG2_THR, fz::WGRAD2_SMEM, st>>>(wa);
+// weight / LayerNorm-parameter gradient launch: two 4-warp CTAs per GEMM problem and split, one per LayerNorm problem
+static void launch_wgrad(const fz::WgradArgs& wa, cudaStream_t st) {
+  fz::k_wgrad2<<<dim3(SPLITS, 2 * wa.n_gemm + wa.n_ln), fz::WG2_THR, fz::WGRAD2_SMEM, st>>>(wa);
 }
 
 int ader::enc_scatter_plan_run(const AderModel* m, int M, int Tcap, const void* ws, void* bwd_ws, Fork& f) {
@@ -1894,8 +1657,6 @@ int ader::enc_scatter_plan_run(const AderModel* m, int M, int Tcap, const void* 
   f.plan_done = true;
   return 0;
 }
-
-bool ader::enc_chain_enabled(const AderModel* m) { return chain_ok(m); }
 
 extern "C" int32_t ader_encoder_bwd_tc(const AderModel* m, const float* theta, const int32_t* ids, int32_t M,
                                        int32_t Tcap, const void* ws, void* bwd_ws, const float* d_rep, float* grad,
@@ -1930,27 +1691,20 @@ int ader::enc_bwd_tc_run(const AderModel* m, const float* theta, const int32_t* 
   const int tile_grid = min(cdiv(Tcap, fz::TM), sm_count());
   fused_attrs();
 
-  const bool chained = chain_ok(m);
-  // token splits of the weight / LayerNorm / position gradient partials: the chained path runs ALL weight gradients in
-  // one launch behind the data-gradient kernel (10 problems x 14 splits = 140 CTAs, one wave)
-  const int splits = chained ? CHAIN_SPLITS : SPLITS;
   // final LayerNorm: data gradient on the chain, parameter gradient beside it
-  const bool drep_here = f.has_drep && !chained;      // the loss group left the d_rep reduction to the kernel below
-  if (f.has_drep && chained) return fail(-3, "encoder_bwd_tc: d_rep partials handed to the chained path");
   auto ln_params = [&] {
     f.edge(st, f.c);
-    k_ln_param_grad<<<splits, dim3(ln_threads, PG_LANES), 0, f.c>>>(d_rep, w.xfinal, w.meanf, w.rstdf, dT, M, w.row_len, w.row_off, d,
+    k_ln_param_grad<<<SPLITS, dim3(ln_threads, PG_LANES), 0, f.c>>>(d_rep, w.xfinal, w.meanf, w.rstdf, dT, M, w.row_len, w.row_off, d,
                                                    part(l.off_lnf), part(l.off_lnf + d), PS);
   };
-  if (!drep_here) ln_params();
-  fz::ChainBwdArgs ca;
-  if (drep_here) {
+  if (f.has_drep) {                           // the loss group left the d_rep reduction to the kernel below
     launch_chain(k_lnf_bwd_drep, dim3(cdiv((long long)(Tcap + M) * 32, 256)), dim3(256), 0, st, f.pdl, f.drep, const_cast<float*>(d_rep),
                  (const float*)w.xfinal, (const float*)w.meanf, (const float*)w.rstdf, theta + l.off_lnf + d, (const int*)w.tok_row,
                  (const int*)w.row_off, (const int*)w.row_len, chain[0], dT, M, Tcap, d);
     ADER_CHECK_LAUNCH("encoder_bwd_tc/final_ln+d_rep");
     ln_params();
-  } else if (!chained) {
+  } else {
+    ln_params();
     // directly behind the d_rep reduction on f.main in the fused step (f.pdl is only set there)
     launch_chain(k_lnf_bwd, dim3(ln_grid), dim3(256), 0, st, f.pdl, d_rep, (const float*)w.xfinal, (const float*)w.meanf, (const float*)w.rstdf,
                  theta + l.off_lnf + d, (const int*)w.tok_row, (const int*)w.row_off, chain[0], dT, d);
@@ -1958,7 +1712,6 @@ int ader::enc_bwd_tc_run(const AderModel* m, const float* theta, const int32_t* 
   }
 
   cudaEvent_t wg_done[8][3];                // weight-gradient pieces of block b finished (f.wg[k]), parallel plans only
-  fz::WgradArgs wgs[fz::CH_MAXB][3];        // chained path: the weight-gradient launches follow the data-gradient kernel
   for (int b = m->num_blocks - 1; b >= 0; --b) {
     const long long bo = l.block(b);
     const float* P = theta + bo;
@@ -1969,7 +1722,7 @@ int ader::enc_bwd_tc_run(const AderModel* m, const float* theta, const int32_t* 
     float *gO = gs[0], *gH = gs[1], *gZ = gs[2], *gY = gs[3], *gQ = gs[4], *gK = gs[5], *gV = gs[6], *gQ1 = gs[7];
     float* gX = chain[ci % 3]; float* gXin = chain[(ci + 1) % 3]; ++ci;
     // this block rewrites the buffer set (and chain buffer) last read by the weight-gradient kernel of block b + 2
-    const bool joined = !chained && f.parallel() && b + 2 < m->num_blocks;
+    const bool joined = f.parallel() && b + 2 < m->num_blocks;
     if (joined) for (int k = 0; k < 3; ++k) cudaStreamWaitEvent(st, wg_done[b + 2][k], 0);
     fz::FfnBwdArgs fa;
     fa.gX = gX; fa.gO = gO; fa.H = H; fa.Y = Y; fa.Q1 = Q1; fa.mean2 = w.mean2[b]; fa.rstd2 = w.rstd2[b];
@@ -1999,53 +1752,22 @@ int ader::enc_bwd_tc_run(const AderModel* m, const float* theta, const int32_t* 
     wa[2].p[0] = {X, gQ1, w.mean1[b], w.rstd1[b], part(bo + l.ln1b), part(bo + l.ln1g)};
     wa[2].n_gemm = 0; wa[2].n_ln = 1;
     for (int k = 0; k < 3; ++k) { wa[k].dT = dT; wa[k].d = d; wa[k].split_stride = PS; }
-    if (chained) {
-      ca.f[b] = fa; ca.at[b] = ab; ca.q[b] = qb;
-      for (int k = 0; k < 3; ++k) wgs[b][k] = wa[k];
-      continue;
-    }
-    // per-sub-layer kernels: each weight-gradient piece is launched on its own stream as soon as its gradients exist, so
+    // each weight-gradient piece is launched on its own stream as soon as its gradients exist, so
     // most of that work is done while the data-gradient chain is still running
     launch_chain(fz::k_ffn_bwd, dim3(tile_grid), dim3(fz::NTHR), fz::FFN_BWD_SMEM, st, f.pdl && !joined, fa);
     f.edge(st, f.wg[0]);
-    launch_wgrad(wa[0], SPLITS, f.wg[0]);
+    launch_wgrad(wa[0], f.wg[0]);
     if (m->num_heads == 1) launch_chain(fz::k_attn_bwd_s1, dim3(cdiv(Tcap, fz::ATT_TOK)), dim3(256), (size_t)fz::att_bwd_smem(L, d), st, f.pdl, ab);
     else fz::k_attn_bwd_w<<<ln_grid, 256, 0, st>>>(ab);
     f.edge(st, f.wg[1]);
-    launch_wgrad(wa[1], SPLITS, f.wg[1]);
+    launch_wgrad(wa[1], f.wg[1]);
     launch_chain(fz::k_qkv_bwd, dim3(tile_grid), dim3(fz::NTHR), fz::QKV_BWD_SMEM, st, f.pdl, qb);
     ADER_CHECK_LAUNCH("encoder_bwd_tc/dgrad");
     f.edge(st, f.wg[2]);
-    launch_wgrad(wa[2], SPLITS, f.wg[2]);
+    launch_wgrad(wa[2], f.wg[2]);
     ADER_CHECK_LAUNCH("encoder_bwd_tc/wgrad");
     if (f.parallel())
       for (int k = 0; k < 3; ++k) { wg_done[b][k] = f.take(); cudaEventRecord(wg_done[b][k], f.wg[k]); }
-  }
-  if (chained) {     // every data gradient of every block in one persistent kernel (a CTA owns whole sessions), then the
-                     // weight-gradient pieces of all blocks side by side
-    ca.nb = m->num_blocks; ca.M = M; ca.row_off = w.row_off; ca.tok_row = w.tok_row;
-    ca.flags = w.flags + CHF_BWD; ca.flag_stride = CHF_STRIDE; ca.done_at = CHF_DONE - CHF_BWD;
-    ca.d_rep = d_rep; ca.xfinal = w.xfinal; ca.meanf = w.meanf; ca.rstdf = w.rstdf; ca.lnf_g = theta + l.off_lnf + d; ca.gx_top = chain[0];
-    launch_chain(fz::k_chain_bwd, dim3(chain_grid(Tcap)), dim3(fz::NTHR), fz::CHAIN_BWD_SMEM, st, f.pdl, ca);
-    ADER_CHECK_LAUNCH("encoder_bwd_tc/chain");
-    fz::WgradArgs wa;                         // the 5 weight matrices (+ biases) of every block: one launch
-    int np = 0;
-    for (int b = m->num_blocks - 1; b >= 0; --b) {
-      wa.p[np++] = wgs[b][0].p[0]; wa.p[np++] = wgs[b][0].p[1];
-      wa.p[np++] = wgs[b][1].p[0]; wa.p[np++] = wgs[b][1].p[1]; wa.p[np++] = wgs[b][1].p[2];
-    }
-    wa.n_gemm = np; wa.n_ln = 0; wa.dT = dT; wa.d = d; wa.split_stride = PS;
-    f.edge(st, f.wg[0]);
-    launch_wgrad(wa, splits, f.wg[0]);
-    for (int k = 1; k < 3; ++k) {             // LayerNorm-parameter gradients of the blocks beside it
-      f.edge(st, f.wg[k]);
-      for (int b = m->num_blocks - 1; b >= 0; --b) {
-        const fz::WgradProb& lp = (k == 1) ? wgs[b][0].p[2] : wgs[b][2].p[0];
-        k_ln_param_grad<<<splits, dim3(ln_threads, PG_LANES), 0, f.wg[k]>>>(lp.grad, lp.act, lp.mean, lp.rstd, dT, 0, nullptr, nullptr, d,
-                                                                        lp.out0, lp.out1, PS);
-      }
-    }
-    ADER_CHECK_LAUNCH("encoder_bwd_tc/wgrad");
   }
   const float* gX0 = chain[ci % 3];          // gradient w.r.t. the (dropout-masked) embedding output
 
@@ -2056,40 +1778,29 @@ int ader::enc_bwd_tc_run(const AderModel* m, const float* theta, const int32_t* 
   if (f.parallel()) { chain_end = f.take(); cudaEventRecord(chain_end, st); }   // for the scatter issued in front of it)
   // item-table scatter (modules.py:127-130): adds to the rows the dE kernel wrote
   if (f.has_table_ready) cudaStreamWaitEvent(st, f.table_ready, 0);
-  // Split table update (f.split_adam): the rows no token touches have their final gradient since the dE kernel, so their
-  // Adam pass (HBM-bound) runs on f.b BESIDE the scatter (latency-bound) once the data-gradient chain has ended -- started
-  // earlier it only slowed the chain kernels down (measured) -- and the touched rows follow the scatter, one warp per item.
-  const bool split = f.adam && f.split_adam && f.plan_done && f.has_table_ready && f.parallel();
   if (f.plan_done) {
     cudaStreamWaitEvent(st, f.plan_ready, 0);
     if (int e = run_scatter_apply(m, l, w, g, gX0, M, Tcap, grad, st)) return e;
   } else if (int e = run_table_scatter(m, l, w, g, gX0, M, Tcap, grad, st)) return e;
   if (f.adam) {                              // ... and the item-table rows here
     cudaStreamWaitEvent(st, f.adam->prep_ready, 0);
-    if (split) { if (int e = run_adam_touched(m, l, w, g, M, Tcap, *f.adam, st)) return e; }
-    else if (int e = adam_table_part(m, *f.adam, st)) return e;
-  }
-  if (split) {
-    cudaStreamWaitEvent(f.b, chain_end, 0);  // f.b carries the dE kernel: stream order covers the gradient
-    cudaStreamWaitEvent(f.b, f.plan_ready, 0);
-    cudaStreamWaitEvent(f.b, f.adam->prep_ready, 0);
-    if (int e = adam_table_untouched(m, *f.adam, g.touched, f.b)) return e;
+    if (int e = adam_table_part(m, *f.adam, st)) return e;
   }
   // position table (ADER.py:41-52) beside the scatter; then all split partials -> dense gradients in fixed order
   if (chain_end) cudaStreamWaitEvent(f.c, chain_end, 0);
-  k_pos_grad<<<dim3(L, splits), dim3(ln_threads, PG_LANES), 0, f.c>>>(gX0, w.row_len, w.row_off, M, L, d, 0.f, 0, nullptr, g.partial, PS);
+  k_pos_grad<<<dim3(L, SPLITS), dim3(ln_threads, PG_LANES), 0, f.c>>>(gX0, w.row_len, w.row_off, M, L, d, 0.f, 0, nullptr, g.partial, PS);
   f.edge(f.c, f.a);
   f.edge(f.wg[1], f.a);
   f.edge(f.wg[2], f.a);
   if (f.adam) {                              // fused step: reduce the partials and update the dense parameters in one launch
     const AdamPlan& ap = *f.adam;
     cudaStreamWaitEvent(f.a, ap.prep_ready, 0);
-    k_reduce_partials_adam<<<cdiv(PS, 256), 256, 0, f.a>>>(g.partial, PS, splits, PS, grad + l.off_pos, ap.theta + l.off_pos,
+    k_reduce_partials_adam<<<cdiv(PS, 256), 256, 0, f.a>>>(g.partial, PS, SPLITS, PS, grad + l.off_pos, ap.theta + l.off_pos,
                                                            ap.m + l.off_pos, ap.v + l.off_pos, ap.state, ap.a.beta1, ap.a.beta2, ap.a.eps,
                                                            ap.a.ewc_lambda, ap.a.fisher ? ap.a.fisher + l.off_pos : nullptr,
                                                            ap.a.theta_star ? ap.a.theta_star + l.off_pos : nullptr);
   } else {
-    k_reduce_partials<<<cdiv(PS, 256), 256, 0, f.a>>>(g.partial, PS, splits, 0, PS, grad + l.off_pos);
+    k_reduce_partials<<<cdiv(PS, 256), 256, 0, f.a>>>(g.partial, PS, SPLITS, 0, PS, grad + l.off_pos);
   }
   f.edge(f.a, st);
   ADER_CHECK_LAUNCH("encoder_bwd_tc/embedding");

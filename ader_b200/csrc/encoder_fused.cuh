@@ -1142,8 +1142,8 @@ struct QkvBwdArgs {
 constexpr size_t QKV_BWD_SMEM = 3 * WMAT_BYTES + 3 * ATILE_BYTES + FTILE_BYTES + 2 * TM * 4 + 16;
 static_assert(3 * ATILE_BYTES >= FTILE_BYTES, "second fp32 tile aliases the operand tiles");
 
-// One 32-token tile: gXin = gK.Wk^T + gV.Wv^T + LN1 backward(gQ.Wq^T + gY).  The K/V products run first (their shadows
-// arrive first in the chained kernel), the Q product second; wait_kv() / wait_q() block until the shadows have landed.
+// One 32-token tile: gXin = gK.Wk^T + gV.Wv^T + LN1 backward(gQ.Wq^T + gY).  The K/V products run first, the Q product
+// second; wait_kv() / wait_q() run in front of each and block until the shadows it reads have landed.
 template <class WaitKV, class WaitQ>
 __device__ __forceinline__ void qkv_bwd_tile(const QkvBwdArgs& a, int t0, int T, uint64_t seed_eff, op_t* __restrict__ A1, op_t* __restrict__ A2,
                                              op_t* __restrict__ A3, float* __restrict__ Ft, float* __restrict__ Ft2, float* __restrict__ rsq,
@@ -1246,24 +1246,25 @@ __global__ void __launch_bounds__(NTHR, 1) k_qkv_bwd(const __grid_constant__ Qkv
                  [&] { if (first) { mbar_wait(bar, 0); first = false; } }, [] {});
 }
 
-// ---- backward: weight / bias / LayerNorm-parameter gradients of one block, ONE launch ------------------
+// ---- backward: weight / bias / LayerNorm-parameter gradients of one block -----------------------------------------
 // dW[c_in][c_out] = sum_t act[t][c_in] * grad[t][c_out] is a [150 x T] x [T x 150] product whose contraction
-// runs over tokens.  TF32 mma.sync.m16n8k8: both operands are read straight from their natural [t][c] fp32
-// layout (cp.async token tiles in a ring of WG_NST stages, row stride 168 words -> conflict-free fragment loads), no
-// transposes and no range scaling (8-bit exponent), 10-bit mantissa.  CTA (split, problem) owns a contiguous
-// range of token tiles and a full 160 x 160 fp32 accumulator in registers (8 warps x 5 x 5 mma tiles); the
-// `splits` partials are reduced afterwards in index order (k_reduce_partials) -> deterministic.
+// runs over tokens.  TF32 mma.sync.m16n8k8: both operands are read straight from their natural [t][c] fp32 layout, no
+// transposes and no range scaling (8-bit exponent), 10-bit mantissa.  A (split, problem) owns a contiguous range of
+// 32-token tiles; the `splits` partials are reduced afterwards in index order (k_reduce_partials) -> deterministic.
 // Problems 0..n_gemm-1: weight + bias gradients; problems n_gemm..: LayerNorm (beta, gamma) gradients
 // (act = LN input x, grad = dout, xhat rebuilt from mean / rstd).
+//   * a tile operand is ONE cp.async.bulk of the contiguous [32 tokens][d] block (19 200 B) completing on an mbarrier, the
+//     next tile in flight behind the one being multiplied (ring depth: see WG2_NST).  Staging a tile with one 8-byte
+//     cp.async per element pair is issue-bound: 6 us from entry to the first tile (profiles/r2/wgrad_phase_timeline.txt);
+//   * shared-memory rows keep the global stride d, and the k slots of a k-step are mapped to tile rows so that the four
+//     rows one fragment load touches are 4 apart (4 * 150 = 24 mod 32 banks): conflict-free without padding.  Summation
+//     over k does not care which token sits in which slot as long as A and B agree;
+//   * a (split, problem) is TWO CTAs of 4 warps, each owning 160 x 80 of the result (the tensor pipe of an SM is saturated by
+//     4 warps with 25 independent accumulators each), so a launch of 3 problems x 21 splits covers 126 SMs;
+//   * partials leave through shared memory as coalesced 8-byte row stores.
+// Bias and LayerNorm-parameter sums run in token order.
 constexpr int WG_TK = 32;                     // tokens per staged tile
-constexpr int WG_LD = 168;                    // fp32 row stride (168 % 32 == 8)
-constexpr int WG_TILE = WG_TK * WG_LD;        // floats per operand tile
-constexpr int WG_NST = 5;                     // ring depth: a CTA's whole token range (T/21 splits ~ 5 tiles at the reference's
-                                              // batch sizes) is in flight at once; with two stages every tile paid its own
-                                              // L2 round trip.  (229 registers x 256 threads already keep every other CTA
-                                              // of the step off the SM, so the 215 KB cost no co-residency.)
-constexpr size_t WGRAD_SMEM = sizeof(float) * 2 * WG_NST * WG_TILE;   // stages x (act, grad) = 215 040 B
-constexpr int WG_MAXP = 10;                   // problems of one launch (chained path: the 5 matrices of 2 blocks)
+constexpr int WG_MAXP = 3;                    // problems of one launch (the largest piece: the Q, K and V matrices)
 struct WgradProb { const float *act, *grad, *mean, *rstd; float *out0, *out1; };   // GEMM: out0 = pW, out1 = pb; LN: out0 = pbeta, out1 = pgamma
 struct WgradArgs { WgradProb p[WG_MAXP]; int n_gemm, n_ln; const int* dT; int d; long long split_stride; };
 
@@ -1277,141 +1278,7 @@ __device__ __forceinline__ void mma_tf32(float (&c)[4], uint32_t a0, uint32_t a1
                : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
                : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
 }
-__device__ __forceinline__ void wg_stage(float* __restrict__ dst, const float* __restrict__ G, int t0, int T, int d) {
-  for (int idx = threadIdx.x; idx < WG_TK * (KP / 2); idx += NTHR) {
-    const int r = idx / (KP / 2), c = (idx % (KP / 2)) * 2;
-    const bool ok = (t0 + r < T) && (c < d);
-    const float* src = ok ? G + (long long)(t0 + r) * d + c : G;
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 8, %2;" ::"r"(smem_u32(dst + r * WG_LD + c)), "l"(src), "r"(ok ? 8 : 0) : "memory");
-  }
-}
 
-#ifdef ADER_TC_TIMELINE      // stamps of problem 0 of the last GEMM launch (rows 0..) and the last LayerNorm-only launch (rows 64..)
-#define WG_TL(slot) do { if (threadIdx.x == 0 && blockIdx.y == 0 && blockIdx.x < 64) { long long t_; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_)); \
-    g_fz_tl[7][blockIdx.x + (is_ln ? 64 : 0)][slot] = t_; } } while (0)
-#else
-#define WG_TL(slot) do { } while (0)
-#endif
-__global__ void __launch_bounds__(NTHR, 1) k_wgrad(const __grid_constant__ WgradArgs a) {
-  extern __shared__ __align__(16) float wsm[];
-  const int T = *a.dT, d = a.d;
-  const int ntiles = (T + WG_TK - 1) / WG_TK;
-  const int chunk = (ntiles + gridDim.x - 1) / gridDim.x;
-  const int tile_lo = blockIdx.x * chunk, tile_hi = min(ntiles, tile_lo + chunk);
-  const WgradProb pr = a.p[blockIdx.y];
-  const bool is_ln = (int)blockIdx.y >= a.n_gemm;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int g = lane >> 2, t4 = lane & 3;
-  const int wm = warp & 1, wn = warp >> 1;           // 5 m16 tiles (rows wm*80..) x 5 n8 tiles (cols wn*40..)
-  float acc[5][5][4];
-#pragma unroll
-  for (int i = 0; i < 5; ++i)
-#pragma unroll
-    for (int j = 0; j < 5; ++j) { acc[i][j][0] = acc[i][j][1] = acc[i][j][2] = acc[i][j][3] = 0.f; }
-  float cs0 = 0.f, cs1 = 0.f;                        // column sums owned by thread tid < 160
-  WG_TL(0);
-  // prologue: WG_NST - 1 tiles in flight (one commit group per tile, empty groups keep the count uniform)
-#pragma unroll
-  for (int s = 0; s < WG_NST - 1; ++s) {
-    if (tile_lo + s < tile_hi) {
-      wg_stage(wsm + s * 2 * WG_TILE, pr.act, (tile_lo + s) * WG_TK, T, d);
-      wg_stage(wsm + s * 2 * WG_TILE + WG_TILE, pr.grad, (tile_lo + s) * WG_TK, T, d);
-    }
-    asm volatile("cp.async.commit_group;" ::: "memory");
-  }
-  for (int tile = tile_lo; tile < tile_hi; ++tile) {
-    const int buf = (tile - tile_lo) % WG_NST;
-    {   // refill the stage the previous iteration released (its readers passed the barrier at the end of that iteration)
-      const int nt = tile + WG_NST - 1, nb = (nt - tile_lo) % WG_NST;
-      if (nt < tile_hi) {
-        wg_stage(wsm + nb * 2 * WG_TILE, pr.act, nt * WG_TK, T, d);
-        wg_stage(wsm + nb * 2 * WG_TILE + WG_TILE, pr.grad, nt * WG_TK, T, d);
-      }
-    }
-    asm volatile("cp.async.commit_group;" ::: "memory");
-    asm volatile("cp.async.wait_group %0;" ::"n"(WG_NST - 1) : "memory");
-    __syncthreads();
-    if (tile - tile_lo < 6) WG_TL(1 + (tile - tile_lo));
-    const float* As = wsm + buf * 2 * WG_TILE;
-    const float* Bs = As + WG_TILE;
-    if (!is_ln) {
-#pragma unroll
-      for (int ks = 0; ks < WG_TK / 8; ++ks) {
-        const float* ar = As + (ks * 8 + t4) * WG_LD + wm * 80 + g;
-        const float* br = Bs + (ks * 8 + t4) * WG_LD + wn * 40 + g;
-        uint32_t bf[5][2];
-#pragma unroll
-        for (int j = 0; j < 5; ++j) { bf[j][0] = to_tf32(br[j * 8]); bf[j][1] = to_tf32(br[4 * WG_LD + j * 8]); }
-#pragma unroll
-        for (int i = 0; i < 5; ++i) {
-          const uint32_t a0 = to_tf32(ar[i * 16]), a1 = to_tf32(ar[i * 16 + 8]);
-          const uint32_t a2 = to_tf32(ar[4 * WG_LD + i * 16]), a3 = to_tf32(ar[4 * WG_LD + i * 16 + 8]);
-#pragma unroll
-          for (int j = 0; j < 5; ++j) mma_tf32(acc[i][j], a0, a1, a2, a3, bf[j][0], bf[j][1]);
-        }
-      }
-      if (tid < KP) {                                 // bias gradient: column sums of grad, token order
-#pragma unroll 8
-        for (int r = 0; r < WG_TK; ++r) cs0 += Bs[r * WG_LD + tid];
-      }
-    } else if (tid < KP) {                            // LayerNorm parameter gradients
-      // rows beyond T were zero-filled by the staging copy (gq = 0 contributes +-0: the sums keep their bits), so the loop
-      // runs over the whole tile and the statistics of eight rows are fetched together instead of one L2 trip per row
-      const int t0 = tile * WG_TK;
-#pragma unroll
-      for (int r8 = 0; r8 < WG_TK; r8 += 8) {
-        float mu[8], rs[8];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) { const int t = min(t0 + r8 + j, T - 1); mu[j] = __ldg(pr.mean + t); rs[j] = __ldg(pr.rstd + t); }
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-          const int r = r8 + j;
-          const float gq = Bs[r * WG_LD + tid];
-          cs0 += gq;
-          cs1 += gq * ((As[r * WG_LD + tid] - mu[j]) * rs[j]);
-        }
-      }
-    }
-    __syncthreads();
-  }
-  asm volatile("cp.async.wait_group 0;" ::: "memory");
-  WG_TL(8);
-  const long long so = (long long)blockIdx.x * a.split_stride;
-  if (!is_ln) {
-#pragma unroll
-    for (int i = 0; i < 5; ++i)
-#pragma unroll
-      for (int j = 0; j < 5; ++j) {
-        const int m = wm * 80 + i * 16 + g, n = wn * 40 + j * 8 + 2 * t4;
-        if (n < d) {
-          if (m < d) *reinterpret_cast<float2*>(pr.out0 + so + (long long)m * d + n) = make_float2(acc[i][j][0], acc[i][j][1]);
-          if (m + 8 < d) *reinterpret_cast<float2*>(pr.out0 + so + (long long)(m + 8) * d + n) = make_float2(acc[i][j][2], acc[i][j][3]);
-        }
-      }
-    if (tid < d) pr.out1[so + tid] = cs0;
-  } else if (tid < d) {
-    pr.out0[so + tid] = cs0;
-    pr.out1[so + tid] = cs1;
-  }
-  WG_TL(9);
-}
-
-
-// ---- second generation of the weight-gradient kernel (default; ADER_B200_WGRAD=1 selects k_wgrad above) -----------------
-// Phase stamps of k_wgrad (scripts/wgrad_timeline.py, profiles/r2/wgrad_phase_timeline.txt): 6 us from entry to the first
-// tile (25 600 8-byte cp.async per CTA: issue-bound), 1.35 us per 32-token tile (tensor pipe 0.92), 2.75 us for the
-// fragment-scattered partial stores.  Here
-//   * a tile operand is ONE cp.async.bulk of the contiguous [32 tokens][d] block (19 200 B) completing on an mbarrier, the
-//     next tile in flight behind the one being multiplied (ring depth: see WG2_NST);
-//   * shared-memory rows keep the global stride d, and the k slots of a k-step are mapped to tile rows so that the four
-//     rows one fragment load touches are 4 apart (4 * 150 = 24 mod 32 banks): conflict-free without padding.  Summation
-//     over k does not care which token sits in which slot as long as A and B agree;
-//   * a (split, problem) is TWO CTAs of 4 warps, each owning 160 x 80 of the result (the tensor pipe of an SM is saturated by
-//     4 warps with 25 independent accumulators each), so a launch of 3 problems x 21 splits covers 126 SMs instead of 63 and
-//     the per-CTA product time halves;
-//   * partials leave through shared memory as coalesced 8-byte row stores.
-// Same token splits and the same fixed-order reduction afterwards: deterministic; bias and LayerNorm-parameter sums keep
-// their exact order (bit-identical to k_wgrad), the weight products differ in the order of additions inside a k-step only.
 constexpr int WG2_THR = 128;
 // ring depth (-DADER_WG2_NST=n): measured in the step on one box, 200 graph replays each, two runs per depth
 // (profiles/r2b/wgrad2_ring_depth.txt): 5 stages (205 KB) 0.2807 / 0.2804 ms, 3 stages (123 KB) 0.2799 / 0.2801,

@@ -47,38 +47,6 @@ __global__ void __launch_bounds__(256) k_adam(float* __restrict__ theta, float* 
   *reinterpret_cast<float2*>(av + e) = v;
 }
 
-// The same update restricted to the table rows no input token of the step touches: for those the gradient is complete once
-// the dE kernel is done (the embedding scatter adds nothing), so they are updated beside the scatter.  touched[row] is
-// written by the scatter plan (encoder.cu); the touched rows are updated by k_adam_touched behind the scatter.
-__global__ void __launch_bounds__(256) k_adam_untouched(float* __restrict__ theta, float* __restrict__ am, float* __restrict__ av,
-                                                        const float* __restrict__ grad, const int* __restrict__ state,
-                                                        const uint8_t* __restrict__ touched, long long n_table, int d, int fits32,
-                                                        float beta1, float beta2, float eps, float ewc_lambda,
-                                                        const float* __restrict__ fisher, const float* __restrict__ theta_star) {
-  // grid-stride over a few CTAs per SM: the kernel runs BESIDE the scatter, and a grid of one CTA per 512 elements would
-  // queue thousands of CTAs in front of every later launch (the block scheduler does not back-fill across streams)
-  const float lr_t = __int_as_float(state[1]);
-  for (long long i2 = ((long long)blockIdx.x * blockDim.x + threadIdx.x) * 2; i2 < n_table; i2 += (long long)gridDim.x * blockDim.x * 2) {
-  const long long e = (long long)d + i2;           // row 0 is the padding row; d is even, so a pair never straddles rows
-  const unsigned row = fits32 ? (unsigned)e / (unsigned)d : (unsigned)(e / d);
-  if (touched[row]) continue;
-  float2 g = *reinterpret_cast<const float2*>(grad + e);
-  float2 th = *reinterpret_cast<const float2*>(theta + e);
-  float2 m = *reinterpret_cast<const float2*>(am + e);
-  float2 v = *reinterpret_cast<const float2*>(av + e);
-  float2 f = make_float2(0.f, 0.f), ts = make_float2(0.f, 0.f);
-  if (ewc_lambda != 0.f) {
-    f = *reinterpret_cast<const float2*>(fisher + e);
-    ts = *reinterpret_cast<const float2*>(theta_star + e);
-  }
-  adam_update_elem(g.x, th.x, m.x, v.x, lr_t, beta1, beta2, eps, ewc_lambda, f.x, ts.x);
-  adam_update_elem(g.y, th.y, m.y, v.y, lr_t, beta1, beta2, eps, ewc_lambda, f.y, ts.y);
-  *reinterpret_cast<float2*>(theta + e) = th;
-  *reinterpret_cast<float2*>(am + e) = m;
-  *reinterpret_cast<float2*>(av + e) = v;
-  }
-}
-
 __global__ void __launch_bounds__(256) k_fisher_acc(const float* __restrict__ grad, double* __restrict__ acc,
                                                     long long n_table, long long table_lo, long long dense_lo,
                                                     long long n_total) {
@@ -132,17 +100,6 @@ int ader::adam_table_part(const AderModel* m, const AdamPlan& p, cudaStream_t st
   k_adam<<<cdiv(n_table / 2 + 1, 256), 256, 0, st>>>(p.theta, p.m, p.v, p.grad, p.state, n_table, (long long)m->d, l.off_pos, n_table,
                                                      p.a.beta1, p.a.beta2, p.a.eps, p.a.ewc_lambda, p.a.fisher, p.a.theta_star);
   ADER_CHECK_LAUNCH("adam table");
-  return 0;
-}
-int ader::adam_table_untouched(const AderModel* m, const AdamPlan& p, const uint8_t* touched, cudaStream_t st) {
-  const long long n_table = (long long)p.a.V * m->d;
-  const int fits32 = ((long long)(p.a.V + 1) * m->d < (1LL << 32)) ? 1 : 0;
-  int sms = 148;
-  { int dev = 0; if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev); }
-  const int need = cdiv(n_table / 2 + 1, 256);
-  k_adam_untouched<<<need < 4 * sms ? need : 4 * sms, 256, 0, st>>>(p.theta, p.m, p.v, p.grad, p.state, touched, n_table, m->d, fits32,
-                                                               p.a.beta1, p.a.beta2, p.a.eps, p.a.ewc_lambda, p.a.fisher, p.a.theta_star);
-  ADER_CHECK_LAUNCH("adam table (untouched rows)");
   return 0;
 }
 extern "C" int32_t ader_fisher_accumulate(const AderModel* m, const float* grad, double* acc, int32_t V, void* stream) {

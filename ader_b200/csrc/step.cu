@@ -16,7 +16,6 @@ namespace ader {
 
 struct StreamPool {
   cudaStream_t s[5];     // side streams, lowest priority (3 general + 2 more for weight-gradient pieces)
-  cudaStream_t hi;       // optional highest-priority chain stream (ADER_B200_DAG_PRIO=1)
   cudaEvent_t ev[128];
   bool ok;
   StreamPool() : ok(false) {}
@@ -26,7 +25,6 @@ struct StreamPool {
     cudaDeviceGetStreamPriorityRange(&least, &greatest);
     for (int i = 0; i < 5; ++i)
       if (cudaStreamCreateWithPriority(&s[i], cudaStreamNonBlocking, least) != cudaSuccess) return fail(-3, "train_fwd_bwd_tc: cannot create a stream");
-    if (cudaStreamCreateWithPriority(&hi, cudaStreamNonBlocking, greatest) != cudaSuccess) return fail(-3, "train_fwd_bwd_tc: cannot create a stream");
     for (int i = 0; i < 128; ++i)
       if (cudaEventCreateWithFlags(&ev[i], cudaEventDisableTiming) != cudaSuccess) return fail(-3, "train_fwd_bwd_tc: cannot create an event");
     ok = true;
@@ -36,9 +34,9 @@ struct StreamPool {
 // one pool per host thread and device (streams belong to the device that was current at creation)
 static thread_local StreamPool g_pool[16];
 
-// switches (read once).  ADER_B200_DAG_PRIO=1 moves the chain to a highest-priority stream: measured slower (the
-// hardware schedules strictly by priority without back-fill, the side streams starve), so the default keeps the chain
-// on the caller's stream.  ADER_B200_PDL=0 turns the programmatic dependent launches of the chain off.
+// switches (read once).  The chain stays on the caller's stream: a highest-priority chain stream measured slower (the
+// hardware schedules strictly by priority without back-fill, the side streams starve; DESIGN §3.4).
+// ADER_B200_PDL=0 turns the programmatic dependent launches of the chain off.
 static int env_flag(const char* name, int dflt) {
   const char* e = getenv(name);
   return e && e[0] ? atoi(e) : dflt;
@@ -64,18 +62,10 @@ static int run_step(const AderModel* m, const float* theta, const int32_t* ids, 
     f.a = p.s[0]; f.b = p.s[1]; f.c = p.s[2];
     f.wg[0] = f.a; f.wg[1] = p.s[3]; f.wg[2] = p.s[4];
     f.ev = p.ev; f.n_ev = 128; f.next_ev = 0;
-    static const int prio = env_flag("ADER_B200_DAG_PRIO", 0);
-    if (prio) { f.main = p.hi; f.edge(st, f.main); }
   }
   static const int pdl = env_flag("ADER_B200_PDL", 1);
   f.pdl = pdl != 0;
-  // ADER_B200_SPLIT_ADAM=1: Adam on the table rows no token touches beside the scatter, on the touched rows behind it
-  // (measured slower: the HBM-bound pass slows the latency-bound tail kernels it runs beside, so the default is ONE Adam
-  // launch over the table behind the scatter); ADER_B200_FUSE_DREP=0: the stand-alone d_rep reduction kernel.  All forms
-  // produce the same bits.
-  static const int split_adam = env_flag("ADER_B200_SPLIT_ADAM", 0), fuse_drep = env_flag("ADER_B200_FUSE_DREP", 1);
-  f.split_adam = f.parallel() && adam && split_adam;
-  f.fuse_drep = f.parallel() && fuse_drep && d_rep && !enc_chain_enabled(m);
+  f.fuse_drep = f.parallel() && d_rep;
   // teacher products / table tiles need nothing from the encoder: start them first, beside it
   f.edge(f.main, f.b);
   if (int e = loss_tc_run(m, theta, nullptr, a, loss_ws, nullptr, nullptr, nullptr, grad, f, 1)) return e;
@@ -92,13 +82,12 @@ static int run_step(const AderModel* m, const float* theta, const int32_t* ids, 
   if (int e = enc_scatter_plan_run(m, M, Tcap, enc_ws, bwd_ws, f)) return e;
   if (int e = loss_tc_run(m, theta, rep, a, loss_ws, loss, row_loss, d_rep, grad, f, 2)) return e;
   if (int e = enc_bwd_tc_run(m, theta, ids, M, Tcap, enc_ws, bwd_ws, d_rep, grad, dropout_rate, seed, d_step, f)) return e;
-  // close the DAG: every side stream (and the priority chain) is ordered before the tail of the caller's stream
+  // close the DAG: every side stream is ordered before the tail of the caller's stream
   f.edge(f.a, st);
   f.edge(f.b, st);
   f.edge(f.c, st);
   f.edge(f.wg[1], st);
   f.edge(f.wg[2], st);
-  f.edge(f.main, st);
   ADER_CHECK_LAUNCH("train step");
   if (adam && !f.adam)        // serial plan: the ordinary optimiser call behind the pass
     return ader_adam_step(m, adam->theta, adam->m, adam->v, adam->grad, adam->state, &adam->a, (void*)st);

@@ -30,10 +30,6 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity, int* er
     }
   }
 }
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-               ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
@@ -89,12 +85,6 @@ __device__ __forceinline__ void tmem_ld_wait16(uint32_t (&r)[16]) {
 }
 __device__ __forceinline__ float ex2(float x) { float y; asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 
-// shared-memory matrix descriptor, no swizzle (cute::UMMA::SmemDescriptor): start>>4 [0,14),
-// LBO>>4 [16,30), SBO>>4 [32,46), version=1 [46,48), layout_type=0 [61,64)
-__device__ __forceinline__ uint64_t make_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-  return (uint64_t)((saddr >> 4) & 0x3FFF) | ((uint64_t)((lbo_bytes >> 4) & 0x3FFF) << 16) |
-         ((uint64_t)((sbo_bytes >> 4) & 0x3FFF) << 32) | (1ull << 46);
-}
 // instruction descriptor (cute::UMMA::InstrDescriptor): c=F32 [4,6), a=BF16 [7,10), b=BF16 [10,13),
 // a_major [15], b_major [16], N>>3 [17,23), M>>4 [24,29)
 __host__ __device__ constexpr uint32_t make_idesc(int M, int N, int a_mn, int b_mn, int a_neg = 0) {
@@ -106,7 +96,8 @@ __device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* tm,
   asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
                ::"r"(dst), "l"(tm), "r"(bar), "r"(c0), "r"(c1) : "memory");
 }
-// shared-memory matrix descriptor, SWIZZLE_128B (layout_type 2 in bits [61,64)), version 1
+// shared-memory matrix descriptor, SWIZZLE_128B (cute::UMMA::SmemDescriptor): start>>4 [0,14), LBO>>4 [16,30),
+// SBO>>4 [32,46), version=1 [46,48), layout_type=2 [61,64)
 __device__ __forceinline__ uint64_t make_desc_sw128(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
   return (uint64_t)((saddr >> 4) & 0x3FFF) | ((uint64_t)((lbo_bytes >> 4) & 0x3FFF) << 16) |
          ((uint64_t)((sbo_bytes >> 4) & 0x3FFF) << 32) | (1ull << 46) | (2ull << 61);

@@ -24,29 +24,8 @@ lib.ader_debug_fz_timeline.argtypes = [C.c_void_p]
 lib.ader_debug_fz_timeline(buf.ctypes.data_as(C.c_void_p))
 names = {0: ("k_qkv_fwd (last = block 1)", ["entry", "setup", "prologue", "weights", "gemmQ", "end"]),
          1: ("k_ffn_bwd (last = block 0)", ["entry", "setup", "stage", "weights", "gemm1+epi", "gemm2+epi", "end"])}
-chain = {2: ("k_chain_fwd", ["entry", "partition", "qkv0", "attn0", "ffn0", "qkv1", "attn1", "ffn1", "lnf"]),
-         3: ("k_chain_bwd", ["entry", "pdl", "lnf", "ffn1", "attn1", "qkv1", "ffn0", "attn0", "qkv0"])}
-for k, (nm, labels) in chain.items():
-    t = buf[k]
-    used = np.nonzero(t[:, 0])[0]
-    if len(used) == 0:
-        continue
-    ntok = t[used, 15]
-    rel = (t[used][:, :len(labels)] - t[used, 0:1]) / 1e3
-    dur = np.diff(rel, axis=1)
-    print("== %s: %d CTAs, tokens per CTA min/median/max %d/%d/%d, start spread %.1f us" % (nm, len(used), ntok.min(), np.median(ntok), ntok.max(),
-          (t[used, 0].max() - t[used, 0].min()) / 1e3))
-    print("   phase durations (us), median over CTAs: " + ", ".join("%s %.1f" % (l, v) for l, v in zip(labels[1:], np.median(dur, axis=0))))
-    print("   max over CTAs:                          " + ", ".join("%s %.1f" % (l, v) for l, v in zip(labels[1:], dur.max(axis=0))))
-    print("   total: median %.1f, max %.1f us" % (np.median(rel[:, -1]), rel[:, -1].max()))
-    for lo, hi in ((0, 16), (17, 32), (33, 48), (49, 64), (65, 200)):
-        sel = (ntok >= lo) & (ntok <= hi)
-        if sel.any():
-            print("   CTAs with %3d..%3d tokens: %3d, median total %.1f us, phases " % (lo, hi, sel.sum(), np.median(rel[sel, -1])) +
-                  ", ".join("%.1f" % v for v in np.median(dur[sel], axis=0)))
 fine = {0: ("qkv_fwd_tile (last tile of block 1)", [6, 7, 2, 3, 4, 8, 5], ["start", "rows loaded+reduced", "LN+tiles+sync", "wait Wq", "gemmQ+epi", "gemmK+epi", "gemmV+epi+sync"]),
         4: ("attn_fwd_group (last group)", [0, 1, 2, 3], ["start", "staged+sync", "keys done", "LN2 done"]),
-        6: ("attn_fwd_tile (block 1)", [0, 1, 2, 3, 4, 5, 6, 7], ["start", "K staged", "scores", "softmax+probs", "sync", "V staged", "PV", "LN2"]),
         5: ("ffn_fwd_tile (last tile)", [0, 1, 2, 5, 3, 4], ["start", "rows+tile+sync", "wait W", "gemm1", "epi1+sync", "gemm2+epi+sync"])}
 for k, (nm, slots, labels) in fine.items():
     t = buf[k]
@@ -58,12 +37,6 @@ for k, (nm, slots, labels) in fine.items():
     print("== %s: %d CTAs" % (nm, len(used)))
     print("   step durations (us) median: " + ", ".join("%s %.2f" % (l, v) for l, v in zip(labels[1:], np.median(dur, axis=0))))
     print("   p90:                        " + ", ".join("%s %.2f" % (l, v) for l, v in zip(labels[1:], np.percentile(dur, 90, axis=0))))
-t2, t7 = buf[2], buf[7]
-used = np.nonzero(t2[:, 0])[0]
-if len(used):
-    for b in range(2):
-        w = (t7[used, b] - t2[used, 2 + 3 * b]) / 1e3
-        print("== chain fwd block %d: publish + neighbour wait + sync: median %.2f, p90 %.2f, max %.2f us" % (b, np.median(w), np.percentile(w, 90), w.max()))
 for k, (nm, labels) in names.items():
     if not np.any(buf[k][:, 0]):
         continue

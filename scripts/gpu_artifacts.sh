@@ -9,7 +9,7 @@ timeout 100 ncu --profile-from-start off --metrics gpu__time_duration.sum --cloc
     --log-file gpurun_out/launches_final.csv python scripts/ncu_step.py 2 > gpurun_out/ncu_launches_final.log 2>&1
 echo "launches rc=$? t=$(( $(date +%s) - T0 ))" >> gpurun_out/legs_artifacts.txt
 timeout 150 ncu --profile-from-start off --set full --clock-control none --import-source on \
-    -k regex:'k_tc_logits|k_scatter_apply|k_adam|k_merge_stats|k_sort_scatter' \
+    -k regex:'k_tc2|k_scatter_apply|k_adam|k_merge_stats|k_sort_scatter' \
     -f -o gpurun_out/final_full python scripts/ncu_step.py 1 > gpurun_out/ncu_final_full.log 2>&1
 echo "full rc=$? t=$(( $(date +%s) - T0 ))" >> gpurun_out/legs_artifacts.txt
 [ -f gpurun_out/final_full.ncu-rep ] && ncu -i gpurun_out/final_full.ncu-rep --page raw --csv > gpurun_out/final_full.raw.csv 2>/dev/null

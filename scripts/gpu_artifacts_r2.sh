@@ -21,7 +21,7 @@ echo "components full rc=$? t=$(( $(date +%s) - T0 ))"
 rm -f gpurun_out/r2_step_full.ncu-rep gpurun_out/r2_components_full.ncu-rep
 # compute-sanitizer (memcheck) over the kernel-level parity tests (SURVEY section 5: race / memory checking)
 timeout 900 compute-sanitizer --tool memcheck --error-exitcode 9 --print-limit 20 python -m pytest tests/test_gpu_parity.py tests/test_gpu_encoder_fused.py tests/test_gpu_eval.py tests/test_gpu_herding.py -m gpu -x -q \
-    -k "encoder_forward or train_grad_kd or tc_loss_path or fused_forward or chained or fused_ranks or second_generation or batched_fisher or adam_matches" \
+    -k "encoder_forward or train_grad_kd or tc_loss_path or fused_forward or fused_ranks or second_generation or batched_fisher or adam_matches" \
     > gpurun_out/r2_sanitizer_memcheck.log 2>&1
 echo "sanitizer rc=$? t=$(( $(date +%s) - T0 ))"; tail -8 gpurun_out/r2_sanitizer_memcheck.log
 ls -la gpurun_out/r2_*

@@ -2,7 +2,7 @@
 
     ncu --profile-from-start off --metrics gpu__time_duration.sum --clock-control none --csv \
         --log-file gpurun_out/launches.csv python scripts/ncu_step.py 2
-    ncu --profile-from-start off --set full --clock-control none --import-source on -k regex:k_tc_logits \
+    ncu --profile-from-start off --set full --clock-control none --import-source on -k regex:k_tc2 \
         -o gpurun_out/tc_full python scripts/ncu_step.py 1
 
 Same shapes / dropout as bench.py (YOOCHOOSE ADER period-4 step), the same C-ABI calls the captured graph holds."""

@@ -1,4 +1,4 @@
-"""The shared-memory addressing of the second-generation weight-gradient kernel (ader_b200/csrc/encoder_fused.cuh: k_wgrad2),
+"""The shared-memory addressing of the weight-gradient kernel (ader_b200/csrc/encoder_fused.cuh: k_wgrad2),
 restated on the CPU: the k slots of a TF32 m16n8k8 step are mapped to rows of the 32-token tile so that
   (a) every tile row is consumed by exactly one (k-step, k slot) -- the product sums over all 32 tokens once, and
   (b) with the tile stored at its natural row stride d = 150 floats (one bulk copy, no padding) the 32 lanes of every
@@ -33,13 +33,3 @@ def test_fragment_loads_are_bank_conflict_free_at_d_150():
             for col0 in (0, 8, 16, 24, 40, 80, 88, 120, 152):       # wm * 80 + i * 16 (+ 8), half * 80 + wn * 40 + j * 8
                 banks = (rows * d + col0 + g) % 32
                 assert len(set(banks.tolist())) == 32, (ks, col0)
-
-
-def test_the_padded_stride_of_the_first_generation_is_conflict_free_too():
-    # k_wgrad: rows ks*8 + t4 (+4) at stride 168 (168 % 32 == 8)
-    t4 = np.arange(32) & 3
-    g = np.arange(32) >> 2
-    for ks in range(4):
-        for off in (0, 4):
-            banks = ((ks * 8 + t4 + off) * 168 + g) % 32
-            assert len(set(banks.tolist())) == 32
