@@ -22,6 +22,7 @@
 //   S tile 128 x 64 fp32 in TMEM (2 buffers x 64 columns), 30 MMAs (M = 128, N = 64, K = 16) per tile.
 // Work: CTA = (row tile, vocabulary chunk); counts are merged with integer atomics (order independent).
 #include "tc_common.cuh"
+#include <limits.h>
 #include <stdlib.h>
 
 namespace ader {
@@ -50,11 +51,17 @@ struct EvalArgs {
   int* flags;                // [0] candidate overflow, [1] pipeline timeout
   // top-k (modes MAX / BOTH)
   float* maxbuf;             // MAX: [n_chunks * 2][R] largest approximate score seen by each (chunk, column half) of a row
-  const float* lo_topk;      // BOTH: [R] columns with S~ >= lo_topk[i] are top-k candidates
+  const float* lo_topk;      // BOTH / RCAND: [R] columns with S~ >= lo_topk[i] are top-k candidates
   int* tk_cnt;               // [R]
   int* tk_cand;              // [R][cap]
+  // recommendation (modes RCAND / RMAX): columns never scored for a row, or NULL
+  const int* excl;           // [R][EXCL_W] ascending, distinct
+  const int* excl_cnt;       // [R]
 };
-enum { EV_RANK = 0, EV_MAX = 1, EV_BOTH = 2 };
+// RCAND: top-k candidates of the eligible (not excluded) columns only, no rank counting.
+// RMAX + s: the 2^s largest approximate scores of eligible columns in every (chunk, column half) of a row.
+enum { EV_RANK = 0, EV_MAX = 1, EV_BOTH = 2, EV_RCAND = 3, EV_RMAX = 4 };
+constexpr int EXCL_W = 64;              // a session holds at most maxlen <= 64 items
 
 // fp32 rows -> [rows_pad][320] bf16 (hi | lo), optional row norms and their maximum (as int bits of a non-negative float)
 __global__ void __launch_bounds__(256) k_pack_hilo(const float* __restrict__ src, long long ld, int n_rows, int d, int rows_pad,
@@ -176,6 +183,59 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_eval_tc(EvalArgs a, const __gri
       }
     }
     __syncwarp();
+  } else if constexpr (MODE >= EV_RCAND) {
+    constexpr int MS = MODE >= EV_RMAX ? 1 << (MODE - EV_RMAX) : 1;
+    const int q = warp & 3, half = (warp - 2) >> 2;
+    const int row = q * 32 + lane, gi = x_tile * TM + row;
+    const uint32_t tlane = (uint32_t)(q * 32) << 16;
+    const bool live = gi < a.R;
+    const float lo_k = (live && MODE == EV_RCAND) ? a.lo_topk[gi] : INFINITY;
+    const int* xl = a.excl + (long long)gi * EXCL_W;
+    const int nx = (live && a.excl_cnt) ? a.excl_cnt[gi] : 0;
+    int cur = 0;                                  // cursor into the row's sorted exclusion list
+    float top[MS];                                // descending; each entry is a different column
+#pragma unroll
+    for (int s = 0; s < MS; ++s) top[s] = -INFINITY;
+    for (int it = 0; it < n_it; ++it) {
+      const int s = it & 1; const uint32_t ph = (it >> 1) & 1;
+      mbar_wait(BAR(B_TFULL + s), ph, err);
+      tc_fence_after();
+      uint32_t r[32];
+      tmem_ld32(tmem + tlane + s * TN + half * 32, r);
+      tc_fence_before();
+      mbar_arrive(BAR(B_TEMPTY + s));
+      const int j0 = (y_lo + it) * TN + half * 32;
+      if (!live) continue;
+      // windows come in ascending column order, so one forward walk of the list serves the whole pass
+      while (cur < nx && xl[cur] < j0) ++cur;
+      unsigned ex = 0u;
+      for (int c = cur; c < nx && xl[c] < j0 + 32; ++c) ex |= 1u << (xl[c] - j0);
+      const bool whole = j0 + 32 <= a.V;
+      unsigned topc = 0u;
+#pragma unroll
+      for (int i = 0; i < 32; ++i) {
+        const float v = __uint_as_float(r[i]);
+        const bool ok = (whole || j0 + i < a.V) && !((ex >> i) & 1u);
+        if constexpr (MODE == EV_RCAND) {
+          topc |= (ok && v >= lo_k) ? (1u << i) : 0u;
+        } else if constexpr (MS == 1) {
+          if (ok) top[0] = fmaxf(top[0], v);
+        } else if (ok && v > top[MS - 1]) {       // insert v into the sorted list, dropping the smallest
+#pragma unroll
+          for (int t = MS - 1; t > 0; --t) top[t] = fmaxf(fminf(v, top[t - 1]), top[t]);
+          top[0] = fmaxf(v, top[0]);
+        }
+      }
+      while (topc) {
+        const int i = __ffs(topc) - 1; topc &= topc - 1;
+        const int pos = atomicAdd(a.tk_cnt + gi, 1);
+        if (pos < a.cap) a.tk_cand[(long long)gi * a.cap + pos] = j0 + i; else atomicExch(a.flags, 1);
+      }
+    }
+    if (live && MODE >= EV_RMAX) {
+#pragma unroll
+      for (int t = 0; t < MS; ++t) a.maxbuf[(long long)((chunk * 2 + half) * MS + t) * a.R + gi] = top[t];
+    }
   } else {
     const int q = warp & 3, half = (warp - 2) >> 2;      // TMEM lane quarter, which 32 of the tile's 64 columns
     const int row = q * 32 + lane, gi = x_tile * TM + row;
@@ -328,6 +388,37 @@ __global__ void __launch_bounds__(256) k_topk_refine(const float* __restrict__ t
   }
 }
 
+// ids [R, L] (left-padded, 0 = empty) -> the row's columns id - 1 < V, ascending and distinct, in excl [R][EXCL_W] + excl_cnt [R].
+// Warp per row, two ids per lane: an id is kept at its first position; its slot is the number of distinct smaller ids.
+__global__ void __launch_bounds__(256) k_excl_lists(const int* __restrict__ ids, int R, int L, int V, int* __restrict__ excl,
+                                                    int* __restrict__ excl_cnt) {
+  const int i = (int)(((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+  if (i >= R) return;
+  int v[2]; bool first[2]; int less[2];
+#pragma unroll
+  for (int h = 0; h < 2; ++h) {
+    const int c = lane + 32 * h;
+    const int id = c < L ? ids[(long long)i * L + c] : 0;
+    v[h] = (id >= 1 && id <= V) ? id - 1 : INT_MAX;
+    first[h] = v[h] != INT_MAX; less[h] = 0;
+  }
+  for (int p = 0; p < 64; ++p) {
+    const int x = __shfl_sync(0xffffffffu, p < 32 ? v[0] : v[1], p & 31);
+#pragma unroll
+    for (int h = 0; h < 2; ++h) if (x == v[h] && p < lane + 32 * h) first[h] = false;
+  }
+  for (int p = 0; p < 64; ++p) {
+    const int x = __shfl_sync(0xffffffffu, p < 32 ? v[0] : v[1], p & 31);
+    const bool fx = __shfl_sync(0xffffffffu, p < 32 ? first[0] : first[1], p & 31);
+#pragma unroll
+    for (int h = 0; h < 2; ++h) less[h] += (fx && x < v[h]) ? 1 : 0;
+  }
+#pragma unroll
+  for (int h = 0; h < 2; ++h) if (first[h]) excl[(long long)i * EXCL_W + less[h]] = v[h];
+  const int n = __popc(__ballot_sync(0xffffffffu, first[0])) + __popc(__ballot_sync(0xffffffffu, first[1]));
+  if (lane == 0) excl_cnt[i] = n;
+}
+
 static int eval_chunks(int n_mtiles, int n_vtiles) {
   int best = 1; double best_eff = 0.0;
   const int cmax = n_vtiles / 8 > 1 ? (n_vtiles / 8 < 128 ? n_vtiles / 8 : 128) : 1;      // >= 8 streamed tiles per CTA, <= 256 top-k slots per row
@@ -442,4 +533,70 @@ extern "C" int32_t ader_eval_rank_topk_tc(const AderModel* m, const float* theta
   ADER_CHECK_ARG(R > 0 && V >= 1 && V < m->v_tab && k >= 1 && k <= 32, "eval_rank_topk_tc: bad sizes");
   ADER_CHECK_ARG(m->d <= HALF, "eval_rank_topk_tc: hidden_units must be <= %d", HALF);
   return eval_tc_run(m, theta, rep, gt, R, V, k, ws, rank, topk_item, topk_score, overflow, (cudaStream_t)stream);
+}
+
+// ---- recommendation: top-k items of unlabelled rows, the row's own items excluded ---------------------------------------
+// The top-k scheme of eval_tc_run without the ground-truth anchor.  The first pass keeps the m largest approximate scores of
+// eligible columns per (chunk, column half), m = the smallest of 1, 2, 4, 8 with 2 * nc * m >= k (so 2 * nc * m <= 256, the
+// slot count k_topk_threshold takes); all of them belong to different eligible items, so at least k eligible items score
+// >= tau - eps and every eligible item whose exact score reaches the k-th one has S~ >= tau - 2 eps.
+static size_t rec_excl_off(int R, int V) { return carve(R, V, ADER_EVAL_CAND_CAP, nullptr).bytes; }
+
+extern "C" size_t ader_recommend_tc_ws_bytes(const AderModel* m, int32_t R, int32_t V) {
+  if (check_model(m) || R <= 0 || V <= 0 || m->d > HALF) return 0;
+  return rec_excl_off(R, V) + align_up(sizeof(int) * (size_t)R * EXCL_W) + align_up(sizeof(int) * (size_t)R);
+}
+
+extern "C" int32_t ader_recommend_topk_tc(const AderModel* m, const float* theta, const float* rep, const int32_t* ids, int32_t R,
+                                          int32_t V, int32_t k, void* ws, int32_t* topk_item, float* topk_score,
+                                          int32_t* overflow, void* stream) {
+  if (int e = check_model(m)) return e;
+  ADER_CHECK_ARG(theta && rep && ws && topk_item && topk_score && overflow, "recommend_topk_tc: NULL pointer");
+  ADER_CHECK_ARG(R > 0 && V >= 1 && V < m->v_tab && k >= 1 && k <= 100, "recommend_topk_tc: bad sizes");
+  ADER_CHECK_ARG(m->d <= HALF, "recommend_topk_tc: hidden_units must be <= %d", HALF);
+  cudaStream_t st = (cudaStream_t)stream;
+  const int d = m->d, cap = ADER_EVAL_CAND_CAP;
+  EvalWs w = carve(R, V, cap, (char*)ws);
+  int* excl = (int*)((char*)ws + rec_excl_off(R, V));
+  int* excl_cnt = (int*)((char*)excl + align_up(sizeof(int) * (size_t)R * EXCL_W));
+  const int nm = cdiv(R, TM), nv = cdiv(V, TN), nc = eval_chunks(nm, nv);
+  int ms = 1;
+  while (ms < 8 && 2 * nc * ms < k) ms *= 2;
+  ADER_CHECK_ARG(2 * nc * ms >= k, "recommend_topk_tc: top-%d needs %d vocabulary chunks per row tile (have %d): use ader_recommend_topk",
+                 k, (k + 15) / 16, nc);
+  static bool attr = false;
+  if (!attr) {
+    cudaFuncSetAttribute(k_eval_tc<EV_RCAND>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_EVAL);
+    cudaFuncSetAttribute(k_eval_tc<EV_RMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_EVAL);
+    cudaFuncSetAttribute(k_eval_tc<EV_RMAX + 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_EVAL);
+    cudaFuncSetAttribute(k_eval_tc<EV_RMAX + 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_EVAL);
+    cudaFuncSetAttribute(k_eval_tc<EV_RMAX + 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_EVAL);
+    attr = true;
+  }
+  CUtensorMap tx, ty;
+  if (int e = make_map2d(&tx, w.x16, D2, (uint64_t)nm * TM, D2 * 2, TM)) return e;
+  if (int e = make_map2d(&ty, w.y16, D2, (uint64_t)nv * TN, D2 * 2, TN)) return e;
+  const float* table1 = theta + d;
+  cudaMemsetAsync(w.max_norm, 0, sizeof(int) * 8, st);          // max_norm + flags
+  cudaMemsetAsync(w.tk_cnt, 0, sizeof(int) * (size_t)R, st);
+  k_pack_hilo<<<cdiv((long long)nv * TN * 32, 256), 256, 0, st>>>(table1, d, V, d, nv * TN, w.y16, nullptr, w.max_norm);
+  k_pack_hilo<<<cdiv((long long)nm * TM * 32, 256), 256, 0, st>>>(rep, d, R, d, nm * TM, w.x16, w.rnorm, nullptr);
+  if (ids) k_excl_lists<<<cdiv((long long)R * 32, 256), 256, 0, st>>>(ids, R, m->maxlen, V, excl, excl_cnt);
+  EvalArgs a = {};
+  a.R = R; a.V = V; a.n_mtiles = nm; a.n_vtiles = nv; a.n_chunks = nc;
+  a.cap = cap; a.flags = w.flags; a.maxbuf = w.maxbuf; a.lo_topk = w.lo_topk; a.tk_cnt = w.tk_cnt; a.tk_cand = w.tk_cand;
+  a.excl = ids ? excl : nullptr; a.excl_cnt = ids ? excl_cnt : nullptr;
+  const int grid = nm * nc;
+  switch (ms) {
+    case 1: k_eval_tc<EV_RMAX><<<grid, NTHREADS, SMEM_EVAL, st>>>(a, tx, ty); break;
+    case 2: k_eval_tc<EV_RMAX + 1><<<grid, NTHREADS, SMEM_EVAL, st>>>(a, tx, ty); break;
+    case 4: k_eval_tc<EV_RMAX + 2><<<grid, NTHREADS, SMEM_EVAL, st>>>(a, tx, ty); break;
+    default: k_eval_tc<EV_RMAX + 3><<<grid, NTHREADS, SMEM_EVAL, st>>>(a, tx, ty); break;
+  }
+  k_topk_threshold<<<cdiv((long long)R * 32, 256), 256, 0, st>>>(w.maxbuf, 2 * nc * ms, R, k, w.rnorm, w.max_norm, w.lo_topk);
+  k_eval_tc<EV_RCAND><<<grid, NTHREADS, SMEM_EVAL, st>>>(a, tx, ty);
+  k_topk_refine<<<cdiv((long long)R * 32, 256), 256, 0, st>>>(table1, rep, R, d, w.tk_cnt, w.tk_cand, cap, k, topk_item, topk_score);
+  cudaMemcpyAsync(overflow, w.flags, sizeof(int), cudaMemcpyDeviceToDevice, st);
+  ADER_CHECK_LAUNCH("recommend_topk_tc");
+  return 0;
 }

@@ -185,6 +185,15 @@ __global__ void __launch_bounds__(256) k_rank_topk_rows(const float* __restrict_
   }
 }
 
+// recommendation: the row's own items (ids [R, L], 0 = empty) become NaN in its score row.  NaN compares false both ways,
+// so k_rank_topk_rows never selects such a column: it is skipped exactly like a column that is not there.
+__global__ void k_mark_seen(float* __restrict__ S, long long ld, const int* __restrict__ ids, int R, int L, int V) {
+  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= (long long)R * L) return;
+  const int id = ids[idx];
+  if (id >= 1 && id <= V) S[(idx / L) * ld + id - 1] = __int_as_float(0x7fc00000);
+}
+
 }  // namespace ader
 
 using namespace ader;
@@ -284,5 +293,20 @@ extern "C" int32_t ader_eval_rank_topk(const AderModel* m, const float* theta, c
   if (int e = run_logits(m, theta, rep, M, V, S, ld, st)) return e;
   k_rank_topk_rows<<<M, 256, 0, st>>>(S, ld, V, gt, k, rank, topk_item, topk_score);
   ADER_CHECK_LAUNCH("rank_topk_rows");
+  return 0;
+}
+
+extern "C" int32_t ader_recommend_topk(const AderModel* m, const float* theta, const float* rep, const int32_t* ids, int32_t R,
+                                       int32_t V, int32_t k, void* ws, int32_t* topk_item, float* topk_score, void* stream) {
+  if (int e = check_model(m)) return e;
+  ADER_CHECK_ARG(theta && rep && ws && topk_item && topk_score, "recommend_topk: NULL pointer");
+  ADER_CHECK_ARG(R > 0 && V >= 1 && V < m->v_tab && k >= 1 && k <= 100, "recommend_topk: bad sizes");
+  cudaStream_t st = (cudaStream_t)stream;
+  const long long ld = logits_ld(V);
+  float* S = (float*)ws;
+  if (int e = run_logits(m, theta, rep, R, V, S, ld, st)) return e;
+  if (ids) k_mark_seen<<<cdiv((long long)R * m->maxlen, 256), 256, 0, st>>>(S, ld, ids, R, m->maxlen, V);
+  k_rank_topk_rows<<<R, 256, 0, st>>>(S, ld, V, nullptr, k, nullptr, topk_item, topk_score);
+  ADER_CHECK_LAUNCH("recommend_topk");
   return 0;
 }

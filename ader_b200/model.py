@@ -359,6 +359,36 @@ class Ader:
         ops.eval_rank_topk(self.ms, self.theta, rep, gt_t, max_item, k, ws, rank, items, scores)
         return rank, items, scores
 
+    def recommend(self, seq, max_item: int, k: int = 20, exclude_seen: bool = True, n_tokens: Optional[int] = None,
+                  force_exact: bool = False):
+        """Top-k next items among 1..max_item for unlabelled sessions: ``seq`` [R, maxlen] left-padded ids (the input rows of
+        ``rank_topk``) -> (items [R, k] int32, best first, ties -> lower id; scores [R, k] fp32, the exact scores of
+        ``logits``).  exclude_seen: the items of the row's own session are never returned.  A row with fewer than k eligible
+        items is padded with item 0 and score -inf.  The tensor-core entry is used where it applies; a batch whose candidate
+        list overflows is rerun on the exact entry (counted in ``eval_fallbacks``).  The lists are the same either way."""
+        if not 1 <= k <= 100:
+            raise ValueError("k must be in 1..100 (got %d)" % k)
+        ids = _to_ids(seq, self.hp.maxlen, self.device)
+        R = ids.shape[0]
+        items = torch.empty((R, k), dtype=torch.int32, device=self.device)
+        scores = torch.empty((R, k), dtype=torch.float32, device=self.device)
+        if R == 0:
+            return items, scores
+        rep = self.encode(ids, n_tokens)[0]
+        self._check_overflow()
+        seen = ids if exclude_seen else None
+        if (not force_exact and self.eval_impl == "tc" and self.hp.hidden_units <= 160
+                and 2 * 8 * ops.eval_topk_chunks(self.ms, R, max_item) >= k):
+            ws = self._eval_ws.get(ops.recommend_tc_ws_bytes(self.ms, R, max_item))
+            over = torch.zeros(1, dtype=torch.int32, device=self.device)
+            ops.recommend_topk_tc(self.ms, self.theta, rep, seen, max_item, k, ws, items, scores, over)
+            if int(over.item()) == 0:
+                return items, scores
+            self.eval_fallbacks += 1          # more than ADER_EVAL_CAND_CAP candidates in a row: exact entry for this batch
+        ws = self._eval_ws.get(ops.eval_ws_bytes(self.ms, R, max_item))
+        ops.recommend_topk(self.ms, self.theta, rep, seen, max_item, k, ws, items, scores)
+        return items, scores
+
     def check_guards(self, guards) -> list:
         """One host read of the guard words collected by rank_topk(guards=...): raises on an encoder token overflow, returns
         the indices of the calls whose candidate band overflowed (the caller re-runs those with force_exact=True)."""

@@ -317,6 +317,29 @@ def eval_rank_topk_tc(ms: AderModel, theta, rep, gt, V: int, k: int, ws, rank, t
                                              _ptr(topk_item), _ptr(topk_score), _ptr(overflow), _stream()), "eval_rank_topk_tc")
 
 
+def recommend_topk(ms: AderModel, theta, rep, ids, V: int, k: int, ws, topk_item, topk_score):
+    """Top-k items 1..V of every row of rep (exact fp32 scores, ties -> lower id); ids [R, maxlen] (or None): the row's own
+    items are left out.  ws: eval_ws_bytes(ms, R, V)."""
+    _require_cuda(theta, rep, ids, ws, topk_item, topk_score)
+    check(_lib.load().ader_recommend_topk(C.byref(ms), _ptr(theta), _ptr(rep), _ptr(ids), rep.shape[0], V, k, _ptr(ws),
+                                          _ptr(topk_item), _ptr(topk_score), _stream()), "recommend_topk")
+
+
+def recommend_tc_ws_bytes(ms: AderModel, R: int, V: int) -> int:
+    n = _lib.load().ader_recommend_tc_ws_bytes(C.byref(ms), R, V)
+    if n == 0:
+        raise _lib.AderError("recommend_tc_ws_bytes: bad model / sizes")
+    return n
+
+
+def recommend_topk_tc(ms: AderModel, theta, rep, ids, V: int, k: int, ws, topk_item, topk_score, overflow):
+    """The same lists on the tensor cores; needs 2 * 8 * eval_topk_chunks(R, V) >= k.  overflow[0] != 0 -> use
+    recommend_topk for this batch."""
+    _require_cuda(theta, rep, ids, ws, topk_item, topk_score, overflow)
+    check(_lib.load().ader_recommend_topk_tc(C.byref(ms), _ptr(theta), _ptr(rep), _ptr(ids), rep.shape[0], V, k, _ptr(ws),
+                                             _ptr(topk_item), _ptr(topk_score), _ptr(overflow), _stream()), "recommend_topk_tc")
+
+
 def herding_ws_bytes(ms: AderModel, N: int) -> int:
     n = _lib.load().ader_herding_ws_bytes(C.byref(ms), N)
     if n == 0:
@@ -411,6 +434,8 @@ _SCHEMAS = {
     "eval_rank_topk": "(int[] model, Tensor theta, Tensor rep, Tensor gt, int V, int k, Tensor(a!) ws, Tensor(b!) rank, Tensor(c!) topk_item, Tensor(d!) topk_score) -> ()",
     "eval_rank_tc": "(int[] model, Tensor theta, Tensor rep, Tensor gt, int V, Tensor(a!) ws, Tensor(b!) rank, Tensor(c!) overflow) -> ()",
     "eval_rank_topk_tc": "(int[] model, Tensor theta, Tensor rep, Tensor gt, int V, int k, Tensor(a!) ws, Tensor(b!) rank, Tensor(c!) topk_item, Tensor(d!) topk_score, Tensor(e!) overflow) -> ()",
+    "recommend_topk": "(int[] model, Tensor theta, Tensor rep, Tensor? ids, int V, int k, Tensor(a!) ws, Tensor(b!) topk_item, Tensor(c!) topk_score) -> ()",
+    "recommend_topk_tc": "(int[] model, Tensor theta, Tensor rep, Tensor? ids, int V, int k, Tensor(a!) ws, Tensor(b!) topk_item, Tensor(c!) topk_score, Tensor(d!) overflow) -> ()",
     "herding_segmented": "(int[] model, Tensor rep, Tensor cand, Tensor seg_off, Tensor quota, Tensor max_steps, Tensor(a!) ws, Tensor(b!) picks, Tensor(c!) n_picked) -> ()",
     "fisher_accumulate": "(int[] model, Tensor grad, Tensor(a!) acc, int V) -> ()",
     "fisher_finalize": "(int[] model, Tensor acc, Tensor(a!) fisher, int V, int n_data) -> ()",
@@ -465,6 +490,8 @@ def register_torch_ops() -> None:
         "eval_rank_topk": lambda model, theta, rep, gt, V, k, ws, rank, items, scores: eval_rank_topk(_ms(model), theta, rep, gt, V, k, ws, rank, items, scores),
         "eval_rank_tc": lambda model, theta, rep, gt, V, ws, rank, overflow: eval_rank_tc(_ms(model), theta, rep, gt, V, ws, rank, overflow),
         "eval_rank_topk_tc": lambda model, theta, rep, gt, V, k, ws, rank, items, scores, overflow: eval_rank_topk_tc(_ms(model), theta, rep, gt, V, k, ws, rank, items, scores, overflow),
+        "recommend_topk": lambda model, theta, rep, ids, V, k, ws, items, scores: recommend_topk(_ms(model), theta, rep, ids, V, k, ws, items, scores),
+        "recommend_topk_tc": lambda model, theta, rep, ids, V, k, ws, items, scores, overflow: recommend_topk_tc(_ms(model), theta, rep, ids, V, k, ws, items, scores, overflow),
         "herding_segmented": lambda model, rep, cand, seg_off, quota, max_steps, ws, picks, n_picked: herding_segmented(_ms(model), rep, cand, seg_off, quota, max_steps, ws, picks, n_picked),
         "fisher_accumulate": lambda model, grad, acc, V: fisher_accumulate(_ms(model), grad, acc, V),
         "fisher_finalize": lambda model, acc, fisher, V, n_data: fisher_finalize(_ms(model), acc, fisher, V, n_data),

@@ -228,6 +228,21 @@ int32_t ader_eval_rank_topk_tc(const AderModel* m, const float* theta, const flo
                                int32_t V, int32_t k, void* ws, int32_t* rank, int32_t* topk_item, float* topk_score,
                                int32_t* overflow, void* stream);
 
+/* ---- recommendation: top-k items for unlabelled sessions -------------------------------- */
+/* top-k items 1..V per row, best first, ties -> lower id, exact fp32 scores; ids [R, maxlen] (or NULL): the row's own
+ * items are never returned; fewer than k eligible items -> item 0, score -inf.  k <= 100. */
+int32_t ader_recommend_topk(const AderModel* m, const float* theta, const float* rep, const int32_t* ids, int32_t R,
+                            int32_t V, int32_t k, void* ws /* ader_eval_ws_bytes */, int32_t* topk_item,
+                            float* topk_score, void* stream);
+/* The same lists on the tcgen05 tensor cores, the [R, V] scores never written: the top-k scheme of ader_eval_rank_topk_tc
+ * without the ground-truth anchor, the row's own items left out of both passes, and m = 1, 2, 4 or 8 approximate maxima
+ * kept per (vocabulary chunk, column half).  Results are identical to ader_recommend_topk.  overflow[0] != 0: a row had
+ * more than ADER_EVAL_CAND_CAP candidates; use ader_recommend_topk for this batch. */
+size_t  ader_recommend_tc_ws_bytes(const AderModel* m, int32_t R, int32_t V);
+int32_t ader_recommend_topk_tc(const AderModel* m, const float* theta, const float* rep, const int32_t* ids, int32_t R,
+                               int32_t V, int32_t k, void* ws, int32_t* topk_item, float* topk_score,
+                               int32_t* overflow, void* stream);   /* needs d <= 160 and 2*ader_eval_topk_chunks*8 >= k */
+
 /* ---- exemplar selection: util.py:401-461 (subsystem 4) ---------------------------------- */
 /* Segmented herding.  rep [N,d]; segment s owns candidate rows cand[seg_off[s] .. seg_off[s+1])
  * (indices into rep, in the reference's sess_by_item order); quota[s] = min(m, n_s);
