@@ -49,18 +49,15 @@ struct EvalArgs {
   int* cand;                 // [R][cap]
   int cap;
   int* flags;                // [0] candidate overflow, [1] pipeline timeout
-  // top-k (modes MAX / BOTH)
-  float* maxbuf;             // MAX: [n_chunks * 2][R] largest approximate score seen by each (chunk, column half) of a row
-  const float* lo_topk;      // BOTH / RCAND: [R] columns with S~ >= lo_topk[i] are top-k candidates
+  // top-k
+  float* maxbuf;             // MS: [n_chunks * 2 * MS][R] the MS largest approximate scores of each (chunk, column half) of a row
+  const float* lo_topk;      // CAND: [R] columns with S~ >= lo_topk[i] are top-k candidates
   int* tk_cnt;               // [R]
   int* tk_cand;              // [R][cap]
-  // recommendation (modes RCAND / RMAX): columns never scored for a row, or NULL
+  // EXCL: columns never scored for a row (a recommended session's own items)
   const int* excl;           // [R][EXCL_W] ascending, distinct
   const int* excl_cnt;       // [R]
 };
-// RCAND: top-k candidates of the eligible (not excluded) columns only, no rank counting.
-// RMAX + s: the 2^s largest approximate scores of eligible columns in every (chunk, column half) of a row.
-enum { EV_RANK = 0, EV_MAX = 1, EV_BOTH = 2, EV_RCAND = 3, EV_RMAX = 4 };
 constexpr int EXCL_W = 64;              // a session holds at most maxlen <= 64 items
 
 // fp32 rows -> [rows_pad][320] bf16 (hi | lo), optional row norms and their maximum (as int bits of a non-negative float)
@@ -106,7 +103,12 @@ __device__ __forceinline__ uint64_t desc_col(uint32_t base, int col, int reg) {
   return make_desc_sw128(base + (col >> 6) * reg + (col & 63) * 2, 16, 1024);
 }
 
-template <int MODE>
+// One pass over the [R, V] approximate scores; its epilogue does what the template parameters ask of each eligible column:
+//   RANK: count the columns certainly above the row's anchor (S~ > hi_thr) and append those in [lo_thr, hi_thr] to cand;
+//   CAND: append the columns with S~ >= lo_topk to tk_cand;
+//   MS:   keep the MS largest scores of every (chunk, column half) of a row, sorted in registers, in maxbuf (0: none);
+//   EXCL: the row's excl list is left out (a column is eligible when it is an item and not excluded).
+template <bool RANK, bool CAND, int MS, bool EXCL>
 __global__ void __launch_bounds__(NTHREADS, 1) k_eval_tc(EvalArgs a, const __grid_constant__ CUtensorMap tm_x,
                                                          const __grid_constant__ CUtensorMap tm_y) {
   extern __shared__ uint8_t smem_raw[];
@@ -183,68 +185,19 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_eval_tc(EvalArgs a, const __gri
       }
     }
     __syncwarp();
-  } else if constexpr (MODE >= EV_RCAND) {
-    constexpr int MS = MODE >= EV_RMAX ? 1 << (MODE - EV_RMAX) : 1;
-    const int q = warp & 3, half = (warp - 2) >> 2;
-    const int row = q * 32 + lane, gi = x_tile * TM + row;
-    const uint32_t tlane = (uint32_t)(q * 32) << 16;
-    const bool live = gi < a.R;
-    const float lo_k = (live && MODE == EV_RCAND) ? a.lo_topk[gi] : INFINITY;
-    const int* xl = a.excl + (long long)gi * EXCL_W;
-    const int nx = (live && a.excl_cnt) ? a.excl_cnt[gi] : 0;
-    int cur = 0;                                  // cursor into the row's sorted exclusion list
-    float top[MS];                                // descending; each entry is a different column
-#pragma unroll
-    for (int s = 0; s < MS; ++s) top[s] = -INFINITY;
-    for (int it = 0; it < n_it; ++it) {
-      const int s = it & 1; const uint32_t ph = (it >> 1) & 1;
-      mbar_wait(BAR(B_TFULL + s), ph, err);
-      tc_fence_after();
-      uint32_t r[32];
-      tmem_ld32(tmem + tlane + s * TN + half * 32, r);
-      tc_fence_before();
-      mbar_arrive(BAR(B_TEMPTY + s));
-      const int j0 = (y_lo + it) * TN + half * 32;
-      if (!live) continue;
-      // windows come in ascending column order, so one forward walk of the list serves the whole pass
-      while (cur < nx && xl[cur] < j0) ++cur;
-      unsigned ex = 0u;
-      for (int c = cur; c < nx && xl[c] < j0 + 32; ++c) ex |= 1u << (xl[c] - j0);
-      const bool whole = j0 + 32 <= a.V;
-      unsigned topc = 0u;
-#pragma unroll
-      for (int i = 0; i < 32; ++i) {
-        const float v = __uint_as_float(r[i]);
-        const bool ok = (whole || j0 + i < a.V) && !((ex >> i) & 1u);
-        if constexpr (MODE == EV_RCAND) {
-          topc |= (ok && v >= lo_k) ? (1u << i) : 0u;
-        } else if constexpr (MS == 1) {
-          if (ok) top[0] = fmaxf(top[0], v);
-        } else if (ok && v > top[MS - 1]) {       // insert v into the sorted list, dropping the smallest
-#pragma unroll
-          for (int t = MS - 1; t > 0; --t) top[t] = fmaxf(fminf(v, top[t - 1]), top[t]);
-          top[0] = fmaxf(v, top[0]);
-        }
-      }
-      while (topc) {
-        const int i = __ffs(topc) - 1; topc &= topc - 1;
-        const int pos = atomicAdd(a.tk_cnt + gi, 1);
-        if (pos < a.cap) a.tk_cand[(long long)gi * a.cap + pos] = j0 + i; else atomicExch(a.flags, 1);
-      }
-    }
-    if (live && MODE >= EV_RMAX) {
-#pragma unroll
-      for (int t = 0; t < MS; ++t) a.maxbuf[(long long)((chunk * 2 + half) * MS + t) * a.R + gi] = top[t];
-    }
   } else {
     const int q = warp & 3, half = (warp - 2) >> 2;      // TMEM lane quarter, which 32 of the tile's 64 columns
     const int row = q * 32 + lane, gi = x_tile * TM + row;
     const uint32_t tlane = (uint32_t)(q * 32) << 16;
     const bool live = gi < a.R;
-    const bool ranking = MODE != EV_MAX;
-    const float lo = (live && ranking) ? a.lo_thr[gi] : INFINITY, hi = (live && ranking) ? a.hi_thr[gi] : INFINITY;
-    const float lo_k = (live && MODE == EV_BOTH) ? a.lo_topk[gi] : INFINITY;
-    float vmax = -INFINITY;
+    const float lo = (live && RANK) ? a.lo_thr[gi] : INFINITY, hi = (live && RANK) ? a.hi_thr[gi] : INFINITY;
+    const float lo_k = (live && CAND) ? a.lo_topk[gi] : INFINITY;
+    const int* xl = a.excl + (long long)gi * EXCL_W;
+    const int nx = (EXCL && live) ? a.excl_cnt[gi] : 0;
+    int cur = 0;                                  // cursor into the row's sorted exclusion list
+    float top[MS > 0 ? MS : 1];                   // descending; each entry is a different column
+#pragma unroll
+    for (int s = 0; s < MS; ++s) top[s] = -INFINITY;
     int above = 0;
     for (int it = 0; it < n_it; ++it) {
       const int s = it & 1; const uint32_t ph = (it >> 1) & 1;
@@ -256,20 +209,32 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_eval_tc(EvalArgs a, const __gri
       mbar_arrive(BAR(B_TEMPTY + s));
       const int j0 = (y_lo + it) * TN + half * 32;
       if (!live) continue;
-      const bool whole = j0 + 32 <= a.V;          // else: zero padding rows of the table matrix are not items
-      if (MODE == EV_MAX) {
-#pragma unroll
-        for (int i = 0; i < 32; ++i) if (whole || j0 + i < a.V) vmax = fmaxf(vmax, __uint_as_float(r[i]));
-        continue;
+      unsigned ex = 0u;
+      if constexpr (EXCL) {
+        // windows come in ascending column order, so one forward walk of the list serves the whole pass
+        while (cur < nx && xl[cur] < j0) ++cur;
+        for (int c = cur; c < nx && xl[c] < j0 + 32; ++c) ex |= 1u << (xl[c] - j0);
       }
+      const bool whole = j0 + 32 <= a.V;          // else: zero padding rows of the table matrix are not items
       unsigned unsure = 0u, topc = 0u;
 #pragma unroll
       for (int i = 0; i < 32; ++i) {
         const float v = __uint_as_float(r[i]);
-        const bool ok = whole || j0 + i < a.V;
-        above += (ok && v > hi) ? 1 : 0;
-        unsure |= (ok && v >= lo && v <= hi) ? (1u << i) : 0u;
-        if (MODE == EV_BOTH) topc |= (ok && v >= lo_k) ? (1u << i) : 0u;
+        const bool ok = (whole || j0 + i < a.V) && !((ex >> i) & 1u);
+        if constexpr (RANK) {
+          above += (ok && v > hi) ? 1 : 0;
+          unsure |= (ok && v >= lo && v <= hi) ? (1u << i) : 0u;
+        }
+        if constexpr (CAND) topc |= (ok && v >= lo_k) ? (1u << i) : 0u;
+        if constexpr (MS == 1) {
+          if (ok) top[0] = fmaxf(top[0], v);
+        } else if constexpr (MS > 1) {
+          if (ok && v > top[MS - 1]) {            // insert v into the sorted list, dropping the smallest
+#pragma unroll
+            for (int t = MS - 1; t > 0; --t) top[t] = fmaxf(fminf(v, top[t - 1]), top[t]);
+            top[0] = fmaxf(v, top[0]);
+          }
+        }
       }
       while (unsure) {                            // rare: a handful of columns per row in the whole pass
         const int i = __ffs(unsure) - 1; unsure &= unsure - 1;
@@ -282,8 +247,11 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_eval_tc(EvalArgs a, const __gri
         if (pos < a.cap) a.tk_cand[(long long)gi * a.cap + pos] = j0 + i; else atomicExch(a.flags, 1);
       }
     }
-    if (live && MODE == EV_MAX) a.maxbuf[(long long)(chunk * 2 + half) * a.R + gi] = vmax;
-    if (live && ranking && above) atomicAdd(a.above + gi, above);
+    if (live) {
+#pragma unroll
+      for (int t = 0; t < MS; ++t) a.maxbuf[(long long)((chunk * 2 + half) * MS + t) * a.R + gi] = top[t];
+    }
+    if (live && RANK && above) atomicAdd(a.above + gi, above);
   }
   __syncthreads();
   if (warp == 1) {
@@ -419,7 +387,8 @@ __global__ void __launch_bounds__(256) k_excl_lists(const int* __restrict__ ids,
   if (lane == 0) excl_cnt[i] = n;
 }
 
-static int eval_chunks(int n_mtiles, int n_vtiles) {
+static int eval_chunks(int R, int V) {
+  const int n_mtiles = cdiv(R, TM), n_vtiles = cdiv(V, TN);
   int best = 1; double best_eff = 0.0;
   const int cmax = n_vtiles / 8 > 1 ? (n_vtiles / 8 < 128 ? n_vtiles / 8 : 128) : 1;      // >= 8 streamed tiles per CTA, <= 256 top-k slots per row
   for (int c = 1; c <= cmax; ++c) {
@@ -436,12 +405,14 @@ struct EvalWs {
   float *rnorm, *sg, *lo, *hi;
   int *max_norm, *above, *cand_cnt, *cand, *flags, *tk_cnt, *tk_cand;
   float *lo_topk, *maxbuf;
+  int *excl, *excl_cnt;
   size_t bytes;
 };
-static EvalWs carve(int R, int V, int cap, char* base) {
+// excl: append the exclusion lists (recommendation); the layout before them is the same either way
+static EvalWs carve(int R, int V, bool excl, char* base) {
   EvalWs w; size_t o = 0;
   auto take = [&](size_t n) { char* p = base ? base + o : nullptr; o += align_up(n); return p; };
-  const int nm = cdiv(R, TM), nv = cdiv(V, TN);
+  const int nm = cdiv(R, TM), nv = cdiv(V, TN), cap = ADER_EVAL_CAND_CAP;
   w.x16 = (__nv_bfloat16*)take((size_t)nm * TM * D2 * 2);
   w.y16 = (__nv_bfloat16*)take((size_t)nv * TN * D2 * 2);
   w.rnorm = (float*)take(sizeof(float) * R);
@@ -456,8 +427,28 @@ static EvalWs carve(int R, int V, int cap, char* base) {
   w.tk_cand = (int*)take(sizeof(int) * (size_t)R * cap);
   w.lo_topk = (float*)take(sizeof(float) * (size_t)R);
   w.maxbuf = (float*)take(sizeof(float) * (size_t)R * 2 * 128);
+  w.excl = excl ? (int*)take(sizeof(int) * (size_t)R * EXCL_W) : nullptr;
+  w.excl_cnt = excl ? (int*)take(sizeof(int) * (size_t)R) : nullptr;
   w.bytes = o;
   return w;
+}
+
+template <bool RANK, bool CAND, int MS, bool EXCL>
+static void eval_pass(const EvalArgs& a, const CUtensorMap& tx, const CUtensorMap& ty, cudaStream_t st) {
+  static const cudaError_t attr =
+      cudaFuncSetAttribute(k_eval_tc<RANK, CAND, MS, EXCL>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_EVAL);
+  (void)attr;                                     // a refusal surfaces as the launch error
+  k_eval_tc<RANK, CAND, MS, EXCL><<<a.n_mtiles * a.n_chunks, NTHREADS, SMEM_EVAL, st>>>(a, tx, ty);
+}
+
+template <bool EXCL>
+static void maxima_pass(int ms, const EvalArgs& a, const CUtensorMap& tx, const CUtensorMap& ty, cudaStream_t st) {
+  switch (ms) {
+    case 1: eval_pass<false, false, 1, EXCL>(a, tx, ty, st); break;
+    case 2: eval_pass<false, false, 2, EXCL>(a, tx, ty, st); break;
+    case 4: eval_pass<false, false, 4, EXCL>(a, tx, ty, st); break;
+    default: eval_pass<false, false, 8, EXCL>(a, tx, ty, st); break;
+  }
 }
 
 }  // namespace ev
@@ -466,49 +457,56 @@ static EvalWs carve(int R, int V, int cap, char* base) {
 using namespace ader;
 using namespace ader::ev;
 
-extern "C" size_t ader_eval_rank_tc_ws_bytes(const AderModel* m, int32_t R, int32_t V) {
-  if (check_model(m) || R <= 0 || V <= 0 || m->d > HALF) return 0;
-  return carve(R, V, ADER_EVAL_CAND_CAP, nullptr).bytes;
-}
-
-static int eval_tc_run(const AderModel* m, const float* theta, const float* rep, const int32_t* gt, int R, int V, int k, void* ws,
-                       int32_t* rank, int32_t* topk_item, float* topk_score, int32_t* overflow, cudaStream_t st) {
+// The pipeline behind the three tensor-core entries.  gt (or NULL): rank of the ground truth, from its exact score
+// (k_gt_band), the counting pass and k_refine.  k > 0: top-k, from a maxima pass, tau (k_topk_threshold), a candidate pass and
+// k_topk_refine.  ids (or NULL, never with gt): each row's own items are left out of the maxima and the candidates.
+// The maxima pass keeps m scores per (chunk, column half), m = the smallest of 1, 2, 4, 8 with 2 * nc * m >= k (the eval
+// entries admit only 2 * nc >= k, so they run with m = 1; 2 * nc * m <= 256, the slot count k_topk_threshold takes).  All
+// kept scores belong to different eligible items, so at least k eligible items score >= tau - eps and every eligible item
+// whose exact score reaches the k-th one has S~ >= tau - 2 eps.
+static int topk_tc_run(const AderModel* m, const float* theta, const float* rep, const int32_t* gt, const int32_t* ids, int R,
+                       int V, int k, void* ws, int32_t* rank, int32_t* topk_item, float* topk_score, int32_t* overflow,
+                       cudaStream_t st) {
   const int d = m->d, cap = ADER_EVAL_CAND_CAP;
-  EvalWs w = carve(R, V, cap, (char*)ws);
-  const int nm = cdiv(R, TM), nv = cdiv(V, TN), nc = eval_chunks(nm, nv);
-  ADER_CHECK_ARG(k == 0 || (2 * nc >= k && 2 * nc <= 256), "eval_rank_tc: top-%d needs %d..128 vocabulary chunks per row tile (have %d): use ader_eval_rank_topk", k, (k + 1) / 2, nc);
-  static bool attr = false;
-  if (!attr) {
-    cudaFuncSetAttribute(k_eval_tc<EV_RANK>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_EVAL);
-    cudaFuncSetAttribute(k_eval_tc<EV_MAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_EVAL);
-    cudaFuncSetAttribute(k_eval_tc<EV_BOTH>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_EVAL);
-    attr = true;
-  }
+  EvalWs w = carve(R, V, ids != nullptr, (char*)ws);
+  const int nm = cdiv(R, TM), nv = cdiv(V, TN), nc = eval_chunks(R, V);
+  int ms = 1;
+  while (ms < 8 && 2 * nc * ms < k) ms *= 2;
   CUtensorMap tx, ty;
   if (int e = make_map2d(&tx, w.x16, D2, (uint64_t)nm * TM, D2 * 2, TM)) return e;
   if (int e = make_map2d(&ty, w.y16, D2, (uint64_t)nv * TN, D2 * 2, TN)) return e;
   const float* table1 = theta + d;                       // item 1 = table row 1 (ADER.py:90-91)
-  cudaMemsetAsync(w.max_norm, 0, sizeof(int) * (8 + 2 * (size_t)R), st);
+  cudaMemsetAsync(w.max_norm, 0, sizeof(int) * (8 + (gt ? 2 * (size_t)R : 0)), st);
+  if (k > 0) cudaMemsetAsync(w.tk_cnt, 0, sizeof(int) * (size_t)R, st);
   k_pack_hilo<<<cdiv((long long)nv * TN * 32, 256), 256, 0, st>>>(table1, d, V, d, nv * TN, w.y16, nullptr, w.max_norm);
   k_pack_hilo<<<cdiv((long long)nm * TM * 32, 256), 256, 0, st>>>(rep, d, R, d, nm * TM, w.x16, w.rnorm, nullptr);
-  k_gt_band<<<cdiv(R, 256), 256, 0, st>>>(table1, rep, gt, R, d, w.rnorm, w.max_norm, w.sg, w.lo, w.hi);
-  EvalArgs a;
+  if (gt) k_gt_band<<<cdiv(R, 256), 256, 0, st>>>(table1, rep, gt, R, d, w.rnorm, w.max_norm, w.sg, w.lo, w.hi);
+  if (ids) k_excl_lists<<<cdiv((long long)R * 32, 256), 256, 0, st>>>(ids, R, m->maxlen, V, w.excl, w.excl_cnt);
+  EvalArgs a = {};
   a.R = R; a.V = V; a.n_mtiles = nm; a.n_vtiles = nv; a.n_chunks = nc;
   a.lo_thr = w.lo; a.hi_thr = w.hi; a.above = w.above; a.cand_cnt = w.cand_cnt; a.cand = w.cand; a.cap = cap; a.flags = w.flags;
   a.maxbuf = w.maxbuf; a.lo_topk = w.lo_topk; a.tk_cnt = w.tk_cnt; a.tk_cand = w.tk_cand;
+  a.excl = w.excl; a.excl_cnt = w.excl_cnt;
   if (k > 0) {
-    cudaMemsetAsync(w.tk_cnt, 0, sizeof(int) * (size_t)R, st);
-    k_eval_tc<EV_MAX><<<nm * nc, NTHREADS, SMEM_EVAL, st>>>(a, tx, ty);
-    k_topk_threshold<<<cdiv((long long)R * 32, 256), 256, 0, st>>>(w.maxbuf, 2 * nc, R, k, w.rnorm, w.max_norm, w.lo_topk);
-    k_eval_tc<EV_BOTH><<<nm * nc, NTHREADS, SMEM_EVAL, st>>>(a, tx, ty);
-    k_topk_refine<<<cdiv((long long)R * 32, 256), 256, 0, st>>>(table1, rep, R, d, w.tk_cnt, w.tk_cand, cap, k, topk_item, topk_score);
-  } else {
-    k_eval_tc<EV_RANK><<<nm * nc, NTHREADS, SMEM_EVAL, st>>>(a, tx, ty);
+    if (ids) maxima_pass<true>(ms, a, tx, ty, st); else maxima_pass<false>(ms, a, tx, ty, st);
+    k_topk_threshold<<<cdiv((long long)R * 32, 256), 256, 0, st>>>(w.maxbuf, 2 * nc * ms, R, k, w.rnorm, w.max_norm, w.lo_topk);
   }
-  k_refine<<<cdiv((long long)R * 32, 256), 256, 0, st>>>(table1, rep, gt, R, d, w.sg, w.above, w.cand_cnt, w.cand, cap, rank);
+  if (gt) {
+    if (k > 0) eval_pass<true, true, 0, false>(a, tx, ty, st); else eval_pass<true, false, 0, false>(a, tx, ty, st);
+  } else {
+    if (ids) eval_pass<false, true, 0, true>(a, tx, ty, st); else eval_pass<false, true, 0, false>(a, tx, ty, st);
+  }
+  if (k > 0)
+    k_topk_refine<<<cdiv((long long)R * 32, 256), 256, 0, st>>>(table1, rep, R, d, w.tk_cnt, w.tk_cand, cap, k, topk_item, topk_score);
+  if (gt) k_refine<<<cdiv((long long)R * 32, 256), 256, 0, st>>>(table1, rep, gt, R, d, w.sg, w.above, w.cand_cnt, w.cand, cap, rank);
   cudaMemcpyAsync(overflow, w.flags, sizeof(int), cudaMemcpyDeviceToDevice, st);
-  ADER_CHECK_LAUNCH("eval_rank_tc");
+  ADER_CHECK_LAUNCH(gt ? "eval_rank_tc" : "recommend_topk_tc");
   return 0;
+}
+
+extern "C" size_t ader_eval_rank_tc_ws_bytes(const AderModel* m, int32_t R, int32_t V) {
+  if (check_model(m) || R <= 0 || V <= 0 || m->d > HALF) return 0;
+  return carve(R, V, false, nullptr).bytes;
 }
 
 extern "C" int32_t ader_eval_rank_tc(const AderModel* m, const float* theta, const float* rep, const int32_t* gt, int32_t R,
@@ -517,12 +515,12 @@ extern "C" int32_t ader_eval_rank_tc(const AderModel* m, const float* theta, con
   ADER_CHECK_ARG(theta && rep && gt && ws && rank && overflow, "eval_rank_tc: NULL pointer");
   ADER_CHECK_ARG(R > 0 && V >= 1 && V < m->v_tab, "eval_rank_tc: bad sizes");
   ADER_CHECK_ARG(m->d <= HALF, "eval_rank_tc: hidden_units must be <= %d", HALF);
-  return eval_tc_run(m, theta, rep, gt, R, V, 0, ws, rank, nullptr, nullptr, overflow, (cudaStream_t)stream);
+  return topk_tc_run(m, theta, rep, gt, nullptr, R, V, 0, ws, rank, nullptr, nullptr, overflow, (cudaStream_t)stream);
 }
 
 extern "C" int32_t ader_eval_topk_chunks(const AderModel* m, int32_t R, int32_t V) {
   if (check_model(m) || R <= 0 || V <= 0) return 0;
-  return eval_chunks(cdiv(R, TM), cdiv(V, TN));
+  return eval_chunks(R, V);
 }
 
 extern "C" int32_t ader_eval_rank_topk_tc(const AderModel* m, const float* theta, const float* rep, const int32_t* gt, int32_t R,
@@ -532,19 +530,14 @@ extern "C" int32_t ader_eval_rank_topk_tc(const AderModel* m, const float* theta
   ADER_CHECK_ARG(theta && rep && gt && ws && rank && overflow && topk_item && topk_score, "eval_rank_topk_tc: NULL pointer");
   ADER_CHECK_ARG(R > 0 && V >= 1 && V < m->v_tab && k >= 1 && k <= 32, "eval_rank_topk_tc: bad sizes");
   ADER_CHECK_ARG(m->d <= HALF, "eval_rank_topk_tc: hidden_units must be <= %d", HALF);
-  return eval_tc_run(m, theta, rep, gt, R, V, k, ws, rank, topk_item, topk_score, overflow, (cudaStream_t)stream);
+  const int nc = eval_chunks(R, V);
+  ADER_CHECK_ARG(2 * nc >= k && 2 * nc <= 256, "eval_rank_tc: top-%d needs %d..128 vocabulary chunks per row tile (have %d): use ader_eval_rank_topk", k, (k + 1) / 2, nc);
+  return topk_tc_run(m, theta, rep, gt, nullptr, R, V, k, ws, rank, topk_item, topk_score, overflow, (cudaStream_t)stream);
 }
-
-// ---- recommendation: top-k items of unlabelled rows, the row's own items excluded ---------------------------------------
-// The top-k scheme of eval_tc_run without the ground-truth anchor.  The first pass keeps the m largest approximate scores of
-// eligible columns per (chunk, column half), m = the smallest of 1, 2, 4, 8 with 2 * nc * m >= k (so 2 * nc * m <= 256, the
-// slot count k_topk_threshold takes); all of them belong to different eligible items, so at least k eligible items score
-// >= tau - eps and every eligible item whose exact score reaches the k-th one has S~ >= tau - 2 eps.
-static size_t rec_excl_off(int R, int V) { return carve(R, V, ADER_EVAL_CAND_CAP, nullptr).bytes; }
 
 extern "C" size_t ader_recommend_tc_ws_bytes(const AderModel* m, int32_t R, int32_t V) {
   if (check_model(m) || R <= 0 || V <= 0 || m->d > HALF) return 0;
-  return rec_excl_off(R, V) + align_up(sizeof(int) * (size_t)R * EXCL_W) + align_up(sizeof(int) * (size_t)R);
+  return carve(R, V, true, nullptr).bytes;
 }
 
 extern "C" int32_t ader_recommend_topk_tc(const AderModel* m, const float* theta, const float* rep, const int32_t* ids, int32_t R,
@@ -554,49 +547,8 @@ extern "C" int32_t ader_recommend_topk_tc(const AderModel* m, const float* theta
   ADER_CHECK_ARG(theta && rep && ws && topk_item && topk_score && overflow, "recommend_topk_tc: NULL pointer");
   ADER_CHECK_ARG(R > 0 && V >= 1 && V < m->v_tab && k >= 1 && k <= 100, "recommend_topk_tc: bad sizes");
   ADER_CHECK_ARG(m->d <= HALF, "recommend_topk_tc: hidden_units must be <= %d", HALF);
-  cudaStream_t st = (cudaStream_t)stream;
-  const int d = m->d, cap = ADER_EVAL_CAND_CAP;
-  EvalWs w = carve(R, V, cap, (char*)ws);
-  int* excl = (int*)((char*)ws + rec_excl_off(R, V));
-  int* excl_cnt = (int*)((char*)excl + align_up(sizeof(int) * (size_t)R * EXCL_W));
-  const int nm = cdiv(R, TM), nv = cdiv(V, TN), nc = eval_chunks(nm, nv);
-  int ms = 1;
-  while (ms < 8 && 2 * nc * ms < k) ms *= 2;
-  ADER_CHECK_ARG(2 * nc * ms >= k, "recommend_topk_tc: top-%d needs %d vocabulary chunks per row tile (have %d): use ader_recommend_topk",
+  const int nc = eval_chunks(R, V);
+  ADER_CHECK_ARG(2 * nc * 8 >= k, "recommend_topk_tc: top-%d needs %d vocabulary chunks per row tile (have %d): use ader_recommend_topk",
                  k, (k + 15) / 16, nc);
-  static bool attr = false;
-  if (!attr) {
-    cudaFuncSetAttribute(k_eval_tc<EV_RCAND>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_EVAL);
-    cudaFuncSetAttribute(k_eval_tc<EV_RMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_EVAL);
-    cudaFuncSetAttribute(k_eval_tc<EV_RMAX + 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_EVAL);
-    cudaFuncSetAttribute(k_eval_tc<EV_RMAX + 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_EVAL);
-    cudaFuncSetAttribute(k_eval_tc<EV_RMAX + 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_EVAL);
-    attr = true;
-  }
-  CUtensorMap tx, ty;
-  if (int e = make_map2d(&tx, w.x16, D2, (uint64_t)nm * TM, D2 * 2, TM)) return e;
-  if (int e = make_map2d(&ty, w.y16, D2, (uint64_t)nv * TN, D2 * 2, TN)) return e;
-  const float* table1 = theta + d;
-  cudaMemsetAsync(w.max_norm, 0, sizeof(int) * 8, st);          // max_norm + flags
-  cudaMemsetAsync(w.tk_cnt, 0, sizeof(int) * (size_t)R, st);
-  k_pack_hilo<<<cdiv((long long)nv * TN * 32, 256), 256, 0, st>>>(table1, d, V, d, nv * TN, w.y16, nullptr, w.max_norm);
-  k_pack_hilo<<<cdiv((long long)nm * TM * 32, 256), 256, 0, st>>>(rep, d, R, d, nm * TM, w.x16, w.rnorm, nullptr);
-  if (ids) k_excl_lists<<<cdiv((long long)R * 32, 256), 256, 0, st>>>(ids, R, m->maxlen, V, excl, excl_cnt);
-  EvalArgs a = {};
-  a.R = R; a.V = V; a.n_mtiles = nm; a.n_vtiles = nv; a.n_chunks = nc;
-  a.cap = cap; a.flags = w.flags; a.maxbuf = w.maxbuf; a.lo_topk = w.lo_topk; a.tk_cnt = w.tk_cnt; a.tk_cand = w.tk_cand;
-  a.excl = ids ? excl : nullptr; a.excl_cnt = ids ? excl_cnt : nullptr;
-  const int grid = nm * nc;
-  switch (ms) {
-    case 1: k_eval_tc<EV_RMAX><<<grid, NTHREADS, SMEM_EVAL, st>>>(a, tx, ty); break;
-    case 2: k_eval_tc<EV_RMAX + 1><<<grid, NTHREADS, SMEM_EVAL, st>>>(a, tx, ty); break;
-    case 4: k_eval_tc<EV_RMAX + 2><<<grid, NTHREADS, SMEM_EVAL, st>>>(a, tx, ty); break;
-    default: k_eval_tc<EV_RMAX + 3><<<grid, NTHREADS, SMEM_EVAL, st>>>(a, tx, ty); break;
-  }
-  k_topk_threshold<<<cdiv((long long)R * 32, 256), 256, 0, st>>>(w.maxbuf, 2 * nc * ms, R, k, w.rnorm, w.max_norm, w.lo_topk);
-  k_eval_tc<EV_RCAND><<<grid, NTHREADS, SMEM_EVAL, st>>>(a, tx, ty);
-  k_topk_refine<<<cdiv((long long)R * 32, 256), 256, 0, st>>>(table1, rep, R, d, w.tk_cnt, w.tk_cand, cap, k, topk_item, topk_score);
-  cudaMemcpyAsync(overflow, w.flags, sizeof(int), cudaMemcpyDeviceToDevice, st);
-  ADER_CHECK_LAUNCH("recommend_topk_tc");
-  return 0;
+  return topk_tc_run(m, theta, rep, nullptr, ids, R, V, k, ws, nullptr, topk_item, topk_score, overflow, (cudaStream_t)stream);
 }

@@ -280,6 +280,18 @@ extern "C" size_t ader_eval_ws_bytes(const AderModel* m, int32_t M, int32_t V) {
   return align_up(sizeof(float) * (size_t)M * logits_ld(V));
 }
 
+// exact scores, the row's own items masked out when ids is set, then the rank of gt (when set) and the top-k of every row
+static int exact_rank_topk(const AderModel* m, const float* theta, const float* rep, const int32_t* gt, const int32_t* ids, int R,
+                           int V, int k, void* ws, int32_t* rank, int32_t* topk_item, float* topk_score, cudaStream_t st) {
+  const long long ld = logits_ld(V);
+  float* S = (float*)ws;
+  if (int e = run_logits(m, theta, rep, R, V, S, ld, st)) return e;
+  if (ids) k_mark_seen<<<cdiv((long long)R * m->maxlen, 256), 256, 0, st>>>(S, ld, ids, R, m->maxlen, V);
+  k_rank_topk_rows<<<R, 256, 0, st>>>(S, ld, V, gt, k, rank, topk_item, topk_score);
+  ADER_CHECK_LAUNCH("rank_topk_rows");
+  return 0;
+}
+
 extern "C" int32_t ader_eval_rank_topk(const AderModel* m, const float* theta, const float* rep, const int32_t* gt,
                                        int32_t M, int32_t V, int32_t k, void* ws, int32_t* rank,
                                        int32_t* topk_item, float* topk_score, void* stream) {
@@ -287,13 +299,7 @@ extern "C" int32_t ader_eval_rank_topk(const AderModel* m, const float* theta, c
   ADER_CHECK_ARG(theta && rep && ws && M > 0 && V >= 1 && V < m->v_tab, "eval_rank_topk: bad argument");
   ADER_CHECK_ARG(k >= 0 && k <= 32 && (k == 0 || (topk_item && topk_score)), "eval_rank_topk: bad k");
   ADER_CHECK_ARG(!gt || rank, "eval_rank_topk: rank is NULL");
-  cudaStream_t st = (cudaStream_t)stream;
-  const long long ld = logits_ld(V);
-  float* S = (float*)ws;
-  if (int e = run_logits(m, theta, rep, M, V, S, ld, st)) return e;
-  k_rank_topk_rows<<<M, 256, 0, st>>>(S, ld, V, gt, k, rank, topk_item, topk_score);
-  ADER_CHECK_LAUNCH("rank_topk_rows");
-  return 0;
+  return exact_rank_topk(m, theta, rep, gt, nullptr, M, V, k, ws, rank, topk_item, topk_score, (cudaStream_t)stream);
 }
 
 extern "C" int32_t ader_recommend_topk(const AderModel* m, const float* theta, const float* rep, const int32_t* ids, int32_t R,
@@ -301,12 +307,5 @@ extern "C" int32_t ader_recommend_topk(const AderModel* m, const float* theta, c
   if (int e = check_model(m)) return e;
   ADER_CHECK_ARG(theta && rep && ws && topk_item && topk_score, "recommend_topk: NULL pointer");
   ADER_CHECK_ARG(R > 0 && V >= 1 && V < m->v_tab && k >= 1 && k <= 100, "recommend_topk: bad sizes");
-  cudaStream_t st = (cudaStream_t)stream;
-  const long long ld = logits_ld(V);
-  float* S = (float*)ws;
-  if (int e = run_logits(m, theta, rep, R, V, S, ld, st)) return e;
-  if (ids) k_mark_seen<<<cdiv((long long)R * m->maxlen, 256), 256, 0, st>>>(S, ld, ids, R, m->maxlen, V);
-  k_rank_topk_rows<<<R, 256, 0, st>>>(S, ld, V, nullptr, k, nullptr, topk_item, topk_score);
-  ADER_CHECK_LAUNCH("recommend_topk");
-  return 0;
+  return exact_rank_topk(m, theta, rep, nullptr, ids, R, V, k, ws, nullptr, topk_item, topk_score, (cudaStream_t)stream);
 }

@@ -77,7 +77,7 @@ class Ader:
         self.encoder_impl = getattr(args, "encoder_impl", None) or ("exact" if self.loss_impl == "exact" else "tc")
         self.infer_encoder_impl = getattr(args, "infer_encoder_impl", "exact")
         # evaluation ranks: "tc" = fused tcgen05 scoring + exact refinement (identical ranks), "exact" = fp32 [M, V] scores
-        self.eval_impl = getattr(args, "eval_impl", None) or os.environ.get("ADER_B200_EVAL", "tc")
+        self.eval_impl = getattr(args, "eval_impl", None) or "tc"
         self.eval_fallbacks = 0
         # how a tc + tc training pass is issued: "dag" = ader_train_fwd_bwd_tc (fork/join over side streams),
         # "serial" = the same entry on one stream, "groups" = the three single-group entry points one after another
@@ -332,31 +332,14 @@ class Ader:
             off = ops.encoder_ws_slot(self.ms, M, tcap_used, -4, 0)
             tok_flag = self._enc_ws.buf[off:off + 4].view(torch.int32).clone()
         rank = torch.empty(M, dtype=torch.int32, device=self.device)
-        if not force_exact and self.eval_impl == "tc" and self.hp.hidden_units <= 160 and (k <= 0 or 2 * ops.eval_topk_chunks(self.ms, M, max_item) >= k):
-            # tcgen05 scores + exact refinement of the columns inside the certainty bands (ader_eval_rank_tc /
-            # ader_eval_rank_topk_tc: identical ranks and top-k lists, the [M, V] scores are never written)
-            ws = self._eval_ws.get(ops.eval_rank_tc_ws_bytes(self.ms, M, max_item))
-            over = torch.zeros(1, dtype=torch.int32, device=self.device)
-            if k <= 0:
-                ops.eval_rank_tc(self.ms, self.theta, rep, gt_t, max_item, ws, rank, over)
-                items = torch.empty((M, 1), dtype=torch.int32, device=self.device)
-                scores = items.float()
-            else:
-                items = torch.empty((M, k), dtype=torch.int32, device=self.device)
-                scores = torch.empty((M, k), dtype=torch.float32, device=self.device)
-                ops.eval_rank_topk_tc(self.ms, self.theta, rep, gt_t, max_item, k, ws, rank, items, scores, over)
-            if guards is not None:
-                guards.append((tok_flag, over))
-                return rank, items, scores
-            if int(over.item()) == 0:
-                return rank, items, scores
-            self.eval_fallbacks += 1          # a band held more than ADER_EVAL_CAND_CAP columns: exact path for this batch
-        if guards is not None:
-            guards.append((tok_flag, torch.zeros(1, dtype=torch.int32, device=self.device)))
-        ws = self._eval_ws.get(ops.eval_ws_bytes(self.ms, M, max_item))
         items = torch.empty((M, max(k, 1)), dtype=torch.int32, device=self.device)
         scores = torch.empty((M, max(k, 1)), dtype=torch.float32, device=self.device)
-        ops.eval_rank_topk(self.ms, self.theta, rep, gt_t, max_item, k, ws, rank, items, scores)
+        # tcgen05 scores + exact refinement inside the certainty bands: identical ranks and top-k, [M, V] never written
+        tc = ((lambda ws, over: ops.eval_rank_tc(self.ms, self.theta, rep, gt_t, max_item, ws, rank, over)) if k <= 0 else
+              (lambda ws, over: ops.eval_rank_topk_tc(self.ms, self.theta, rep, gt_t, max_item, k, ws, rank, items, scores, over)))
+        self._tc_or_exact(M, max_item, k, 1, ops.eval_rank_tc_ws_bytes, tc,
+                          lambda ws: ops.eval_rank_topk(self.ms, self.theta, rep, gt_t, max_item, k, ws, rank, items, scores),
+                          force_exact, guards, tok_flag)
         return rank, items, scores
 
     def recommend(self, seq, max_item: int, k: int = 20, exclude_seen: bool = True, n_tokens: Optional[int] = None,
@@ -377,17 +360,30 @@ class Ader:
         rep = self.encode(ids, n_tokens)[0]
         self._check_overflow()
         seen = ids if exclude_seen else None
-        if (not force_exact and self.eval_impl == "tc" and self.hp.hidden_units <= 160
-                and 2 * 8 * ops.eval_topk_chunks(self.ms, R, max_item) >= k):
-            ws = self._eval_ws.get(ops.recommend_tc_ws_bytes(self.ms, R, max_item))
-            over = torch.zeros(1, dtype=torch.int32, device=self.device)
-            ops.recommend_topk_tc(self.ms, self.theta, rep, seen, max_item, k, ws, items, scores, over)
-            if int(over.item()) == 0:
-                return items, scores
-            self.eval_fallbacks += 1          # more than ADER_EVAL_CAND_CAP candidates in a row: exact entry for this batch
-        ws = self._eval_ws.get(ops.eval_ws_bytes(self.ms, R, max_item))
-        ops.recommend_topk(self.ms, self.theta, rep, seen, max_item, k, ws, items, scores)
+        self._tc_or_exact(R, max_item, k, 8, ops.recommend_tc_ws_bytes,
+                          lambda ws, over: ops.recommend_topk_tc(self.ms, self.theta, rep, seen, max_item, k, ws, items, scores, over),
+                          lambda ws: ops.recommend_topk(self.ms, self.theta, rep, seen, max_item, k, ws, items, scores),
+                          force_exact)
         return items, scores
+
+    def _tc_or_exact(self, R: int, max_item: int, k: int, m_max: int, tc_ws_bytes, run_tc, run_exact, force_exact: bool,
+                     guards: Optional[list] = None, tok_flag=None):
+        """``run_tc(ws, over)`` where the tensor-core entry applies (hidden_units <= 160, 2 * m_max * chunks >= k: up to m_max
+        maxima per (chunk, column half)); else, or after a candidate overflow (counted in ``eval_fallbacks``), ``run_exact(ws)``.
+        guards: see ``rank_topk``; ``(tok_flag, overflow word)`` is appended instead of read."""
+        if (not force_exact and self.eval_impl == "tc" and self.hp.hidden_units <= 160
+                and 2 * m_max * ops.eval_topk_chunks(self.ms, R, max_item) >= k):
+            over = torch.zeros(1, dtype=torch.int32, device=self.device)
+            run_tc(self._eval_ws.get(tc_ws_bytes(self.ms, R, max_item)), over)
+            if guards is not None:
+                guards.append((tok_flag, over))
+                return
+            if int(over.item()) == 0:
+                return
+            self.eval_fallbacks += 1          # more than ADER_EVAL_CAND_CAP candidates in a row: exact entry for this batch
+        if guards is not None:
+            guards.append((tok_flag, torch.zeros(1, dtype=torch.int32, device=self.device)))
+        run_exact(self._eval_ws.get(ops.eval_ws_bytes(self.ms, R, max_item)))
 
     def check_guards(self, guards) -> list:
         """One host read of the guard words collected by rank_topk(guards=...): raises on an encoder token overflow, returns
