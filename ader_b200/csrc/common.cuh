@@ -58,9 +58,19 @@ static inline int check_model(const AderModel* m) {
   return 0;
 }
 
-// Teacher of a distillation (mode 1) call: stored logits (`teacher`) or a frozen snapshot (`teacher_rep` + the table the
-// entry reads: fp32 rows for the exact entry, the bf16 shadow for the tcgen05 ones) -- exactly one of the two.
-static inline int check_teacher(const AderLossArgs* a, const char* who, bool tc) {
+// The fields of AderLossArgs (a != NULL), as every logits + CE + distillation entry takes them.  The teacher of a
+// distillation (mode 1) call is stored logits (`teacher`) or a frozen snapshot (`teacher_rep` + the table the entry reads:
+// fp32 rows for the exact entry, the bf16 shadow for the tcgen05 ones `tc`) -- exactly one of the two.
+static inline int check_loss_args(const AderModel* m, const AderLossArgs* a, const char* who, bool tc) {
+  if (a->M != a->n_train + a->n_ex || a->M <= 0)
+    return fail(-1, "%s: M (%d) != n_train + n_ex (%d + %d)", who, a->M, a->n_train, a->n_ex);
+  if (a->V < 1 || a->V >= m->v_tab) return fail(-1, "%s: max_item %d outside table of %d rows", who, a->V, m->v_tab);
+  if (a->mode < 0 || a->mode > 2) return fail(-1, "%s: bad mode %d", who, a->mode);
+  if (a->n_train > 0 && !a->pos) return fail(-1, "%s: pos is NULL", who);
+  if (a->n_ex <= 0) return 0;
+  if (a->mode == 0) return fail(-1, "%s: exemplar rows given in vanilla mode", who);
+  if (a->mode == 2 && !a->ex_pos) return fail(-1, "%s: exemplar_pos is NULL", who);
+  if (a->mode != 1) return 0;
   const bool stored = a->teacher != nullptr, frozen = a->teacher_rep != nullptr;
   if (stored == frozen)
     return fail(-1, "%s: mode 1 takes exactly one teacher source: teacher (stored logits) or teacher_rep (frozen snapshot)", who);

@@ -37,7 +37,6 @@
 // online (max, sumexp) per chunk, merged into lse_t), then
 //   MODE_TP  : recomputes the T tiles and writes Pc = coef * exp(T - lse_t) as bf16 straight into the matrix MODE_TU / MODE_DE read
 #include "tc_common.cuh"
-#include <stdlib.h>
 
 namespace ader {
 namespace tc {
@@ -738,12 +737,15 @@ static int tc_chunks(int n_mtiles, int n_vtiles) {
   }
   return best;
 }
-// V = columns of this shard (local), Vp_local = how many of them are teacher columns (0 = no distillation)
-static TcWs carve_tc(const AderModel* m, int M, int V, int n_ex, int Vp_local, char* base, bool frozen = false) {
+// workspace of a call over logits columns [v_lo, v_hi); its teacher columns are the part of [0, V_prev) inside that range
+static TcWs carve_tc(const AderLossArgs* a, int v_lo, int v_hi, char* base) {
   TcWs w; size_t o = 0;
   auto take = [&](size_t n) { char* p = base ? base + o : nullptr; o += align_up(n); return p; };
+  const int M = a->M, V = v_hi - v_lo, n_ex = a->n_ex;
+  const int t_hi = a->V_prev < v_hi ? a->V_prev : v_hi;
+  const int Vp_local = n_ex > 0 && a->mode == 1 && t_hi > v_lo ? t_hi - v_lo : 0;
   const int nm = cdiv(M, TILE), nv = cdiv(V, TILE), nc = tc_chunks(nm, nv);
-  const bool kd = n_ex > 0 && Vp_local > 0;
+  const bool kd = Vp_local > 0;
   w.x0_t = kd ? (M - n_ex) / TILE : 0;
   w.n_et = kd ? (M - 1) / TILE - w.x0_t + 1 : 0;
   w.n_vtp = kd ? cdiv(Vp_local, TILE) : 0;
@@ -759,7 +761,7 @@ static TcWs carve_tc(const AderModel* m, int M, int V, int n_ex, int Vp_local, c
   w.u = (float*)take(sizeof(float) * ((size_t)w.n_et * TILE * KP + 4));
   w.udot = (float*)take(sizeof(float) * ((size_t)w.n_et * TILE + 4));
   w.err = (int*)take(sizeof(int) * 4);
-  const bool fz = frozen && kd;
+  const bool fz = a->teacher_rep && kd;
   w.trep16 = fz ? (uint8_t*)take((size_t)w.n_et * TILE * ROW16 * 2) : nullptr;
   w.tstats = fz ? (float*)take(sizeof(float) * 4 * (size_t)w.n_chunks_t * 2 * w.n_et * TILE) : nullptr;
   w.lse_tt = fz ? (float*)take(sizeof(float) * (size_t)w.n_et * TILE) : nullptr;
@@ -769,7 +771,7 @@ static TcWs carve_tc(const AderModel* m, int M, int V, int n_ex, int Vp_local, c
 
 extern "C" size_t ader_loss_tc_ws_bytes(const AderModel* m, const AderLossArgs* a) {
   if (check_model(m) || !a || a->M <= 0 || a->V <= 0) return 0;
-  return carve_tc(m, a->M, a->V, a->n_ex, a->mode == 1 ? a->V_prev : 0, nullptr, a->teacher_rep != nullptr).bytes;
+  return carve_tc(a, 0, a->V, nullptr).bytes;
 }
 
 extern "C" size_t ader_table16_ws_bytes(const AderModel* m, int32_t V) {
@@ -777,18 +779,6 @@ extern "C" size_t ader_table16_ws_bytes(const AderModel* m, int32_t V) {
   return (size_t)cdiv(V, TILE) * TILE * ROW16 * 2;
 }
 
-// ---- TMA tensor maps over the row-major bf16 operand matrices ---------------------------------------------------------
-struct TcMaps { CUtensorMap rep, e, pt, trep, ttab; };     // trep / ttab: frozen teacher only
-static int make_tc_maps(const TcWs& w, int nm, int nv, TcMaps& mp) {
-  if (int e = make_map2d(&mp.rep, w.rep_tiles, ROW16, (uint64_t)nm * TILE, ROW16 * 2)) return e;
-  if (int e = make_map2d(&mp.e, w.e_tiles, ROW16, (uint64_t)nv * TILE, ROW16 * 2)) return e;
-  if (w.n_et > 0 && w.n_vtp > 0) {
-    if (int e = make_map2d(&mp.pt, w.pt_tiles, (uint64_t)w.n_vtp * TILE, (uint64_t)w.n_et * TILE, (uint64_t)w.n_vtp * TILE * 2)) return e;
-  } else mp.pt = mp.e;       // never dereferenced (no teacher tiles), but the parameter must be a valid map
-  return 0;
-}
-
-// launches shared by the single-GPU and vocab-parallel entry points -----------------------------------------------
 static void set_tc_attrs() {
   static bool attr_set = false;
   if (attr_set) return;
@@ -799,6 +789,43 @@ static void set_tc_attrs() {
   cudaFuncSetAttribute(k_tc2<MODE_TP>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tc2(MODE_TP));
   attr_set = true;
 }
+
+// TMA tensor maps over the row-major bf16 operand matrices
+struct TcMaps { CUtensorMap rep, e, pt, trep, ttab; };     // trep / ttab: frozen teacher only
+
+// The tcgen05 plan of one call over logits columns [v_lo, v_hi) -- the single-GPU loss is the one shard [0, V): workspace,
+// kernel arguments and tensor maps.  grad (or NULL) receives dE in item-table rows v_lo+1 .. v_hi.  Host work only.
+static int tc_plan(const AderModel* m, const AderLossArgs* a, int v_lo, int v_hi, void* ws, float* grad,
+                   TcWs& w, TcArgs& t, TcMaps& mp) {
+  const int d = m->d, M = a->M, V = v_hi - v_lo;
+  w = carve_tc(a, v_lo, v_hi, (char*)ws);
+  const int nm = cdiv(M, TILE), nv = cdiv(V, TILE), nc = tc_chunks(nm, nv);
+  set_tc_attrs();
+
+  t.M = M; t.V = V; t.V_total = a->V; t.v_off = v_lo; t.n_mtiles = nm; t.n_vtiles = nv; t.n_chunks = nc;
+  t.n_train = a->n_train; t.n_ex = a->n_ex; t.V_prev = a->V_prev; t.mode = a->n_ex > 0 ? a->mode : 0;
+  t.coef_train = a->n_train > 0 ? 1.0f / (float)(a->n_train_global > 0 ? a->n_train_global : a->n_train) : 0.f;
+  t.coef_ex = a->n_ex > 0 ? a->lambda_ / (float)(a->n_ex_global > 0 ? a->n_ex_global : a->n_ex) : 0.f;
+  t.pos = a->pos; t.ex_pos = a->ex_pos;
+  t.lse = w.lse; t.lse_t = w.lse_t; t.stats = w.stats; t.drep_part = w.drep_part;
+  t.grad_table = grad ? grad + (size_t)(1 + v_lo) * d : nullptr;
+  t.d = d; t.err = w.err;
+  t.x0_t = w.x0_t; t.n_et = w.n_et; t.n_vtp = w.n_vtp; t.n_chunks_t = w.n_chunks_t; t.u_part = w.u_part;
+  t.pt_out = nullptr; t.t_row_lo = t.t_row_hi = 0;
+
+  if (int e = make_map2d(&mp.rep, w.rep_tiles, ROW16, (uint64_t)nm * TILE, ROW16 * 2)) return e;
+  if (int e = make_map2d(&mp.e, w.e_tiles, ROW16, (uint64_t)nv * TILE, ROW16 * 2)) return e;
+  if (w.n_et > 0 && w.n_vtp > 0) {
+    if (int e = make_map2d(&mp.pt, w.pt_tiles, (uint64_t)w.n_vtp * TILE, (uint64_t)w.n_et * TILE, (uint64_t)w.n_vtp * TILE * 2)) return e;
+  } else mp.pt = mp.e;       // never dereferenced (no teacher tiles), but the parameter must be a valid map
+  if (w.trep16) {            // frozen teacher
+    if (int e = make_map2d(&mp.trep, w.trep16, ROW16, (uint64_t)w.n_et * TILE, ROW16 * 2)) return e;
+    if (int e = make_map2d(&mp.ttab, a->teacher_table16, ROW16, (uint64_t)w.n_vtp * TILE, ROW16 * 2)) return e;
+  }
+  return 0;
+}
+
+// launches shared by the single-GPU and vocab-parallel entry points -----------------------------------------------
 // teacher statistics + tiles + uc partials (rep-independent), then u = sum of partials and udot = rep . u
 // frozen teacher: Pc from the snapshot (packed reps -> MODE_FWD statistics of T = trep . E_prev^T -> lse_t -> MODE_TP tiles)
 static void launch_teacher_frozen(const AderLossArgs* a, const TcWs& w, const TcArgs& t, int d, cudaStream_t st, const TcMaps& mp) {
@@ -866,46 +893,18 @@ int ader::loss_tc_run(const AderModel* m, const float* theta, const float* rep, 
   ADER_CHECK_ARG(theta && a && ws, "loss_fwd_bwd_tc: NULL pointer");
   ADER_CHECK_ARG(!(phase_mask & 2) || (rep && loss && row_loss), "loss_fwd_bwd_tc: NULL pointer");
   ADER_CHECK_ARG(m->d <= KP && m->d % 2 == 0, "loss_fwd_bwd_tc: hidden_units must be <= %d", KP);
-  ADER_CHECK_ARG(a->M == a->n_train + a->n_ex && a->M > 0, "loss_fwd_bwd_tc: M != n_train + n_ex");
-  ADER_CHECK_ARG(a->V >= 1 && a->V < m->v_tab, "loss_fwd_bwd_tc: max_item outside the table");
-  ADER_CHECK_ARG(a->mode >= 0 && a->mode <= 2, "loss_fwd_bwd_tc: bad mode");
-  ADER_CHECK_ARG(a->n_train == 0 || a->pos, "loss_fwd_bwd_tc: pos is NULL");
-  if (a->n_ex > 0) {
-    ADER_CHECK_ARG(a->mode != 0, "loss_fwd_bwd_tc: exemplar rows given in vanilla mode");
-    if (a->mode == 1) { if (int e = check_teacher(a, "loss_fwd_bwd_tc", true)) return e; }
-    if (a->mode == 2) ADER_CHECK_ARG(a->ex_pos, "loss_fwd_bwd_tc: exemplar_pos is NULL");
-  }
+  if (int e = check_loss_args(m, a, "loss_fwd_bwd_tc", true)) return e;
   cudaStream_t st = f.main, sb = f.b;
   const int d = m->d, M = a->M, V = a->V;
   const bool kd = a->n_ex > 0 && a->mode == 1;
-  TcWs w = carve_tc(m, M, V, a->n_ex, kd ? a->V_prev : 0, (char*)ws, a->teacher_rep != nullptr);
-  const int nm = cdiv(M, TILE), nv = cdiv(V, TILE), nc = tc_chunks(nm, nv);
-  set_tc_attrs();
-
-  TcArgs t;
-  t.M = M; t.V = V; t.V_total = V; t.v_off = 0; t.n_mtiles = nm; t.n_vtiles = nv; t.n_chunks = nc;
-  t.n_train = a->n_train; t.n_ex = a->n_ex; t.V_prev = a->V_prev; t.mode = a->n_ex > 0 ? a->mode : 0;
-  t.coef_train = a->n_train > 0 ? 1.0f / (float)(a->n_train_global > 0 ? a->n_train_global : a->n_train) : 0.f;
-  t.coef_ex = a->n_ex > 0 ? a->lambda_ / (float)(a->n_ex_global > 0 ? a->n_ex_global : a->n_ex) : 0.f;
-  t.pos = a->pos; t.ex_pos = a->ex_pos;
-  t.lse = w.lse; t.lse_t = w.lse_t; t.stats = w.stats; t.drep_part = w.drep_part; t.grad_table = grad ? grad + d : nullptr;
-  t.d = d; t.err = w.err;
-  t.x0_t = w.x0_t; t.n_et = w.n_et; t.n_vtp = w.n_vtp; t.n_chunks_t = w.n_chunks_t; t.u_part = w.u_part;
-  t.pt_out = nullptr; t.t_row_lo = t.t_row_hi = 0;
-
-  TcMaps mp;
-  if (int e = make_tc_maps(w, nm, nv, mp)) return e;
-  if (kd && a->teacher_rep) {
-    if (int e = make_map2d(&mp.trep, w.trep16, ROW16, (uint64_t)w.n_et * TILE, ROW16 * 2)) return e;
-    if (int e = make_map2d(&mp.ttab, a->teacher_table16, ROW16, (uint64_t)w.n_vtp * TILE, ROW16 * 2)) return e;
-  }
+  TcWs w; TcArgs t; TcMaps mp;
+  if (int e = tc_plan(m, a, 0, V, ws, grad, w, t, mp)) return e;
+  const int nm = t.n_mtiles, nv = t.n_vtiles, nc = t.n_chunks;
   if (phase_mask == 4) {      // measurement only: the three tensor-core kernels on an already prepared workspace, launched as
-                              // in the step: programmatic dependent launches along the chain (ADER_B200_PDL=0: plain)
-    const char* pe = getenv("ADER_B200_PDL");
-    const bool pdl = !(pe && pe[0] == '0');
-    launch_chain(k_tc2<MODE_FWD>, dim3(nm * nc), dim3(NTHREADS), (size_t)smem_tc2(MODE_FWD), st, pdl, t, mp.rep, mp.e, mp.pt);
-    launch_chain(k_tc2<MODE_DREP>, dim3(nm * nc), dim3(NTHREADS), (size_t)smem_tc2(MODE_DREP), st, pdl, t, mp.rep, mp.e, mp.pt);
-    if (grad) launch_chain(k_tc2<MODE_DE>, dim3(nv), dim3(NTHREADS), (size_t)smem_tc2(MODE_DE), st, pdl, t, mp.rep, mp.e, mp.pt);
+                              // in the step: programmatic dependent launches along the chain
+    launch_chain(k_tc2<MODE_FWD>, dim3(nm * nc), dim3(NTHREADS), (size_t)smem_tc2(MODE_FWD), st, true, t, mp.rep, mp.e, mp.pt);
+    launch_chain(k_tc2<MODE_DREP>, dim3(nm * nc), dim3(NTHREADS), (size_t)smem_tc2(MODE_DREP), st, true, t, mp.rep, mp.e, mp.pt);
+    if (grad) launch_chain(k_tc2<MODE_DE>, dim3(nv), dim3(NTHREADS), (size_t)smem_tc2(MODE_DE), st, true, t, mp.rep, mp.e, mp.pt);
     ADER_CHECK_LAUNCH("tc kernels");
     return 0;
   }
@@ -960,51 +959,20 @@ extern "C" int32_t ader_debug_tc_timeline(long long* out) {
 #endif
 
 // ---- vocab-parallel variant (SURVEY 8e): this rank owns logits columns [v_lo, v_hi) ---------------------
-static int vp_teacher_cols(const AderLossArgs* a, int v_lo, int v_hi) {      // teacher columns inside this shard
-  if (!(a->n_ex > 0 && a->mode == 1)) return 0;
-  const int hi = a->V_prev < v_hi ? a->V_prev : v_hi;
-  return hi > v_lo ? hi - v_lo : 0;
-}
-static int vp_setup(const AderModel* m, const float* theta, const float* rep, const AderLossArgs* a, int v_lo, int v_hi,
-                    void* ws, cudaStream_t st, TcWs& w, TcArgs& t, bool pack, TcMaps& mp) {
-  const int d = m->d, M = a->M, Vl = v_hi - v_lo;
-  w = carve_tc(m, M, Vl, a->n_ex, vp_teacher_cols(a, v_lo, v_hi), (char*)ws);
-  const int nm = cdiv(M, TILE), nv = cdiv(Vl, TILE), nc = tc_chunks(nm, nv);
-  set_tc_attrs();
-  if (int e = make_tc_maps(w, nm, nv, mp)) return e;
-  if (pack) {
-    cudaMemsetAsync(w.err, 0, sizeof(int) * 4, st);
-    launch_pack(rep, d, M, d, nm, w.rep_tiles, st);
-    launch_pack(theta + (size_t)(1 + v_lo) * d, d, Vl, d, nv, w.e_tiles, st);
-  }
-  t.M = M; t.V = Vl; t.V_total = a->V; t.v_off = v_lo;
-  t.n_mtiles = nm; t.n_vtiles = nv; t.n_chunks = nc;
-  t.n_train = a->n_train; t.n_ex = a->n_ex; t.V_prev = a->V_prev; t.mode = a->n_ex > 0 ? a->mode : 0;
-  t.coef_train = a->n_train > 0 ? 1.0f / (float)(a->n_train_global > 0 ? a->n_train_global : a->n_train) : 0.f;
-  t.coef_ex = a->n_ex > 0 ? a->lambda_ / (float)(a->n_ex_global > 0 ? a->n_ex_global : a->n_ex) : 0.f;
-  t.pos = a->pos; t.ex_pos = a->ex_pos;
-  t.lse = w.lse; t.lse_t = w.lse_t; t.stats = w.stats; t.drep_part = w.drep_part; t.grad_table = nullptr;
-  t.d = d; t.err = w.err;
-  t.x0_t = w.x0_t; t.n_et = w.n_et; t.n_vtp = w.n_vtp; t.n_chunks_t = w.n_chunks_t; t.u_part = w.u_part;
-  t.pt_out = nullptr; t.t_row_lo = t.t_row_hi = 0;
-  if (pack && w.n_et > 0) launch_teacher_u(a, w, t, v_lo, rep, d, st, mp);
-  return 0;
-}
-
+// the arguments of ader_loss_fwd_bwd_tc except a frozen teacher, and a 128-aligned shard inside [0, V)
 static int vp_check(const AderModel* m, const AderLossArgs* a, int v_lo, int v_hi) {
   if (int e = check_model(m)) return e;
-  ADER_CHECK_ARG(a && a->M == a->n_train + a->n_ex && a->M > 0, "loss_tc_vp: bad row counts");
-  ADER_CHECK_ARG(a->V >= 1 && a->V < m->v_tab && a->mode >= 0 && a->mode <= 2, "loss_tc_vp: bad V / mode");
+  ADER_CHECK_ARG(a, "loss_tc_vp: NULL pointer");
+  ADER_CHECK_ARG(!a->teacher_rep, "loss_tc_vp: a frozen teacher (teacher_rep) is not supported by the vocab-parallel entries");
+  if (int e = check_loss_args(m, a, "loss_tc_vp", true)) return e;
   ADER_CHECK_ARG(v_lo >= 0 && v_lo < v_hi && v_hi <= a->V && v_lo % TILE == 0, "loss_tc_vp: shard [%d,%d) must be 128-aligned inside [0,%d)", v_lo, v_hi, a->V);
   ADER_CHECK_ARG(m->d <= KP, "loss_tc_vp: hidden_units too large");
-  ADER_CHECK_ARG(!a->teacher_rep, "loss_tc_vp: a frozen teacher (teacher_rep) is not supported by the vocab-parallel entries");
-  if (a->n_ex > 0 && a->mode == 1) ADER_CHECK_ARG(a->teacher && a->V_prev >= 1 && a->V_prev <= a->V, "loss_tc_vp: bad teacher");
   return 0;
 }
 
 extern "C" size_t ader_loss_tc_vp_ws_bytes(const AderModel* m, const AderLossArgs* a, int32_t v_lo, int32_t v_hi) {
   if (check_model(m) || !a || a->M <= 0 || v_hi <= v_lo || a->teacher_rep) return 0;
-  return carve_tc(m, a->M, v_hi - v_lo, a->n_ex, vp_teacher_cols(a, v_lo, v_hi), nullptr).bytes;
+  return carve_tc(a, v_lo, v_hi, nullptr).bytes;
 }
 
 extern "C" int32_t ader_loss_tc_vp_fwd(const AderModel* m, const float* theta, const float* rep, const AderLossArgs* a,
@@ -1012,8 +980,13 @@ extern "C" int32_t ader_loss_tc_vp_fwd(const AderModel* m, const float* theta, c
   if (int e = vp_check(m, a, v_lo, v_hi)) return e;
   ADER_CHECK_ARG(theta && rep && ws && stats, "loss_tc_vp_fwd: NULL pointer");
   cudaStream_t st = (cudaStream_t)stream;
+  const int d = m->d;
   TcWs w; TcArgs t; TcMaps mp;
-  if (int e = vp_setup(m, theta, rep, a, v_lo, v_hi, ws, st, w, t, true, mp)) return e;
+  if (int e = tc_plan(m, a, v_lo, v_hi, ws, nullptr, w, t, mp)) return e;
+  cudaMemsetAsync(w.err, 0, sizeof(int) * 4, st);
+  launch_pack(rep, d, a->M, d, t.n_mtiles, w.rep_tiles, st);
+  launch_pack(theta + (size_t)(1 + v_lo) * d, d, t.V, d, t.n_vtiles, w.e_tiles, st);
+  if (w.n_et > 0) launch_teacher_u(a, w, t, v_lo, rep, d, st, mp);
   k_tc2<MODE_FWD><<<t.n_mtiles * t.n_chunks, NTHREADS, smem_tc2(MODE_FWD), st>>>(t, mp.rep, mp.e, mp.pt);
   k_merge_stats<<<cdiv((long long)a->M * 32, 256), 256, 0, st>>>(w.stats, a->M, t.n_chunks * 2, a->n_train, t.mode, nullptr, nullptr, stats,
                                                  w.n_et > 0 ? w.udot : nullptr, w.x0_t, t.coef_ex);
@@ -1028,9 +1001,8 @@ extern "C" int32_t ader_loss_tc_vp_bwd(const AderModel* m, const float* theta, c
   ADER_CHECK_ARG(theta && rep && ws && lse, "loss_tc_vp_bwd: NULL pointer");
   cudaStream_t st = (cudaStream_t)stream;
   TcWs w; TcArgs t; TcMaps mp;
-  if (int e = vp_setup(m, theta, rep, a, v_lo, v_hi, ws, st, w, t, false, mp)) return e;     // operands were packed by the forward call
+  if (int e = tc_plan(m, a, v_lo, v_hi, ws, grad, w, t, mp)) return e;     // operands were packed by the forward call
   t.lse = lse;
-  t.grad_table = grad ? grad + (size_t)(1 + v_lo) * m->d : nullptr;
   if (d_rep_partial) {
     k_tc2<MODE_DREP><<<t.n_mtiles * t.n_chunks, NTHREADS, smem_tc2(MODE_DREP), st>>>(t, mp.rep, mp.e, mp.pt);
     k_reduce_drep<<<cdiv((long long)a->M * m->d, 256), 256, 0, st>>>(w.drep_part, t.n_chunks, t.n_mtiles * TILE, a->M, m->d, d_rep_partial,

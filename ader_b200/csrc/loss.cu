@@ -216,15 +216,7 @@ extern "C" int32_t ader_loss_fwd_bwd(const AderModel* m, const float* theta, con
                                      float* d_rep, float* grad, void* stream) {
   if (int e = check_model(m)) return e;
   ADER_CHECK_ARG(theta && rep && a && ws && loss && row_loss, "loss_fwd_bwd: NULL pointer");
-  ADER_CHECK_ARG(a->M == a->n_train + a->n_ex && a->M > 0, "loss_fwd_bwd: M (%d) != n_train + n_ex (%d + %d)", a->M, a->n_train, a->n_ex);
-  ADER_CHECK_ARG(a->V >= 1 && a->V < m->v_tab, "loss_fwd_bwd: max_item %d outside table of %d rows", a->V, m->v_tab);
-  ADER_CHECK_ARG(a->mode >= 0 && a->mode <= 2, "loss_fwd_bwd: bad mode %d", a->mode);
-  ADER_CHECK_ARG(a->n_train == 0 || a->pos, "loss_fwd_bwd: pos is NULL");
-  if (a->n_ex > 0) {
-    ADER_CHECK_ARG(a->mode != 0, "loss_fwd_bwd: exemplar rows given in vanilla mode");
-    if (a->mode == 1) { if (int e = check_teacher(a, "loss_fwd_bwd", false)) return e; }
-    if (a->mode == 2) ADER_CHECK_ARG(a->ex_pos, "loss_fwd_bwd: exemplar_pos is NULL");
-  }
+  if (int e = check_loss_args(m, a, "loss_fwd_bwd", false)) return e;
   cudaStream_t st = (cudaStream_t)stream;
   const int d = m->d, M = a->M, V = a->V;
   const long long ld = logits_ld(V);

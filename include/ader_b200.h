@@ -138,8 +138,8 @@ int32_t ader_debug_loss_tc_kernels(const AderModel* m, const float* theta, const
  *   fwd  -> stats [M,4] = this shard's per-row (max, sum exp(s - max), label logit or 0, KD dot);
  *           the caller all-reduces them (max; rescaled sum; sums) into lse [M];
  *   bwd  -> d_rep_partial [M,d] (to be all-reduce-summed) and grad rows v_lo+1 .. v_hi of the item table.
- * `a->V` stays the GLOBAL max_item.  The workspace must persist between the two calls.  Stored teacher logits only
- * (a frozen teacher is rejected). */
+ * `a->V` stays the GLOBAL max_item.  The workspace must persist between the two calls.  Both take the same argument
+ * checks as ader_loss_fwd_bwd_tc; stored teacher logits only (a frozen teacher is rejected). */
 size_t  ader_loss_tc_vp_ws_bytes(const AderModel* m, const AderLossArgs* a, int32_t v_lo, int32_t v_hi);
 int32_t ader_loss_tc_vp_fwd(const AderModel* m, const float* theta, const float* rep, const AderLossArgs* a,
                             int32_t v_lo, int32_t v_hi, void* ws, float* stats, void* stream);
