@@ -61,6 +61,7 @@ SIGNATURES = {
     "ader_param_count": (C.c_int64, [_MP]),
     "ader_param_offset": (C.c_int64, [_MP, C.c_int32]),
     "ader_dense_count": (C.c_int64, [_MP]),
+    "ader_path_check": (C.c_int32, [_MP, C.c_int32]),
     "ader_encoder_ws_bytes": (C.c_size_t, [_MP, C.c_int32, C.c_int32]),
     "ader_encoder_bwd_ws_bytes": (C.c_size_t, [_MP, C.c_int32, C.c_int32]),
     "ader_encoder_ws_slot": (C.c_int64, [_MP, C.c_int32, C.c_int32, C.c_int32, C.c_int32]),

@@ -58,6 +58,24 @@ static inline int check_model(const AderModel* m) {
   return 0;
 }
 
+// ---- shape limits of the kernel paths (ader_path_check) ----------------------------------------
+// The exact attention kernels (encoder.cu) hold one whole session row per CTA in shared memory: K^T and V^T
+// [d][LP] plus the row's queries (forward) or Q, K, dY and the [L][LP] score tiles (backward).
+constexpr int ATT_THREADS = 256, ATT_WARPS = 8;
+__host__ __device__ inline int att_lp(int L) { return (L + 3) / 4 * 4; }
+__host__ __device__ inline int al4(int x) { return (x + 3) & ~3; }
+constexpr size_t ATTN_FWD_SMEM_MAX = 200 * 1024, ATTN_BWD_SMEM_MAX = 220 * 1024;
+static inline size_t attn_fwd_smem(int d, int L) {
+  return sizeof(float) * (2 * (size_t)d * att_lp(L) + (size_t)al4(L * d) + ATT_WARPS * 256);
+}
+static inline size_t attn_bwd_smem(int d, int L) {
+  return sizeof(float) * (2 * (size_t)d * att_lp(L) + 3 * (size_t)al4(L * d) + 3 * (size_t)L * att_lp(L));
+}
+// widest model of the fused encoder, the tcgen05 loss / evaluation and the on-chip herding (operands padded to 160 columns)
+constexpr int PATH_TC_MAX_D = 160;
+// 0 if `path` (ADER_PATH_*) serves the (already checked) model, else -1; the message is set only when `report`
+int path_check(const AderModel* m, int path, bool report = true);
+
 // The fields of AderLossArgs (a != NULL), as every logits + CE + distillation entry takes them.  The teacher of a
 // distillation (mode 1) call is stored logits (`teacher`) or a frozen snapshot (`teacher_rep` + the table the entry reads:
 // fp32 rows for the exact entry, the bf16 shadow for the tcgen05 ones `tc`) -- exactly one of the two.

@@ -14,6 +14,7 @@ namespace ader {
 constexpr int NSLOT = 8;          // per-block [Tcap,d] activation slots
 constexpr int SPLITS = 21;        // split-K partials for weight / LN / bias gradients (21 x 7 problems = 147 CTAs: one wave of 148 SMs)
 constexpr int PG_LANES = 6;       // token lanes per column in the LN / position gradient reductions (160 x 6 = 960 threads)
+constexpr int PG_LANES_WIDE = 4;  // the same for hidden_units > 160 (256 x 4 = 1024 threads)
 
 // workspace flag words: packing / overflow flags.  k_row_len (first kernel of every forward) zeroes them.
 constexpr int N_WS_FLAGS = 4;
@@ -329,15 +330,16 @@ __global__ void k_lnf_bwd_drep(const DrepFuse df, float* d_rep, const float* __r
 // partial LN parameter gradients: dbeta[c] = sum_t dout[t,c]; dgamma[c] = sum_t dout[t,c]*xhat[t,c]
 // split s sums tokens [s*chunk, (s+1)*chunk) sequentially -> deterministic.
 // rows != nullptr: "last token" mode (dout indexed by row, x by last token of the row, count = M).
+template <int LANES>
 __global__ void k_ln_param_grad(const float* __restrict__ dout, const float* __restrict__ x,
                                 const float* __restrict__ mean, const float* __restrict__ rstd,
                                 const int* __restrict__ dT, int count_host,
                                 const int* __restrict__ row_len, const int* __restrict__ row_off,
                                 int d, float* __restrict__ pbeta, float* __restrict__ pgamma,
                                 long long split_stride) {
-  // blockDim = (ceil32(d), PG_LANES): thread (c, k) sums tokens lo+k, lo+k+PG_LANES, ... ; the
-  // PG_LANES partial sums are then added in lane order -> deterministic.
-  __shared__ float sb_s[PG_LANES][256], sg_s[PG_LANES][256];
+  // blockDim = (ceil32(d), LANES): thread (c, k) sums tokens lo+k, lo+k+LANES, ... ; the
+  // LANES partial sums are then added in lane order -> deterministic.
+  __shared__ float sb_s[LANES][256], sg_s[LANES][256];
   const int c = threadIdx.x, k = threadIdx.y;
   const int s = blockIdx.x;
   const int count = row_off ? count_host : *dT;
@@ -345,7 +347,7 @@ __global__ void k_ln_param_grad(const float* __restrict__ dout, const float* __r
   const int lo = s * chunk, hi = min(count, lo + chunk);
   float sb = 0.f, sg = 0.f;
   if (c < d) {
-    for (int i = lo + k; i < hi; i += PG_LANES) {
+    for (int i = lo + k; i < hi; i += LANES) {
       long long xo, go; float mu, rs;
       if (row_off) {
         if (row_len[i] == 0) continue;
@@ -360,7 +362,7 @@ __global__ void k_ln_param_grad(const float* __restrict__ dout, const float* __r
   if (k == 0 && c < d) {
     float tb = 0.f, tg = 0.f;
 #pragma unroll
-    for (int q = 0; q < PG_LANES; ++q) { tb += sb_s[q][c]; tg += sg_s[q][c]; }
+    for (int q = 0; q < LANES; ++q) { tb += sb_s[q][c]; tg += sg_s[q][c]; }
     pbeta[(long long)s * split_stride + c] = tb;
     pgamma[(long long)s * split_stride + c] = tg;
   }
@@ -404,9 +406,7 @@ __device__ __forceinline__ void stage_rows_t(const float* __restrict__ src, floa
 // Attention kernels: one CTA (8 warps) per session row.  A warp owns a block of 4 queries (or 4 keys in
 // the transposed products); operands are staged so that the per-k inner step is one conflict-free LDS
 // (lanes over keys / features) + one broadcast LDS.128 (the 4 queries) feeding 4 independent FMA chains.
-constexpr int ATT_THREADS = 256, ATT_WARPS = 8;
-__host__ __device__ inline int att_lp(int L) { return (L + 3) / 4 * 4; }
-__host__ __device__ inline int al4(int x) { return (x + 3) & ~3; }
+// Tile sizes and shared-memory budgets: common.cuh (attn_fwd_smem / attn_bwd_smem).
 
 __global__ void __launch_bounds__(ATT_THREADS) k_attn_fwd(const float* __restrict__ Q, const float* __restrict__ K,
                                                           const float* __restrict__ V, const float* __restrict__ Q1,
@@ -679,24 +679,25 @@ __global__ void k_reduce_partials(const float* __restrict__ partial, long long s
 }
 
 // position-table gradient: dP[p,c] = sum over rows having position p of dx0[token(r,p), c]
+template <int LANES>
 __global__ void k_pos_grad(const float* __restrict__ gx, const int* __restrict__ row_len,
                            const int* __restrict__ row_off, int M, int L, int d,
                            float drop_p, uint64_t seed0, const int* __restrict__ d_step, float* __restrict__ gpos,
                            long long split_stride) {
   const uint64_t seed = seed0 + (d_step ? (uint64_t)(uint32_t)__ldg(d_step) : 0ull);
   // grid (L, splits): CTA (p, s) sums the rows of chunk s that have position p into partial slot s.
-  // blockDim = (ceil32(d), PG_LANES): thread (c, k) sums rows lo+k, lo+k+PG_LANES, ...; lanes reduced in fixed order.
+  // blockDim = (ceil32(d), LANES): thread (c, k) sums rows lo+k, lo+k+LANES, ...; lanes reduced in fixed order.
   // (Round 2 tried eight rows per trip and ten positions per CTA with the row lengths fetched once: 23 us and 34 us in the
   // step against 16-19 us for this form -- the tail kernels run beside the last weight-gradient CTAs, and what a variant
   // gains in dependent trips it loses to registers / shared memory that no longer fit beside them.)
-  __shared__ float part[PG_LANES][256];
+  __shared__ float part[LANES][256];
   const int p = blockIdx.x, c = threadIdx.x, k = threadIdx.y;
   const int chunk = (M + gridDim.y - 1) / gridDim.y;
   const int lo = blockIdx.y * chunk, hi = min(M, lo + chunk);
   gpos += (long long)blockIdx.y * split_stride;
   float s = 0.f;
   if (c < d) {
-    for (int r = lo + k; r < hi; r += PG_LANES) {
+    for (int r = lo + k; r < hi; r += LANES) {
       int n = row_len[r];
       if (n >= L - p) {
         long long e = (long long)(row_off[r] + p - (L - n)) * d + c;
@@ -711,9 +712,23 @@ __global__ void k_pos_grad(const float* __restrict__ gx, const int* __restrict__
   if (k == 0 && c < d) {
     float t = 0.f;
 #pragma unroll
-    for (int q = 0; q < PG_LANES; ++q) t += part[q][c];
+    for (int q = 0; q < LANES; ++q) t += part[q][c];
     gpos[p * d + c] = t;
   }
+}
+
+// block (ceil32(d) columns, token lanes) of the two reductions above: PG_LANES lanes up to d = 160, PG_LANES_WIDE above
+template <typename... Args>
+static void launch_ln_param_grad(dim3 grid, int d, cudaStream_t st, Args... args) {
+  const int cols = ((d + 31) / 32) * 32;
+  if (cols * PG_LANES <= 1024) k_ln_param_grad<PG_LANES><<<grid, dim3(cols, PG_LANES), 0, st>>>(args...);
+  else k_ln_param_grad<PG_LANES_WIDE><<<grid, dim3(cols, PG_LANES_WIDE), 0, st>>>(args...);
+}
+template <typename... Args>
+static void launch_pos_grad(dim3 grid, int d, cudaStream_t st, Args... args) {
+  const int cols = ((d + 31) / 32) * 32;
+  if (cols * PG_LANES <= 1024) k_pos_grad<PG_LANES><<<grid, dim3(cols, PG_LANES), 0, st>>>(args...);
+  else k_pos_grad<PG_LANES_WIDE><<<grid, dim3(cols, PG_LANES_WIDE), 0, st>>>(args...);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1005,9 +1020,8 @@ static int run_embedding_grads(const AderModel* m, const Layout& l, const EncWs&
   const int d = m->d, L = m->maxlen;
   const int* dT = w.row_off + M;
   const long long PS = l.dense_count();
-  const int ln_threads = ((d + 31) / 32) * 32;
   // position table (ADER.py:41-52): per-row-chunk partials into the first L*d entries of the split slots
-  k_pos_grad<<<dim3(L, SPLITS), dim3(ln_threads, PG_LANES), 0, st>>>(gX, w.row_len, w.row_off, M, L, d, p, seed, d_step, g.partial, PS);
+  launch_pos_grad(dim3(L, SPLITS), d, st, gX, w.row_len, w.row_off, M, L, d, p, seed, d_step, g.partial, PS);
   // dense parameter gradients (position table included): reduce the split partials in fixed order
   k_reduce_partials<<<cdiv(PS, 256), 256, 0, st>>>(g.partial, PS, SPLITS, 0, PS, grad + l.off_pos);
   return run_table_scatter(m, l, w, g, gX, M, Tcap, grad, st);
@@ -1088,6 +1102,7 @@ extern "C" int32_t ader_encoder_fwd(const AderModel* m, const float* theta, cons
                                     int32_t Tcap, void* ws, float* rep, float dropout_rate, uint64_t seed,
                                     void* stream) {
   if (int e = check_model(m)) return e;
+  if (int e = path_check(m, ADER_PATH_ENCODER_FWD)) return e;
   ADER_CHECK_ARG(theta && ids && ws && rep, "encoder_fwd: NULL pointer");
   ADER_CHECK_ARG(M > 0 && Tcap > 0 && (long long)Tcap <= (long long)M * m->maxlen, "encoder_fwd: bad M/Tcap (%d, %d)", M, Tcap);
   ADER_CHECK_ARG(dropout_rate >= 0.f && dropout_rate < 1.f, "encoder_fwd: dropout_rate out of range");
@@ -1103,13 +1118,12 @@ extern "C" int32_t ader_encoder_fwd(const AderModel* m, const float* theta, cons
                                                            dropout_rate, seed, w.slot[0][0]);
   ADER_CHECK_LAUNCH("encoder_fwd/pack+embed");
 
-  const size_t attn_smem = sizeof(float) * (2 * (size_t)d * att_lp(L) + (size_t)al4(L * d) + ATT_WARPS * 256);
+  const size_t attn_smem = attn_fwd_smem(d, L);
   static bool attr_set = false;
   if (!attr_set) {
-    cudaFuncSetAttribute(k_attn_fwd, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    cudaFuncSetAttribute(k_attn_fwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ATTN_FWD_SMEM_MAX);
     attr_set = true;
   }
-  ADER_CHECK_ARG(attn_smem <= 200 * 1024, "encoder_fwd: attention tile does not fit shared memory");
   const int ln_grid = cdiv((long long)Tcap * 32, 256);
 
   for (int b = 0; b < m->num_blocks; ++b) {
@@ -1391,6 +1405,7 @@ extern "C" int32_t ader_encoder_bwd(const AderModel* m, const float* theta, cons
                                     int32_t Tcap, const void* ws, void* bwd_ws, const float* d_rep, float* grad,
                                     float dropout_rate, uint64_t seed, void* stream) {
   if (int e = check_model(m)) return e;
+  if (int e = path_check(m, ADER_PATH_ENCODER_BWD)) return e;
   ADER_CHECK_ARG(theta && ids && ws && bwd_ws && d_rep && grad, "encoder_bwd: NULL pointer");
   ADER_CHECK_ARG(M > 0 && Tcap > 0, "encoder_bwd: bad M/Tcap");
   return enc_bwd_exact(m, theta, ids, M, Tcap, ws, bwd_ws, d_rep, grad, dropout_rate, seed, (cudaStream_t)stream, nullptr);
@@ -1411,21 +1426,19 @@ static int enc_bwd_exact(const AderModel* m, const float* theta, const int32_t* 
         *gQ = g.g[6], *gK = g.g[7], *gV = g.g[8], *gQ1 = g.g[9];
   const int ln_grid = cdiv((long long)Tcap * 32, 256);
   const int el_grid = cdiv((long long)Tcap * d, 256);
-  const int ln_threads = ((d + 31) / 32) * 32;
 
-  const size_t attn_smem = sizeof(float) * (2 * (size_t)d * att_lp(L) + 3 * (size_t)al4(L * d) + 3 * (size_t)L * att_lp(L));
+  const size_t attn_smem = attn_bwd_smem(d, L);      // within ATTN_BWD_SMEM_MAX: the entries ran path_check
   static bool attr_set = false;
   if (!attr_set) {
-    cudaFuncSetAttribute(k_attn_bwd, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024);
+    cudaFuncSetAttribute(k_attn_bwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ATTN_BWD_SMEM_MAX);
     attr_set = true;
   }
-  ADER_CHECK_ARG(attn_smem <= 220 * 1024, "encoder_bwd: attention tile does not fit shared memory");
 
   // final LayerNorm (ADER.py:82): only the last token of each row carries gradient
   k_lnf_bwd<<<ln_grid, 256, 0, st>>>(d_rep, w.xfinal, w.meanf, w.rstdf, theta + l.off_lnf + d, w.tok_row, w.row_off, gX, dT, d);
   if (fh) k_fisher_ln<<<1, 160, 0, st>>>(d_rep, w.xfinal, w.meanf, w.rstdf, w.tok_row, dT, M, w.row_len, w.row_off, d,
                                          fh->acc + l.off_lnf, fh->acc + l.off_lnf + d);
-  else k_ln_param_grad<<<SPLITS, dim3(ln_threads, PG_LANES), 0, st>>>(d_rep, w.xfinal, w.meanf, w.rstdf, dT, M, w.row_len, w.row_off, d,
+  else launch_ln_param_grad(dim3(SPLITS), d, st, d_rep, w.xfinal, w.meanf, w.rstdf, dT, M, w.row_len, w.row_off, d,
                                                  part(l.off_lnf), part(l.off_lnf + d), PS);
   ADER_CHECK_LAUNCH("encoder_bwd/final_ln");
 
@@ -1454,7 +1467,7 @@ static int enc_bwd_exact(const AderModel* m, const float* theta, const int32_t* 
     k_ln_bwd<<<ln_grid, 256, 0, st>>>(gZ, Y, w.mean2[b], w.rstd2[b], P + l.ln2g, gY, dT, d, 0);
     if (fh) k_fisher_ln<<<1, 160, 0, st>>>(gZ, Y, w.mean2[b], w.rstd2[b], w.tok_row, dT, 0, nullptr, nullptr, d,
                                            fh->acc + bo + l.ln2b, fh->acc + bo + l.ln2g);
-    else k_ln_param_grad<<<SPLITS, dim3(ln_threads, PG_LANES), 0, st>>>(gZ, Y, w.mean2[b], w.rstd2[b], dT, 0, nullptr, nullptr, d,
+    else launch_ln_param_grad(dim3(SPLITS), d, st, gZ, Y, w.mean2[b], w.rstd2[b], dT, 0, nullptr, nullptr, d,
                                                    part(bo + l.ln2b), part(bo + l.ln2g), PS);
     k_attn_bwd<<<M, ATT_THREADS, attn_smem, st>>>(Qp, Kp, Vp, w.probs[b], gY, w.row_len, w.row_off, d, m->num_heads, L, Tcap,
                                           p, seed, 1u + 3u * b, gQ, gK, gV);
@@ -1475,7 +1488,7 @@ static int enc_bwd_exact(const AderModel* m, const float* theta, const int32_t* 
     k_ln_bwd<<<ln_grid, 256, 0, st>>>(gQ1, X, w.mean1[b], w.rstd1[b], P + l.ln1g, gXin, dT, d, 1);
     if (fh) k_fisher_ln<<<1, 160, 0, st>>>(gQ1, X, w.mean1[b], w.rstd1[b], w.tok_row, dT, 0, nullptr, nullptr, d,
                                            fh->acc + bo + l.ln1b, fh->acc + bo + l.ln1g);
-    else k_ln_param_grad<<<SPLITS, dim3(ln_threads, PG_LANES), 0, st>>>(gQ1, X, w.mean1[b], w.rstd1[b], dT, 0, nullptr, nullptr, d,
+    else launch_ln_param_grad(dim3(SPLITS), d, st, gQ1, X, w.mean1[b], w.rstd1[b], dT, 0, nullptr, nullptr, d,
                                                    part(bo + l.ln1b), part(bo + l.ln1g), PS);
     ADER_CHECK_LAUNCH("encoder_bwd/block");
     float* t = gX; gX = gXin; gXin = t;
@@ -1494,7 +1507,7 @@ static int enc_bwd_exact(const AderModel* m, const float* theta, const int32_t* 
 constexpr int FISHER_CHUNK = 256;
 static long long fisher_ld(int V) { return ((long long)V + 3) / 4 * 4; }
 extern "C" size_t ader_fisher_batched_ws_bytes(const AderModel* m, int32_t S, int32_t V) {
-  if (check_model(m) || S <= 0 || V <= 0 || m->d > 160) return 0;
+  if (check_model(m) || S <= 0 || V <= 0 || path_check(m, ADER_PATH_FISHER_BATCHED)) return 0;
   return 2 * align_up(sizeof(float) * (size_t)S * m->d) + align_up(sizeof(float) * (size_t)S) +
          align_up(sizeof(float) * (size_t)FISHER_CHUNK * fisher_ld(V));
 }
@@ -1502,9 +1515,9 @@ extern "C" size_t ader_fisher_batched_ws_bytes(const AderModel* m, int32_t S, in
 extern "C" int32_t ader_fisher_batched(const AderModel* m, const float* theta, const int32_t* ids, const int32_t* pos, int32_t S,
                                        int32_t Tcap, int32_t V, void* enc_ws, void* bwd_ws, void* ws, double* acc, void* stream) {
   if (int e = check_model(m)) return e;
+  if (int e = path_check(m, ADER_PATH_FISHER_BATCHED)) return e;
   ADER_CHECK_ARG(theta && ids && pos && enc_ws && bwd_ws && ws && acc, "fisher_batched: NULL pointer");
   ADER_CHECK_ARG(S > 0 && Tcap > 0 && V >= 1 && V < m->v_tab, "fisher_batched: bad sizes");
-  ADER_CHECK_ARG(m->d <= 160, "fisher_batched: hidden_units must be <= 160");
   cudaStream_t st = (cudaStream_t)stream;
   const int d = m->d;
   const Layout l = make_layout(m);
@@ -1539,11 +1552,7 @@ extern "C" int32_t ader_fisher_batched(const AderModel* m, const float* theta, c
 // fused tensor-core path (encoder_fused.cuh): same contract, same workspace slots
 // ------------------------------------------------------------------------------------------
 namespace ader {
-static int fused_check(const AderModel* m) {
-  if (m->d > fz::KP) return fail(-1, "fused encoder path needs hidden_units <= %d (got %d): use the exact path", fz::KP, m->d);
-  if (m->maxlen > 64) return fail(-1, "fused encoder path needs maxlen <= 64");
-  return 0;
-}
+static_assert(PATH_TC_MAX_D == fz::KP, "the fused encoder pads features to KP columns");
 static int sm_count() {
   static int n = 0;
   if (!n) { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev); if (n <= 0) n = 148; }
@@ -1583,7 +1592,7 @@ extern "C" int32_t ader_encoder_fwd_tc(const AderModel* m, const float* theta, c
 int ader::enc_fwd_tc_run(const AderModel* m, const float* theta, const int32_t* ids, int M, int Tcap, void* ws, float* rep,
                          float dropout_rate, uint64_t seed, const int32_t* d_step, Fork& f) {
   if (int e = check_model(m)) return e;
-  if (int e = fused_check(m)) return e;
+  if (int e = path_check(m, ADER_PATH_ENCODER_TC)) return e;
   ADER_CHECK_ARG(theta && ids && ws && rep, "encoder_fwd_tc: NULL pointer");
   ADER_CHECK_ARG(M > 0 && Tcap > 0 && (long long)Tcap <= (long long)M * m->maxlen, "encoder_fwd_tc: bad M/Tcap (%d, %d)", M, Tcap);
   ADER_CHECK_ARG(dropout_rate >= 0.f && dropout_rate < 1.f, "encoder_fwd_tc: dropout_rate out of range");
@@ -1672,7 +1681,7 @@ extern "C" int32_t ader_encoder_bwd_tc(const AderModel* m, const float* theta, c
 int ader::enc_bwd_tc_run(const AderModel* m, const float* theta, const int32_t* ids, int M, int Tcap, const void* ws, void* bwd_ws,
                          const float* d_rep, float* grad, float dropout_rate, uint64_t seed, const int32_t* d_step, Fork& f) {
   if (int e = check_model(m)) return e;
-  if (int e = fused_check(m)) return e;
+  if (int e = path_check(m, ADER_PATH_ENCODER_TC)) return e;
   ADER_CHECK_ARG(theta && ids && ws && bwd_ws && d_rep && grad, "encoder_bwd_tc: NULL pointer");
   ADER_CHECK_ARG(M > 0 && Tcap > 0, "encoder_bwd_tc: bad M/Tcap");
   cudaStream_t st = f.main;
@@ -1694,7 +1703,7 @@ int ader::enc_bwd_tc_run(const AderModel* m, const float* theta, const int32_t* 
   // final LayerNorm: data gradient on the chain, parameter gradient beside it
   auto ln_params = [&] {
     f.edge(st, f.c);
-    k_ln_param_grad<<<SPLITS, dim3(ln_threads, PG_LANES), 0, f.c>>>(d_rep, w.xfinal, w.meanf, w.rstdf, dT, M, w.row_len, w.row_off, d,
+    k_ln_param_grad<PG_LANES><<<SPLITS, dim3(ln_threads, PG_LANES), 0, f.c>>>(d_rep, w.xfinal, w.meanf, w.rstdf, dT, M, w.row_len, w.row_off, d,
                                                    part(l.off_lnf), part(l.off_lnf + d), PS);
   };
   if (f.has_drep) {                           // the loss group left the d_rep reduction to the kernel below
@@ -1788,7 +1797,7 @@ int ader::enc_bwd_tc_run(const AderModel* m, const float* theta, const int32_t* 
   }
   // position table (ADER.py:41-52) beside the scatter; then all split partials -> dense gradients in fixed order
   if (chain_end) cudaStreamWaitEvent(f.c, chain_end, 0);
-  k_pos_grad<<<dim3(L, SPLITS), dim3(ln_threads, PG_LANES), 0, f.c>>>(gX0, w.row_len, w.row_off, M, L, d, 0.f, 0, nullptr, g.partial, PS);
+  k_pos_grad<PG_LANES><<<dim3(L, SPLITS), dim3(ln_threads, PG_LANES), 0, f.c>>>(gX0, w.row_len, w.row_off, M, L, d, 0.f, 0, nullptr, g.partial, PS);
   f.edge(f.c, f.a);
   f.edge(f.wg[1], f.a);
   f.edge(f.wg[2], f.a);

@@ -31,6 +31,7 @@ using namespace ader::tc;
 
 constexpr int D2 = 320;                 // hi | lo columns of the operand matrices
 constexpr int HALF = 160;               // column of lo[0]
+static_assert(HALF == PATH_TC_MAX_D, "ADER_PATH_EVAL_TC: rows of d <= HALF columns");
 constexpr int NREG = 5;
 constexpr int XREG = 128 * 128, YREG = 64 * 128;
 constexpr int XBYTES = NREG * XREG, YBYTES = NREG * YREG;
@@ -505,16 +506,16 @@ static int topk_tc_run(const AderModel* m, const float* theta, const float* rep,
 }
 
 extern "C" size_t ader_eval_rank_tc_ws_bytes(const AderModel* m, int32_t R, int32_t V) {
-  if (check_model(m) || R <= 0 || V <= 0 || m->d > HALF) return 0;
+  if (check_model(m) || R <= 0 || V <= 0 || path_check(m, ADER_PATH_EVAL_TC)) return 0;
   return carve(R, V, false, nullptr).bytes;
 }
 
 extern "C" int32_t ader_eval_rank_tc(const AderModel* m, const float* theta, const float* rep, const int32_t* gt, int32_t R,
                                      int32_t V, void* ws, int32_t* rank, int32_t* overflow, void* stream) {
   if (int e = check_model(m)) return e;
+  if (int e = path_check(m, ADER_PATH_EVAL_TC)) return e;
   ADER_CHECK_ARG(theta && rep && gt && ws && rank && overflow, "eval_rank_tc: NULL pointer");
   ADER_CHECK_ARG(R > 0 && V >= 1 && V < m->v_tab, "eval_rank_tc: bad sizes");
-  ADER_CHECK_ARG(m->d <= HALF, "eval_rank_tc: hidden_units must be <= %d", HALF);
   return topk_tc_run(m, theta, rep, gt, nullptr, R, V, 0, ws, rank, nullptr, nullptr, overflow, (cudaStream_t)stream);
 }
 
@@ -527,16 +528,16 @@ extern "C" int32_t ader_eval_rank_topk_tc(const AderModel* m, const float* theta
                                           int32_t V, int32_t k, void* ws, int32_t* rank, int32_t* topk_item, float* topk_score,
                                           int32_t* overflow, void* stream) {
   if (int e = check_model(m)) return e;
+  if (int e = path_check(m, ADER_PATH_EVAL_TC)) return e;
   ADER_CHECK_ARG(theta && rep && gt && ws && rank && overflow && topk_item && topk_score, "eval_rank_topk_tc: NULL pointer");
   ADER_CHECK_ARG(R > 0 && V >= 1 && V < m->v_tab && k >= 1 && k <= 32, "eval_rank_topk_tc: bad sizes");
-  ADER_CHECK_ARG(m->d <= HALF, "eval_rank_topk_tc: hidden_units must be <= %d", HALF);
   const int nc = eval_chunks(R, V);
   ADER_CHECK_ARG(2 * nc >= k && 2 * nc <= 256, "eval_rank_tc: top-%d needs %d..128 vocabulary chunks per row tile (have %d): use ader_eval_rank_topk", k, (k + 1) / 2, nc);
   return topk_tc_run(m, theta, rep, gt, nullptr, R, V, k, ws, rank, topk_item, topk_score, overflow, (cudaStream_t)stream);
 }
 
 extern "C" size_t ader_recommend_tc_ws_bytes(const AderModel* m, int32_t R, int32_t V) {
-  if (check_model(m) || R <= 0 || V <= 0 || m->d > HALF) return 0;
+  if (check_model(m) || R <= 0 || V <= 0 || path_check(m, ADER_PATH_EVAL_TC)) return 0;
   return carve(R, V, true, nullptr).bytes;
 }
 
@@ -544,9 +545,9 @@ extern "C" int32_t ader_recommend_topk_tc(const AderModel* m, const float* theta
                                           int32_t V, int32_t k, void* ws, int32_t* topk_item, float* topk_score,
                                           int32_t* overflow, void* stream) {
   if (int e = check_model(m)) return e;
+  if (int e = path_check(m, ADER_PATH_EVAL_TC)) return e;
   ADER_CHECK_ARG(theta && rep && ws && topk_item && topk_score && overflow, "recommend_topk_tc: NULL pointer");
   ADER_CHECK_ARG(R > 0 && V >= 1 && V < m->v_tab && k >= 1 && k <= 100, "recommend_topk_tc: bad sizes");
-  ADER_CHECK_ARG(m->d <= HALF, "recommend_topk_tc: hidden_units must be <= %d", HALF);
   const int nc = eval_chunks(R, V);
   ADER_CHECK_ARG(2 * nc * 8 >= k, "recommend_topk_tc: top-%d needs %d vocabulary chunks per row tile (have %d): use ader_recommend_topk",
                  k, (k + 15) / 16, nc);

@@ -377,10 +377,13 @@ k_herding_big(const float* __restrict__ rep, int d, const int* __restrict__ cand
 
 using namespace ader;
 
+// Dn: rows of stride 160 (spill of k_herding_big) or d (k_herding, the only form of hidden_units > 160)
+static size_t dn_floats(const AderModel* m, int32_t N) { return (size_t)N * (m->d > 160 ? m->d : 160); }
+
 extern "C" size_t ader_herding_ws_bytes(const AderModel* m, int32_t N) {
   if (check_model(m) || N <= 0) return 0;
-  // [Dn fp32 N x d (global-memory fallback for segments > 2800)] [selected N] [class lists 4 x N] [counters]
-  return align_up(sizeof(float) * (size_t)N * 160) + align_up(sizeof(int) * (size_t)N) + 4 * align_up(sizeof(int) * (size_t)N) + 256;
+  // [Dn fp32 (global-memory fallback for segments > 2800)] [selected N] [class lists 4 x N] [counters]
+  return align_up(sizeof(float) * dn_floats(m, N)) + align_up(sizeof(int) * (size_t)N) + 4 * align_up(sizeof(int) * (size_t)N) + 256;
 }
 
 extern "C" int32_t ader_herding_segmented(const AderModel* m, const float* rep, int32_t N, const int32_t* cand,
@@ -393,13 +396,13 @@ extern "C" int32_t ader_herding_segmented(const AderModel* m, const float* rep, 
   cudaStream_t st = (cudaStream_t)stream;
   char* base = (char*)ws; size_t o = 0;
   auto take = [&](size_t n) { char* p = base + o; o += align_up(n); return p; };
-  float* Dn = (float*)take(sizeof(float) * (size_t)N * 160);
+  float* Dn = (float*)take(sizeof(float) * dn_floats(m, N));
   int* selected = (int*)take(sizeof(int) * (size_t)N);
   int* lists[4];
   for (int k = 0; k < 4; ++k) lists[k] = (int*)take(sizeof(int) * (size_t)N);
   int* cnt = (int*)take(256);
   static const bool v1 = [] { const char* e = getenv("ADER_B200_HERDING"); return e && e[0] == '1'; }();
-  if (v1 || m->d > 160) {                          // first generation: CTA per segment, D in global memory
+  if (v1 || path_check(m, ADER_PATH_HERDING_ONCHIP, false)) {   // first generation: CTA per segment, D in global memory
     k_herding<<<n_seg, 256, 0, st>>>(rep, m->d, cand, seg_off, quota, max_steps, Dn, selected, picks, n_picked, nullptr, nullptr);
     ADER_CHECK_LAUNCH("herding");
     return 0;

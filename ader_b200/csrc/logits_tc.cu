@@ -43,6 +43,7 @@ namespace tc {
 
 constexpr int TILE = 128;
 constexpr int KP = 160;                       // padded feature dim
+static_assert(KP == PATH_TC_MAX_D, "ADER_PATH_LOSS_TC: rows of d <= KP columns");
 constexpr int TILE_BYTES = TILE * KP * 2;     // 40960: one 128-row tile of an operand matrix in HBM
 constexpr int DS_BYTES = TILE * TILE * 2;     // 32768: one 128 x 128 tile of the teacher-probability matrix in HBM
 constexpr int KSTEPS1 = KP / 16;              // 10 MMAs per S tile
@@ -775,7 +776,7 @@ extern "C" size_t ader_loss_tc_ws_bytes(const AderModel* m, const AderLossArgs* 
 }
 
 extern "C" size_t ader_table16_ws_bytes(const AderModel* m, int32_t V) {
-  if (check_model(m) || V <= 0 || m->d > KP) return 0;
+  if (check_model(m) || V <= 0 || path_check(m, ADER_PATH_LOSS_TC)) return 0;
   return (size_t)cdiv(V, TILE) * TILE * ROW16 * 2;
 }
 
@@ -890,9 +891,9 @@ extern "C" int32_t ader_debug_loss_tc_kernels(const AderModel* m, const float* t
 int ader::loss_tc_run(const AderModel* m, const float* theta, const float* rep, const AderLossArgs* a, void* ws, float* loss,
                       float* row_loss, float* d_rep, float* grad, Fork& f, int phase_mask) {
   if (int e = check_model(m)) return e;
+  if (int e = path_check(m, ADER_PATH_LOSS_TC)) return e;
   ADER_CHECK_ARG(theta && a && ws, "loss_fwd_bwd_tc: NULL pointer");
   ADER_CHECK_ARG(!(phase_mask & 2) || (rep && loss && row_loss), "loss_fwd_bwd_tc: NULL pointer");
-  ADER_CHECK_ARG(m->d <= KP && m->d % 2 == 0, "loss_fwd_bwd_tc: hidden_units must be <= %d", KP);
   if (int e = check_loss_args(m, a, "loss_fwd_bwd_tc", true)) return e;
   cudaStream_t st = f.main, sb = f.b;
   const int d = m->d, M = a->M, V = a->V;
@@ -962,11 +963,11 @@ extern "C" int32_t ader_debug_tc_timeline(long long* out) {
 // the arguments of ader_loss_fwd_bwd_tc except a frozen teacher, and a 128-aligned shard inside [0, V)
 static int vp_check(const AderModel* m, const AderLossArgs* a, int v_lo, int v_hi) {
   if (int e = check_model(m)) return e;
+  if (int e = path_check(m, ADER_PATH_LOSS_TC)) return e;
   ADER_CHECK_ARG(a, "loss_tc_vp: NULL pointer");
   ADER_CHECK_ARG(!a->teacher_rep, "loss_tc_vp: a frozen teacher (teacher_rep) is not supported by the vocab-parallel entries");
   if (int e = check_loss_args(m, a, "loss_tc_vp", true)) return e;
   ADER_CHECK_ARG(v_lo >= 0 && v_lo < v_hi && v_hi <= a->V && v_lo % TILE == 0, "loss_tc_vp: shard [%d,%d) must be 128-aligned inside [0,%d)", v_lo, v_hi, a->V);
-  ADER_CHECK_ARG(m->d <= KP, "loss_tc_vp: hidden_units too large");
   return 0;
 }
 
@@ -1015,9 +1016,9 @@ extern "C" int32_t ader_loss_tc_vp_bwd(const AderModel* m, const float* theta, c
 
 extern "C" int32_t ader_pack_table16(const AderModel* m, const float* rows, int32_t V, void* out, void* stream) {
   if (int e = check_model(m)) return e;
+  if (int e = path_check(m, ADER_PATH_LOSS_TC)) return e;
   ADER_CHECK_ARG(rows && out, "pack_table16: NULL pointer");
   ADER_CHECK_ARG(V >= 1 && V < m->v_tab, "pack_table16: V=%d outside the table of %d rows", V, m->v_tab);
-  ADER_CHECK_ARG(m->d <= KP, "pack_table16: hidden_units must be <= %d", KP);
   const long long rows_pad = (long long)cdiv(V, TILE) * TILE;
   k_pack_rows16<<<cdiv(rows_pad * (ROW16 / 8), 256), 256, 0, (cudaStream_t)stream>>>(rows, m->d, V, m->d, (int)rows_pad,
                                                                                      reinterpret_cast<__nv_bfloat16*>(out), nullptr);

@@ -267,7 +267,7 @@ class FrozenTeacher:
         self._rows = model.theta[:(self.width + 1) * d].clone()
         self.table = self._rows[d:].view(self.width, d)
         self.table16 = None
-        if d <= 160:
+        if ops.path_check(model.ms, ops.PATH_LOSS_TC) is None:
             self.table16 = torch.empty(ops.table16_bytes(model.ms, self.width), dtype=torch.uint8, device=model.device)
             ops.pack_table16(model.ms, self.table, self.width, self.table16)
 

@@ -448,6 +448,7 @@ def run(args) -> dict:
         raise ValueError("Invalid dataset name")
     args.dropout_rate = 0 if (args.ewc or args.finetune) else args.dropout_rate      # main.py:141
     model = Ader(item_num, args) if not args.ewc else Ewc(item_num, args)
+    model.check_trainable()                                    # a shape no training path serves fails here, not at step 1
     dp = None
     if args.dp_world > 1:
         from .dist import make_comm

@@ -82,8 +82,16 @@ class Ader:
         # how a tc + tc training pass is issued: "dag" = ader_train_fwd_bwd_tc (fork/join over side streams),
         # "serial" = the same entry on one stream, "groups" = the three single-group entry points one after another
         self.step_impl = getattr(args, "step_impl", None) or os.environ.get("ADER_B200_STEP_IMPL", "dag")
-        if self.hp.hidden_units > 160:
+        # the library says which kernel path serves this shape (ops.path_check); a refused fast path falls back to fp32
+        if ops.path_check(self.ms, ops.PATH_ENCODER_TC) is not None:
             self.encoder_impl = self.infer_encoder_impl = "exact"
+        if ops.path_check(self.ms, ops.PATH_LOSS_TC) is not None:
+            self.loss_impl = "exact"
+        if ops.path_check(self.ms, ops.PATH_EVAL_TC) is not None:
+            self.eval_impl = "exact"
+        # inference (rep, evaluation, recommendation, herding) runs at every accepted shape; training also needs the
+        # backward of its encoder.  A refusal is kept here and raised before the first launch of a training call.
+        self.train_refusal = ops.path_check(self.ms, ops.PATH_ENCODER_BWD) if self.encoder_impl == "exact" else None
         self.global_step = 0            # host mirror of adam_state[0] (drives the dropout stream)
         self._enc_ws = ops.Workspace(self.device)
         self._bwd_ws = ops.Workspace(self.device)
@@ -165,6 +173,11 @@ class Ader:
         return r, self.logits(r, max_item)
 
     # ---- training step ------------------------------------------------------------------------
+    def check_trainable(self):
+        """Raise if no training path serves this model shape (the message names the limit, hidden_units and maxlen)."""
+        if self.train_refusal is not None:
+            raise ops._lib.AderError("this model cannot be trained: " + self.train_refusal)
+
     def loss_and_grad(self, seq, pos, max_item: int, exemplar_logits=None, exemplar_pos=None,
                       teacher_rows=None, dropout_rate: float = 0.0, n_tokens: Optional[int] = None,
                       mode: Optional[int] = None, lambda_: Optional[float] = None, _events=None,
@@ -174,6 +187,7 @@ class Ader:
         ADER.py:20), a device tensor [E, V_prev] indexed by ``teacher_rows`` [M_e], or a ``data.FrozenTeacher``
         whose reps ``teacher_rows`` indexes the same way."""
         from .data import FrozenTeacher
+        self.check_trainable()
         mode = self.mode if mode is None else mode
         lam = self.lambda_ if lambda_ is None else lambda_
         ids = _to_ids(seq, self.hp.maxlen, self.device)
@@ -288,6 +302,7 @@ class Ader:
         """sess.run(model.train_op, feed) (main.py:233-256).  Returns the device scalar loss."""
         lr = self.args.lr if lr is None else lr
         p = self.args.dropout_rate if dropout_rate is None else dropout_rate
+        self.check_trainable()
         self._opt_applied = False
         if self.dp is not None:          # peer back end: every rank has finished the previous update (first launch of the step)
             self.dp.begin_step(self)
@@ -368,10 +383,10 @@ class Ader:
 
     def _tc_or_exact(self, R: int, max_item: int, k: int, m_max: int, tc_ws_bytes, run_tc, run_exact, force_exact: bool,
                      guards: Optional[list] = None, tok_flag=None):
-        """``run_tc(ws, over)`` where the tensor-core entry applies (hidden_units <= 160, 2 * m_max * chunks >= k: up to m_max
+        """``run_tc(ws, over)`` where the tensor-core entry applies (eval_impl "tc", 2 * m_max * chunks >= k: up to m_max
         maxima per (chunk, column half)); else, or after a candidate overflow (counted in ``eval_fallbacks``), ``run_exact(ws)``.
         guards: see ``rank_topk``; ``(tok_flag, overflow word)`` is appended instead of read."""
-        if (not force_exact and self.eval_impl == "tc" and self.hp.hidden_units <= 160
+        if (not force_exact and self.eval_impl == "tc"
                 and 2 * m_max * ops.eval_topk_chunks(self.ms, R, max_item) >= k):
             over = torch.zeros(1, dtype=torch.int32, device=self.device)
             run_tc(self._eval_ws.get(tc_ws_bytes(self.ms, R, max_item)), over)
@@ -502,12 +517,15 @@ class Ewc(Ader):
         accumulated in float64, divided by len(data).  Consumes the Python RNG like the reference
         (Sampler shuffle at construction and at wrap)."""
         from .data import Sampler
+        # the batched pass where the library serves it, else one training pass per sample
+        batched = self.fisher_impl == "batched" and ops.path_check(self.ms, ops.PATH_FISHER_BATCHED) is None
+        if not batched:
+            self.check_trainable()
         sampler = Sampler(data, self.hp.maxlen, batch_size, is_subseq=True)
         if self._fisher_acc is None:
             self._fisher_acc = torch.zeros(self.layout.total, dtype=torch.float64, device=self.device)
         acc = self._fisher_acc
         acc.zero_()
-        batched = self.fisher_impl == "batched" and self.hp.hidden_units <= 160
         rows_ids, rows_pos = [], []
         for _ in range(sampler.batch_num()):
             seq, pos = sampler.sampler_arrays()

@@ -36,6 +36,19 @@ def model_struct(hp: Hyper) -> AderModel:
     return AderModel(hp.v_tab, hp.hidden_units, hp.maxlen, hp.num_blocks, hp.num_heads)
 
 
+# kernel paths of ader_path_check (include/ader_b200.h ADER_PATH_*)
+PATH_ENCODER_FWD, PATH_ENCODER_BWD, PATH_ENCODER_TC, PATH_LOSS_TC, PATH_EVAL_TC, PATH_FISHER_BATCHED, PATH_HERDING_ONCHIP = range(7)
+
+
+def path_check(ms: AderModel, path: int) -> Optional[str]:
+    """None when the kernel path ``path`` (PATH_*) serves the model shape, else the library's refusal, which names the
+    limit, hidden_units and maxlen.  Host only: needs no device."""
+    lib = _lib.load()
+    if lib.ader_path_check(C.byref(ms), path) == 0:
+        return None
+    return lib.ader_last_error().decode("utf-8", "replace")
+
+
 class Workspace:
     """Grow-only caller-owned device scratch (the C ABI never allocates)."""
 

@@ -47,6 +47,22 @@ int64_t     ader_param_count(const AderModel* m);
 int64_t     ader_param_offset(const AderModel* m, int32_t idx);
 int64_t     ader_dense_count(const AderModel* m);      /* everything after the item table */
 
+/* ---- which kernel path serves a model shape ------------------------------------------------
+ * Every model that passes the model check (even hidden_units <= 256, maxlen 1..64, num_heads dividing hidden_units,
+ * num_blocks 1..8) is accepted by the library, but each path has its own limits.  ader_path_check needs no device:
+ * it returns 0 when `path` serves the model, else -1 with ader_last_error() naming the limit, hidden_units and maxlen.
+ * The entries of a path run the same check before their first launch and refuse with the same message. */
+#define ADER_PATH_ENCODER_FWD    0   /* exact encoder forward: attention tile of one session in 200 KB of shared memory  */
+#define ADER_PATH_ENCODER_BWD    1   /* exact encoder backward: attention tile in 220 KB (loss_impl=exact training,
+                                        hidden_units > 160 training, batched Fisher)                                      */
+#define ADER_PATH_ENCODER_TC     2   /* fused tensor-core encoder (ader_encoder_*_tc): hidden_units <= 160              */
+#define ADER_PATH_LOSS_TC        3   /* tcgen05 loss entries, ader_train_*_tc, the bf16 table shadow: hidden_units <= 160 */
+#define ADER_PATH_EVAL_TC        4   /* tcgen05 evaluation ranks / top-k and recommendation: hidden_units <= 160         */
+#define ADER_PATH_FISHER_BATCHED 5   /* ader_fisher_batched: hidden_units <= 160 and both exact encoder paths            */
+#define ADER_PATH_HERDING_ONCHIP 6   /* herding with candidates on chip: hidden_units <= 160; wider models are served by
+                                        the first-generation kernel (candidates in the workspace)                         */
+int32_t     ader_path_check(const AderModel* m, int32_t path);
+
 /* ---- encoder: modules.py:23-271 + ADER.py:25-85 (subsystem 1) ------------------------- */
 /* Activation workspace (saved for backward) for M rows and a capacity of Tcap real tokens
  * (Tcap <= M * maxlen; the exact token count is computed on the device, overflow is flagged

@@ -106,7 +106,7 @@ def test_every_compute_entry_point_is_a_torch_op(lib):
     import torch
     ops.register_torch_ops()
     host_only = ("_ws_bytes", "_ws_slot", "abi_version", "last_error", "param_count", "param_offset", "dense_count", "ipc_",
-                 "dp_status", "debug_", "eval_topk_chunks")
+                 "dp_status", "debug_", "eval_topk_chunks", "path_check")
     want = sorted(s[len("ader_"):] for s in _declared_symbols() if not any(h in s for h in host_only))
     assert want == ops.registered_op_names()
     for name in want:
