@@ -94,6 +94,9 @@ SIGNATURES = {
     "ader_recommend_topk": (C.c_int32, [_MP, _P, _P, _P, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P, _P]),
     "ader_recommend_tc_ws_bytes": (C.c_size_t, [_MP, C.c_int32, C.c_int32]),
     "ader_recommend_topk_tc": (C.c_int32, [_MP, _P, _P, _P, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P, _P, _P]),
+    "ader_logsumexp": (C.c_int32, [_MP, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P]),
+    "ader_logsumexp_tc_ws_bytes": (C.c_size_t, [_MP, C.c_int32, C.c_int32]),
+    "ader_logsumexp_tc": (C.c_int32, [_MP, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P]),
     "ader_herding_ws_bytes": (C.c_size_t, [_MP, C.c_int32]),
     "ader_herding_segmented": (C.c_int32, [_MP, _P, C.c_int32, _P, _P, C.c_int32, _P, _P, _P, _P, _P, _P]),
     "ader_fisher_accumulate": (C.c_int32, [_MP, _P, _P, C.c_int32, _P]),

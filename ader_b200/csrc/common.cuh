@@ -99,6 +99,20 @@ static inline int check_loss_args(const AderModel* m, const AderLossArgs* a, con
   return 0;
 }
 
+// The arguments of the two log-sum-exp entries (ader_logsumexp, ader_logsumexp_tc): nll is written exactly when gt is given.
+static inline int check_lse_args(const AderModel* m, const float* theta, const float* rep, const int32_t* gt, int R, int V,
+                                 const void* ws, const float* lse, const float* nll, const char* who) {
+  if (!theta) return fail(-1, "%s: theta is NULL", who);
+  if (!rep) return fail(-1, "%s: rep is NULL", who);
+  if (!ws) return fail(-1, "%s: ws is NULL", who);
+  if (!lse) return fail(-1, "%s: lse is NULL", who);
+  if (R <= 0) return fail(-1, "%s: R must be > 0 (got %d)", who, R);
+  if (V < 1 || V >= m->v_tab) return fail(-1, "%s: V=%d outside the items 1..%d of the table", who, V, m->v_tab - 1);
+  if (gt && !nll) return fail(-1, "%s: gt is given but nll is NULL", who);
+  if (!gt && nll) return fail(-1, "%s: nll is given but gt is NULL", who);
+  return 0;
+}
+
 // ---- programmatic dependent launch (PDL) -----------------------------------------------------------------
 // Chain kernels call pdl_wait() before their first access to data of the preceding kernel (a no-op for a normal
 // launch) and pdl_go() right behind it; launch_chain() sets the programmatic-stream-serialization attribute when

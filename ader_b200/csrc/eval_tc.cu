@@ -21,6 +21,10 @@
 //   Y (streamed)  :  64 rows of the table = 5 regions x  8 KB = 40 KB, ring of 3
 //   S tile 128 x 64 fp32 in TMEM (2 buffers x 64 columns), 30 MMAs (M = 128, N = 64, K = 16) per tile.
 // Work: CTA = (row tile, vocabulary chunk); counts are merged with integer atomics (order independent).
+//
+// Log-sum-exp (the normaliser of the next-item softmax, ADER.py:91-93): the same pass keeps a running (max, sum exp) of
+// its row per (chunk, column half) over the approximate scores of items 1..V, and k_lse_merge combines a row's slots in a
+// fixed order.  Every S~ is within eps_i of s, so |lse~ - lse| <= eps_i plus the rounding of the sums.
 #include "tc_common.cuh"
 #include <limits.h>
 #include <stdlib.h>
@@ -108,10 +112,13 @@ __device__ __forceinline__ uint64_t desc_col(uint32_t base, int col, int reg) {
 //   RANK: count the columns certainly above the row's anchor (S~ > hi_thr) and append those in [lo_thr, hi_thr] to cand;
 //   CAND: append the columns with S~ >= lo_topk to tk_cand;
 //   MS:   keep the MS largest scores of every (chunk, column half) of a row, sorted in registers, in maxbuf (0: none);
-//   EXCL: the row's excl list is left out (a column is eligible when it is an item and not excluded).
-template <bool RANK, bool CAND, int MS, bool EXCL>
+//   EXCL: the row's excl list is left out (a column is eligible when it is an item and not excluded);
+//   LSE:  keep (max, sum exp(S~ - max)) of every (chunk, column half) of a row in lse_part [n_chunks * 2][R].
+// lse_part is a parameter of its own behind the tensor maps, so EvalArgs and the maps sit at the same offsets in every
+// instance.
+template <bool RANK, bool CAND, int MS, bool EXCL, bool LSE>
 __global__ void __launch_bounds__(NTHREADS, 1) k_eval_tc(EvalArgs a, const __grid_constant__ CUtensorMap tm_x,
-                                                         const __grid_constant__ CUtensorMap tm_y) {
+                                                         const __grid_constant__ CUtensorMap tm_y, float2* __restrict__ lse_part) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   uint8_t* sX = smem;
@@ -200,6 +207,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_eval_tc(EvalArgs a, const __gri
 #pragma unroll
     for (int s = 0; s < MS; ++s) top[s] = -INFINITY;
     int above = 0;
+    float lmax = -INFINITY, lsum = 0.f;           // LSE: running max and sum exp(S~ - lmax) of the slot
     for (int it = 0; it < n_it; ++it) {
       const int s = it & 1; const uint32_t ph = (it >> 1) & 1;
       mbar_wait(BAR(B_TFULL + s), ph, err);
@@ -237,6 +245,18 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_eval_tc(EvalArgs a, const __gri
           }
         }
       }
+      if constexpr (LSE) {
+        // window max first, so each score takes one exp; the window's 32 terms are summed before they join the slot's sum
+        constexpr float LOG2E = 1.4426950408889634f;
+        float wm = -INFINITY;
+#pragma unroll
+        for (int i = 0; i < 32; ++i) if (whole || j0 + i < a.V) wm = fmaxf(wm, __uint_as_float(r[i]));
+        if (wm > lmax) { lsum *= exp2f((lmax - wm) * LOG2E); lmax = wm; }
+        float ws = 0.f;
+#pragma unroll
+        for (int i = 0; i < 32; ++i) ws += (whole || j0 + i < a.V) ? exp2f((__uint_as_float(r[i]) - lmax) * LOG2E) : 0.f;
+        lsum += ws;
+      }
       while (unsure) {                            // rare: a handful of columns per row in the whole pass
         const int i = __ffs(unsure) - 1; unsure &= unsure - 1;
         const int pos = atomicAdd(a.cand_cnt + gi, 1);
@@ -251,6 +271,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_eval_tc(EvalArgs a, const __gri
     if (live) {
 #pragma unroll
       for (int t = 0; t < MS; ++t) a.maxbuf[(long long)((chunk * 2 + half) * MS + t) * a.R + gi] = top[t];
+      if constexpr (LSE) lse_part[(long long)(chunk * 2 + half) * a.R + gi] = make_float2(lmax, lsum);
     }
     if (live && RANK && above) atomicAdd(a.above + gi, above);
   }
@@ -357,6 +378,35 @@ __global__ void __launch_bounds__(256) k_topk_refine(const float* __restrict__ t
   }
 }
 
+// lse[i] = log sum over the row's n_slots (max, sum) pairs, combined in a fixed order (lane-strided, then a butterfly), in
+// fp64; nll[i] = lse[i] - sg[i] when sg is given.  Warp per row; a slot without items is (-inf, 0).
+__global__ void __launch_bounds__(256) k_lse_merge(const float2* __restrict__ part, int n_slots, int R, const float* __restrict__ sg,
+                                                   float* __restrict__ lse, float* __restrict__ nll) {
+  const int i = (int)(((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+  if (i >= R) return;
+  double m = -INFINITY, s = 0.0;
+  auto join = [&](double m2, double s2) {         // (m, s) <- (m, s) + (m2, s2); -inf maxima carry a zero sum
+    const double mx = fmax(m, m2);
+    if (mx == -INFINITY) return;
+    s = (m == mx ? s : s * exp(m - mx)) + (m2 == mx ? s2 : s2 * exp(m2 - mx));
+    m = mx;
+  };
+  for (int t = lane; t < n_slots; t += 32) {
+    const float2 p = part[(long long)t * R + i];
+    join(p.x, p.y);
+  }
+#pragma unroll
+  for (int o = 16; o; o >>= 1) {
+    const double m2 = __shfl_xor_sync(0xffffffffu, m, o), s2 = __shfl_xor_sync(0xffffffffu, s, o);
+    join(m2, s2);
+  }
+  if (lane == 0) {
+    const float l = (float)(m + log(s));
+    lse[i] = l;
+    if (sg) nll[i] = l - sg[i];
+  }
+}
+
 // ids [R, L] (left-padded, 0 = empty) -> the row's columns id - 1 < V, ascending and distinct, in excl [R][EXCL_W] + excl_cnt [R].
 // Warp per row, two ids per lane: an id is kept at its first position; its slot is the number of distinct smaller ids.
 __global__ void __launch_bounds__(256) k_excl_lists(const int* __restrict__ ids, int R, int L, int V, int* __restrict__ excl,
@@ -407,10 +457,12 @@ struct EvalWs {
   int *max_norm, *above, *cand_cnt, *cand, *flags, *tk_cnt, *tk_cand;
   float *lo_topk, *maxbuf;
   int *excl, *excl_cnt;
+  float2* lse_part;
   size_t bytes;
 };
-// excl: append the exclusion lists (recommendation); the layout before them is the same either way
-static EvalWs carve(int R, int V, bool excl, char* base) {
+// excl: append the exclusion lists (recommendation); lse: append the (max, sum) slots of the log-sum-exp pass.  The layout
+// before them is the same either way.
+static EvalWs carve(int R, int V, bool excl, bool lse, char* base) {
   EvalWs w; size_t o = 0;
   auto take = [&](size_t n) { char* p = base ? base + o : nullptr; o += align_up(n); return p; };
   const int nm = cdiv(R, TM), nv = cdiv(V, TN), cap = ADER_EVAL_CAND_CAP;
@@ -430,16 +482,18 @@ static EvalWs carve(int R, int V, bool excl, char* base) {
   w.maxbuf = (float*)take(sizeof(float) * (size_t)R * 2 * 128);
   w.excl = excl ? (int*)take(sizeof(int) * (size_t)R * EXCL_W) : nullptr;
   w.excl_cnt = excl ? (int*)take(sizeof(int) * (size_t)R) : nullptr;
+  w.lse_part = lse ? (float2*)take(sizeof(float2) * (size_t)R * 2 * eval_chunks(R, V)) : nullptr;
   w.bytes = o;
   return w;
 }
 
-template <bool RANK, bool CAND, int MS, bool EXCL>
-static void eval_pass(const EvalArgs& a, const CUtensorMap& tx, const CUtensorMap& ty, cudaStream_t st) {
+template <bool RANK, bool CAND, int MS, bool EXCL, bool LSE = false>
+static void eval_pass(const EvalArgs& a, const CUtensorMap& tx, const CUtensorMap& ty, cudaStream_t st,
+                      float2* lse_part = nullptr) {
   static const cudaError_t attr =
-      cudaFuncSetAttribute(k_eval_tc<RANK, CAND, MS, EXCL>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_EVAL);
+      cudaFuncSetAttribute(k_eval_tc<RANK, CAND, MS, EXCL, LSE>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_EVAL);
   (void)attr;                                     // a refusal surfaces as the launch error
-  k_eval_tc<RANK, CAND, MS, EXCL><<<a.n_mtiles * a.n_chunks, NTHREADS, SMEM_EVAL, st>>>(a, tx, ty);
+  k_eval_tc<RANK, CAND, MS, EXCL, LSE><<<a.n_mtiles * a.n_chunks, NTHREADS, SMEM_EVAL, st>>>(a, tx, ty, lse_part);
 }
 
 template <bool EXCL>
@@ -458,18 +512,20 @@ static void maxima_pass(int ms, const EvalArgs& a, const CUtensorMap& tx, const 
 using namespace ader;
 using namespace ader::ev;
 
-// The pipeline behind the three tensor-core entries.  gt (or NULL): rank of the ground truth, from its exact score
-// (k_gt_band), the counting pass and k_refine.  k > 0: top-k, from a maxima pass, tau (k_topk_threshold), a candidate pass and
-// k_topk_refine.  ids (or NULL, never with gt): each row's own items are left out of the maxima and the candidates.
+// The pipeline behind the tensor-core entries.  gt (or NULL): the exact score of the ground truth (k_gt_band); with rank, the
+// rank of the ground truth from it, the counting pass and k_refine.  k > 0: top-k, from a maxima pass, tau (k_topk_threshold),
+// a candidate pass and k_topk_refine.  ids (or NULL, never with gt): each row's own items are left out of the maxima and the
+// candidates.  lse (or NULL): the log-sum-exp pass over items 1..V and k_lse_merge, and with gt nll = lse - s_gt.
+// overflow may be NULL when no candidate list is collected.
 // The maxima pass keeps m scores per (chunk, column half), m = the smallest of 1, 2, 4, 8 with 2 * nc * m >= k (the eval
 // entries admit only 2 * nc >= k, so they run with m = 1; 2 * nc * m <= 256, the slot count k_topk_threshold takes).  All
 // kept scores belong to different eligible items, so at least k eligible items score >= tau - eps and every eligible item
 // whose exact score reaches the k-th one has S~ >= tau - 2 eps.
 static int topk_tc_run(const AderModel* m, const float* theta, const float* rep, const int32_t* gt, const int32_t* ids, int R,
                        int V, int k, void* ws, int32_t* rank, int32_t* topk_item, float* topk_score, int32_t* overflow,
-                       cudaStream_t st) {
+                       float* lse, float* nll, cudaStream_t st) {
   const int d = m->d, cap = ADER_EVAL_CAND_CAP;
-  EvalWs w = carve(R, V, ids != nullptr, (char*)ws);
+  EvalWs w = carve(R, V, ids != nullptr, lse != nullptr, (char*)ws);
   const int nm = cdiv(R, TM), nv = cdiv(V, TN), nc = eval_chunks(R, V);
   int ms = 1;
   while (ms < 8 && 2 * nc * ms < k) ms *= 2;
@@ -477,7 +533,7 @@ static int topk_tc_run(const AderModel* m, const float* theta, const float* rep,
   if (int e = make_map2d(&tx, w.x16, D2, (uint64_t)nm * TM, D2 * 2, TM)) return e;
   if (int e = make_map2d(&ty, w.y16, D2, (uint64_t)nv * TN, D2 * 2, TN)) return e;
   const float* table1 = theta + d;                       // item 1 = table row 1 (ADER.py:90-91)
-  cudaMemsetAsync(w.max_norm, 0, sizeof(int) * (8 + (gt ? 2 * (size_t)R : 0)), st);
+  cudaMemsetAsync(w.max_norm, 0, sizeof(int) * (8 + (rank ? 2 * (size_t)R : 0)), st);
   if (k > 0) cudaMemsetAsync(w.tk_cnt, 0, sizeof(int) * (size_t)R, st);
   k_pack_hilo<<<cdiv((long long)nv * TN * 32, 256), 256, 0, st>>>(table1, d, V, d, nv * TN, w.y16, nullptr, w.max_norm);
   k_pack_hilo<<<cdiv((long long)nm * TM * 32, 256), 256, 0, st>>>(rep, d, R, d, nm * TM, w.x16, w.rnorm, nullptr);
@@ -492,22 +548,26 @@ static int topk_tc_run(const AderModel* m, const float* theta, const float* rep,
     if (ids) maxima_pass<true>(ms, a, tx, ty, st); else maxima_pass<false>(ms, a, tx, ty, st);
     k_topk_threshold<<<cdiv((long long)R * 32, 256), 256, 0, st>>>(w.maxbuf, 2 * nc * ms, R, k, w.rnorm, w.max_norm, w.lo_topk);
   }
-  if (gt) {
+  if (rank) {
     if (k > 0) eval_pass<true, true, 0, false>(a, tx, ty, st); else eval_pass<true, false, 0, false>(a, tx, ty, st);
-  } else {
+  } else if (k > 0) {
     if (ids) eval_pass<false, true, 0, true>(a, tx, ty, st); else eval_pass<false, true, 0, false>(a, tx, ty, st);
   }
   if (k > 0)
     k_topk_refine<<<cdiv((long long)R * 32, 256), 256, 0, st>>>(table1, rep, R, d, w.tk_cnt, w.tk_cand, cap, k, topk_item, topk_score);
-  if (gt) k_refine<<<cdiv((long long)R * 32, 256), 256, 0, st>>>(table1, rep, gt, R, d, w.sg, w.above, w.cand_cnt, w.cand, cap, rank);
-  cudaMemcpyAsync(overflow, w.flags, sizeof(int), cudaMemcpyDeviceToDevice, st);
-  ADER_CHECK_LAUNCH(gt ? "eval_rank_tc" : "recommend_topk_tc");
+  if (rank) k_refine<<<cdiv((long long)R * 32, 256), 256, 0, st>>>(table1, rep, gt, R, d, w.sg, w.above, w.cand_cnt, w.cand, cap, rank);
+  if (lse) {
+    eval_pass<false, false, 0, false, true>(a, tx, ty, st, w.lse_part);
+    k_lse_merge<<<cdiv((long long)R * 32, 256), 256, 0, st>>>(w.lse_part, 2 * nc, R, gt ? w.sg : nullptr, lse, nll);
+  }
+  if (overflow) cudaMemcpyAsync(overflow, w.flags, sizeof(int), cudaMemcpyDeviceToDevice, st);
+  ADER_CHECK_LAUNCH(lse ? "logsumexp_tc" : gt ? "eval_rank_tc" : "recommend_topk_tc");
   return 0;
 }
 
 extern "C" size_t ader_eval_rank_tc_ws_bytes(const AderModel* m, int32_t R, int32_t V) {
   if (check_model(m) || R <= 0 || V <= 0 || path_check(m, ADER_PATH_EVAL_TC)) return 0;
-  return carve(R, V, false, nullptr).bytes;
+  return carve(R, V, false, false, nullptr).bytes;
 }
 
 extern "C" int32_t ader_eval_rank_tc(const AderModel* m, const float* theta, const float* rep, const int32_t* gt, int32_t R,
@@ -516,7 +576,7 @@ extern "C" int32_t ader_eval_rank_tc(const AderModel* m, const float* theta, con
   if (int e = path_check(m, ADER_PATH_EVAL_TC)) return e;
   ADER_CHECK_ARG(theta && rep && gt && ws && rank && overflow, "eval_rank_tc: NULL pointer");
   ADER_CHECK_ARG(R > 0 && V >= 1 && V < m->v_tab, "eval_rank_tc: bad sizes");
-  return topk_tc_run(m, theta, rep, gt, nullptr, R, V, 0, ws, rank, nullptr, nullptr, overflow, (cudaStream_t)stream);
+  return topk_tc_run(m, theta, rep, gt, nullptr, R, V, 0, ws, rank, nullptr, nullptr, overflow, nullptr, nullptr, (cudaStream_t)stream);
 }
 
 extern "C" int32_t ader_eval_topk_chunks(const AderModel* m, int32_t R, int32_t V) {
@@ -533,12 +593,13 @@ extern "C" int32_t ader_eval_rank_topk_tc(const AderModel* m, const float* theta
   ADER_CHECK_ARG(R > 0 && V >= 1 && V < m->v_tab && k >= 1 && k <= 32, "eval_rank_topk_tc: bad sizes");
   const int nc = eval_chunks(R, V);
   ADER_CHECK_ARG(2 * nc >= k && 2 * nc <= 256, "eval_rank_tc: top-%d needs %d..128 vocabulary chunks per row tile (have %d): use ader_eval_rank_topk", k, (k + 1) / 2, nc);
-  return topk_tc_run(m, theta, rep, gt, nullptr, R, V, k, ws, rank, topk_item, topk_score, overflow, (cudaStream_t)stream);
+  return topk_tc_run(m, theta, rep, gt, nullptr, R, V, k, ws, rank, topk_item, topk_score, overflow, nullptr, nullptr,
+                     (cudaStream_t)stream);
 }
 
 extern "C" size_t ader_recommend_tc_ws_bytes(const AderModel* m, int32_t R, int32_t V) {
   if (check_model(m) || R <= 0 || V <= 0 || path_check(m, ADER_PATH_EVAL_TC)) return 0;
-  return carve(R, V, true, nullptr).bytes;
+  return carve(R, V, true, false, nullptr).bytes;
 }
 
 extern "C" int32_t ader_recommend_topk_tc(const AderModel* m, const float* theta, const float* rep, const int32_t* ids, int32_t R,
@@ -551,5 +612,19 @@ extern "C" int32_t ader_recommend_topk_tc(const AderModel* m, const float* theta
   const int nc = eval_chunks(R, V);
   ADER_CHECK_ARG(2 * nc * 8 >= k, "recommend_topk_tc: top-%d needs %d vocabulary chunks per row tile (have %d): use ader_recommend_topk",
                  k, (k + 15) / 16, nc);
-  return topk_tc_run(m, theta, rep, nullptr, ids, R, V, k, ws, nullptr, topk_item, topk_score, overflow, (cudaStream_t)stream);
+  return topk_tc_run(m, theta, rep, nullptr, ids, R, V, k, ws, nullptr, topk_item, topk_score, overflow, nullptr, nullptr,
+                     (cudaStream_t)stream);
+}
+
+extern "C" size_t ader_logsumexp_tc_ws_bytes(const AderModel* m, int32_t R, int32_t V) {
+  if (check_model(m) || R <= 0 || V <= 0 || path_check(m, ADER_PATH_EVAL_TC)) return 0;
+  return carve(R, V, false, true, nullptr).bytes;
+}
+
+extern "C" int32_t ader_logsumexp_tc(const AderModel* m, const float* theta, const float* rep, const int32_t* gt, int32_t R,
+                                     int32_t V, void* ws, float* lse, float* nll, void* stream) {
+  if (int e = check_model(m)) return e;
+  if (int e = path_check(m, ADER_PATH_EVAL_TC)) return e;
+  if (int e = check_lse_args(m, theta, rep, gt, R, V, ws, lse, nll, "logsumexp_tc")) return e;
+  return topk_tc_run(m, theta, rep, gt, nullptr, R, V, 0, ws, nullptr, nullptr, nullptr, nullptr, lse, nll, (cudaStream_t)stream);
 }

@@ -194,6 +194,32 @@ __global__ void k_mark_seen(float* __restrict__ S, long long ld, const int* __re
   if (id >= 1 && id <= V) S[(idx / L) * ld + id - 1] = __int_as_float(0x7fc00000);
 }
 
+// ---- log-normaliser of the next-item softmax (ADER.py:91-93) over an exact logits row -------------------------------
+// one CTA per row: max, then sum exp(s_j - max) accumulated in fp64 in a fixed order; lse in fp32, nll = lse - s[gt - 1]
+__global__ void __launch_bounds__(256) k_lse_rows(const float* __restrict__ S, long long ld, int V, const int* __restrict__ gt,
+                                                  float* __restrict__ lse, float* __restrict__ nll) {
+  __shared__ float sh[32];
+  __shared__ double shd[8];
+  const int i = blockIdx.x, lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  const float* s = S + (long long)i * ld;
+  float mx = -INFINITY;
+  for (int j = threadIdx.x; j < V; j += blockDim.x) mx = fmaxf(mx, s[j]);
+  mx = block_reduce(mx, true, sh);
+  double sum = 0.0;
+  for (int j = threadIdx.x; j < V; j += blockDim.x) sum += (double)expf(s[j] - mx);
+#pragma unroll
+  for (int o = 16; o; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
+  if (lane == 0) shd[wid] = sum;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double t = 0.0;
+    for (int w = 0; w < 8; ++w) t += shd[w];
+    const float l = (float)((double)mx + log(t));
+    lse[i] = l;
+    if (gt) nll[i] = l - s[gt[i] - 1];
+  }
+}
+
 }  // namespace ader
 
 using namespace ader;
@@ -292,6 +318,19 @@ extern "C" int32_t ader_eval_rank_topk(const AderModel* m, const float* theta, c
   ADER_CHECK_ARG(k >= 0 && k <= 32 && (k == 0 || (topk_item && topk_score)), "eval_rank_topk: bad k");
   ADER_CHECK_ARG(!gt || rank, "eval_rank_topk: rank is NULL");
   return exact_rank_topk(m, theta, rep, gt, nullptr, M, V, k, ws, rank, topk_item, topk_score, (cudaStream_t)stream);
+}
+
+extern "C" int32_t ader_logsumexp(const AderModel* m, const float* theta, const float* rep, const int32_t* gt, int32_t R,
+                                  int32_t V, void* ws, float* lse, float* nll, void* stream) {
+  if (int e = check_model(m)) return e;
+  if (int e = check_lse_args(m, theta, rep, gt, R, V, ws, lse, nll, "logsumexp")) return e;
+  cudaStream_t st = (cudaStream_t)stream;
+  const long long ld = logits_ld(V);
+  float* S = (float*)ws;
+  if (int e = run_logits(m, theta, rep, R, V, S, ld, st)) return e;
+  k_lse_rows<<<R, 256, 0, st>>>(S, ld, V, gt, lse, nll);
+  ADER_CHECK_LAUNCH("logsumexp");
+  return 0;
 }
 
 extern "C" int32_t ader_recommend_topk(const AderModel* m, const float* theta, const float* rep, const int32_t* ids, int32_t R,

@@ -320,12 +320,16 @@ def load_exemplars(exemplar_pre) -> "ExemplarSet":                              
 # ---- util.py:276-350 -----------------------------------------------------------------------------
 class Evaluator:
     def __init__(self, data: list, is_subseq: bool, maxlen: int, batch_size: int, max_item: int, mode: str,
-                 model, sess=None, chunk_rows: int = 8192, dp=None, cache: Optional[dict] = None):
+                 model, sess=None, chunk_rows: int = 8192, dp=None, cache: Optional[dict] = None, nll: bool = False):
         """cache: a dict the caller keeps for as long as `data` is unchanged (main.py builds a new Evaluator over the SAME
         validation rows after every epoch, main.py:263): the packed row matrices and their device copies are stored in it
         by the first Evaluator and reused by the next ones (the Sampler itself is rebuilt every time: its constructor
-        draws from `random`, util.py:148-149)."""
+        draws from `random`, util.py:148-149).
+        nll: also keep each row's negative log-likelihood of its ground truth (the training loss of the row, measured on
+        held-out rows) in ``self.nll``, in the order of ``self.ranks``; its mean joins the display line."""
         self.max_item, self.model, self.mode = max_item, model, mode
+        self.want_nll = nll
+        self.nll: Optional[np.ndarray] = None
         self.cache = cache
         self.dp = dp                      # (rank, world): rows of a pass are sharded over the ranks, ranks all-gathered
         self.ranks: List[int] = []
@@ -362,11 +366,14 @@ class Evaluator:
             self.cache.update(n=len(s.prepared_data), packed=s.packed(), dev=self._rows_dev)
         order_d = torch.from_numpy(order).to(dev)
         guards, spans = [], []
+        nlls = []
         for lo in range(0, len(order), self.chunk_rows):
             idx = order[lo:lo + self.chunk_rows]
             idx_d = order_d[lo:lo + self.chunk_rows]
+            nll = torch.empty(len(idx), dtype=torch.float32, device=dev) if self.want_nll else None
             r, items, _ = self.model.rank_topk(ids_d.index_select(0, idx_d), label_d.index_select(0, idx_d), self.max_item, k,
-                                               n_tokens=int(n_in[idx].sum()), guards=guards)
+                                               n_tokens=int(n_in[idx].sum()), guards=guards, nll=nll)
+            nlls.append(nll)
             ranks.append(r)
             tops.append(items)
             spans.append((lo, idx))
@@ -390,6 +397,14 @@ class Evaluator:
             parts = [torch.empty_like(mine) for _ in range(world)]
             dist.all_gather(parts, mine)
             ranks = [p[:n] for p, n in zip(parts, sizes)]
+            if self.want_nll:
+                mine_n = torch.full((cap,), float("nan"), dtype=torch.float32, device=dev)
+                if nlls:
+                    n_loc = torch.cat(nlls)
+                    mine_n[:n_loc.numel()] = n_loc
+                parts_n = [torch.empty_like(mine_n) for _ in range(world)]
+                dist.all_gather(parts_n, mine_n)
+                nlls = [p[:n] for p, n in zip(parts_n, sizes)]
             if k > 0:
                 mine_t = torch.zeros((cap, k), dtype=torch.int32, device=dev)
                 if tops:
@@ -401,9 +416,17 @@ class Evaluator:
         if ranks and n_all > 0:
             self.ranks = torch.cat(ranks).cpu().numpy().tolist()
             self.topk = torch.cat(tops) if k > 0 else None
+            self.nll = torch.cat(nlls).cpu().numpy() if self.want_nll else None
         else:
             self.ranks = []
+            self.nll = np.zeros(0, np.float32) if self.want_nll else None
         return self.display(epoch)
+
+    def mean_nll(self) -> Optional[float]:
+        """Mean negative log-likelihood of the pass's rows (None unless the Evaluator was built with nll=True)."""
+        if self.nll is None:
+            return None
+        return float(np.mean(self.nll, dtype=np.float64)) if len(self.nll) else float("nan")
 
     def results(self):                                                           # util.py:329-339
         n = len(self.ranks)
@@ -417,6 +440,8 @@ class Evaluator:
         res = self.results()
         info = "epoch:%d, %s (MRR@20: %.4f, RECALL@20: %.4f, MRR@10: %.4f, RECALL@10: %.4f)" % (
             epoch, self.mode, res[0], res[1], res[2], res[3])
+        if self.nll is not None:
+            info += " NLL: %.4f" % self.mean_nll()
         print(info)
         return info
 

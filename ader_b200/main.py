@@ -81,6 +81,9 @@ def build_parser() -> argparse.ArgumentParser:             # main.py:75-108 (typ
     # losses use the global-mean denominators, gradients are summed (ader_b200/dist.py), evaluation rows are sharded.
     p.add_argument("--epoch_queue", default=True, type=lambda v: str(v).lower() not in ("0", "false", "no"))  # host out of the step loop
     p.add_argument("--dp", default=False, type=lambda v: str(v).lower() not in ("0", "false", "no"))
+    # held-out log-likelihood: validation and test passes also report the mean NLL of the ground truth under the softmax
+    # over items 1..max_item (the training objective on unseen rows; it moves before a rank-20 cutoff does)
+    p.add_argument("--eval_nll", action="store_true")
     return p
 
 
@@ -466,6 +469,7 @@ def run(args) -> dict:
     best_epoch, item_num_prev = 0, 0
     t_start = time.time()
     metrics = {"MRR_20": [], "Recall_20": [], "MRR_10": [], "Recall_10": []}
+    eval_nll = bool(getattr(args, "eval_nll", False))
     stats = []
     fast_exemplar = None
     ckpt = {}                                                  # (period, epoch) -> state (tf.train.Saver max_to_keep=1)
@@ -566,7 +570,7 @@ def run(args) -> dict:
                 rnd = random.sample(exemplar_subseq, min(len(exemplar_subseq), args.ewc_sample_num))
                 model.compute_fisher(None, rnd, 50, max_item)
             valid_evaluator = Evaluator(valid_subseq, True, args.maxlen, args.test_batch, max_item, "valid", model, None, dp=dp,
-                                        cache=valid_cache)
+                                        cache=valid_cache, nll=eval_nll)
             t0 = time.time()
             info = valid_evaluator.evaluate(epoch)
             eval_time += time.time() - t0                         # evaluate() ends with the ranks on the host
@@ -574,6 +578,8 @@ def run(args) -> dict:
             logs.write(info + "\n")
             performance = valid_evaluator.results()[1]
             rec["valid"].append(valid_evaluator.results())
+            if eval_nll:
+                rec.setdefault("valid_nll", []).append(valid_evaluator.mean_nll())
             if best_performance >= performance:                # main.py:272-280
                 stop_counter += 1
                 if stop_counter >= args.stop:
@@ -584,7 +590,8 @@ def run(args) -> dict:
                 best_performance = performance
                 ckpt = {(period, epoch): model.state_dict()}
         model.load_state_dict(ckpt[(period, best_epoch)])      # main.py:283
-        test_evaluator = Evaluator(test_sess, False, args.maxlen, args.test_batch, max_item, "test", model, None, dp=dp)
+        test_evaluator = Evaluator(test_sess, False, args.maxlen, args.test_batch, max_item, "test", model, None, dp=dp,
+                                   nll=eval_nll)
         t0 = time.time()
         info = test_evaluator.evaluate(best_epoch)
         eval_time += time.time() - t0
@@ -594,6 +601,9 @@ def run(args) -> dict:
         rec["best_epoch"], rec["test"], rec["test_ranks"] = best_epoch, r, list(test_evaluator.ranks)
         metrics["MRR_20"].append(r[0]); metrics["Recall_20"].append(r[1])
         metrics["MRR_10"].append(r[2]); metrics["Recall_10"].append(r[3])
+        if eval_nll:
+            rec["test_nll"] = test_evaluator.mean_nll()
+            metrics.setdefault("NLL", []).append(rec["test_nll"])
         sps = trainer.rows_seen / max(train_time, 1e-9)
         stats.append({"period": period, "train_rows": trainer.rows_seen, "train_s": train_time, "sessions_per_s": sps,
                       "eval_rows": eval_rows, "eval_s": eval_time, "eval_rows_per_s": eval_rows / max(eval_time, 1e-9),

@@ -330,12 +330,14 @@ class Ader:
 
     # ---- evaluation ---------------------------------------------------------------------------
     def rank_topk(self, seq, gt, max_item: int, k: int = 20, n_tokens: Optional[int] = None, guards: Optional[list] = None,
-                  force_exact: bool = False):
+                  force_exact: bool = False, nll: Optional[torch.Tensor] = None):
         """Rank of the ground-truth item among items 1..max_item (== pred_last[row, gt-1],
         ADER.py:103 + util.py:325; ties -> lower index first) and the top-k item ids.
         guards: None = the two guard words of the call (encoder token overflow, candidate-band overflow of the fused path)
         are read here (two small host syncs); a list = they are appended as device tensors ``(tokens, band)`` and the CALLER
-        reads them later (``check_guards``) - an evaluation pass then launches all its chunks without a host sync."""
+        reads them later (``check_guards``) - an evaluation pass then launches all its chunks without a host sync.
+        nll (fp32 [M] device tensor, or None): also receives each row's negative log-likelihood of its ground truth under the
+        softmax over items 1..max_item (``logsumexp``), from the representations this call encodes."""
         ids = _to_ids(seq, self.hp.maxlen, self.device)
         gt_t = _to_i32(gt, self.device)
         rep, tcap_used = self.encode(ids, n_tokens)
@@ -355,15 +357,44 @@ class Ader:
         self._tc_or_exact(M, max_item, k, 1, ops.eval_rank_tc_ws_bytes, tc,
                           lambda ws: ops.eval_rank_topk(self.ms, self.theta, rep, gt_t, max_item, k, ws, rank, items, scores),
                           force_exact, guards, tok_flag)
+        if nll is not None:
+            self.logsumexp(rep, max_item, gt_t, force_exact=force_exact, nll=nll)
         return rank, items, scores
 
+    def logsumexp(self, rep: torch.Tensor, max_item: int, gt=None, force_exact: bool = False,
+                  nll: Optional[torch.Tensor] = None):
+        """(lse [R], nll [R] or None) of representations ``rep`` [R, d]: lse = log sum_{j=1..max_item} exp(rep . E_j), the
+        log-normaliser of the next-item softmax (ADER.py:91-93), so p(j | session) = exp(score_j - lse); with ``gt`` [R]
+        (ids 1..max_item), nll = lse - score_gt, the row's cross-entropy.  The tensor-core entry (within
+        eps = 2^-12 ||rep|| max_j ||E_j|| of the exact value) is used where it applies, else the exact fp32 / fp64 one.
+        nll: an fp32 [R] device tensor to write into (allocated when None)."""
+        R = rep.shape[0]
+        lse = torch.empty(R, dtype=torch.float32, device=self.device)
+        gt_t = None if gt is None else _to_i32(gt, self.device)
+        if gt_t is None:
+            nll = None
+        elif nll is None:
+            nll = torch.empty(R, dtype=torch.float32, device=self.device)
+        if R == 0:
+            return lse, nll
+        rep = rep.contiguous()
+        if not force_exact and self.eval_impl == "tc":
+            ops.logsumexp_tc(self.ms, self.theta, rep, gt_t, max_item,
+                             self._eval_ws.get(ops.logsumexp_tc_ws_bytes(self.ms, R, max_item)), lse, nll)
+        else:
+            ops.logsumexp(self.ms, self.theta, rep, gt_t, max_item, self._eval_ws.get(ops.eval_ws_bytes(self.ms, R, max_item)),
+                          lse, nll)
+        return lse, nll
+
     def recommend(self, seq, max_item: int, k: int = 20, exclude_seen: bool = True, n_tokens: Optional[int] = None,
-                  force_exact: bool = False):
+                  force_exact: bool = False, probs: bool = False):
         """Top-k next items among 1..max_item for unlabelled sessions: ``seq`` [R, maxlen] left-padded ids (the input rows of
         ``rank_topk``) -> (items [R, k] int32, best first, ties -> lower id; scores [R, k] fp32, the exact scores of
         ``logits``).  exclude_seen: the items of the row's own session are never returned.  A row with fewer than k eligible
         items is padded with item 0 and score -inf.  The tensor-core entry is used where it applies; a batch whose candidate
-        list overflows is rerun on the exact entry (counted in ``eval_fallbacks``).  The lists are the same either way."""
+        list overflows is rerun on the exact entry (counted in ``eval_fallbacks``).  The lists are the same either way.
+        probs: the second tensor holds p(item | session) = exp(score - lse) instead, lse over all items 1..max_item, the
+        session's own items included (``logsumexp``); padding entries get 0."""
         if not 1 <= k <= 100:
             raise ValueError("k must be in 1..100 (got %d)" % k)
         ids = _to_ids(seq, self.hp.maxlen, self.device)
@@ -379,6 +410,9 @@ class Ader:
                           lambda ws, over: ops.recommend_topk_tc(self.ms, self.theta, rep, seen, max_item, k, ws, items, scores, over),
                           lambda ws: ops.recommend_topk(self.ms, self.theta, rep, seen, max_item, k, ws, items, scores),
                           force_exact)
+        if probs:
+            lse = self.logsumexp(rep, max_item, force_exact=force_exact)[0]
+            scores = torch.exp(scores - lse[:, None])
         return items, scores
 
     def _tc_or_exact(self, R: int, max_item: int, k: int, m_max: int, tc_ws_bytes, run_tc, run_exact, force_exact: bool,

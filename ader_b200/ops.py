@@ -353,6 +353,29 @@ def recommend_topk_tc(ms: AderModel, theta, rep, ids, V: int, k: int, ws, topk_i
                                              _ptr(topk_item), _ptr(topk_score), _ptr(overflow), _stream()), "recommend_topk_tc")
 
 
+def logsumexp(ms: AderModel, theta, rep, gt, V: int, ws, lse, nll):
+    """lse [R] = log sum_{j=1..V} exp(rep . E_j) from the exact fp32 scores (fp64 sums); gt [R] (or None): nll [R] =
+    lse - the ground-truth score (nll None when gt is).  ws: eval_ws_bytes(ms, R, V)."""
+    _require_cuda(theta, rep, gt, ws, lse, nll)
+    check(_lib.load().ader_logsumexp(C.byref(ms), _ptr(theta), _ptr(rep), _ptr(gt), rep.shape[0], V, _ptr(ws), _ptr(lse),
+                                     _ptr(nll), _stream()), "logsumexp")
+
+
+def logsumexp_tc_ws_bytes(ms: AderModel, R: int, V: int) -> int:
+    n = _lib.load().ader_logsumexp_tc_ws_bytes(C.byref(ms), R, V)
+    if n == 0:
+        raise _lib.AderError("logsumexp_tc_ws_bytes: bad model / sizes")
+    return n
+
+
+def logsumexp_tc(ms: AderModel, theta, rep, gt, V: int, ws, lse, nll):
+    """The same on the tensor cores ([R, V] never written): within eps_i = 2^-12 ||rep_i|| max_j ||E_j|| of the exact lse;
+    nll uses the exact ground-truth score."""
+    _require_cuda(theta, rep, gt, ws, lse, nll)
+    check(_lib.load().ader_logsumexp_tc(C.byref(ms), _ptr(theta), _ptr(rep), _ptr(gt), rep.shape[0], V, _ptr(ws), _ptr(lse),
+                                        _ptr(nll), _stream()), "logsumexp_tc")
+
+
 def herding_ws_bytes(ms: AderModel, N: int) -> int:
     n = _lib.load().ader_herding_ws_bytes(C.byref(ms), N)
     if n == 0:
@@ -449,6 +472,8 @@ _SCHEMAS = {
     "eval_rank_topk_tc": "(int[] model, Tensor theta, Tensor rep, Tensor gt, int V, int k, Tensor(a!) ws, Tensor(b!) rank, Tensor(c!) topk_item, Tensor(d!) topk_score, Tensor(e!) overflow) -> ()",
     "recommend_topk": "(int[] model, Tensor theta, Tensor rep, Tensor? ids, int V, int k, Tensor(a!) ws, Tensor(b!) topk_item, Tensor(c!) topk_score) -> ()",
     "recommend_topk_tc": "(int[] model, Tensor theta, Tensor rep, Tensor? ids, int V, int k, Tensor(a!) ws, Tensor(b!) topk_item, Tensor(c!) topk_score, Tensor(d!) overflow) -> ()",
+    "logsumexp": "(int[] model, Tensor theta, Tensor rep, Tensor? gt, int V, Tensor(a!) ws, Tensor(b!) lse, Tensor(c!)? nll) -> ()",
+    "logsumexp_tc": "(int[] model, Tensor theta, Tensor rep, Tensor? gt, int V, Tensor(a!) ws, Tensor(b!) lse, Tensor(c!)? nll) -> ()",
     "herding_segmented": "(int[] model, Tensor rep, Tensor cand, Tensor seg_off, Tensor quota, Tensor max_steps, Tensor(a!) ws, Tensor(b!) picks, Tensor(c!) n_picked) -> ()",
     "fisher_accumulate": "(int[] model, Tensor grad, Tensor(a!) acc, int V) -> ()",
     "fisher_finalize": "(int[] model, Tensor acc, Tensor(a!) fisher, int V, int n_data) -> ()",
@@ -505,6 +530,8 @@ def register_torch_ops() -> None:
         "eval_rank_topk_tc": lambda model, theta, rep, gt, V, k, ws, rank, items, scores, overflow: eval_rank_topk_tc(_ms(model), theta, rep, gt, V, k, ws, rank, items, scores, overflow),
         "recommend_topk": lambda model, theta, rep, ids, V, k, ws, items, scores: recommend_topk(_ms(model), theta, rep, ids, V, k, ws, items, scores),
         "recommend_topk_tc": lambda model, theta, rep, ids, V, k, ws, items, scores, overflow: recommend_topk_tc(_ms(model), theta, rep, ids, V, k, ws, items, scores, overflow),
+        "logsumexp": lambda model, theta, rep, gt, V, ws, lse, nll: logsumexp(_ms(model), theta, rep, gt, V, ws, lse, nll),
+        "logsumexp_tc": lambda model, theta, rep, gt, V, ws, lse, nll: logsumexp_tc(_ms(model), theta, rep, gt, V, ws, lse, nll),
         "herding_segmented": lambda model, rep, cand, seg_off, quota, max_steps, ws, picks, n_picked: herding_segmented(_ms(model), rep, cand, seg_off, quota, max_steps, ws, picks, n_picked),
         "fisher_accumulate": lambda model, grad, acc, V: fisher_accumulate(_ms(model), grad, acc, V),
         "fisher_finalize": lambda model, acc, fisher, V, n_data: fisher_finalize(_ms(model), acc, fisher, V, n_data),

@@ -1,12 +1,17 @@
 """Top-k next-item lists for a file of sessions, from the checkpoint a training run writes.
 
     python -m ader_b200.recommend --checkpoint results/DIGINETICA-ADER/checkpoint.pt --sessions sessions.txt --out topk.txt
-        [--k 20] [--keep_seen] [--max_item N] [--scores] [--batch 4096]
+        [--k 20] [--keep_seen] [--max_item N] [--scores | --probs] [--batch 4096]
 
 Input: one session per line, item ids separated by whitespace, oldest first.  The model reads the last ``maxlen`` items of
 each session, right-aligned, as it read the sessions it was trained on.  Output: one line per input line with ``k`` ids,
-best first (``id:score`` pairs with ``--scores``).  A session's own items are never recommended unless ``--keep_seen``;
-a session with fewer than ``k`` items left to recommend is padded with item 0 (score -inf).
+best first (``id:score`` pairs with ``--scores``, ``id:probability`` pairs with ``--probs``).  A session's own items are
+never recommended unless ``--keep_seen``; a session with fewer than ``k`` items left to recommend is padded with item 0
+(score -inf, probability 0).
+
+The probability is the model's next-item softmax, p(j | session) = exp(score_j - lse) with lse = log sum exp(score) over
+ALL items 1..max_item, the session's own items included (the distribution the model was trained to fit).  A line's listed
+probabilities therefore sum to at most 1: the rest belongs to the items not listed, excluded ones among them.
 """
 from __future__ import annotations
 
@@ -30,7 +35,9 @@ def build_parser() -> argparse.ArgumentParser:
     p.add_argument("--k", default=20, type=int, help="items per session, 1..100")
     p.add_argument("--keep_seen", action="store_true", help="allow a session's own items in its list")
     p.add_argument("--max_item", default=None, type=int, help="rank items 1..max_item (default: the largest item seen in training)")
-    p.add_argument("--scores", action="store_true", help="write id:score pairs")
+    out = p.add_mutually_exclusive_group()
+    out.add_argument("--scores", action="store_true", help="write id:score pairs")
+    out.add_argument("--probs", action="store_true", help="write id:probability pairs (softmax over all items 1..max_item)")
     p.add_argument("--batch", default=4096, type=int, help="sessions per device pass")
     return p
 
@@ -99,12 +106,15 @@ def load_model(path: str, device=None):
     return model, int(np.max(st["item_set"]))
 
 
-def recommend_sessions(model, sessions, max_item: int, k: int = 20, exclude_seen: bool = True, batch: int = 4096):
-    """items [N, k] int32 and scores [N, k] fp32 (host arrays) for a list of sessions."""
+def recommend_sessions(model, sessions, max_item: int, k: int = 20, exclude_seen: bool = True, batch: int = 4096,
+                       probs: bool = False):
+    """items [N, k] int32 and scores [N, k] fp32 (host arrays) for a list of sessions; probs: probabilities instead of
+    scores (``Ader.recommend``)."""
     ids, n_in = session_rows(sessions, model.hp.maxlen)
     items, scores = [], []
     for lo in range(0, len(sessions), batch):
-        it, sc = model.recommend(ids[lo:lo + batch], max_item, k, exclude_seen, n_tokens=int(n_in[lo:lo + batch].sum()))
+        it, sc = model.recommend(ids[lo:lo + batch], max_item, k, exclude_seen, n_tokens=int(n_in[lo:lo + batch].sum()),
+                                 probs=probs)
         items.append(it.cpu().numpy()); scores.append(sc.cpu().numpy())
     if not items:
         return np.zeros((0, k), np.int32), np.zeros((0, k), np.float32)
@@ -126,10 +136,10 @@ def main(argv=None) -> None:
         sessions = read_sessions(a.sessions, model.hp.v_tab)
     except ValueError as e:
         raise SystemExit(str(e)) from None
-    items, scores = recommend_sessions(model, sessions, max_item, a.k, not a.keep_seen, a.batch)
+    items, scores = recommend_sessions(model, sessions, max_item, a.k, not a.keep_seen, a.batch, probs=a.probs)
     with open(a.out, "w") as f:
         for r in range(items.shape[0]):
-            f.write(format_line(items[r], scores[r] if a.scores else None) + "\n")
+            f.write(format_line(items[r], scores[r] if (a.scores or a.probs) else None) + "\n")
 
 
 if __name__ == "__main__":

@@ -57,7 +57,8 @@ int64_t     ader_dense_count(const AderModel* m);      /* everything after the i
                                         hidden_units > 160 training, batched Fisher)                                      */
 #define ADER_PATH_ENCODER_TC     2   /* fused tensor-core encoder (ader_encoder_*_tc): hidden_units <= 160              */
 #define ADER_PATH_LOSS_TC        3   /* tcgen05 loss entries, ader_train_*_tc, the bf16 table shadow: hidden_units <= 160 */
-#define ADER_PATH_EVAL_TC        4   /* tcgen05 evaluation ranks / top-k and recommendation: hidden_units <= 160         */
+#define ADER_PATH_EVAL_TC        4   /* tcgen05 evaluation ranks / top-k, recommendation and log-sum-exp:
+                                        hidden_units <= 160                                                              */
 #define ADER_PATH_FISHER_BATCHED 5   /* ader_fisher_batched: hidden_units <= 160 and both exact encoder paths            */
 #define ADER_PATH_HERDING_ONCHIP 6   /* herding with candidates on chip: hidden_units <= 160; wider models are served by
                                         the first-generation kernel (candidates in the workspace)                         */
@@ -258,6 +259,20 @@ size_t  ader_recommend_tc_ws_bytes(const AderModel* m, int32_t R, int32_t V);
 int32_t ader_recommend_topk_tc(const AderModel* m, const float* theta, const float* rep, const int32_t* ids, int32_t R,
                                int32_t V, int32_t k, void* ws, int32_t* topk_item, float* topk_score,
                                int32_t* overflow, void* stream);   /* needs d <= 160 and 2*ader_eval_topk_chunks*8 >= k */
+
+/* ---- next-item probabilities and held-out log-likelihood ---------------------------------- */
+/* lse[i] = log sum_{j=1..V} exp(rep_i . E_j) -- the log-normaliser of the next-item softmax (ADER.py:91-93);
+ * gt (or NULL): nll[i] = lse[i] - rep_i . E_gt[i] (nll may be NULL when gt is).  Exact fp32 scores, fp64 sums. */
+int32_t ader_logsumexp(const AderModel* m, const float* theta, const float* rep, const int32_t* gt, int32_t R, int32_t V,
+                       void* ws /* ader_eval_ws_bytes */, float* lse, float* nll, void* stream);
+/* The same on the tcgen05 tensor cores, [R, V] never written: |lse - exact| <= eps_i + rounding (eps_i of
+ * ader_eval_rank_tc); nll uses the exact ground-truth score.  Needs hidden_units <= 160.
+ * The approximate scores are summed per (vocabulary chunk, column half) and the partial sums merged in a fixed order, so
+ * repeated calls with the same (R, V) give the same bits; the chunk count depends on R (ader_eval_topk_chunks), so the same
+ * session in batches of different R may differ in the last bits, within the bound. */
+size_t  ader_logsumexp_tc_ws_bytes(const AderModel* m, int32_t R, int32_t V);
+int32_t ader_logsumexp_tc(const AderModel* m, const float* theta, const float* rep, const int32_t* gt, int32_t R, int32_t V,
+                          void* ws, float* lse, float* nll, void* stream);
 
 /* ---- exemplar selection: util.py:401-461 (subsystem 4) ---------------------------------- */
 /* Segmented herding.  rep [N,d]; segment s owns candidate rows cand[seg_off[s] .. seg_off[s+1])
