@@ -1408,6 +1408,7 @@ extern "C" int32_t ader_encoder_bwd(const AderModel* m, const float* theta, cons
   if (int e = path_check(m, ADER_PATH_ENCODER_BWD)) return e;
   ADER_CHECK_ARG(theta && ids && ws && bwd_ws && d_rep && grad, "encoder_bwd: NULL pointer");
   ADER_CHECK_ARG(M > 0 && Tcap > 0, "encoder_bwd: bad M/Tcap");
+  ADER_CHECK_ARG(dropout_rate >= 0.f && dropout_rate < 1.f, "encoder_bwd: dropout_rate out of range");
   return enc_bwd_exact(m, theta, ids, M, Tcap, ws, bwd_ws, d_rep, grad, dropout_rate, seed, (cudaStream_t)stream, nullptr);
 }
 
@@ -1684,6 +1685,7 @@ int ader::enc_bwd_tc_run(const AderModel* m, const float* theta, const int32_t* 
   if (int e = path_check(m, ADER_PATH_ENCODER_TC)) return e;
   ADER_CHECK_ARG(theta && ids && ws && bwd_ws && d_rep && grad, "encoder_bwd_tc: NULL pointer");
   ADER_CHECK_ARG(M > 0 && Tcap > 0, "encoder_bwd_tc: bad M/Tcap");
+  ADER_CHECK_ARG(dropout_rate >= 0.f && dropout_rate < 1.f, "encoder_bwd_tc: dropout_rate out of range");
   cudaStream_t st = f.main;
   const Layout l = make_layout(m);
   const int d = m->d, L = m->maxlen;

@@ -40,9 +40,11 @@ using namespace ader;
 static int run_step(const AderModel* m, const float* theta, const int32_t* ids, int32_t M, int32_t Tcap,
                     const AderLossArgs* a, void* enc_ws, void* bwd_ws, void* loss_ws, float* rep,
                     float* loss, float* row_loss, float* d_rep, float* grad, float dropout_rate,
-                    uint64_t seed, const int32_t* d_step, int32_t serial, cudaStream_t st, AdamPlan* adam) {
+                    uint64_t seed, const int32_t* d_step, int32_t serial, cudaStream_t st, AdamPlan* adam,
+                    const char* entry) {
   ADER_CHECK_ARG(m && theta && ids && a && enc_ws && bwd_ws && loss_ws && rep && loss && row_loss && d_rep && grad,
                  "train step: NULL pointer");
+  ADER_CHECK_ARG(dropout_rate >= 0.f && dropout_rate < 1.f, "%s: dropout_rate out of range", entry);
   ADER_CHECK_ARG(a->M == M, "train step: loss rows (%d) != encoder rows (%d)", a->M, M);
   Fork f = Fork::serial(st);
   if (!serial) {
@@ -92,7 +94,7 @@ extern "C" int32_t ader_train_fwd_bwd_tc(const AderModel* m, const float* theta,
                                          float* loss, float* row_loss, float* d_rep, float* grad, float dropout_rate,
                                          uint64_t seed, const int32_t* d_step, int32_t serial, void* stream) {
   return run_step(m, theta, ids, M, Tcap, a, enc_ws, bwd_ws, loss_ws, rep, loss, row_loss, d_rep, grad, dropout_rate, seed,
-                  d_step, serial, (cudaStream_t)stream, nullptr);
+                  d_step, serial, (cudaStream_t)stream, nullptr, "train_fwd_bwd_tc");
 }
 
 extern "C" int32_t ader_train_step_tc(const AderModel* m, float* theta, const int32_t* ids, int32_t M, int32_t Tcap,
@@ -106,5 +108,5 @@ extern "C" int32_t ader_train_step_tc(const AderModel* m, float* theta, const in
   AdamPlan plan;
   plan.theta = theta; plan.m = adam_m; plan.v = adam_v; plan.grad = grad; plan.state = state; plan.a = *opt; plan.prep_ready = nullptr;
   return run_step(m, theta, ids, M, Tcap, a, enc_ws, bwd_ws, loss_ws, rep, loss, row_loss, d_rep, grad, dropout_rate, seed,
-                  d_step, serial, (cudaStream_t)stream, &plan);
+                  d_step, serial, (cudaStream_t)stream, &plan, "train_step_tc");
 }

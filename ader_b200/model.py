@@ -22,6 +22,18 @@ from . import ops
 from .params import Hyper, ParamLayout
 
 
+# Odd 32-bit constant that separates the dropout streams of data-parallel ranks (see dropout_seed).
+DROPOUT_RANK_SALT = 0x9E3779B9
+
+
+def dropout_seed(random_seed: int, rank: int = 0) -> int:
+    """Dropout seed of step 0; step t draws its masks from ``dropout_seed(...) + t`` (csrc/common.cuh: drop_site).
+    The high 32 bits carry ``random_seed`` plus ``rank * DROPOUT_RANK_SALT``: every rank numbers its packed tokens
+    from 0, so without the salt token t of every rank would get the same masks.  Rank 0 (and a single GPU) keeps the
+    unsalted stream ``random_seed << 32``."""
+    return ((int(random_seed) + int(rank) * DROPOUT_RANK_SALT) << 32) & 0xFFFFFFFFFFFFFFFF
+
+
 def _to_ids(seq, maxlen: int, device) -> torch.Tensor:
     """Accept the reference's tuple-of-arrays batches, ndarrays or device tensors -> int32 [M, L] on device."""
     if isinstance(seq, torch.Tensor):
@@ -235,7 +247,8 @@ class Ader:
         # dropout stream: (seed, step).  Under CUDA-graph capture the step is read on the device from the Adam
         # state (incremented by the optimiser kernel), so every replay draws fresh masks.
         d_step = self.adam_state if (_device_step and self.encoder_impl == "tc") else None   # exact encoder: graphs only at p = 0
-        seed = (self.seed << 32) + (0 if _device_step else self.global_step)
+        rank = self.dp.rank if self.dp is not None else 0
+        seed = dropout_seed(self.seed, rank) + (0 if _device_step else self.global_step)
         gc = global_counts if global_counts is not None else self.global_counts
         a = ops.make_loss_args(M, n_train, n_ex, max_item, v_prev, mode if n_ex > 0 else self.VANILLA, lam,
                                pos_t, ex_pos_t, teacher, trow, *(gc or (0, 0)),

@@ -113,8 +113,9 @@ def normalize(x, beta, gamma, eps: float = 1e-8):
     return gamma * ((x - mean) / (var + eps) ** 0.5) + beta
 
 
-def multihead_attention(q, keys, wq, bq, wk, bk, wv, bv, num_heads: int, id_mask=None):
-    """modules.py:172-223 with causality=True, dropout 0."""
+def multihead_attention(q, keys, wq, bq, wk, bk, wv, bv, num_heads: int, id_mask=None, drop=None):
+    """modules.py:172-223 with causality=True.  drop: None (dropout 0) or the [h*M, T, T] multipliers of the
+    attention weights (modules.py:214; oracle/dropout.py draws the library's own)."""
     Q = q @ wq + bq                                                   # :172
     K = keys @ wk + bk                                                # :173
     V = keys @ wv + bv                                                # :174
@@ -133,30 +134,40 @@ def multihead_attention(q, keys, wq, bq, wk, bk, wv, bv, num_heads: int, id_mask
     out = torch.softmax(out, dim=-1)                                  # :205
     query_masks = (torch.sign(torch.abs(q.sum(-1))) if literal else id_mask).repeat(num_heads, 1)[:, :, None]  # :208-210
     out = out * query_masks                                           # :211
+    if drop is not None:
+        out = out * drop                                              # :214
     out = out @ V_                                                    # :217
     out = torch.cat(torch.chunk(out, num_heads, dim=0), dim=2)        # :220
     return out + q                                                    # :223 residual on queries
 
 
-def feedforward(z, w1, b1, w2, b2):
-    """modules.py:254-266 -- conv1d(k=1) == dense; residual on the (normalised) input."""
-    return torch.relu(z @ w1 + b1) @ w2 + b2 + z
+def feedforward(z, w1, b1, w2, b2, drop=None):
+    """modules.py:254-266 -- conv1d(k=1) == dense; residual on the (normalised) input.  drop: None (dropout 0)
+    or the (inner, output) multipliers, each [M, T, d] (modules.py:257, 262)."""
+    if drop is None:
+        return torch.relu(z @ w1 + b1) @ w2 + b2 + z
+    return (torch.relu(z @ w1 + b1) * drop[0] @ w2 + b2) * drop[1] + z
 
 
-def forward_rep(params: Sequence[torch.Tensor], ids: torch.Tensor, hp: Hyper) -> torch.Tensor:
-    """ADER.py:25-85: ids [M, maxlen] int -> rep [M, d] (eval mode / dropout 0)."""
+def forward_rep(params: Sequence[torch.Tensor], ids: torch.Tensor, hp: Hyper, drop=None) -> torch.Tensor:
+    """ADER.py:25-85: ids [M, maxlen] int -> rep [M, d].  drop: None (eval mode / dropout 0) or a dict site ->
+    multipliers in the padded layout (oracle.dropout.dense_multipliers: the library's masks)."""
     d = hp.hidden_units
     table, pos_table = params[0], params[1]
     mask = (ids != 0).to(table.dtype)[..., None]                          # ADER.py:25
     e0 = torch.cat([torch.zeros(1, d, dtype=table.dtype), table[1:]], 0)  # modules.py:124-126
     seq = e0[ids.long()] * (d ** 0.5)                                     # modules.py:127-130
     seq = seq + pos_table[torch.arange(ids.shape[1])][None]               # ADER.py:41-52
+    if drop is not None:
+        drop = {k: torch.as_tensor(v).to(table.dtype) for k, v in drop.items()}
+        seq = seq * drop[0]                                               # ADER.py:55-58
     seq = seq * mask                                                      # ADER.py:60
     for b in range(hp.num_blocks):
         (ln1b, ln1g, wq, bq, wk, bk, wv, bv, ln2b, ln2g, w1, b1, w2, b2) = params[2 + 14 * b: 16 + 14 * b]
+        d_att, d_ffn = (None, None) if drop is None else (drop[1 + 3 * b], (drop[2 + 3 * b], drop[3 + 3 * b]))
         seq = multihead_attention(normalize(seq, ln1b, ln1g), seq, wq, bq, wk, bk, wv, bv,
-                                  hp.num_heads, id_mask=mask[..., 0])     # ADER.py:66-74
-        seq = feedforward(normalize(seq, ln2b, ln2g), w1, b1, w2, b2)     # ADER.py:77
+                                  hp.num_heads, id_mask=mask[..., 0], drop=d_att)  # ADER.py:66-74
+        seq = feedforward(normalize(seq, ln2b, ln2g), w1, b1, w2, b2, drop=d_ffn)  # ADER.py:77
         seq = seq * mask                                                  # ADER.py:80
     seq = normalize(seq, params[-2], params[-1])                          # ADER.py:82
     return seq[:, -1, :]                                                  # ADER.py:85
@@ -173,19 +184,20 @@ def ce_rows(logits: torch.Tensor, pos: torch.Tensor) -> torch.Tensor:
     return lse - logits.gather(1, (pos.long() - 1)[:, None])[:, 0]
 
 
-def loss_vanilla(params, ids, pos, max_item: int, hp: Hyper):
-    """ADER.py:93 (set_vanilla_loss, ADER.py:105-106)."""
-    rep = forward_rep(params, ids, hp)
+def loss_vanilla(params, ids, pos, max_item: int, hp: Hyper, drop=None):
+    """ADER.py:93 (set_vanilla_loss, ADER.py:105-106).  drop: see forward_rep."""
+    rep = forward_rep(params, ids, hp, drop)
     return ce_rows(logits_of(rep, params[0], max_item), pos).mean()
 
 
 def loss_ader(params, ids, pos, max_item: int, hp: Hyper, lambda_: float,
               exemplar_logits: Optional[torch.Tensor] = None,
-              exemplar_pos: Optional[torch.Tensor] = None):
+              exemplar_pos: Optional[torch.Tensor] = None, drop=None):
     """ADER.py:108-138 (update_loss).  Exemplar rows are the LAST rows of ``ids``; ``pos``
     covers only the leading train rows.  KD branch: student softmax over the first V_prev
-    columns only (ADER.py:134); ER branch: one-hot CE on the exemplar rows (ADER.py:126-131)."""
-    rep = forward_rep(params, ids, hp)
+    columns only (ADER.py:134); ER branch: one-hot CE on the exemplar rows (ADER.py:126-131).  drop: see
+    forward_rep."""
+    rep = forward_rep(params, ids, hp, drop)
     logits = logits_of(rep, params[0], max_item)
     n_ex = exemplar_logits.shape[0] if exemplar_logits is not None else exemplar_pos.shape[0]
     n_train = ids.shape[0] - n_ex
