@@ -5,6 +5,7 @@
 #include <stdio.h>
 #include <stdarg.h>
 #include <math.h>
+#include <atomic>
 #include "../../include/ader_b200.h"
 
 #if defined(__CUDA_ARCH__) && (__CUDA_ARCH__ < 1000)
@@ -18,6 +19,32 @@ int fail(int code, const char* fmt, ...);
 #define ADER_CHECK_ARG(cond, ...) do { if (!(cond)) return ::ader::fail(-1, __VA_ARGS__); } while (0)
 #define ADER_CHECK_LAUNCH(name) do { cudaError_t e__ = cudaGetLastError(); \
     if (e__ != cudaSuccess) return ::ader::fail(-3, "%s: %s", name, cudaGetErrorString(e__)); } while (0)
+
+// Prepares kernel K for launches on the current device: 0, or -3 with a message naming the kernel.  The first call per
+// (kernel, device) sets K's dynamic shared-memory limit to smem_bytes (0 for a kernel that only needs its module loaded
+// before the first launch), which also loads K's module; later calls cost one cudaGetDevice and one atomic load, so a
+// stream capture after an eager first call reaches no other CUDA call.  Kernel attributes are per device.  Every caller
+// of one K passes the same smem_bytes, so threads racing on the first call set the same value.
+template <auto K>
+int kernel_ready(int smem_bytes, const char* name) {
+  static std::atomic<uint64_t> ready{0};                 // bit i: prepared on device i
+  int dev = 0;
+  cudaError_t e = cudaGetDevice(&dev);
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    return fail(-3, "%s: no current device: %s", name, cudaGetErrorString(e));
+  }
+  if (dev >= 64) return fail(-3, "%s: device %d is beyond the 64 the library serves", name, dev);
+  const uint64_t bit = 1ull << dev;
+  if (ready.load(std::memory_order_acquire) & bit) return 0;
+  e = cudaFuncSetAttribute(K, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    return fail(-3, "%s: cannot reserve %d B of shared memory on device %d: %s", name, smem_bytes, dev, cudaGetErrorString(e));
+  }
+  ready.fetch_or(bit, std::memory_order_release);
+  return 0;
+}
 
 static inline int cdiv(long long a, long long b) { return (int)((a + b - 1) / b); }
 static inline size_t align_up(size_t x, size_t a = 256) { return (x + a - 1) / a * a; }

@@ -281,29 +281,19 @@ using namespace ader::dp;
 
 // CUDA loads kernels lazily, and a first-use load may wait for the context to drain: it must not happen while an
 // arrive kernel is already spinning (several emulated ranks in one process would stall until the timeout), so
-// every kernel of this file is loaded before the first launch of any of them.
-static void dp_preload() {
-  static bool done = false;
-  if (done) return;
-  cudaFuncAttributes fa;
-  cudaFuncGetAttributes(&fa, k_dp_adam<2>);
-  cudaFuncGetAttributes(&fa, k_dp_adam<4>);
-  cudaFuncGetAttributes(&fa, k_dp_adam<8>);
-  cudaFuncGetAttributes(&fa, k_dp_adam<16>);
-  cudaFuncGetAttributes(&fa, k_dp_adam_mc);
-  cudaFuncGetAttributes(&fa, k_dp_publish);
-  cudaFuncGetAttributes(&fa, k_dp_arrive);
-  cudaFuncGetAttributes(&fa, k_dp_wait);
-  cudaGetLastError();
-  done = true;
-}
-
+// every kernel of this file is loaded on the device before the first launch of any of them.
 static int check_comm(const AderDpComm* c) {
-  dp_preload();
   ADER_CHECK_ARG(c, "dp: comm is NULL");
   ADER_CHECK_ARG(c->world >= 1 && c->world <= ADER_DP_MAX_RANKS && c->rank >= 0 && c->rank < c->world, "dp: bad rank %d / world %d", c->rank, c->world);
   for (int r = 0; r < c->world; ++r) ADER_CHECK_ARG(c->theta[r] && c->grad[r] && c->flags[r], "dp: NULL pointer for rank %d", r);
-  return 0;
+  if (int e = kernel_ready<k_dp_adam<2>>(0, "k_dp_adam<2>")) return e;
+  if (int e = kernel_ready<k_dp_adam<4>>(0, "k_dp_adam<4>")) return e;
+  if (int e = kernel_ready<k_dp_adam<8>>(0, "k_dp_adam<8>")) return e;
+  if (int e = kernel_ready<k_dp_adam<16>>(0, "k_dp_adam<16>")) return e;
+  if (int e = kernel_ready<k_dp_adam_mc>(0, "k_dp_adam_mc")) return e;
+  if (int e = kernel_ready<k_dp_publish>(0, "k_dp_publish")) return e;
+  if (int e = kernel_ready<k_dp_arrive>(0, "k_dp_arrive")) return e;
+  return kernel_ready<k_dp_wait>(0, "k_dp_wait");
 }
 
 extern "C" int32_t ader_dp_wait(const AderDpComm* c, void* stream) {

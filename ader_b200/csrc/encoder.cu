@@ -1107,6 +1107,7 @@ extern "C" int32_t ader_encoder_fwd(const AderModel* m, const float* theta, cons
   ADER_CHECK_ARG(M > 0 && Tcap > 0 && (long long)Tcap <= (long long)M * m->maxlen, "encoder_fwd: bad M/Tcap (%d, %d)", M, Tcap);
   ADER_CHECK_ARG(dropout_rate >= 0.f && dropout_rate < 1.f, "encoder_fwd: dropout_rate out of range");
   cudaStream_t st = (cudaStream_t)stream;
+  if (int e = kernel_ready<k_attn_fwd>((int)ATTN_FWD_SMEM_MAX, "k_attn_fwd")) return e;
   const Layout l = make_layout(m);
   const int d = m->d, L = m->maxlen;
   EncWs w = carve_enc(m, M, Tcap, (char*)ws);
@@ -1119,11 +1120,6 @@ extern "C" int32_t ader_encoder_fwd(const AderModel* m, const float* theta, cons
   ADER_CHECK_LAUNCH("encoder_fwd/pack+embed");
 
   const size_t attn_smem = attn_fwd_smem(d, L);
-  static bool attr_set = false;
-  if (!attr_set) {
-    cudaFuncSetAttribute(k_attn_fwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ATTN_FWD_SMEM_MAX);
-    attr_set = true;
-  }
   const int ln_grid = cdiv((long long)Tcap * 32, 256);
 
   for (int b = 0; b < m->num_blocks; ++b) {
@@ -1415,6 +1411,7 @@ extern "C" int32_t ader_encoder_bwd(const AderModel* m, const float* theta, cons
 static int enc_bwd_exact(const AderModel* m, const float* theta, const int32_t* ids, int32_t M, int32_t Tcap, const void* ws,
                          void* bwd_ws, const float* d_rep, float* grad, float dropout_rate, uint64_t seed, cudaStream_t st,
                          const FisherHook* fh) {
+  if (int e = kernel_ready<k_attn_bwd>((int)ATTN_BWD_SMEM_MAX, "k_attn_bwd")) return e;
   const Layout l = make_layout(m);
   const int d = m->d, L = m->maxlen;
   const float p = dropout_rate;
@@ -1429,11 +1426,6 @@ static int enc_bwd_exact(const AderModel* m, const float* theta, const int32_t* 
   const int el_grid = cdiv((long long)Tcap * d, 256);
 
   const size_t attn_smem = attn_bwd_smem(d, L);      // within ATTN_BWD_SMEM_MAX: the entries ran path_check
-  static bool attr_set = false;
-  if (!attr_set) {
-    cudaFuncSetAttribute(k_attn_bwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ATTN_BWD_SMEM_MAX);
-    attr_set = true;
-  }
 
   // final LayerNorm (ADER.py:82): only the last token of each row carries gradient
   k_lnf_bwd<<<ln_grid, 256, 0, st>>>(d_rep, w.xfinal, w.meanf, w.rstdf, theta + l.off_lnf + d, w.tok_row, w.row_off, gX, dT, d);
@@ -1554,22 +1546,21 @@ extern "C" int32_t ader_fisher_batched(const AderModel* m, const float* theta, c
 // ------------------------------------------------------------------------------------------
 namespace ader {
 static_assert(PATH_TC_MAX_D == fz::KP, "the fused encoder pads features to KP columns");
+// SMs of the current device (a cached query of the runtime): the tile kernels launch at most one CTA per SM
 static int sm_count() {
-  static int n = 0;
-  if (!n) { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev); if (n <= 0) n = 148; }
+  int dev = 0, n = 0;
+  cudaGetDevice(&dev);
+  cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
   return n;
 }
-static void fused_attrs() {
-  static bool done = false;
-  if (done) return;
-  cudaFuncSetAttribute(fz::k_qkv_fwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fz::QKV_FWD_SMEM);
-  cudaFuncSetAttribute(fz::k_ffn_fwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fz::FFN_FWD_SMEM);
-  cudaFuncSetAttribute(fz::k_ffn_bwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fz::FFN_BWD_SMEM);
-  cudaFuncSetAttribute(fz::k_qkv_bwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fz::QKV_BWD_SMEM);
-  cudaFuncSetAttribute(fz::k_wgrad2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fz::WGRAD2_SMEM);
-  cudaFuncSetAttribute(fz::k_attn_ln_fwd, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * fz::att_rows_cap(64) * fz::KP * 4);
-  cudaFuncSetAttribute(fz::k_attn_bwd_s1, cudaFuncAttributeMaxDynamicSharedMemorySize, fz::att_bwd_smem(64, fz::KP));
-  done = true;
+static int fused_ready() {
+  if (int e = kernel_ready<fz::k_qkv_fwd>((int)fz::QKV_FWD_SMEM, "k_qkv_fwd")) return e;
+  if (int e = kernel_ready<fz::k_ffn_fwd>((int)fz::FFN_FWD_SMEM, "k_ffn_fwd")) return e;
+  if (int e = kernel_ready<fz::k_ffn_bwd>((int)fz::FFN_BWD_SMEM, "k_ffn_bwd")) return e;
+  if (int e = kernel_ready<fz::k_qkv_bwd>((int)fz::QKV_BWD_SMEM, "k_qkv_bwd")) return e;
+  if (int e = kernel_ready<fz::k_wgrad2>((int)fz::WGRAD2_SMEM, "k_wgrad2")) return e;
+  if (int e = kernel_ready<fz::k_attn_ln_fwd>(2 * fz::att_rows_cap(64) * fz::KP * 4, "k_attn_ln_fwd")) return e;
+  return kernel_ready<fz::k_attn_bwd_s1>(fz::att_bwd_smem(64, fz::KP), "k_attn_bwd_s1");
 }
 static const fz::op_t* shadow_of(const EncWs& w, int b, int which, int orient) {
   return (const fz::op_t*)w.wshadow + (size_t)((b * 5 + which) * 2 + orient) * (fz::KP * fz::LDS);
@@ -1597,12 +1588,12 @@ int ader::enc_fwd_tc_run(const AderModel* m, const float* theta, const int32_t* 
   ADER_CHECK_ARG(theta && ids && ws && rep, "encoder_fwd_tc: NULL pointer");
   ADER_CHECK_ARG(M > 0 && Tcap > 0 && (long long)Tcap <= (long long)M * m->maxlen, "encoder_fwd_tc: bad M/Tcap (%d, %d)", M, Tcap);
   ADER_CHECK_ARG(dropout_rate >= 0.f && dropout_rate < 1.f, "encoder_fwd_tc: dropout_rate out of range");
+  if (int e = fused_ready()) return e;
   cudaStream_t st = f.main;
   const Layout l = make_layout(m);
   const int d = m->d, L = m->maxlen;
   EncWs w = carve_enc(m, M, Tcap, (char*)ws);
   const int* dT = w.row_off + M;
-  fused_attrs();
 
   // weight shadows depend on theta only: off the packing chain (joined before the first tile kernel)
   f.edge(st, f.a);
@@ -1686,6 +1677,7 @@ int ader::enc_bwd_tc_run(const AderModel* m, const float* theta, const int32_t* 
   ADER_CHECK_ARG(theta && ids && ws && bwd_ws && d_rep && grad, "encoder_bwd_tc: NULL pointer");
   ADER_CHECK_ARG(M > 0 && Tcap > 0, "encoder_bwd_tc: bad M/Tcap");
   ADER_CHECK_ARG(dropout_rate >= 0.f && dropout_rate < 1.f, "encoder_bwd_tc: dropout_rate out of range");
+  if (int e = fused_ready()) return e;
   cudaStream_t st = f.main;
   const Layout l = make_layout(m);
   const int d = m->d, L = m->maxlen;
@@ -1700,7 +1692,6 @@ int ader::enc_bwd_tc_run(const AderModel* m, const float* theta, const int32_t* 
   const int ln_grid = cdiv((long long)Tcap * 32, 256);
   const int ln_threads = ((d + 31) / 32) * 32;
   const int tile_grid = min(cdiv(Tcap, fz::TM), sm_count());
-  fused_attrs();
 
   // final LayerNorm: data gradient on the chain, parameter gradient beside it
   auto ln_params = [&] {

@@ -488,21 +488,20 @@ static EvalWs carve(int R, int V, bool excl, bool lse, char* base) {
 }
 
 template <bool RANK, bool CAND, int MS, bool EXCL, bool LSE = false>
-static void eval_pass(const EvalArgs& a, const CUtensorMap& tx, const CUtensorMap& ty, cudaStream_t st,
-                      float2* lse_part = nullptr) {
-  static const cudaError_t attr =
-      cudaFuncSetAttribute(k_eval_tc<RANK, CAND, MS, EXCL, LSE>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_EVAL);
-  (void)attr;                                     // a refusal surfaces as the launch error
+static int eval_pass(const EvalArgs& a, const CUtensorMap& tx, const CUtensorMap& ty, cudaStream_t st,
+                     float2* lse_part = nullptr) {
+  if (int e = kernel_ready<k_eval_tc<RANK, CAND, MS, EXCL, LSE>>(SMEM_EVAL, "k_eval_tc")) return e;
   k_eval_tc<RANK, CAND, MS, EXCL, LSE><<<a.n_mtiles * a.n_chunks, NTHREADS, SMEM_EVAL, st>>>(a, tx, ty, lse_part);
+  return 0;
 }
 
 template <bool EXCL>
-static void maxima_pass(int ms, const EvalArgs& a, const CUtensorMap& tx, const CUtensorMap& ty, cudaStream_t st) {
+static int maxima_pass(int ms, const EvalArgs& a, const CUtensorMap& tx, const CUtensorMap& ty, cudaStream_t st) {
   switch (ms) {
-    case 1: eval_pass<false, false, 1, EXCL>(a, tx, ty, st); break;
-    case 2: eval_pass<false, false, 2, EXCL>(a, tx, ty, st); break;
-    case 4: eval_pass<false, false, 4, EXCL>(a, tx, ty, st); break;
-    default: eval_pass<false, false, 8, EXCL>(a, tx, ty, st); break;
+    case 1: return eval_pass<false, false, 1, EXCL>(a, tx, ty, st);
+    case 2: return eval_pass<false, false, 2, EXCL>(a, tx, ty, st);
+    case 4: return eval_pass<false, false, 4, EXCL>(a, tx, ty, st);
+    default: return eval_pass<false, false, 8, EXCL>(a, tx, ty, st);
   }
 }
 
@@ -545,19 +544,19 @@ static int topk_tc_run(const AderModel* m, const float* theta, const float* rep,
   a.maxbuf = w.maxbuf; a.lo_topk = w.lo_topk; a.tk_cnt = w.tk_cnt; a.tk_cand = w.tk_cand;
   a.excl = w.excl; a.excl_cnt = w.excl_cnt;
   if (k > 0) {
-    if (ids) maxima_pass<true>(ms, a, tx, ty, st); else maxima_pass<false>(ms, a, tx, ty, st);
+    if (int e = ids ? maxima_pass<true>(ms, a, tx, ty, st) : maxima_pass<false>(ms, a, tx, ty, st)) return e;
     k_topk_threshold<<<cdiv((long long)R * 32, 256), 256, 0, st>>>(w.maxbuf, 2 * nc * ms, R, k, w.rnorm, w.max_norm, w.lo_topk);
   }
   if (rank) {
-    if (k > 0) eval_pass<true, true, 0, false>(a, tx, ty, st); else eval_pass<true, false, 0, false>(a, tx, ty, st);
+    if (int e = k > 0 ? eval_pass<true, true, 0, false>(a, tx, ty, st) : eval_pass<true, false, 0, false>(a, tx, ty, st)) return e;
   } else if (k > 0) {
-    if (ids) eval_pass<false, true, 0, true>(a, tx, ty, st); else eval_pass<false, true, 0, false>(a, tx, ty, st);
+    if (int e = ids ? eval_pass<false, true, 0, true>(a, tx, ty, st) : eval_pass<false, true, 0, false>(a, tx, ty, st)) return e;
   }
   if (k > 0)
     k_topk_refine<<<cdiv((long long)R * 32, 256), 256, 0, st>>>(table1, rep, R, d, w.tk_cnt, w.tk_cand, cap, k, topk_item, topk_score);
   if (rank) k_refine<<<cdiv((long long)R * 32, 256), 256, 0, st>>>(table1, rep, gt, R, d, w.sg, w.above, w.cand_cnt, w.cand, cap, rank);
   if (lse) {
-    eval_pass<false, false, 0, false, true>(a, tx, ty, st, w.lse_part);
+    if (int e = eval_pass<false, false, 0, false, true>(a, tx, ty, st, w.lse_part)) return e;
     k_lse_merge<<<cdiv((long long)R * 32, 256), 256, 0, st>>>(w.lse_part, 2 * nc, R, gt ? w.sg : nullptr, lse, nll);
   }
   if (overflow) cudaMemcpyAsync(overflow, w.flags, sizeof(int), cudaMemcpyDeviceToDevice, st);

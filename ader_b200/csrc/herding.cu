@@ -409,12 +409,8 @@ extern "C" int32_t ader_herding_segmented(const AderModel* m, const float* rep, 
   }
   constexpr int SMEM_MID = (HM_MAX * 160 + 2 * 160 + HM_MAX) * 4;
   constexpr int SMEM_BIG = (HB_PER * 160 + 4 * 160 + HB_PER) * 4 + HB_BM_WORDS * 4;
-  static bool attr = false;
-  if (!attr) {
-    cudaFuncSetAttribute(k_herding_mid, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_MID);
-    cudaFuncSetAttribute(k_herding_big, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BIG);
-    attr = true;
-  }
+  if (int e = kernel_ready<k_herding_mid>(SMEM_MID, "k_herding_mid")) return e;
+  if (int e = kernel_ready<k_herding_big>(SMEM_BIG, "k_herding_big")) return e;
   cudaMemsetAsync(cnt, 0, 256, st);
   k_herding_classify<<<cdiv(n_seg, 256), 256, 0, st>>>(seg_off, quota, n_seg, cnt, lists[0], lists[1], lists[2], lists[3], n_picked);
   // grids are upper bounds of the class sizes (a class-c segment has more than its lower size bound of candidates);

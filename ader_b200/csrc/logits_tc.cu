@@ -780,15 +780,12 @@ extern "C" size_t ader_table16_ws_bytes(const AderModel* m, int32_t V) {
   return (size_t)cdiv(V, TILE) * TILE * ROW16 * 2;
 }
 
-static void set_tc_attrs() {
-  static bool attr_set = false;
-  if (attr_set) return;
-  cudaFuncSetAttribute(k_tc2<MODE_FWD>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tc2(MODE_FWD));
-  cudaFuncSetAttribute(k_tc2<MODE_DREP>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tc2(MODE_DREP));
-  cudaFuncSetAttribute(k_tc2<MODE_DE>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tc2(MODE_DE));
-  cudaFuncSetAttribute(k_tc2<MODE_TU>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tc2(MODE_TU));
-  cudaFuncSetAttribute(k_tc2<MODE_TP>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tc2(MODE_TP));
-  attr_set = true;
+static int tc_ready() {
+  if (int e = kernel_ready<k_tc2<MODE_FWD>>(smem_tc2(MODE_FWD), "k_tc2<MODE_FWD>")) return e;
+  if (int e = kernel_ready<k_tc2<MODE_DREP>>(smem_tc2(MODE_DREP), "k_tc2<MODE_DREP>")) return e;
+  if (int e = kernel_ready<k_tc2<MODE_DE>>(smem_tc2(MODE_DE), "k_tc2<MODE_DE>")) return e;
+  if (int e = kernel_ready<k_tc2<MODE_TU>>(smem_tc2(MODE_TU), "k_tc2<MODE_TU>")) return e;
+  return kernel_ready<k_tc2<MODE_TP>>(smem_tc2(MODE_TP), "k_tc2<MODE_TP>");
 }
 
 // TMA tensor maps over the row-major bf16 operand matrices
@@ -801,7 +798,7 @@ static int tc_plan(const AderModel* m, const AderLossArgs* a, int v_lo, int v_hi
   const int d = m->d, M = a->M, V = v_hi - v_lo;
   w = carve_tc(a, v_lo, v_hi, (char*)ws);
   const int nm = cdiv(M, TILE), nv = cdiv(V, TILE), nc = tc_chunks(nm, nv);
-  set_tc_attrs();
+  if (int e = tc_ready()) return e;
 
   t.M = M; t.V = V; t.V_total = a->V; t.v_off = v_lo; t.n_mtiles = nm; t.n_vtiles = nv; t.n_chunks = nc;
   t.n_train = a->n_train; t.n_ex = a->n_ex; t.V_prev = a->V_prev; t.mode = a->n_ex > 0 ? a->mode : 0;

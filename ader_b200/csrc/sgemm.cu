@@ -176,8 +176,7 @@ __global__ void __launch_bounds__(256, 2) sgemm_kernel(GemmArgs g, int a_vec2, i
 
 template <bool AK, bool BK_>
 static int launch_one(const GemmArgs& g, dim3 grid, int av, int bv, cudaStream_t st) {
-  static bool attr = false;
-  if (!attr) { cudaFuncSetAttribute(sgemm_kernel<AK, BK_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SGEMM_SMEM); attr = true; }
+  if (int e = kernel_ready<sgemm_kernel<AK, BK_>>((int)SGEMM_SMEM, "sgemm_kernel")) return e;
   sgemm_kernel<AK, BK_><<<grid, 256, SGEMM_SMEM, st>>>(g, av, bv);
   return 0;
 }
@@ -193,10 +192,11 @@ int launch_gemm(const GemmArgs& g, cudaStream_t st) {
   };
   const int av = ak ? vec_ok(g.A, g.a_cs, g.a_rs) : vec_ok(g.A, g.a_rs, g.a_cs);
   const int bv = bk ? vec_ok(g.B, g.b_rs, g.b_cs) : vec_ok(g.B, g.b_cs, g.b_rs);
-  if (ak && bk) launch_one<true, true>(g, grid, av, bv, st);
-  else if (ak) launch_one<true, false>(g, grid, av, bv, st);
-  else if (bk) launch_one<false, true>(g, grid, av, bv, st);
-  else launch_one<false, false>(g, grid, av, bv, st);
+  const int e = ak && bk ? launch_one<true, true>(g, grid, av, bv, st)
+              : ak       ? launch_one<true, false>(g, grid, av, bv, st)
+              : bk       ? launch_one<false, true>(g, grid, av, bv, st)
+                         : launch_one<false, false>(g, grid, av, bv, st);
+  if (e) return e;
   ADER_CHECK_LAUNCH("sgemm_kernel");
   return 0;
 }

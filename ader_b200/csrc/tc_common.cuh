@@ -111,16 +111,14 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 // bf16 matrix [rows][cols], row pitch in bytes (multiple of 16); box = 64 columns (128 B, one swizzle span) x 128 rows
 static inline int make_map2d(CUtensorMap* tm, const void* base, uint64_t cols, uint64_t rows, uint64_t pitch_bytes, uint32_t box_rows = 128) {
-  static EncodeTiledFn enc = nullptr;
-  if (!enc) {
+  static const EncodeTiledFn enc = [] {          // one lookup per process: the entry point does not depend on the device
     void* fn = nullptr;
     cudaDriverEntryPointQueryResult qr;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qr) != cudaSuccess || !fn) {
-      cudaGetLastError();
-      return ::ader::fail(-3, "loss_tc: cuTensorMapEncodeTiled is unavailable (driver too old?)");
-    }
-    enc = (EncodeTiledFn)fn;
-  }
+    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qr) == cudaSuccess) return (EncodeTiledFn)fn;
+    cudaGetLastError();
+    return (EncodeTiledFn)nullptr;
+  }();
+  if (!enc) return ::ader::fail(-3, "loss_tc: cuTensorMapEncodeTiled is unavailable (driver too old?)");
   const cuuint64_t gdim[2] = {cols, rows};
   const cuuint64_t gstr[1] = {pitch_bytes};
   const cuuint32_t box[2] = {64, box_rows};
