@@ -79,7 +79,6 @@ def build_parser() -> argparse.ArgumentParser:             # main.py:75-108 (typ
     # SURVEY 8e: data parallel under torchrun (one process per GPU).  Every rank runs the same host protocol with the same
     # seeds (identical batches, splits, exemplar sets); a step's train rows and exemplar rows are split over the ranks,
     # losses use the global-mean denominators, gradients are summed (ader_b200/dist.py), evaluation rows are sharded.
-    p.add_argument("--epoch_queue", default=True, type=lambda v: str(v).lower() not in ("0", "false", "no"))  # host out of the step loop
     p.add_argument("--dp", default=False, type=lambda v: str(v).lower() not in ("0", "false", "no"))
     # held-out log-likelihood: validation and test passes also report the mean NLL of the ground truth under the softmax
     # over items 1..max_item (the training objective on unseen rows; it moves before a rank-20 cutoff does)
@@ -91,23 +90,34 @@ class PeriodTrainer:
     """One period's epoch loop on GPU-resident rows (main.py:217-256)."""
 
     def __init__(self, model: Ader, train_sampler: Sampler, exemplar_sampler, args, max_item: int):
+        # exemplar rows reach the loss as their labels (one-hot replay) or as row ids into a device-resident teacher
+        # (ExemplarSet.teacher: stored logits or a FrozenTeacher); a sampler fed the reference's [session, logits] lists has
+        # its teacher on the host, and no step here reads it from there
+        self.teacher = None
+        if exemplar_sampler is not None and not model.disable_distillation:
+            self.teacher = getattr(exemplar_sampler, "teacher", None)
+            if self.teacher is None:
+                raise ValueError("distillation needs the exemplars' teacher on the device: feed the exemplar sampler an "
+                                 "ExemplarSet, not a list of [session, logits]")
         self.model, self.args, self.max_item = model, args, max_item
         self.ts, self.es = train_sampler, exemplar_sampler
         dev = model.device
         self.t_ids, self.t_lab = train_sampler.device_rows(dev)
         self.t_nin = train_sampler.packed()[2]
+        self.e_ids = self.e_aux = None  # e_aux, per exemplar row: its label (one-hot replay) or its teacher row (distillation)
         if exemplar_sampler is not None:
-            self.e_ids, self.e_lab = exemplar_sampler.device_rows(dev)
+            self.e_ids, e_lab = exemplar_sampler.device_rows(dev)
             self.e_nin = exemplar_sampler.packed()[2]
+            self.e_aux = e_lab if model.disable_distillation else \
+                torch.as_tensor(np.asarray(exemplar_sampler.logits, dtype=np.int32)).to(dev)
         self.rows_seen = 0
-        self.trace = None
-        self.trace_rows = None
+        self.trace = None               # list: receives every step's loss, read once per epoch
+        self.trace_rows = None          # list: receives every step's (row losses, ids), read after each step (debug)
         # the step as CUDA graphs, one GraphStep per batch geometry (n_train, n_ex).  The reference drops rows of length <= 1
         # from a batch (util.py:228-229), so a few rows are missing from about half of the batches of some periods: the
         # full geometry is captured at once, any other after its third appearance (at most MAX_GEOM of them)
         self.gs_map = {}
         self._geom_seen = {}
-        self._graph_off = False
         self.n_eager = 0                # steps issued launch by launch (rare batch geometry / no graph)
         # data parallel: this rank's shard of every batch (train rows and exemplar rows split separately, main.py:229 order kept)
         self.rank, self.world = getattr(args, "dp_rank", 0), getattr(args, "dp_world", 1)
@@ -149,51 +159,42 @@ class PeriodTrainer:
         if gs is not None:
             return gs
         m, args = self.model, self.args
-        if self._graph_off or not getattr(args, "graph", True):
+        if not getattr(args, "graph", True):
             return None
         if self.world > 1 and (n_train < self.world or (self.es is not None and n_ex < self.world)):
             return None                 # a rank would be left without rows: rare tail batch, eager on every rank
         if m.encoder_impl != "tc" and args.dropout_rate > 0:
-            self._graph_off = True
-            return None
+            return None                 # the exact encoder has no device-side dropout counter: no replay
         full = (args.batch_size, self.es.batch_size if self.es is not None else 0)
         seen = self._geom_seen[key] = self._geom_seen.get(key, 0) + 1
         if key != full and (seen < 3 or len(self.gs_map) >= self.MAX_GEOM):
             return None
-        dev = m.device
-        e_ids = e_aux = teacher = None
-        if self.es is not None:
-            if m.disable_distillation:
-                e_aux = self.e_lab
-            elif getattr(self.es, "teacher", None) is not None:
-                e_aux = torch.as_tensor(np.asarray(self.es.logits, dtype=np.int32)).to(dev)
-                teacher = self.es.teacher
-            else:
-                self._graph_off = True   # host-resident teacher lists (reference feed): eager path
-                return None
-            e_ids = self.e_ids
         (tl, th), (el, eh) = self._shard(n_train, n_ex)
         if self.world > 1:
             m.global_counts = (n_train, n_ex)       # baked into the captured loss arguments
         n_train, n_ex = th - tl, eh - el
         mean_tok = n_train * float(np.mean(self.t_nin)) + (n_ex * float(np.mean(self.e_nin)) if self.es is not None else 0.0)
         caps = [int(mean_tok * f) + 64 for f in (1.1, 1.3, 1.7)]
-        gs = m.graph_step(n_train, n_ex, self.max_item, args.lr, args.dropout_rate, teacher=teacher,
-                          sources=(self.t_ids, self.t_lab, e_ids, e_aux) if self.es is not None
-                          else (self.t_ids, self.t_lab, None, None), tcaps=caps, queue=(self.q, self.q_off, self.q_counter))
+        gs = m.graph_step(n_train, n_ex, self.max_item, args.lr, args.dropout_rate, teacher=self.teacher,
+                          sources=(self.t_ids, self.t_lab, self.e_ids, self.e_aux),
+                          tcaps=caps, queue=(self.q, self.q_off, self.q_counter))
         self.gs_map[key] = gs
         return gs
 
     def run_epoch(self, n_steps: int):
         """One epoch (main.py:220-256) with the host out of the loop: the samplers are advanced a chunk of steps ahead of the
-        GPU (same calls in the same order as step-by-step, so both host RNG streams move identically), the row indices go to
-        the device chunk by chunk, and every step is a graph replay that gathers its batch from that queue.  A step whose
-        batch geometry has no graph (rare tail batches) runs eagerly from the same queue."""
+        GPU (the same calls in the same order as the reference's batch loop, so both host RNG streams move identically), the
+        row indices go to the device chunk by chunk, and every step is a graph replay that gathers its batch from that queue.
+        A step whose batch geometry has no graph (rare tail batches, or no graph at all: --graph false, the exact encoder
+        with dropout) runs eagerly from the same queue.  With ``trace`` set, every step's loss is copied into a device
+        buffer right behind the step (the next step overwrites it) and the buffer is read once, at the end of the epoch."""
         m = self.model
         if self._q_copied is not None:
             self._q_copied.synchronize()                         # last epoch's queue copies have left the pinned buffers
         qh, oh = self._q_host.numpy(), self._qoff_host.numpy()
         self.q_counter.zero_()
+        losses = torch.empty(n_steps, dtype=torch.float32, device=m.device) if self.trace is not None else None
+        group = self.GROUP if losses is None else 1              # one step per replay: every step's loss is recorded
         o, s0, loss = 0, 0, None
         # planned and launched in chunks, so the host plans chunk k+1 while the GPU runs chunk k (first chunk short: the
         # GPU starts after a few steps' worth of planning)
@@ -225,7 +226,7 @@ class PeriodTrainer:
                 # runs of GROUP consecutive steps of one batch geometry go out as ONE graph replay (capacity = the largest
                 # of their buckets): the replay-to-replay launch gap is paid once per GROUP steps
                 key, _, _, n_tok = plan[i]
-                n = self.GROUP
+                n = group
                 if n > 1 and i + n <= len(plan) and all(plan[i + k][0] == key for k in range(1, n)):
                     gs = self.gs_map.get(key)
                     if gs is not None and self._geom_multi(key):
@@ -235,12 +236,18 @@ class PeriodTrainer:
                         i += n
                         continue
                 loss = self._launch_queued(*plan[i])
+                if losses is not None:
+                    losses[s0 + i:s0 + i + 1].copy_(loss)
+                    if self.trace_rows is not None:
+                        self.trace_rows.append((m.last_row_loss.cpu().numpy(), m._keep[0].cpu().numpy()))
                 i += 1
             self.host_s["launch"] += time.time() - t1
             s0 = s1
         if self._q_copied is None:
             self._q_copied = torch.cuda.Event()
         self._q_copied.record()
+        if losses is not None:
+            self.trace.extend(losses.tolist())
         return loss
 
     CHUNK0, CHUNK = 8, 48
@@ -253,7 +260,7 @@ class PeriodTrainer:
         return key == full
 
     def _launch_queued(self, key, nt, ne, n_tok):
-        """One step of a queued epoch: graph replay, or (rare batch geometry) eager launches from the same queue."""
+        """One step of a queued epoch: graph replay, or (rare batch geometry / no graph) eager launches from the same queue."""
         m, dev, L = self.model, self.model.device, self.model.hp.maxlen
         gs = self._graph(*key) if (key[0] > 0 and (self.es is None or key[1] > 0)) else None
         if self.world > 1:
@@ -264,73 +271,15 @@ class PeriodTrainer:
         ids = torch.empty((nt + ne, L), dtype=torch.int32, device=dev)
         pos = torch.empty(nt, dtype=torch.int32, device=dev)
         aux = torch.empty(max(ne, 1), dtype=torch.int32, device=dev)
-        e_aux = None
-        if self.es is not None:
-            e_aux = self.e_lab if m.disable_distillation else self._teacher_rows()
-        ops.gather_batch_q(self.t_ids, self.t_lab, nt, self.e_ids if ne else None, e_aux if ne else None, ne, self.q, self.q_off,
-                           self.q_counter, ids, pos, aux[:ne] if ne else None)
+        ops.gather_batch_q(self.t_ids, self.t_lab, nt, self.e_ids if ne else None, self.e_aux if ne else None, ne, self.q,
+                           self.q_off, self.q_counter, ids, pos, aux[:ne] if ne else None)
         ops.queue_advance(self.q_counter)
-        if self.es is None or ne == 0:
+        if ne == 0:
             return m.train_step(ids, pos, self.max_item, self.args.lr, self.args.dropout_rate, n_tokens=n_tok)
         if m.disable_distillation:
             return m.train_step(ids, pos, self.max_item, self.args.lr, self.args.dropout_rate, exemplar_pos=aux[:ne], n_tokens=n_tok)
-        return m.train_step(ids, pos, self.max_item, self.args.lr, self.args.dropout_rate, exemplar_logits=self.es.teacher,
+        return m.train_step(ids, pos, self.max_item, self.args.lr, self.args.dropout_rate, exemplar_logits=self.teacher,
                             teacher_rows=aux[:ne], n_tokens=n_tok)
-
-    def _teacher_rows(self):
-        if getattr(self, "_trows", None) is None:
-            self._trows = torch.as_tensor(np.asarray(self.es.logits, dtype=np.int32)).to(self.model.device)
-        return self._trows
-
-    def can_queue(self) -> bool:
-        """The queued epoch needs GPU-resident exemplar logits (ExemplarSet.teacher) or no exemplars at all."""
-        if not getattr(self.args, "graph", True):
-            return False
-        m = self.model
-        if m.encoder_impl != "tc" and self.args.dropout_rate > 0:
-            return False
-        return self.es is None or m.disable_distillation or getattr(self.es, "teacher", None) is not None
-
-    def step(self):
-        loss = self._step()
-        if self.trace is not None:
-            self.trace.append(float(loss.item()))
-            if self.trace_rows is not None:
-                self.trace_rows.append((self.model.last_row_loss.cpu().numpy(), self.model._keep[0].cpu().numpy()))
-        return loss
-
-    def _step(self):
-        m, dev, L = self.model, self.model.device, self.model.hp.maxlen
-        ti = self.ts.next_indices()
-        ei = self.es.next_indices() if self.es is not None else np.zeros(0, np.int64)
-        gs = self._graph(len(ti), len(ei)) if (len(ti) > 0 and (self.es is None or len(ei) > 0)) else None
-        self.rows_seen += len(ti) + len(ei)                      # rows of the whole step (all ranks)
-        if self.world > 1:                                       # keep this rank's rows; the means stay global
-            m.global_counts = (len(ti), len(ei))
-            (tl, th), (el, eh) = self._shard(len(ti), len(ei))
-            ti, ei = ti[tl:th], ei[el:eh]
-        n_tok = int(self.t_nin[ti].sum()) + (int(self.e_nin[ei].sum()) if self.es is not None else 0)
-        if gs is not None:
-            return gs.run_indices(ti, ei if self.es is not None else None, n_tok)
-        self.n_eager += 1                                        # rare batch geometry / no graph
-        ti_d = torch.from_numpy(ti.astype(np.int32)).pin_memory().to(dev, non_blocking=True)
-        ids = torch.empty((len(ti) + len(ei), L), dtype=torch.int32, device=dev)
-        ops.gather_rows_i32(self.t_ids, ti_d, ids[:len(ti)])
-        pos = self.t_lab[ti_d.long()]
-        if self.es is None:
-            return m.train_step(ids, pos, self.max_item, self.args.lr, self.args.dropout_rate, n_tokens=n_tok)
-        ei_d = torch.from_numpy(ei.astype(np.int32)).pin_memory().to(dev, non_blocking=True)
-        if len(ei):
-            ops.gather_rows_i32(self.e_ids, ei_d, ids[len(ti):])
-        if m.disable_distillation:
-            return m.train_step(ids, pos, self.max_item, self.args.lr, self.args.dropout_rate,
-                                exemplar_pos=self.e_lab[ei_d.long()], n_tokens=n_tok)
-        if getattr(self.es, "teacher", None) is not None:
-            rows = torch.as_tensor(np.asarray([self.es.logits[i] for i in ei], dtype=np.int32)).to(dev)
-            return m.train_step(ids, pos, self.max_item, self.args.lr, self.args.dropout_rate,
-                                exemplar_logits=self.es.teacher, teacher_rows=rows, n_tokens=n_tok)
-        lg = np.asarray([self.es.logits[i] for i in ei], dtype=np.float32)
-        return m.train_step(ids, pos, self.max_item, self.args.lr, self.args.dropout_rate, exemplar_logits=lg, n_tokens=n_tok)
 
 
 # ---- per-period checkpoint (SURVEY 8(f)1) -------------------------------------------------------------------
@@ -551,11 +500,7 @@ def run(args) -> dict:
             gc_on = gc.isenabled()
             gc.disable()
             try:
-                if trainer.trace is None and trainer.can_queue() and getattr(args, "epoch_queue", True):
-                    trainer.run_epoch(batch_num)
-                else:
-                    for _ in range(batch_num):
-                        trainer.step()
+                trainer.run_epoch(batch_num)
             finally:
                 if gc_on:
                     gc.enable()

@@ -80,7 +80,6 @@ class Ader:
         self.disable_distillation = bool(getattr(args, "disable_distillation", False))
         self.mode = self.VANILLA
         self.lambda_ = 0.0
-        self.grad_sync = None           # optional callable run between backward and the optimiser (legacy hook)
         self.dp = None                  # data parallel back end (ader_b200.dist.PeerComm / NcclComm): sums gradients over ranks
         self.global_counts = None       # data parallel: (n_train, n_ex) over all ranks -> global means
         self.loss_impl = getattr(args, "loss_impl", "tc")   # "tc": tcgen05 fused logits+CE+KD; "exact": fp32
@@ -264,7 +263,7 @@ class Ader:
             rep = torch.empty((M, self.hp.hidden_units), dtype=torch.float32, device=self.device)
             d_rep = torch.empty_like(rep)
             self._opt_applied = False
-            if _opt is not None and self.grad_sync is None and self.dp is None:
+            if _opt is not None and self.dp is None:
                 # one GPU: the optimiser joins the DAG (table rows right behind the scatter, dense parameters behind
                 # their partial reduction)
                 V_, lr_, lam_, fis_, star_ = _opt
@@ -275,8 +274,6 @@ class Ader:
             else:
                 ops.train_fwd_bwd_tc(self.ms, self.theta, ids, tcap, a, ews, bws, lws, rep, self._loss, row_loss, d_rep,
                                      self.grad, dropout_rate, seed, d_step, serial=(self.step_impl == "serial"))
-            if self.grad_sync is not None:
-                self.grad_sync()
             self.last_row_loss = row_loss
             self._keep = (ids, pos_t, teacher, trow, ex_pos_t, rep, d_rep, frozen)
             return self._loss
@@ -297,8 +294,6 @@ class Ader:
                         impl=self.encoder_impl, d_step=d_step)
         if _events:
             _events[2].record()
-        if self.grad_sync is not None:      # data parallel: NCCL all-reduce of the flat gradient
-            self.grad_sync()
         self.last_row_loss = row_loss
         self._keep = (ids, pos_t, teacher, trow, ex_pos_t, rep, d_rep, frozen)   # keep alive until the stream is done
         return self._loss

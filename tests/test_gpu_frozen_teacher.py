@@ -311,15 +311,6 @@ def test_driver_frozen_resume_reproduces_the_uninterrupted_run(tmp_path, selecti
         run(_e2e_args(tmp_path / "cut", selection=selection, teacher="logits", resume=True, **kw))
 
 
-@pytest.mark.parametrize("kw", [dict(), dict(loss_impl="tc", dropout_rate=0.3)], ids=["exact", "tc_dropout"])
-def test_driver_frozen_epoch_queue_equals_step_by_step(tmp_path, kw):
-    from ader_b200.main import run
-    a = run(_e2e_args(tmp_path / "q", selection="random", teacher="frozen", trace=False, epoch_queue=True, **kw))
-    b = run(_e2e_args(tmp_path / "s", selection="random", teacher="frozen", trace=False, epoch_queue=False, **kw))
-    assert torch.equal(a["model"].theta, b["model"].theta)
-    assert a["per_period"] == b["per_period"]
-
-
 def test_frozen_selection_builds_no_vocabulary_wide_matrix():
     """In the frozen form selection keeps [E, d] reps and the [V_prev, d] table copy, and never allocates anything with
     V_prev columns, not even transiently: the peak device memory of herding selection grows by far less than the

@@ -770,19 +770,44 @@ def test_resume_after_a_period_reproduces_the_uninterrupted_run(tmp_path, select
 
 
 @pytest.mark.parametrize("kw", [dict(selection="random"), dict(selection="random", loss_impl="tc", dropout_rate=0.3),
-                                dict(selection="loss", disable_distillation=True), dict(finetune=True)],
-                         ids=["exact_kd", "tc_dropout_kd", "exact_er", "finetune"])
-def test_epoch_queue_run_equals_step_by_step_run(tmp_path, kw):
-    """SURVEY 8(f): the epoch-resident index queue (all row indices of an epoch uploaded once, every step a graph replay
-    that gathers its batch on the device) is the same computation as feeding the indices step by step: same samplers,
-    same RNG consumption, same kernels -- final weights, metrics and exemplar sets are bit-identical."""
+                                dict(selection="loss", disable_distillation=True), dict(finetune=True),
+                                dict(selection="random", teacher="frozen", loss_impl="tc", dropout_rate=0.3),
+                                dict(selection="random", dropout_rate=0.3), dict(selection="random", graph=False),
+                                dict(ewc=True, selection="random", ewc_sample_num=30, lambda_=50.0)],
+                         ids=["exact_kd", "tc_dropout_kd", "exact_er", "finetune", "frozen_tc", "exact_dropout", "no_graph", "ewc"])
+def test_traced_run_equals_untraced_run(tmp_path, kw):
+    """Every epoch runs through the epoch-resident index queue (PeriodTrainer.run_epoch).  A traced run also copies each
+    step's loss into a device buffer behind the step and replays one step per graph launch; that must not perturb the
+    run: final weights, Adam slots, metrics and rows trained on are bit-identical to the untraced run.  The end-to-end
+    tests against the oracle driver check the traced run itself (exact_dropout and no_graph run every step eagerly from
+    the queue)."""
     from ader_b200.main import run
-    a = run(_e2e_args(tmp_path / "q", trace=False, epoch_queue=True, **kw))
-    b = run(_e2e_args(tmp_path / "s", trace=False, epoch_queue=False, **kw))
+    a = run(_e2e_args(tmp_path / "t", trace=True, **kw))
+    b = run(_e2e_args(tmp_path / "u", trace=False, **kw))
     assert torch.equal(a["model"].theta, b["model"].theta)
     assert torch.equal(a["model"].adam_v, b["model"].adam_v)
     assert a["per_period"] == b["per_period"]
     assert [t["train_rows"] for t in a["throughput"]] == [t["train_rows"] for t in b["throughput"]]
+
+
+def test_period_trainer_refuses_host_teacher_lists(tmp_path):
+    """Distillation reads the exemplars' teacher from the device (ExemplarSet.teacher).  An exemplar sampler fed the
+    reference's [session, logits] lists keeps it on the host: PeriodTrainer refuses it before any device work."""
+    from ader_b200.data import Sampler
+    from ader_b200.main import PeriodTrainer
+    from ader_b200.model import Ader
+    a = _e2e_args(tmp_path)
+    m = Ader(a.item_num, a)
+    m.update_loss(0.8)
+    ts = Sampler([[1, 2, 3, 4], [5, 6, 7]], a.maxlen, 2)
+    es = Sampler([], a.maxlen, 1)
+    es.add_exemplar([[[1, 2, 3], [0.5] * 9], [[4, 5, 6], [0.25] * 9]])
+    with pytest.raises(ValueError, match="ExemplarSet"):
+        PeriodTrainer(m, ts, es, a, 9)
+    assert ts._dev is None and es._dev is None          # no rows went to the device
+    m.disable_distillation = True                       # one-hot replay needs only the labels: accepted
+    m.update_loss(0.8)
+    PeriodTrainer(m, ts, es, a, 9)
 
 
 @pytest.mark.parametrize("mode,shards", [("vanilla", 2), ("kd", 3), ("er", 2)])
